@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""bench.py — SWTPG hot-path throughput on B200 (contract: see the task brief / DESIGN.md §6).
+"""bench.py — SWTPG hot-path throughput on B200 (see DESIGN.md §6).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            native arm (CUDA kernels through the C ABI)
+  python bench.py ... --dump-outputs DIR                         also write the TP list of the last timed step as DIR/tp_<field>.npy
   python bench.py --impl reference [--steps K] [--warmup W]      the reference's own AVX2 code on the host cores
 
 A "step" = one superchunk batch: every link of this GPU's shard advances by `frames` WIBEth frames through the fused
@@ -60,7 +61,29 @@ def parse_args():
     ap.add_argument("--module-links", type=int, default=6000, help="config[2] as written: links of the whole module, split over the GPUs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-variants", action="store_true", help="skip the FIR / running-sum / WIB2 / stress side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the TP list of the last timed step (rank 0's links) to DIR/tp_<field>.npy")
     return ap.parse_args()
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_tps(out_dir: str, tps):
+    """One float64 array per TP field, in the canonical (time_start, link, channel) order, so that two builds can be compared
+    element for element (every field fits float64 exactly: timestamps stay below 2^53). A list over DUMP_MAX_BYTES is cut
+    to a fixed, seeded sample of its rows."""
+    import numpy as np
+
+    from fdreadoutlibs_b200 import frames as F
+
+    tps = F.sort_tps(tps)
+    names = tps.dtype.names
+    keep = DUMP_MAX_BYTES // (8 * len(names))
+    if tps.size > keep:
+        tps = tps[np.sort(np.random.default_rng(0).choice(tps.size, keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for name in names:
+        np.save(os.path.join(out_dir, f"tp_{name}.npy"), tps[name].astype(np.float64))
 
 
 def peaks():
@@ -332,6 +355,8 @@ def main():
             gen.process_device(d_frames.data_ptr(), frames, stream=stream)
         ev1.record()
         torch.cuda.synchronize()
+        if args.dump_outputs and rank == 0:
+            dump_tps(args.dump_outputs, gen.fetch_tps(cap=1 << 22))
         # long enough for nvidia-smi to see the load: repeat untimed launches for ~1 s, collecting per-launch times
         t_end = time.time() + 1.0
         while time.time() < t_end:

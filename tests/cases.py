@@ -12,6 +12,7 @@ import numpy as np
 
 import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import frames as F
+from oracle import binding as B
 
 GOLDEN_TS0 = 79554162068719943  # docs/README.md:136-146
 GOLDEN_PATTERN = [500, 502, 504, 505, 506, 505, 504, 502, 500]
@@ -140,3 +141,125 @@ def make_input(case: dict) -> np.ndarray:
     if case["fmt"] == "wib2":
         return S.gen_wib2_host(p, case["n_links"], case["n_units"])
     return S.gen_wibeth_host(p, case["n_links"], case["n_units"])
+
+
+# ---- differential cases against the reference's own compiled code ----------------------------------------------------------
+# Each run returns the oracle's outputs for one input as {name: array}. What the reference returned for that input is stored in
+# tests/golden/reference_outputs.npz under "<key>__<name>" (tests/golden/record_reference_outputs.py); the tests assert the
+# oracle's outputs, or the GPU's, equal to it (util.assert_same_as_reference). Reference impl codes: oracle/binding.py.
+def reference_outputs():
+    import os
+
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_outputs.npz"))
+
+
+WIBETH_DIFF = [(11, 0.02, 60), (12, 0.3, 20), (13, 0.9, 8), (14, 0.9, 0), (15, 0.05, 3)]  # seed, pulse rate, threshold
+WIBETH_DIFF_IMPLS = [(0, B.REF_ETH_SIMPLE_AVX2, 0), (0, B.REF_ETH_SIMPLE_NAIVE, 1), (1, B.REF_ETH_ABSRS_AVX2, 0),
+                     (2, B.REF_ETH_STDRS_AVX2, 0)]  # algorithm, reference impl, oracle flavour
+ACC_LIMITS = [1, 3, 10, 50, 0, -2]
+WIB2_DIFF = [(31, 0.05), (32, 0.6)]
+WIB2_DIFF_IMPLS = [(0, B.REF_WIB2_SIMPLE_AVX2, 0, 100), (0, B.REF_WIB2_SIMPLE_AVX2, 0, 30), (3, B.REF_WIB2_FIR_AVX2, 0, 5),
+                   (3, B.REF_WIB2_FIR_NAIVE, 1, 5), (3, B.REF_WIB2_FIR_AVX2, 0, 2), (1, B.REF_WIB2_ABSRS_AVX2, 0, 60),
+                   (1, B.REF_WIB2_ABSRS_AVX2, 0, 5), (1, B.REF_WIB2_ABSRS_AVX2, 0, 1), (1, B.REF_WIB2_ABSRS_AVX2, 0, 500)]
+ANY_TAPS = [([2, 5, 11, 17, 9, 4, 1], 6), ([-3, 7, 20, 31, 20, 7, -3], 6), ([1, 3, 8, 10, 8, 3, 1], 5), ([300, -700, 1200, 2000, 1200, -700, 300], 6),
+            ([0, 0, 0, 64, 0, 0, 0], 6)]
+LANE_PRODUCT_THRESHOLDS = (11, 40, 700)  # 102*64*11 = 71808 > 65535: lanes overflow into each other
+GPU_RS_DIFF = ["AbsRS", "StandardRS"]
+GPU_WIB2_DIFF = [("SimpleThreshold", 60), ("FIR", 5)]
+CONFIG1_THRESHOLDS = [60, 20]
+
+
+def wibeth_diff(seed, rate, thr, algo, flav):
+    fr = S.gen_wibeth_host(S.gen_params(seed, rate), 1, 150)[0]
+    o = B.Oracle(B.make_config(algorithm=algo, threshold=thr, rs_memory_factor=8, rs_scale_factor=5), flav)
+    tps, ped, _ = o.process(fr, dump=True)
+    return {"tps": tps, "pedestal": ped[:, 63, :], "accum": o.state()["accum"]}  # pedestal after every frame
+
+
+def acc_limit_diff(L):
+    fr = S.gen_wibeth_host(S.gen_params(21, 0.2), 1, 60)[0]
+    tps, ped, _ = B.Oracle(B.make_config(threshold=25, acc_limit=L)).process(fr, dump=True)
+    return {"tps": tps, "pedestal": ped[:, 63, :]}
+
+
+def memory_factor_diff():
+    fr = S.gen_wibeth_host(S.gen_params(22, 0.2), 1, 80)[0]
+    o = B.Oracle(B.make_config(algorithm=1, threshold=30))
+    o.set_memory_factor(np.where(np.arange(64) % 3 == 0, 0, 8).astype(np.uint16))
+    return {"tps": o.process(fr)}
+
+
+def _wib2_state(o, quartiles):
+    st = o.state()
+    return {"pedestal": st["pedestal"], **({"quantile25": st["quantile25"], "quantile75": st["quantile75"]} if quartiles else {})}
+
+
+def wib2_diff(seed, rate, algo, flav, thr):
+    sc = S.gen_wib2_host(S.gen_params(seed, rate), 1, 250)[0]
+    o = B.Oracle(B.make_config(fmt="wib2", algorithm=algo, threshold=thr), flav)
+    return {"tps": o.process(sc), **_wib2_state(o, algo in (1, 3))}
+
+
+def taps_diff(taps, exponent, flav):
+    sc = S.gen_wib2_host(S.gen_params(34, 0.5), 1, 200)[0]
+    o = B.Oracle(B.make_config(fmt="wib2", algorithm=3, threshold=5, fir_taps=taps, tap_exponent=exponent), flav)
+    return {"tps": o.process(sc), **_wib2_state(o, True)}
+
+
+def lane_product_diff(thr):
+    sc = S.gen_wib2_host(S.gen_params(33, 0.4, noise_q8=40 * 256), 1, 200)[0]  # wide noise -> sigma at its clamp of 102
+    return {"tps": B.Oracle(B.make_config(fmt="wib2", algorithm=3, threshold=thr)).process(sc)}
+
+
+def gpu_rs_input():
+    return S.gen_wibeth_host(S.gen_params(72, 0.3), 1, 300)
+
+
+def gpu_rs_diff(algorithm):
+    cfg = B.make_config(algorithm=S.ALGORITHMS[algorithm], threshold=30, rs_memory_factor=8, rs_scale_factor=5)
+    return {"tps": B.Oracle(cfg).process(gpu_rs_input()[0], cap=1 << 20)}
+
+
+def gpu_wib2_input():
+    return S.gen_wib2_host(S.gen_params(73, 0.3), 1, 600)
+
+
+def gpu_wib2_diff(algorithm, thr):
+    cfg = B.make_config(fmt="wib2", algorithm=S.ALGORITHMS[algorithm], threshold=thr)
+    return {"tps": B.Oracle(cfg).process(gpu_wib2_input()[0], cap=1 << 20)}
+
+
+def config1_input():
+    return S.gen_wibeth_host(S.gen_params(1, 0.05), 1, 10000)
+
+
+def config1_diff(thr):
+    return {"tps": B.Oracle(B.make_config(threshold=thr)).process(config1_input()[0], cap=1 << 20)}
+
+
+def taps_key(taps, exponent):
+    return "taps_" + "_".join(str(t) for t in taps) + f"_exp{exponent}"
+
+
+def reference_runs():
+    """(key, run) of every case whose reference output tests/golden/reference_outputs.npz holds."""
+    for seed, rate, thr in WIBETH_DIFF:
+        for algo, impl, flav in WIBETH_DIFF_IMPLS:
+            yield f"wibeth_{seed}_thr{thr}_impl{impl}", lambda a=(seed, rate, thr, algo, flav): wibeth_diff(*a)
+    for L in ACC_LIMITS:
+        yield f"acc_limit_{L}", lambda L=L: acc_limit_diff(L)
+    yield "memory_factor_per_channel", memory_factor_diff
+    for seed, rate in WIB2_DIFF:
+        for algo, impl, flav, thr in WIB2_DIFF_IMPLS:
+            yield f"wib2_{seed}_thr{thr}_impl{impl}", lambda a=(seed, rate, algo, flav, thr): wib2_diff(*a)
+    for taps, exponent in ANY_TAPS:
+        yield taps_key(taps, exponent), lambda a=(taps, exponent, 0): taps_diff(*a)
+    for thr in LANE_PRODUCT_THRESHOLDS:
+        yield f"lane_product_thr{thr}", lambda thr=thr: lane_product_diff(thr)
+    for algorithm in GPU_RS_DIFF:
+        yield f"gpu_rs_{algorithm}", lambda a=algorithm: gpu_rs_diff(a)
+    for algorithm, thr in GPU_WIB2_DIFF:
+        yield f"gpu_wib2_{algorithm}_thr{thr}", lambda a=(algorithm, thr): gpu_wib2_diff(*a)
+    for thr in CONFIG1_THRESHOLDS:
+        yield f"config1_thr{thr}", lambda thr=thr: config1_diff(thr)
+

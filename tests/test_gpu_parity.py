@@ -12,7 +12,7 @@ import cases
 import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import frames as F
 from oracle import binding as B
-from util import assert_same_tps, oracle_config
+from util import assert_same_as_reference, assert_same_tps, oracle_config
 
 pytestmark = pytest.mark.gpu
 
@@ -749,14 +749,15 @@ def test_full_size_one_apa_properties():
         assert_same_tps(fir_one[fir_one["link"] == l], want, f"FIR link {l} vs oracle")
 
 
-@pytest.mark.parametrize("thr", [60, 20])
+@pytest.mark.parametrize("thr", cases.CONFIG1_THRESHOLDS)
 def test_config1_single_link_10k_frames(thr):
     """BASELINE config[0]: one WIBEth link (64 ch x 64 ticks/frame), 10 000 synthetic frames (40.96 M samples), SimpleThreshold,
     accumulator limit 10 — the run the reference's (absent) emulator app would do with AVX and NAIVE implementations.
-    GPU == AVX2 flavour on every field; == the reference's own compiled code where oracle/_ref travelled with the snapshot;
+    GPU == AVX2 flavour on every field; == what the reference's own compiled code returned (tests/golden/reference_outputs.npz);
     == NAIVE flavour after its position->channel mapping wherever the integral did not overflow 15 bits (SURVEY H1, H3)."""
     n_frames = 10000
-    units = S.gen_wibeth_host(S.gen_params(1, 0.05), 1, n_frames)
+    units = cases.config1_input()
+    assert units.shape[1] == n_frames
     with S.TPGenerator(1, 2500, threshold=thr, tp_capacity=1 << 20) as g:
         g.start()
         got = np.concatenate([g.process_host(np.ascontiguousarray(units[:, u:u + 2500])) for u in range(0, n_frames, 2500)])
@@ -769,34 +770,30 @@ def test_config1_single_link_10k_frames(thr):
     naive = B.Oracle(B.make_config(threshold=thr), B.FLAVOUR_NAIVE).process(units[0], cap=1 << 20)
     keep = lambda a: a[a["adc_integral"] <= 32767]
     assert_same_tps(keep(got), keep(naive), "NAIVE flavour (integrals <= 32767)")
-    if B.reference_available():
-        ref = B.ReferenceWibEth(B.REF_ETH_SIMPLE_AVX2, thr, 10).process(units[0], cap=1 << 20)
-        assert_same_tps(got, ref, "reference process_window_avx2 itself")
+    assert_same_as_reference({"tps": got}, cases.reference_outputs(), f"config1_thr{thr}")  # process_window_avx2 itself
 
 
-@pytest.mark.skipif(not B.reference_available(), reason="oracle/_ref/libswtpg_ref.so did not travel with the snapshot")
 @pytest.mark.parametrize("algorithm,impl", [("AbsRS", B.REF_ETH_ABSRS_AVX2), ("StandardRS", B.REF_ETH_STDRS_AVX2)])
 def test_running_sums_against_the_reference_itself(algorithm, impl):
-    """GPU vs the reference's own process_window_rs_avx2 / process_window_standard_rs_avx2 (compiled from its headers), no
-    restatement in between."""
-    units = S.gen_wibeth_host(S.gen_params(72, 0.3), 1, 300)
-    ref = B.ReferenceWibEth(impl, 30, 10, 8, 5).process(units[0], cap=1 << 20)
+    """GPU vs what the reference's own process_window_rs_avx2 / process_window_standard_rs_avx2 (compiled from its headers)
+    returned for this input (tests/golden/reference_outputs.npz), no restatement in between."""
+    assert algorithm in cases.GPU_RS_DIFF
+    units = cases.gpu_rs_input()
     with S.TPGenerator(1, 100, algorithm=algorithm, threshold=30, rs_memory_factor=8, rs_scale_factor=5) as g:
         g.start()
         got = np.concatenate([g.process_host(np.ascontiguousarray(units[:, u:u + 100])) for u in range(0, 300, 100)])
-    assert ref.size > 500
-    assert_same_tps(got, ref, algorithm)
+    assert got.size > 500
+    assert_same_as_reference({"tps": got}, cases.reference_outputs(), f"gpu_rs_{algorithm}")
 
 
-@pytest.mark.skipif(not B.reference_available(), reason="oracle/_ref/libswtpg_ref.so did not travel with the snapshot")
 @pytest.mark.parametrize("algorithm,impl,thr", [("SimpleThreshold", B.REF_WIB2_SIMPLE_AVX2, 60), ("FIR", B.REF_WIB2_FIR_AVX2, 5)])
 def test_wib2_against_the_reference_itself(algorithm, impl, thr):
-    """BASELINE config[4]: GPU vs the reference's own swtpg_wib2::process_window_avx2 (SimpleThreshold and FIR + IQR), both
-    register selectors."""
-    units = S.gen_wib2_host(S.gen_params(73, 0.3), 1, 600)
-    ref = B.ReferenceWib2(impl, thr).process(units[0], cap=1 << 20)
+    """BASELINE config[4]: GPU vs what the reference's own swtpg_wib2::process_window_avx2 (SimpleThreshold and FIR + IQR), both
+    register selectors, returned for this input (tests/golden/reference_outputs.npz)."""
+    assert (algorithm, thr) in cases.GPU_WIB2_DIFF
+    units = cases.gpu_wib2_input()
     with S.TPGenerator(1, 200, fmt="wib2", algorithm=algorithm, threshold=thr) as g:
         g.start()
         got = np.concatenate([g.process_host(np.ascontiguousarray(units[:, u:u + 200])) for u in range(0, 600, 200)])
-    assert ref.size > 300
-    assert_same_tps(got, ref, f"wib2 {algorithm}")
+    assert got.size > 300
+    assert_same_as_reference({"tps": got}, cases.reference_outputs(), f"gpu_wib2_{algorithm}_thr{thr}")
