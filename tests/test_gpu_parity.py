@@ -441,12 +441,13 @@ def test_more_links_than_persistent_warps_whole_batches():
 
 
 @pytest.mark.skipif(os.environ.get("SWTPG_PARTS") is not None, reason="already running with forced slicing")
-@pytest.mark.parametrize("parts", [2, 8])
+@pytest.mark.parametrize("parts", [2, 4, 8])
 def test_links_handed_out_in_slices(parts):
     """A launch with more links than persistent warps hands every link out in slices (wibeth_kernel: a later slice continues from
     the state its predecessor stored, and may run on another warp). SWTPG_PARTS forces that for EVERY launch of a process, so
     the ragged / empty / carried-state / dump / hand-out cases above are repeated under it: units fewer than slices (empty
-    slices), hits open across a slice boundary, FIR ring phase, running sums, the scalar policies."""
+    slices), hits open across a slice boundary, FIR ring phase, running sums, the scalar policies. 4 is the slice count of
+    the production launches (tests/test_gpu_launch_geometry.py runs those in their default geometries)."""
     env = dict(os.environ, SWTPG_PARTS=str(parts))
     sel = ("test_more_links_than_persistent_warps_ragged or test_more_links_than_persistent_warps_whole_batches or "
            "test_ragged_and_empty_batches or test_against_oracle_with_state_and_dumps or "

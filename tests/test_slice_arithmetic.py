@@ -4,7 +4,8 @@ every unit count incl. fewer units than slices: (1) the slices partition [0, n);
 (it is the one that re-arms the link's counter); (3) `slices_before` equals the number of non-empty slices in front of a slice
 wherever the kernel uses it (a slice that waits, a slice that publishes); (4) processing the items of a launch in claim order with
 any number of persistent warps never dead-locks and leaves every counter at zero. No GPU: this pins the formulas, the CUDA side
-is covered by tests/test_gpu_parity.py::test_links_handed_out_in_slices."""
+is covered by tests/test_gpu_parity.py::test_links_handed_out_in_slices (forced slice counts) and by
+tests/test_gpu_launch_geometry.py (the production launch geometries, every link against the oracle)."""
 import numpy as np
 import pytest
 
