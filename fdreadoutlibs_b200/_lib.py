@@ -41,6 +41,23 @@ class SwtpgConfig(C.Structure):
     ]
 
 
+MAX_LINK_CONFIGS = 16  # SWTPG_MAX_LINK_CONFIGS
+
+
+class SwtpgLinkConfig(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_uint32),
+        ("algorithm", C.c_int32),
+        ("threshold", C.c_uint16),
+        ("frugal_acc_limit", C.c_int16),
+        ("rs_memory_factor", C.c_uint16),
+        ("rs_scale_factor", C.c_uint16),
+        ("fir_taps", C.c_int16 * 8),
+        ("tap_exponent", C.c_uint8),
+        ("reserved0", C.c_uint8 * 3),
+    ]
+
+
 class SwtpgCounters(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in (
         "units_processed", "samples_processed", "tps_emitted", "tps_dropped_overflow", "batches", "submit_busy",
@@ -59,6 +76,7 @@ EXPORTS = {
     "swtpg_stop": (C.c_int, [C.c_void_p]),
     "swtpg_set_rs_memory_factor": (C.c_int, [C.c_void_p, C.c_void_p]),
     "swtpg_set_link_rs_memory_factor": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p]),
+    "swtpg_set_link_config": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(SwtpgLinkConfig)]),
     "swtpg_process_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "swtpg_process_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
     "swtpg_fetch_tps": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),

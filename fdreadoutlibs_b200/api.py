@@ -12,7 +12,7 @@ import numpy as np
 
 from . import frames as F
 from ._lib import (ALGO_ABS_RS, ALGO_FIR_IQR, ALGO_SIMPLE_THRESHOLD, ALGO_STANDARD_RS, FORMAT_WIB2, FORMAT_WIBETH,
-                   SWTPG_ERR_BUSY, SWTPG_ERR_OVERFLOW, SWTPG_OK, SwtpgConfig, SwtpgCounters, lib)
+                   SWTPG_ERR_BUSY, SWTPG_ERR_OVERFLOW, SWTPG_OK, SwtpgConfig, SwtpgCounters, SwtpgLinkConfig, lib)
 
 ALGORITHMS = {
     # tpg_algorithm strings of the reference (src/wibeth/WIBEthFrameProcessor.cpp:180-197)
@@ -130,6 +130,30 @@ class TPGenerator:
         a = np.ascontiguousarray(by_channel, dtype=np.uint16)
         assert a.size == self.channels
         self._check(lib.swtpg_set_link_rs_memory_factor(self._h, link, a.ctypes.data))
+
+    def set_link_config(self, link: int, *, algorithm: Optional[str] = None, threshold: Optional[int] = None,
+                        acc_limit: Optional[int] = None, rs_memory_factor: Optional[int] = None, rs_scale_factor: Optional[int] = None,
+                        fir_taps: Optional[Sequence[int]] = None, tap_exponent: Optional[int] = None, reset: bool = False):
+        """swtpg_set_link_config: the TPG parameters of one link. A field left as None takes the handle's value; reset=True
+        returns the link to the handle's configuration. Only while the handle is stopped; takes effect at the next start()."""
+        if reset:
+            self._check(lib.swtpg_set_link_config(self._h, link, None))
+            return
+        if algorithm is not None and algorithm not in ALGORITHMS:
+            raise TPGAlgorithmInexistent(algorithm)
+        h = self.cfg
+        c = SwtpgLinkConfig()
+        c.struct_size = C.sizeof(SwtpgLinkConfig)
+        c.algorithm = h.algorithm if algorithm is None else ALGORITHMS[algorithm]
+        c.threshold = h.threshold if threshold is None else threshold
+        c.frugal_acc_limit = h.frugal_acc_limit if acc_limit is None else acc_limit
+        c.rs_memory_factor = h.rs_memory_factor if rs_memory_factor is None else rs_memory_factor
+        c.rs_scale_factor = h.rs_scale_factor if rs_scale_factor is None else rs_scale_factor
+        taps = list(h.fir_taps) if fir_taps is None else list(fir_taps)
+        for i in range(8):
+            c.fir_taps[i] = int(taps[i]) if i < len(taps) else 0
+        c.tap_exponent = h.tap_exponent if tap_exponent is None else tap_exponent
+        self._check(lib.swtpg_set_link_config(self._h, link, C.byref(c)))
 
     # -- batch entry points ----------------------------------------------------------------------------------------------
     def _nunits(self, n_units):

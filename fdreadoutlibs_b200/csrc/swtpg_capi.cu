@@ -18,13 +18,16 @@
 #include <vector>
 
 using namespace swtpg;
+using swtpg_internal::ConfGroup;
 using swtpg_internal::fail;
+using swtpg_internal::TpgConf;
 
 // Layouts the ctypes binding (fdreadoutlibs_b200/_lib.py, frames.py) relies on.
 static_assert(sizeof(swtpg_tp) == 32, "swtpg_tp must stay 32 bytes (two 16-byte device stores)");
 static_assert(sizeof(swtpg_config) == 72, "swtpg_config layout changed: bump SWTPG_ABI_VERSION and the bindings");
 static_assert(sizeof(swtpg_channel_state) == 48, "swtpg_channel_state layout changed");
 static_assert(sizeof(swtpg_counters) == 80, "swtpg_counters layout changed");
+static_assert(sizeof(swtpg_link_config) == 36, "swtpg_link_config layout changed");
 
 namespace {
 thread_local std::string g_create_error;
@@ -278,73 +281,124 @@ launch_wib2(const KernelParams& kp, cudaStream_t s)
 
 template<bool DUMP>
 cudaError_t
-launch(const swtpg_handle* h, const KernelParams& kp, cudaStream_t s)
+launch(const swtpg_handle* h, const TpgConf& c, const KernelParams& kp, cudaStream_t s)
 {
   if (h->cfg.format == SWTPG_FORMAT_WIB2) {
-    switch (h->cfg.algorithm) {
+    switch (c.algorithm) {
       case SWTPG_ALGO_SIMPLE_THRESHOLD:
-        return h->fast_simple ? launch_wib2<PackedSimpleWib2, DUMP>(kp, s)
+        return c.fast_simple ? launch_wib2<PackedSimpleWib2, DUMP>(kp, s)
                               : launch_wib2<ScalarAlgo<SWTPG_ALGO_SIMPLE_THRESHOLD, true>, DUMP>(kp, s);
       case SWTPG_ALGO_FIR_IQR:
-        return h->fast_fir       ? launch_wib2<PackedFirIqr, DUMP>(kp, s)
-               : h->fast_fir_any ? launch_wib2<PackedFirIqrAnyTaps, DUMP>(kp, s)
+        return c.fast_fir       ? launch_wib2<PackedFirIqr, DUMP>(kp, s)
+               : c.fast_fir_any ? launch_wib2<PackedFirIqrAnyTaps, DUMP>(kp, s)
                                  : launch_wib2<ScalarAlgo<SWTPG_ALGO_FIR_IQR, true>, DUMP>(kp, s);
       case SWTPG_ALGO_ABS_RS:
-        return h->fast_rs_wib2 ? launch_wib2<PackedRsIqrWib2, DUMP>(kp, s) : launch_wib2<ScalarAlgo<SWTPG_ALGO_ABS_RS, true>, DUMP>(kp, s);
+        return c.fast_rs_wib2 ? launch_wib2<PackedRsIqrWib2, DUMP>(kp, s) : launch_wib2<ScalarAlgo<SWTPG_ALGO_ABS_RS, true>, DUMP>(kp, s);
       default: return cudaErrorNotSupported;
     }
   }
   if (h->cfg.format == SWTPG_FORMAT_WIBETH) {
-    switch (h->cfg.algorithm) {
+    switch (c.algorithm) {
       case SWTPG_ALGO_SIMPLE_THRESHOLD:
-        return h->fast_simple ? launch_wibeth<PackedSimpleWibEth, DUMP>(kp, s)
+        return c.fast_simple ? launch_wibeth<PackedSimpleWibEth, DUMP>(kp, s)
                               : launch_wibeth<ScalarAlgo<SWTPG_ALGO_SIMPLE_THRESHOLD, false>, DUMP>(kp, s);
       case SWTPG_ALGO_ABS_RS:
-        return h->fast_rs ? launch_wibeth<PackedRsWibEth<false>, DUMP>(kp, s) : launch_wibeth<ScalarAlgo<SWTPG_ALGO_ABS_RS, false>, DUMP>(kp, s);
+        return c.fast_rs ? launch_wibeth<PackedRsWibEth<false>, DUMP>(kp, s) : launch_wibeth<ScalarAlgo<SWTPG_ALGO_ABS_RS, false>, DUMP>(kp, s);
       case SWTPG_ALGO_STANDARD_RS:
-        return h->fast_rs ? launch_wibeth<PackedRsWibEth<true>, DUMP>(kp, s)
+        return c.fast_rs ? launch_wibeth<PackedRsWibEth<true>, DUMP>(kp, s)
                           : launch_wibeth<ScalarAlgo<SWTPG_ALGO_STANDARD_RS, false>, DUMP>(kp, s);
       case SWTPG_ALGO_FIR_IQR:
-        return h->fast_fir       ? launch_wibeth<PackedFirIqr, DUMP>(kp, s)
-               : h->fast_fir_any ? launch_wibeth<PackedFirIqrAnyTaps, DUMP>(kp, s)
+        return c.fast_fir       ? launch_wibeth<PackedFirIqr, DUMP>(kp, s)
+               : c.fast_fir_any ? launch_wibeth<PackedFirIqrAnyTaps, DUMP>(kp, s)
                                  : launch_wibeth<ScalarAlgo<SWTPG_ALGO_FIR_IQR, false>, DUMP>(kp, s);
     }
   }
   return cudaErrorNotSupported;
 }
 
+// Kernel parameters of one configuration group's launch.
 KernelParams
-make_params(const swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t stride, swtpg_tp* d_tps, unsigned* d_count,
-            int16_t* ped, int16_t* wav)
+make_params(const swtpg_handle* h, const ConfGroup& g, const void* d_frames, const uint32_t* d_nunits, uint32_t stride, swtpg_tp* d_tps,
+            unsigned* d_count, int16_t* ped, int16_t* wav)
 {
+  const TpgConf& c = h->confs[g.conf];
   KernelParams kp{};
   kp.frames = static_cast<const uint8_t*>(d_frames);
   kp.n_units = d_nunits;
   kp.units_stride = stride;
-  kp.n_links = h->cfg.n_links;
+  kp.n_links = g.n_links;
+  kp.link_ids = g.d_links;
   kp.state = h->d_state;
   kp.group_flags = h->d_flags;
-  kp.link_cursor = h->d_link_cursor;
-  kp.link_done = h->d_link_cursor + 2;
+  kp.link_cursor = g.d_cursor;
+  kp.link_done = h->d_link_cursor + 2 * SWTPG_MAX_LINK_CONFIGS;
   kp.parts_log2 = 0;
   kp.sink.buf = d_tps;
   kp.sink.count = d_count;
   kp.sink.cap = h->tp_capacity;
   kp.pedestal_out = ped;
   kp.waveform_out = wav;
-  kp.threshold = h->cfg.threshold;
-  kp.acc_limit = h->cfg.frugal_acc_limit;
-  kp.acc_limit_neg = 0u - (uint32_t(h->cfg.frugal_acc_limit) & 0xFFFFu);
-  kp.rs_scale = int16_t(h->cfg.rs_scale_factor);
-  kp.tap_exponent = h->cfg.tap_exponent;
+  kp.threshold = c.threshold;
+  kp.acc_limit = c.frugal_acc_limit;
+  kp.acc_limit_neg = 0u - (uint32_t(c.frugal_acc_limit) & 0xFFFFu);
+  kp.rs_scale = int16_t(c.rs_scale_factor);
+  kp.tap_exponent = c.tap_exponent;
   for (int i = 0; i < 8; ++i)
-    kp.taps[i] = h->cfg.fir_taps[i];
+    kp.taps[i] = c.fir_taps[i];
   kp.wib2_adc_offset = h->cfg.wib2_adc_offset;
   static const bool force_exact = [] { const char* e = getenv("SWTPG_FIR_FORCE_EXACT"); return e && atoi(e) != 0; }();
-  kp.debug_flags = (force_exact || h->fir_force_exact) ? 1u : 0u;
+  kp.debug_flags = (force_exact || c.fir_force_exact) ? 1u : 0u;
   kp.all_ones = 0xFFFFFFFFu;
   kp.one = 1u;
   return kp;
+}
+
+// One batch = one launch per configuration group. The groups run one after another on the same stream, never concurrently:
+// a warp's first work item is fixed by its warp index rather than claimed, so a later slice of a link can wait for a warp of
+// its own grid that is not resident yet. Every persistent grid is sized to the whole GPU, so two sliced grids running at once
+// could fill the SMs with warps that all spin on warps of their own grid which can never become resident: a deadlock.
+template<bool DUMP>
+cudaError_t
+launch_groups(const swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t stride, swtpg_tp* d_tps, unsigned* d_count,
+              int16_t* ped, int16_t* wav, cudaStream_t s)
+{
+  for (const ConfGroup& g : h->conf_groups) {
+    const cudaError_t e = launch<DUMP>(h, h->confs[g.conf], make_params(h, g, d_frames, d_nunits, stride, d_tps, d_count, ped, wav), s);
+    if (e != cudaSuccess)
+      return e;
+  }
+  return cudaSuccess;
+}
+
+// The configuration groups of the links' current configurations (swtpg_start): one per entry of h->confs in use, its links in
+// ascending order. A handle whose links all run one configuration launches as before any link had its own: link_ids = nullptr.
+swtpg_status
+form_conf_groups(swtpg_handle* h)
+{
+  std::vector<uint32_t> links;
+  std::vector<ConfGroup> groups;
+  for (uint32_t c = 0; c < h->confs.size(); ++c) {
+    const size_t first = links.size();
+    for (uint32_t l = 0; l < h->cfg.n_links; ++l)
+      if (h->link_conf[l] == c)
+        links.push_back(l);
+    if (links.size() == first)
+      continue;
+    ConfGroup g;
+    g.conf = c;
+    g.n_links = uint32_t(links.size() - first);
+    g.d_links = h->d_group_links + first;
+    g.d_cursor = h->d_link_cursor + 2 * groups.size();
+    groups.push_back(g);
+  }
+  if (groups.size() == 1)
+    groups[0].d_links = nullptr;
+  else
+    SW_CUDA(h, cudaMemcpyAsync(h->d_group_links, links.data(), links.size() * 4, cudaMemcpyHostToDevice, h->stream));
+  SW_CUDA(h, cudaStreamSynchronize(h->stream));
+  h->conf_groups = std::move(groups);
+  h->conf_groups_stale = false;
+  return SWTPG_OK;
 }
 
 swtpg_status
@@ -355,8 +409,8 @@ reset_state(swtpg_handle* h)
   for (uint32_t g = 0; g < h->n_groups; ++g) {
     const uint32_t link = g / h->groups_per_link, sub = g % h->groups_per_link;
     for (uint32_t lane = 0; lane < 32; ++lane) {
-      uint32_t lo = h->cfg.rs_memory_factor, hi = h->cfg.rs_memory_factor;
-      if (h->h_rs_factor) {
+      uint32_t lo = h->link_rs_factor[link], hi = lo;
+      if (h->h_rs_factor && h->rs_table_link[link]) {
         const uint16_t* f = h->h_rs_factor + size_t(link) * h->channels + sub * 64 + 2 * lane;
         lo = f[0];
         hi = f[1];
@@ -366,12 +420,12 @@ reset_state(swtpg_handle* h)
   }
   SW_CUDA(h, cudaMemcpyAsync(h->d_state, st.data(), st.size() * 4, cudaMemcpyHostToDevice, h->stream));
   SW_CUDA(h, cudaMemsetAsync(h->d_flags, 0, size_t(h->n_groups) * 4, h->stream));
-  SW_CUDA(h, cudaMemsetAsync(h->d_link_cursor, 0, (2 + size_t(h->cfg.n_links)) * sizeof(uint32_t), h->stream));
+  SW_CUDA(h, cudaMemsetAsync(h->d_link_cursor, 0, (2 * SWTPG_MAX_LINK_CONFIGS + size_t(h->cfg.n_links)) * sizeof(uint32_t), h->stream));
   SW_CUDA(h, cudaStreamSynchronize(h->stream));
   return SWTPG_OK;
 }
 
-// Rewrites the SV_RS_FACTOR rows of links [link0, link0 + n) from h->h_rs_factor (or the configured factor): ONE strided
+// Rewrites the SV_RS_FACTOR rows of links [link0, link0 + n) from h->h_rs_factor (or each link's configured factor): ONE strided
 // asynchronous copy on the compute stream, i.e. ordered before every kernel launched after this call and after every kernel
 // launched before it. The source is pageable, so the runtime has staged it when the call returns.
 swtpg_status
@@ -382,8 +436,8 @@ upload_rs_factor_rows(swtpg_handle* h, uint32_t link0, uint32_t n)
   for (uint32_t g = 0; g < ng; ++g) {
     const uint32_t link = (g0 + g) / h->groups_per_link, sub = (g0 + g) % h->groups_per_link;
     for (uint32_t lane = 0; lane < 32; ++lane) {
-      uint32_t lo = h->cfg.rs_memory_factor, hi = lo;
-      if (h->h_rs_factor) {
+      uint32_t lo = h->link_rs_factor[link], hi = lo;
+      if (h->h_rs_factor && h->rs_table_link[link]) {
         const uint16_t* f = h->h_rs_factor + size_t(link) * h->channels + sub * 64 + 2 * lane;
         lo = f[0];
         hi = f[1];
@@ -435,9 +489,11 @@ enqueue_batch(swtpg_handle* h, const void* d_frames, const uint32_t* n_units, ui
   }
   SW_CUDA(h, cudaMemsetAsync(h->d_count, 0, sizeof(unsigned), s));
   if (stride) {
-    KernelParams kp = make_params(h, d_frames, d_nu, stride, h->d_tps, h->d_count, dump ? h->d_ped : nullptr, dump ? h->d_wav : nullptr);
+    int16_t* ped = dump ? h->d_ped : nullptr;
+    int16_t* wav = dump ? h->d_wav : nullptr;
     SW_CUDA(h, cudaEventRecord(h->ev0, s));
-    SW_CUDA(h, dump ? launch<true>(h, kp, s) : launch<false>(h, kp, s));
+    SW_CUDA(h, dump ? launch_groups<true>(h, d_frames, d_nu, stride, h->d_tps, h->d_count, ped, wav, s)
+                    : launch_groups<false>(h, d_frames, d_nu, stride, h->d_tps, h->d_count, ped, wav, s));
     SW_CUDA(h, cudaEventRecord(h->ev1, s));
     h->timed = true;
   }
@@ -482,14 +538,110 @@ fetch(swtpg_handle* h, cudaStream_t s, swtpg_tp* out, size_t cap, size_t* n_out)
   return SWTPG_OK;
 }
 
+// Checks one TPG configuration of a handle of `format`, normalises it and picks the policy that runs it (the packed fast paths'
+// validity ranges). swtpg_create and swtpg_set_link_config both go through here. On failure *why says what is wrong.
+swtpg_status
+classify_config(int32_t format, const swtpg_link_config& in, TpgConf* out, const char** why)
+{
+  const bool wib2 = format == SWTPG_FORMAT_WIB2;
+  if (in.algorithm < SWTPG_ALGO_SIMPLE_THRESHOLD || in.algorithm > SWTPG_ALGO_FIR_IQR)
+    return *why = "unknown tpg_algorithm (reference: TPGAlgorithmInexistent)", SWTPG_ERR_UNSUPPORTED;
+  if (wib2 && in.algorithm == SWTPG_ALGO_STANDARD_RS)
+    return *why = "StandardRS does not exist for the WIB2 format (reference: SimpleThreshold and AbsRS only)", SWTPG_ERR_UNSUPPORTED;
+  if (wib2 && in.algorithm == SWTPG_ALGO_ABS_RS && in.threshold == 0)
+    return *why = "WIB2 AbsRS needs threshold >= 1 (sigmaMax = 2^15 / (multiplier * threshold))", SWTPG_ERR_INVALID_ARG;
+  if (in.tap_exponent > 14)
+    return *why = "tap_exponent out of range", SWTPG_ERR_INVALID_ARG;
+  TpgConf c;
+  c.algorithm = in.algorithm;
+  c.threshold = in.threshold;
+  c.frugal_acc_limit = in.frugal_acc_limit;
+  c.rs_scale_factor = in.rs_scale_factor;
+  c.tap_exponent = in.tap_exponent == 0 ? 6 : in.tap_exponent;
+  bool any_tap = false;
+  for (int i = 0; i < 8; ++i) {
+    c.fir_taps[i] = in.fir_taps[i];
+    any_tap |= in.fir_taps[i] != 0;
+  }
+  if (!any_tap) { // src/wib2/WIB2FrameProcessor.cpp:93-94
+    swtpg_firwin_int(7, 0.1, 1 << c.tap_exponent, c.fir_taps);
+    c.fir_taps[7] = 0;
+  }
+  const bool scalar_forced = getenv("SWTPG_FORCE_SCALAR") != nullptr;
+  // Packed fast path validity (see PackedSimpleWibEth)
+  c.fast_simple = c.algorithm == SWTPG_ALGO_SIMPLE_THRESHOLD && c.threshold <= 32767 &&
+                  (wib2 || (c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000)) && !scalar_forced;
+
+  c.fast_rs = !wib2 && (c.algorithm == SWTPG_ALGO_ABS_RS || c.algorithm == SWTPG_ALGO_STANDARD_RS) && c.threshold <= 32767 &&
+              c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000 && !scalar_forced;
+  // WIB2 AbsRS fast path validity (see PackedRsIqrWib2); threshold >= 1 is enforced above for the algorithm as such
+  if (wib2 && c.algorithm == SWTPG_ALGO_ABS_RS && c.threshold >= 1) {
+    const uint32_t e = c.tap_exponent, mult = 1u << e;
+    const uint64_t sigma_max = (1u << 15) / (uint64_t(mult) * c.threshold);
+    // thresholds sigma * threshold are compared by the bf16 comparator (valid up to 32640) and built by a packed multiply-add
+    // (no carry between the halves while (sigmaMax + 3) * threshold < 2^16); outside that range every group takes the
+    // exact-threshold tier (plain signed compares on the 64-bit-lane product, like the reference's _mm256_cmpgt_epi16)
+    const bool packed_ok = e >= 1 && e <= 10 && !scalar_forced;
+    const bool range_ok = (sigma_max + 3) * c.threshold < 65536 && sigma_max * c.threshold <= 32640;
+    c.fast_rs_wib2 = packed_ok;
+    c.fir_force_exact = packed_ok && !range_ok;
+  }
+  // Packed FIR fast path validity (see PackedFirIqr): binomial taps, and (sigmaMax + 3) * multiplier * threshold < 2^16
+  {
+    static const int16_t kBinomial[8] = { 1, 6, 15, 20, 15, 6, 1, 0 };
+    bool taps_ok = true;
+    for (int i = 0; i < 8; ++i)
+      taps_ok &= c.fir_taps[i] == kBinomial[i];
+    const uint32_t e = c.tap_exponent, mult = 1u << e;
+    const uint64_t sigma_max = (1u << 15) / (mult * 5u);
+    // The packed policies build sigma * multiplier * threshold with one multiply-add (no carry between the halves while
+    // (sigmaMax + 3) * K < 2^16) and compare through the bf16 comparator, which orders like signed int16 only up to 32640:
+    // K = multiplier * threshold with sigmaMax * K <= 32640 (threshold <= 5 at the reference's exponent 6). Beyond that the
+    // reference's _mm256_cmpgt_epi16 sees the product as a NEGATIVE int16 once a channel's IQR is large enough, so such
+    // configurations run the same packed trackers and filter with the exact-threshold tier forced on for every group.
+    const uint64_t K = uint64_t(mult) * c.threshold;
+    const bool packed_ok = c.algorithm == SWTPG_ALGO_FIR_IQR && e >= 1 && e <= 10 && !scalar_forced;
+    const bool range_ok = (sigma_max + 3) * K < 65536 && sigma_max * K <= 32640;
+    c.fast_fir = packed_ok && taps_ok;      // binomial cascade
+    c.fast_fir_any = packed_ok && !taps_ok; // any other taps[0..6]: packed multiply-add chain (PackedFirIqrAnyTaps)
+    if (packed_ok && !range_ok)
+      c.fir_force_exact = true;
+  }
+  *out = c;
+  return SWTPG_OK;
+}
+
+// Whether links of configurations a and b can run in one launch: they agree in every field their algorithm reads (the kernel
+// parameters the policies of launch() consume). The policy flags follow from those fields. rs_memory_factor is per-link state
+// (SV_RS_FACTOR rows), not a kernel parameter, so it never splits a group.
+bool
+same_group(int32_t format, const TpgConf& a, const TpgConf& b)
+{
+  if (a.algorithm != b.algorithm || a.threshold != b.threshold)
+    return false;
+  const bool wib2 = format == SWTPG_FORMAT_WIB2;
+  const bool acc = !wib2 && a.algorithm != SWTPG_ALGO_FIR_IQR; // WIB2 and the FIR finder hard-wire 10 (wib2/tpg/ProcessAVX2.hpp:79)
+  const bool scale = !wib2 && a.algorithm == SWTPG_ALGO_ABS_RS; // StandardRS adds s' unscaled (ProcessStandardRSAVX2.hpp:140-144)
+  const bool exponent = wib2 || a.algorithm == SWTPG_ALGO_FIR_IQR; // the charge shift of WIB2, the multiplier of FIR + IQR
+  const bool taps = a.algorithm == SWTPG_ALGO_FIR_IQR;
+  if (acc && a.frugal_acc_limit != b.frugal_acc_limit)
+    return false;
+  if (scale && a.rs_scale_factor != b.rs_scale_factor)
+    return false;
+  if (exponent && a.tap_exponent != b.tap_exponent)
+    return false;
+  if (taps && memcmp(a.fir_taps, b.fir_taps, sizeof a.fir_taps) != 0)
+    return false;
+  return true;
+}
+
 } // namespace
 
 cudaError_t
 swtpg_internal::launch_batch_kernel(swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t units_stride, swtpg_tp* d_tps,
                                     unsigned* d_count, cudaStream_t s)
 {
-  const KernelParams kp = make_params(h, d_frames, d_nunits, units_stride, d_tps, d_count, nullptr, nullptr);
-  return launch<false>(h, kp, s);
+  return launch_groups<false>(h, d_frames, d_nunits, units_stride, d_tps, d_count, nullptr, nullptr, s);
 }
 
 extern "C" void swtpg_internal_ingest_counts(swtpg_handle* h, uint64_t* zero_copy, uint64_t* staged); // swtpg_stream.cu
@@ -558,16 +710,22 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "max_units must stay below 2^18 units per batch (hit records carry the unit index in 18 bits)");
   if (cfg->format != SWTPG_FORMAT_WIBETH && cfg->format != SWTPG_FORMAT_WIB2)
     return fail(nullptr, SWTPG_ERR_UNSUPPORTED, "unknown frame format");
-  if (cfg->algorithm < SWTPG_ALGO_SIMPLE_THRESHOLD || cfg->algorithm > SWTPG_ALGO_FIR_IQR)
-    return fail(nullptr, SWTPG_ERR_UNSUPPORTED, "unknown tpg_algorithm (reference: TPGAlgorithmInexistent)");
-  if (cfg->format == SWTPG_FORMAT_WIB2 && cfg->algorithm == SWTPG_ALGO_STANDARD_RS)
-    return fail(nullptr, SWTPG_ERR_UNSUPPORTED, "StandardRS does not exist for the WIB2 format (reference: SimpleThreshold and AbsRS only)");
-  if (cfg->format == SWTPG_FORMAT_WIB2 && cfg->algorithm == SWTPG_ALGO_ABS_RS && cfg->threshold == 0)
-    return fail(nullptr, SWTPG_ERR_INVALID_ARG, "WIB2 AbsRS needs threshold >= 1 (sigmaMax = 2^15 / (multiplier * threshold))");
+  swtpg_link_config own{};
+  own.struct_size = sizeof own;
+  own.algorithm = cfg->algorithm;
+  own.threshold = cfg->threshold;
+  own.frugal_acc_limit = cfg->frugal_acc_limit;
+  own.rs_memory_factor = cfg->rs_memory_factor;
+  own.rs_scale_factor = cfg->rs_scale_factor;
+  memcpy(own.fir_taps, cfg->fir_taps, sizeof own.fir_taps);
+  own.tap_exponent = cfg->tap_exponent;
+  TpgConf conf;
+  const char* why = nullptr;
+  const swtpg_status cs = classify_config(cfg->format, own, &conf, &why);
+  if (cs != SWTPG_OK)
+    return fail(nullptr, cs, why);
   if (cfg->wib2_adc_offset % 4 != 0 || cfg->wib2_adc_offset > SWTPG_WIB2_FRAME_BYTES - 448)
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "wib2_adc_offset must be a multiple of 4 and leave room for the 448-byte ADC block");
-  if (cfg->tap_exponent > 14)
-    return fail(nullptr, SWTPG_ERR_INVALID_ARG, "tap_exponent out of range");
   if (cfg->flags & ~SWTPG_FLAG_SORTED_TPS)
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "unknown bits in swtpg_config.flags");
 
@@ -598,71 +756,30 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
     h->cfg.n_slots = 4; // measured: 2 slots 38.0, 3 slots 45.4, 4 slots 47.1, 6 slots 47.2 GB/s (profiles/r02_streaming_slots_probe.txt)
   if (h->cfg.n_slots < 2)
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "n_slots must be >= 2");
-  if (h->cfg.tap_exponent == 0)
-    h->cfg.tap_exponent = 6;
+  h->cfg.tap_exponent = conf.tap_exponent;
+  memcpy(h->cfg.fir_taps, conf.fir_taps, sizeof conf.fir_taps);
   if (h->cfg.wib2_adc_offset == 0)
     h->cfg.wib2_adc_offset = 20;
-  bool any_tap = false;
-  for (int i = 0; i < 8; ++i)
-    any_tap |= h->cfg.fir_taps[i] != 0;
-  if (!any_tap) { // src/wib2/WIB2FrameProcessor.cpp:93-94
-    swtpg_firwin_int(7, 0.1, 1 << h->cfg.tap_exponent, h->cfg.fir_taps);
-    h->cfg.fir_taps[7] = 0;
-  }
+  h->confs.assign(1, conf);
+  h->conf_links.assign(1, cfg->n_links);
+  h->link_conf.assign(cfg->n_links, 0);
+  h->link_rs_factor.assign(cfg->n_links, cfg->rs_memory_factor);
+  h->rs_table_link.assign(cfg->n_links, 0);
   // TP buffer: explicit, else samples/128 per batch clamped to [64 Ki, 16 Mi] records (physical TP rates are orders of
   // magnitude below one per 128 samples; the high-occupancy stress configuration sets tp_capacity itself).
   const uint64_t samples = uint64_t(cfg->n_links) * cfg->max_units * h->channels * h->ticks;
   uint64_t cap = cfg->tp_capacity ? cfg->tp_capacity : std::min<uint64_t>(std::max<uint64_t>(samples / 128, 1u << 16), 1u << 24);
   cap = std::min<uint64_t>(cap, std::max<uint64_t>(samples / 2, 1));
   h->tp_capacity = uint32_t(cap);
-  // Packed fast path validity (see PackedSimpleWibEth)
-  h->fast_simple = cfg->algorithm == SWTPG_ALGO_SIMPLE_THRESHOLD && cfg->threshold <= 32767 &&
-                   (wib2 || (cfg->frugal_acc_limit >= 1 && cfg->frugal_acc_limit <= 1000)) && getenv("SWTPG_FORCE_SCALAR") == nullptr;
-
-  h->fast_rs = !wib2 && (cfg->algorithm == SWTPG_ALGO_ABS_RS || cfg->algorithm == SWTPG_ALGO_STANDARD_RS) && cfg->threshold <= 32767 &&
-               cfg->frugal_acc_limit >= 1 && cfg->frugal_acc_limit <= 1000 && getenv("SWTPG_FORCE_SCALAR") == nullptr;
-  // WIB2 AbsRS fast path validity (see PackedRsIqrWib2); threshold >= 1 is enforced below for the algorithm as such
-  if (wib2 && cfg->algorithm == SWTPG_ALGO_ABS_RS && cfg->threshold >= 1) {
-    const uint32_t e = h->cfg.tap_exponent, mult = 1u << e;
-    const uint64_t sigma_max = (1u << 15) / (uint64_t(mult) * cfg->threshold);
-    // thresholds sigma * threshold are compared by the bf16 comparator (valid up to 32640) and built by a packed multiply-add
-    // (no carry between the halves while (sigmaMax + 3) * threshold < 2^16); outside that range every group takes the
-    // exact-threshold tier (plain signed compares on the 64-bit-lane product, like the reference's _mm256_cmpgt_epi16)
-    const bool packed_ok = e >= 1 && e <= 10 && getenv("SWTPG_FORCE_SCALAR") == nullptr;
-    const bool range_ok = (sigma_max + 3) * cfg->threshold < 65536 && sigma_max * cfg->threshold <= 32640;
-    h->fast_rs_wib2 = packed_ok;
-    h->fir_force_exact = packed_ok && !range_ok;
-  }
-  // Packed FIR fast path validity (see PackedFirIqr): binomial taps, and (sigmaMax + 3) * multiplier * threshold < 2^16
-  {
-    static const int16_t kBinomial[8] = { 1, 6, 15, 20, 15, 6, 1, 0 };
-    bool taps_ok = true;
-    for (int i = 0; i < 8; ++i)
-      taps_ok &= h->cfg.fir_taps[i] == kBinomial[i];
-    const uint32_t e = h->cfg.tap_exponent, mult = 1u << e;
-    const uint64_t sigma_max = (1u << 15) / (mult * 5u);
-    // The packed policies build sigma * multiplier * threshold with one multiply-add (no carry between the halves while
-    // (sigmaMax + 3) * K < 2^16) and compare through the bf16 comparator, which orders like signed int16 only up to 32640:
-    // K = multiplier * threshold with sigmaMax * K <= 32640 (threshold <= 5 at the reference's exponent 6). Beyond that the
-    // reference's _mm256_cmpgt_epi16 sees the product as a NEGATIVE int16 once a channel's IQR is large enough, so such
-    // configurations run the same packed trackers and filter with the exact-threshold tier forced on for every group.
-    const uint64_t K = uint64_t(mult) * cfg->threshold;
-    const bool packed_ok = cfg->algorithm == SWTPG_ALGO_FIR_IQR && e >= 1 && e <= 10 && getenv("SWTPG_FORCE_SCALAR") == nullptr;
-    const bool range_ok = (sigma_max + 3) * K < 65536 && sigma_max * K <= 32640;
-    h->fast_fir = packed_ok && taps_ok;      // binomial cascade
-    h->fast_fir_any = packed_ok && !taps_ok; // any other taps[0..6]: packed multiply-add chain (PackedFirIqrAnyTaps)
-    if (packed_ok && !range_ok)
-      h->fir_force_exact = true;
-  }
-
   swtpg_handle* hp = h.get();
   SW_CUDA(hp, cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
   SW_CUDA(hp, cudaEventCreate(&h->ev0));
   SW_CUDA(hp, cudaEventCreate(&h->ev1));
   SW_CUDA(hp, cudaMalloc(&h->d_state, size_t(h->n_groups) * kStateWordsPerGroup * 4));
   SW_CUDA(hp, cudaMalloc(&h->d_flags, size_t(h->n_groups) * 4));
-  SW_CUDA(hp, cudaMalloc(&h->d_link_cursor, (2 + size_t(h->cfg.n_links)) * sizeof(uint32_t)));
-  SW_CUDA(hp, cudaMemset(h->d_link_cursor, 0, (2 + size_t(h->cfg.n_links)) * sizeof(uint32_t)));
+  SW_CUDA(hp, cudaMalloc(&h->d_link_cursor, (2 * SWTPG_MAX_LINK_CONFIGS + size_t(h->cfg.n_links)) * sizeof(uint32_t)));
+  SW_CUDA(hp, cudaMemset(h->d_link_cursor, 0, (2 * SWTPG_MAX_LINK_CONFIGS + size_t(h->cfg.n_links)) * sizeof(uint32_t)));
+  SW_CUDA(hp, cudaMalloc(&h->d_group_links, size_t(h->cfg.n_links) * sizeof(uint32_t)));
   SW_CUDA(hp, cudaMalloc(&h->d_tps, size_t(h->tp_capacity) * sizeof(swtpg_tp)));
   SW_CUDA(hp, cudaMalloc(&h->d_count, sizeof(unsigned)));
   SW_CUDA(hp, cudaMallocHost(&h->h_count, sizeof(unsigned)));
@@ -696,6 +813,7 @@ swtpg_destroy(swtpg_handle* h)
   if (h->d_state) cudaFree(h->d_state);
   if (h->d_flags) cudaFree(h->d_flags);
   if (h->d_link_cursor) cudaFree(h->d_link_cursor);
+  if (h->d_group_links) cudaFree(h->d_group_links);
   if (h->d_tps) cudaFree(h->d_tps);
   if (h->d_count) cudaFree(h->d_count);
   if (h->h_count) cudaFreeHost(h->h_count);
@@ -721,7 +839,10 @@ swtpg_start(swtpg_handle* h)
   if (!h)
     return SWTPG_ERR_INVALID_ARG;
   SW_CUDA(h, cudaSetDevice(h->cfg.device));
-  swtpg_status s = reset_state(h);
+  swtpg_status s = SWTPG_OK;
+  if (h->conf_groups_stale && (s = form_conf_groups(h)) != SWTPG_OK)
+    return s;
+  s = reset_state(h);
   if (s != SWTPG_OK)
     return s;
   s = swtpg_internal::engine_reset(h); // streaming path: idle, rings empty, undelivered TPs of the previous run dropped
@@ -755,6 +876,7 @@ swtpg_set_rs_memory_factor(swtpg_handle* h, const uint16_t* by_link_channel)
     h->h_rs_factor = new uint16_t[n];
     memcpy(h->h_rs_factor, by_link_channel, n * sizeof(uint16_t));
   }
+  std::fill(h->rs_table_link.begin(), h->rs_table_link.end(), by_link_channel ? 1 : 0);
   if (h->started) { // only the factor rows change; carried state is preserved
     SW_CUDA(h, cudaSetDevice(h->cfg.device));
     return upload_rs_factor_rows(h, 0, h->cfg.n_links);
@@ -769,17 +891,63 @@ swtpg_set_link_rs_memory_factor(swtpg_handle* h, uint32_t link, const uint16_t* 
     return SWTPG_ERR_INVALID_ARG;
   {
     std::lock_guard<std::mutex> lk(h->engine_mu); // several links' threads may arrive here with their first frames
-    if (!h->h_rs_factor) {
-      const size_t n = size_t(h->cfg.n_links) * h->channels;
-      h->h_rs_factor = new uint16_t[n];
-      std::fill(h->h_rs_factor, h->h_rs_factor + n, h->cfg.rs_memory_factor);
-    }
+    if (!h->h_rs_factor) // the other links keep their configuration's factor (rs_table_link)
+      h->h_rs_factor = new uint16_t[size_t(h->cfg.n_links) * h->channels];
     memcpy(h->h_rs_factor + size_t(link) * h->channels, by_channel, size_t(h->channels) * sizeof(uint16_t));
+    h->rs_table_link[link] = 1;
   }
   if (!h->started)
     return SWTPG_OK; // swtpg_start uploads the table
   SW_CUDA(h, cudaSetDevice(h->cfg.device));
   return upload_rs_factor_rows(h, link, 1);
+}
+
+swtpg_status
+swtpg_set_link_config(swtpg_handle* h, uint32_t link, const swtpg_link_config* c)
+{
+  if (!h)
+    return fail(nullptr, SWTPG_ERR_INVALID_ARG, "handle is NULL");
+  if (h->started)
+    return fail(h, SWTPG_ERR_STATE, "a link's configuration can only change while the handle is stopped");
+  if (link >= h->cfg.n_links)
+    return fail(h, SWTPG_ERR_INVALID_ARG, "link out of range");
+  TpgConf conf = h->confs[0];
+  uint16_t rs_factor = h->cfg.rs_memory_factor;
+  if (c) {
+    if (c->struct_size != sizeof(swtpg_link_config))
+      return fail(h, SWTPG_ERR_INVALID_ARG, "swtpg_link_config.struct_size mismatch");
+    const char* why = nullptr;
+    const swtpg_status s = classify_config(h->cfg.format, *c, &conf, &why);
+    if (s != SWTPG_OK)
+      return fail(h, s, why);
+    rs_factor = c->rs_memory_factor;
+  }
+  std::lock_guard<std::mutex> lk(h->engine_mu); // links' conf() calls may arrive from several threads
+  const uint32_t old = h->link_conf[link];
+  --h->conf_links[old];
+  auto in_use = [&](uint32_t i) { return i == 0 || h->conf_links[i] != 0; }; // the handle's own always counts
+  uint32_t at = uint32_t(h->confs.size());
+  for (uint32_t i = 0; i < h->confs.size() && at == h->confs.size(); ++i)
+    if (in_use(i) && same_group(h->cfg.format, h->confs[i], conf))
+      at = i;
+  for (uint32_t i = 1; i < h->confs.size() && at == h->confs.size(); ++i)
+    if (!in_use(i))
+      at = i; // a free entry
+  if (at == h->confs.size()) {
+    if (at == SWTPG_MAX_LINK_CONFIGS) {
+      ++h->conf_links[old];
+      return fail(h, SWTPG_ERR_INVALID_ARG, "more than SWTPG_MAX_LINK_CONFIGS distinct link configurations");
+    }
+    h->confs.push_back(conf);
+    h->conf_links.push_back(0);
+  } else if (!in_use(at)) {
+    h->confs[at] = conf;
+  }
+  ++h->conf_links[at];
+  h->link_conf[link] = uint8_t(at);
+  h->link_rs_factor[link] = rs_factor;
+  h->conf_groups_stale = true;
+  return SWTPG_OK;
 }
 
 swtpg_status

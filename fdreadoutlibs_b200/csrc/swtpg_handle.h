@@ -19,6 +19,30 @@
 namespace swtpg_internal {
 struct StreamEngine;
 struct TpSorter;
+
+// One TPG configuration (swtpg_create's or a link's, swtpg_set_link_config), normalised — default taps and tap exponent
+// filled in — and classified: which policy of the launch table runs it. classify_config (swtpg_capi.cu) is the only place
+// that makes one.
+struct TpgConf
+{
+  int32_t algorithm = 0;
+  uint16_t threshold = 0;
+  int16_t frugal_acc_limit = 0;
+  uint16_t rs_scale_factor = 0;
+  int16_t fir_taps[SWTPG_MAX_TAPS] = {};
+  uint8_t tap_exponent = 0;
+  bool fast_simple = false, fast_fir = false, fast_rs = false, fast_rs_wib2 = false, fast_fir_any = false;
+  bool fir_force_exact = false; // packed FIR / WIB2-AbsRS trackers with the exact-threshold tier on every group (classify_config)
+};
+
+// Links of one handle whose configurations run as one launch of the batch kernel (formed at swtpg_start).
+struct ConfGroup
+{
+  uint32_t conf = 0;                  // index into swtpg_handle::confs
+  uint32_t n_links = 0;
+  const uint32_t* d_links = nullptr;  // the group's links in ascending order; nullptr = every link of the handle
+  uint32_t* d_cursor = nullptr;       // its own {claimed, finished} pair of the kernels' dynamic link hand-out
+};
 }
 
 struct swtpg_handle
@@ -26,9 +50,20 @@ struct swtpg_handle
   swtpg_config cfg{};
   uint32_t unit_bytes = 0, channels = 0, ticks = 0, groups_per_link = 0, n_groups = 0;
   uint32_t tp_capacity = 0;
-  bool fast_simple = false, fast_fir = false, fast_rs = false, fast_rs_wib2 = false, fast_fir_any = false;
-  bool fir_force_exact = false; // packed FIR / WIB2-AbsRS trackers with the exact-threshold tier on every group (see swtpg_create)
   std::atomic<bool> started{ false };
+
+  // TPG configurations: confs[0] is the handle's own (swtpg_create), the others come from swtpg_set_link_config; link l runs
+  // confs[link_conf[l]]. No two entries in use run the same (same_group), and there are at most SWTPG_MAX_LINK_CONFIGS.
+  std::vector<swtpg_internal::TpgConf> confs;
+  std::vector<uint32_t> conf_links;    // links using each entry of confs; an entry other than 0 with none is free
+  std::vector<uint8_t> link_conf;      // [n_links]
+  std::vector<uint16_t> link_rs_factor; // [n_links] rs_memory_factor of each link's configuration
+  // Configuration groups: one per entry of confs in use, formed by swtpg_start when a link's configuration has changed, and
+  // frozen while the handle is started (the streaming engine's threads read them without a lock, so swtpg_set_link_config
+  // refuses to run then).
+  std::vector<swtpg_internal::ConfGroup> conf_groups;
+  bool conf_groups_stale = true;
+  uint32_t* d_group_links = nullptr;   // [n_links]: the groups' link lists, back to back
 
   cudaStream_t stream = nullptr; // batch path + all kernels (state is carried batch to batch: kernels are ordered)
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -37,8 +72,9 @@ struct swtpg_handle
 
   uint32_t* d_state = nullptr;
   uint32_t* d_flags = nullptr;
-  uint32_t* d_link_cursor = nullptr; // {claimed, finished}: dynamic link hand-out of the kernels, self-resetting; followed by
-                                     // [n_links] slices done per link (wibeth_kernel's sliced hand-out, self-resetting too)
+  uint32_t* d_link_cursor = nullptr; // SWTPG_MAX_LINK_CONFIGS x {claimed, finished}: dynamic link hand-out of the kernels, one
+                                     // pair per configuration group, self-resetting; followed by [n_links] slices done per link
+                                     // (wibeth_kernel's sliced hand-out, self-resetting too)
   swtpg_tp* d_tps = nullptr;
   unsigned* d_count = nullptr;
   unsigned* h_count = nullptr;
@@ -54,6 +90,7 @@ struct swtpg_handle
   int16_t* d_wav = nullptr;
   size_t d_dump_elems = 0;
   uint16_t* h_rs_factor = nullptr; // [n_links][channels] or null
+  std::vector<uint8_t> rs_table_link; // [n_links] 1 = the link's rows of h_rs_factor were set (else its configuration's factor)
   swtpg_internal::TpSorter* sorter = nullptr; // SWTPG_FLAG_SORTED_TPS: device-side ordering of TP lists (swtpg_sort.cu)
 
   // streaming path (swtpg_stream.cu), created on the first swtpg_submit / swtpg_register_buffer

@@ -77,11 +77,14 @@ struct KernelParams
   const uint8_t* frames;   // link-major units
   const uint32_t* n_units; // per link, or nullptr = units_stride everywhere
   uint32_t units_stride;
-  uint32_t n_links;
+  uint32_t n_links;        // links this launch works on: its configuration group's
+  const uint32_t* link_ids; // [n_links] the group's links (ascending), nullptr = links 0 .. n_links-1. Work item i of the launch
+                            // is link link_ids[i mod n_links]; frames, n_units, state, flags, link_done, TPs and dumps are
+                            // indexed by that link
   uint32_t* state;         // [n_groups][SV_COUNT][32]
   uint32_t* group_flags;   // [n_groups]: bit 0 initialized, bits 8..10 FIR ring phase (absTimeModNTAPS)
   uint32_t* link_cursor;   // [2] {links claimed beyond each warp's first, warps finished}; zero between launches (WIBEth kernel)
-  uint32_t* link_done;     // [n_links] slices of the link finished in THIS launch; zero between launches (wibeth_kernel, sliced)
+  uint32_t* link_done;     // [links of the handle] slices of the link finished in THIS launch; zero between launches (wibeth_kernel, sliced)
   uint32_t parts_log2;     // wibeth_kernel: a link's units are handed out in 2^parts_log2 consecutive slices (0 = whole links)
   uint32_t slice_geom;     // ... of equal length (0) or halving: n/2, n/4, ..., and the rest (1)
   TpSink sink;
@@ -1669,7 +1672,7 @@ wibeth_kernel(const KernelParams p)
     --fifo_n;
     return link;
   };
-  // Work items: item i = slice (i / n_links) of link (i % n_links); slice k of a link with n units is its units
+  // Work items: item i = slice (i / n_links) of the group's link (i % n_links); slice k of a link with n units is its units
   // [k n >> parts_log2, (k + 1) n >> parts_log2), or, with slice_geom, halving slices (what the launch's last round leaves idle is
   // at most one LAST slice, so small last slices shorten the tail without more state round trips per link). Items are claimed
   // in increasing order, so every first slice is handed out before any second one.
@@ -1680,6 +1683,8 @@ wibeth_kernel(const KernelParams p)
       link -= p.n_links;
       ++part;
     }
+    if (p.link_ids != nullptr) // one configuration group of several: its (item mod n_links)-th link
+      link = p.link_ids[link];
     const uint32_t n = units_of(link);
     if (p.slice_geom) { // halving slices: n/2, n/4, ... and the rest (slice k starts ceil(n / 2^k) units before the end)
       u0 = n - ((n + (1u << part) - 1u) >> part);
@@ -1870,6 +1875,7 @@ wibeth_kernel(const KernelParams p)
 // Ragged batches: a quad runs for the longest of its links; a consumer whose link is shorter (or absent) only keeps step.
 // =====================================================================================================================
 constexpr int kQuad = 4;
+constexpr uint32_t kNoLink = 0xFFFFFFFFu; // quad position without a link (past the end of the group)
 constexpr uint32_t kQuadFifo = 4; // quads in flight: the producer is at most NSTAGE chunks ahead, a quad has >= kChunksPerUnit chunks
 
 template<int NSTAGE, int CHUNK_TICKS>
@@ -1907,6 +1913,7 @@ wibeth_quad_kernel(const KernelParams p)
 
   auto units_of = [&](uint32_t link) -> uint32_t { return p.n_units ? p.n_units[link] : p.units_stride; };
   auto base_of = [&](uint32_t link) -> const uint8_t* { return p.frames + size_t(link) * p.units_stride * SWTPG_WIBETH_FRAME_BYTES; };
+  auto link_of = [&](uint32_t item) -> uint32_t { return p.link_ids != nullptr ? p.link_ids[item] : item; }; // the group's item-th link
 
   if (threadIdx.x == 0) {
 #pragma unroll
@@ -1928,7 +1935,7 @@ wibeth_quad_kernel(const KernelParams p)
       if (round != 0)
         mbar_wait_producer(&empty[slot], (round - 1u) & 1u);
     };
-    uint32_t first_link = blockIdx.x * kQuad; // the CTA's first quad; every further one is claimed from the cursor
+    uint32_t first_link = blockIdx.x * kQuad; // the CTA's first quad (work items); every further one is claimed from the cursor
     for (bool first = true;;) {
       uint32_t nu[kQuad], longest = 0;
       for (;;) { // next quad that has data
@@ -1939,8 +1946,8 @@ wibeth_quad_kernel(const KernelParams p)
         if (first_link >= p.n_links)
           break;
 #pragma unroll
-        for (int c = 0; c < kQuad; ++c) {
-          nu[c] = first_link + c < p.n_links ? units_of(first_link + c) : 0u;
+        for (int c = 0; c < kQuad; ++c) { // a group's last quad may be partial
+          nu[c] = first_link + c < p.n_links ? units_of(link_of(first_link + c)) : 0u;
           longest = max(longest, nu[c]);
         }
         if (longest != 0)
@@ -1954,13 +1961,15 @@ wibeth_quad_kernel(const KernelParams p)
         mbar_arrive(&full[slot]);
         break;
       }
-      const uint8_t* src0 = base_of(first_link) + 32;                             // link c of the quad: + c * link_stride
+      const uint8_t* src0 = p.frames + 32;                                        // link l of the quad: + l * link_stride
       const size_t link_stride = size_t(p.units_stride) * SWTPG_WIBETH_FRAME_BYTES;
       for (uint32_t unit = 0; unit < longest; ++unit) {
         for (uint32_t ch = 0; ch < kChunksPerUnit; ++ch) {
           wait_slot();
           if (unit == 0 && ch == 0) { // published before the arrive below releases it to the consumers
-            entry[0] = first_link;
+#pragma unroll
+            for (int c = 0; c < kQuad; ++c)
+              entry[c] = first_link + c < p.n_links ? link_of(first_link + c) : kNoLink;
             entry[4] = longest;
             entry[5] = 0u;
             ++pushed;
@@ -1974,7 +1983,7 @@ wibeth_quad_kernel(const KernelParams p)
 #pragma unroll
           for (int c = 0; c < kQuad; ++c)
             if (unit < nu[c])
-              bulk_g2s(stages + (slot * kQuad + c) * kChunkBytes, src + c * link_stride, kChunkBytes, &full[slot]);
+              bulk_g2s(stages + (slot * kQuad + c) * kChunkBytes, src + link_of(first_link + c) * link_stride, kChunkBytes, &full[slot]);
           if (++slot == NSTAGE) {
             slot = 0;
             ++round;
@@ -2006,9 +2015,11 @@ wibeth_quad_kernel(const KernelParams p)
     const volatile uint32_t* entry = fifo + (popped & (kQuadFifo - 1u)) * 8u;
     if (entry[5] != 0u)
       break;
-    const uint32_t link = entry[0] + warp, longest = entry[4];
-    const uint32_t n_units = link < p.n_links ? units_of(link) : 0u;
-    const uint8_t* link_base = base_of(link < p.n_links ? link : 0u);
+    // the position's link through a reduction: a uniform register, as the link index was before groups (ptxas otherwise
+    // needs up to 7 more registers for this kernel)
+    const uint32_t link = __reduce_max_sync(0xFFFFFFFFu, entry[warp]), longest = entry[4];
+    const uint32_t n_units = link != kNoLink ? units_of(link) : 0u;
+    const uint8_t* link_base = base_of(link != kNoLink ? link : 0u);
     uint32_t* st = p.state + size_t(link) * kStateWordsPerGroup;
     uint32_t flags = 0;
     bool need_seed = false;
@@ -2151,20 +2162,21 @@ wib2_kernel(const KernelParams p)
       if (round != 0)
         mbar_wait_producer(&empty[slot], (round - 1u) & 1u);
     };
-    uint32_t link = blockIdx.x; // the CTA's first link; every further one is claimed from the cursor (as in wibeth_kernel)
+    uint32_t item = blockIdx.x; // the CTA's first work item; every further one is claimed from the cursor (as in wibeth_kernel)
     for (bool first = true;; first = false) {
-      uint32_t n_units = 0;
+      uint32_t n_units = 0, link = 0;
       for (;;) {
         if (!first)
-          link = gridDim.x + atomicAdd(p.link_cursor, 1u);
+          item = gridDim.x + atomicAdd(p.link_cursor, 1u);
         first = false;
-        if (link >= p.n_links)
+        if (item >= p.n_links)
           break;
+        link = p.link_ids != nullptr ? p.link_ids[item] : item; // the group's item-th link
         n_units = units_of(link);
         if (n_units != 0)
           break;
       }
-      if (link >= p.n_links) { // end marker: a stage that completes without data
+      if (item >= p.n_links) { // end marker: a stage that completes without data
         wait_slot();
         fifo[pushed & (kWib2Fifo - 1u)] = kNoMoreLinks;
         mbar_arrive(&full[slot]);

@@ -76,13 +76,20 @@ TpgEngine::attach(FrameProcessorBase* p)
 }
 
 void
-TpgEngine::configure(const swtpg_config& a)
+TpgEngine::configure(uint32_t link, const swtpg_config& a)
 {
   std::lock_guard<std::mutex> lk(m_mu);
-  if (m_configured) {
-    if (a.algorithm != m_cfg.algorithm || a.threshold != m_cfg.threshold || a.frugal_acc_limit != m_cfg.frugal_acc_limit ||
-        a.rs_memory_factor != m_cfg.rs_memory_factor || a.rs_scale_factor != m_cfg.rs_scale_factor)
-      throw std::runtime_error("TpgEngine: the links of one device must share one TPG configuration");
+  if (m_configured) { // every link parses its own RawDataProcessorConf (src/wibeth/WIBEthFrameProcessor.cpp:175-230)
+    swtpg_link_config c{};
+    c.struct_size = sizeof c;
+    c.algorithm = a.algorithm;
+    c.threshold = a.threshold;
+    c.frugal_acc_limit = a.frugal_acc_limit;
+    c.rs_memory_factor = a.rs_memory_factor;
+    c.rs_scale_factor = a.rs_scale_factor;
+    memcpy(c.fir_taps, a.fir_taps, sizeof c.fir_taps);
+    c.tap_exponent = a.tap_exponent;
+    check(m_h, swtpg_set_link_config(m_h, link, &c), "swtpg_set_link_config");
     return;
   }
   m_cfg.algorithm = a.algorithm;
@@ -290,8 +297,8 @@ WIBEthFrameProcessor::conf(const RawDataProcessorConf& config)
     a.frugal_acc_limit = m_tpg_frugal_streaming_accumulator_limit;
     a.rs_memory_factor = m_tpg_rs_memory_factor;
     a.rs_scale_factor = m_tpg_rs_scale_factor;
-    m_engine->configure(a);
     m_wibeth_frame_handler->link = m_engine->attach(this);
+    m_engine->configure(m_wibeth_frame_handler->link, a);
     inherited::add_postprocess_task([this](constframeptr fp) { find_hits(fp, m_wibeth_frame_handler.get()); });
   }
   inherited::conf(config);
@@ -527,8 +534,8 @@ WIB2FrameProcessor::conf(const RawDataProcessorConf& config)
     m_channel_map = make_map(config.channel_map_name);
     a.threshold = config.tpg_threshold;
     a.frugal_acc_limit = 10;
-    m_engine->configure(a);
     m_handler->link = m_engine->attach(this);
+    m_engine->configure(m_handler->link, a);
     inherited::add_postprocess_task([this](constframeptr fp) { find_hits(fp, m_handler.get()); });
   }
   inherited::conf(config);
@@ -818,6 +825,15 @@ struct swtpg_host_conf
   uint32_t sink_capacity; // per link; try_send fails beyond it (0 = unbounded)
 };
 
+// The TPG fields of one link's RawDataProcessorConf, overriding those of swtpg_host_conf (swtpg_host_create_links).
+struct swtpg_host_link_conf
+{
+  char tpg_algorithm[32];
+  float tpg_rs_memory_factor, tpg_rs_scale_factor;
+  uint16_t tpg_threshold;
+  int16_t tpg_frugal_streaming_accumulator_limit;
+};
+
 struct swtpg_host_tp
 {
   uint64_t time_start, time_peak, time_over_threshold;
@@ -851,8 +867,8 @@ swtpg_host_last_error(void)
   return g_host_error.c_str();
 }
 
-swtpg_host*
-swtpg_host_create(const swtpg_host_conf* c)
+static swtpg_host*
+host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links)
 {
   try {
     auto h = std::make_unique<swtpg_host>();
@@ -881,6 +897,13 @@ swtpg_host_create(const swtpg_host_conf* c)
       rc.channel_map_name = c->reversed_map ? "reversed" : "linear";
       rc.enable_simple_threshold_on_collection = c->enable_simple_threshold_on_collection != 0;
       rc.block_on_backpressure = c->block_on_backpressure != 0;
+      if (links) {
+        rc.tpg_algorithm = links[l].tpg_algorithm;
+        rc.tpg_threshold = links[l].tpg_threshold;
+        rc.tpg_rs_memory_factor = links[l].tpg_rs_memory_factor;
+        rc.tpg_rs_scale_factor = links[l].tpg_rs_scale_factor;
+        rc.tpg_frugal_streaming_accumulator_limit = links[l].tpg_frugal_streaming_accumulator_limit;
+      }
       swtpg_host* hp = h.get();
       auto sink = [hp, l](TriggerPrimitiveTypeAdapter&& tp) {
         if (hp->count_only) {
@@ -910,6 +933,19 @@ swtpg_host_create(const swtpg_host_conf* c)
     g_host_error = e.what();
   }
   return nullptr;
+}
+
+swtpg_host*
+swtpg_host_create(const swtpg_host_conf* c)
+{
+  return host_create(c, nullptr);
+}
+
+// links[n_links]: each frame processor's conf() gets its own TPG fields (one engine, links with different configurations)
+swtpg_host*
+swtpg_host_create_links(const swtpg_host_conf* c, const swtpg_host_link_conf* links)
+{
+  return host_create(c, links);
 }
 
 void

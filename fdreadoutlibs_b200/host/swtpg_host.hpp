@@ -228,7 +228,9 @@ public:
   ~TpgEngine();
   TpgEngine(const TpgEngine&) = delete;
   uint32_t attach(FrameProcessorBase* p);      // conf(): returns the link index
-  void configure(const swtpg_config& algo);    // first conf() fixes the algorithm parameters; later ones must agree
+  // conf() of the processor attached as `link`: the first one creates the handle with its parameters, every later one sets its
+  // own link's (swtpg_set_link_config), so links of one device may run different algorithms and thresholds. Before start().
+  void configure(uint32_t link, const swtpg_config& algo);
   void start();                                // idempotent per run: the first processor to start creates the handle state
   void stop();                                 // flush + drain; the last processor to stop ends the run
   // per-position RS memory factor of one link, by FRAME channel (src/wibeth/WIBEthFrameProcessor.cpp:437-456 + setState)

@@ -21,6 +21,11 @@ class HostConf(C.Structure):
                 ("block_on_backpressure", C.c_uint8), ("count_only_sink", C.c_uint8), ("n_slots", C.c_uint8), ("sink_capacity", C.c_uint32)]
 
 
+class HostLinkConf(C.Structure):
+    _fields_ = [("tpg_algorithm", C.c_char * 32), ("tpg_rs_memory_factor", C.c_float), ("tpg_rs_scale_factor", C.c_float),
+                ("tpg_threshold", C.c_uint16), ("tpg_frugal_streaming_accumulator_limit", C.c_int16)]
+
+
 HOST_TP_DTYPE = np.dtype([("time_start", "<u8"), ("time_peak", "<u8"), ("time_over_threshold", "<u8"), ("channel", "<u4"),
                           ("adc_integral", "<u4"), ("adc_peak", "<u2"), ("detid", "<u2"), ("type", "<u4"), ("algorithm", "<u4"),
                           ("version", "<u2"), ("flag", "<u2")], align=True)
@@ -49,7 +54,7 @@ class TpHandlerInfo(C.Structure):
 
 EXPORTS = ["swtpg_host_tpsets_create", "swtpg_host_tpsets_destroy", "swtpg_host_tpsets_receive", "swtpg_host_tpsets_cycle",
            "swtpg_host_tpsets_cutoff", "swtpg_host_tpsets_count", "swtpg_host_tpsets_get", "swtpg_host_tpsets_info",
-           "swtpg_host_push_parallel", "swtpg_host_push_feeders", "swtpg_host_tp_count", "swtpg_host_counters", "swtpg_host_stream_timing", "swtpg_host_last_error", "swtpg_host_create", "swtpg_host_destroy", "swtpg_host_start", "swtpg_host_stop", "swtpg_host_push",
+           "swtpg_host_push_parallel", "swtpg_host_push_feeders", "swtpg_host_tp_count", "swtpg_host_counters", "swtpg_host_stream_timing", "swtpg_host_last_error", "swtpg_host_create", "swtpg_host_create_links", "swtpg_host_destroy", "swtpg_host_start", "swtpg_host_stop", "swtpg_host_push",
            "swtpg_host_take_tps", "swtpg_host_get_info", "swtpg_host_error_count", "swtpg_host_misconfigurations",
            "swtpg_host_last_daq_time", "swtpg_host_register_channel_map", "swtpg_host_register_buffer"]
 
@@ -63,6 +68,8 @@ def host_lib():
         lib.swtpg_host_last_error.restype = C.c_char_p
         lib.swtpg_host_create.restype = C.c_void_p
         lib.swtpg_host_create.argtypes = [C.POINTER(HostConf)]
+        lib.swtpg_host_create_links.restype = C.c_void_p
+        lib.swtpg_host_create_links.argtypes = [C.POINTER(HostConf), C.POINTER(HostLinkConf)]
         lib.swtpg_host_destroy.argtypes = [C.c_void_p]
         lib.swtpg_host_start.argtypes = [C.c_void_p]
         lib.swtpg_host_stop.argtypes = [C.c_void_p]
@@ -113,7 +120,9 @@ class FrameProcessors:
                  crate_id: int = 1, slot_id: int = 0, first_link_id: int = 0, enable_tpg: bool = True, emulator_mode: bool = False,
                  correct_channel_lookup: bool = False, reversed_map: bool = False, collection_simple_threshold: bool = False,
                  sink_capacity: int = 0, block_on_backpressure: bool = True, device: int = 0, count_only_sink: bool = False,
-                 n_slots: int = 4):
+                 n_slots: int = 4, link_confs=None):
+        """link_confs: optional list of n_links dicts, each overriding algorithm, threshold, rs_memory_factor, rs_scale_factor
+        and acc_limit for its link's conf(); the keys it leaves out take the arguments above."""
         c = HostConf()
         c.device, c.format, c.n_links, c.superchunk_units = device, 1 if fmt == "wib2" else 0, n_links, superchunk_units
         c.tpg_algorithm = algorithm.encode()
@@ -131,7 +140,18 @@ class FrameProcessors:
         c.n_slots = n_slots
         self.lib = host_lib()
         self.n_links = n_links
-        self.h = self.lib.swtpg_host_create(C.byref(c))
+        if link_confs is None:
+            self.h = self.lib.swtpg_host_create(C.byref(c))
+        else:
+            assert len(link_confs) == n_links
+            links = (HostLinkConf * n_links)()
+            for l, lc in enumerate(link_confs):
+                links[l].tpg_algorithm = lc.get("algorithm", algorithm).encode()
+                links[l].tpg_threshold = lc.get("threshold", threshold)
+                links[l].tpg_rs_memory_factor = lc.get("rs_memory_factor", rs_memory_factor)
+                links[l].tpg_rs_scale_factor = lc.get("rs_scale_factor", rs_scale_factor)
+                links[l].tpg_frugal_streaming_accumulator_limit = lc.get("acc_limit", acc_limit)
+            self.h = self.lib.swtpg_host_create_links(C.byref(c), links)
         if not self.h:
             raise HostError(self.lib.swtpg_host_last_error().decode())
 

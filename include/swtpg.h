@@ -164,6 +164,31 @@ swtpg_status swtpg_set_rs_memory_factor(swtpg_handle* h, const uint16_t* by_link
  * against the other links' calls and against batches in flight. */
 swtpg_status swtpg_set_link_rs_memory_factor(swtpg_handle* h, uint32_t link, const uint16_t* by_channel);
 
+/* Per-link TPG configuration. Every frame processor of the reference parses its own RawDataProcessorConf
+ * (src/wibeth/WIBEthFrameProcessor.cpp:175-230), so two links of one application may run different algorithms or thresholds.
+ * Links whose configurations agree in every field their algorithm reads form one configuration group; each group is one
+ * launch of the batch kernel, and the groups of a batch run one after another on the same stream. */
+#define SWTPG_MAX_LINK_CONFIGS 16u /* distinct configurations per handle, the handle's own included */
+typedef struct swtpg_link_config
+{
+  uint32_t struct_size;      /* = sizeof(swtpg_link_config) */
+  int32_t algorithm;         /* swtpg_algorithm */
+  uint16_t threshold;
+  int16_t frugal_acc_limit;
+  uint16_t rs_memory_factor, rs_scale_factor; /* already x10 / 10/x, as in swtpg_config */
+  int16_t fir_taps[SWTPG_MAX_TAPS];           /* all zero = firwin_int(7, 0.1, 1 << tap_exponent) + {0} */
+  uint8_t tap_exponent;      /* 0 = 6 */
+  uint8_t reserved0[3];
+} swtpg_link_config;
+/* The TPG parameters of ONE link (the rest of its conf(): src/wibeth/WIBEthFrameProcessor.cpp:175-230). NULL = back to the
+ * handle's swtpg_config. Only while the handle is not started (before swtpg_start or after swtpg_stop): SWTPG_ERR_STATE
+ * otherwise. Takes effect at the next swtpg_start, which gives every link fresh state. SWTPG_ERR_INVALID_ARG for a bad
+ * struct_size, link >= n_links, a field out of range or a configuration that would make more than SWTPG_MAX_LINK_CONFIGS
+ * distinct ones (configurations that differ only in fields their algorithm does not read, or only in rs_memory_factor,
+ * count as one); SWTPG_ERR_UNSUPPORTED for an unknown algorithm or StandardRS on WIB2, as swtpg_create. A per-channel table
+ * of swtpg_set_*rs_memory_factor takes precedence over the link's rs_memory_factor, as over the handle's. */
+swtpg_status swtpg_set_link_config(swtpg_handle* h, uint32_t link, const swtpg_link_config* c);
+
 /*
  * Batch entry points. `frames` is link-major: unit u of link l starts at ((l * units_stride) + u) * unit_bytes.
  * n_units[l] <= units_stride <= cfg.max_units valid units for link l (ragged batches allowed; NULL = all links
