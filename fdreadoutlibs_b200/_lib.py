@@ -77,6 +77,7 @@ EXPORTS = {
     "swtpg_set_rs_memory_factor": (C.c_int, [C.c_void_p, C.c_void_p]),
     "swtpg_set_link_rs_memory_factor": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p]),
     "swtpg_set_link_config": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(SwtpgLinkConfig)]),
+    "swtpg_set_link_thresholds": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p]),
     "swtpg_process_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "swtpg_process_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
     "swtpg_fetch_tps": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),

@@ -155,6 +155,15 @@ class TPGenerator:
         c.tap_exponent = h.tap_exponent if tap_exponent is None else tap_exponent
         self._check(lib.swtpg_set_link_config(self._h, link, C.byref(c)))
 
+    def set_link_thresholds(self, link: int, by_channel: Optional[np.ndarray]):
+        """swtpg_set_link_thresholds: per-channel hit thresholds of one link, by frame channel (0..32767 each); None returns the
+        link to its configuration's threshold. SimpleThreshold and the WIBEth running sums only. Only while the handle is
+        stopped; takes effect at the next start() and stays until reset."""
+        a = None if by_channel is None else np.ascontiguousarray(by_channel, dtype=np.uint16)
+        if a is not None:
+            assert a.size == self.channels
+        self._check(lib.swtpg_set_link_thresholds(self._h, link, _ptr(a)))
+
     # -- batch entry points ----------------------------------------------------------------------------------------------
     def _nunits(self, n_units):
         if n_units is None:

@@ -404,10 +404,12 @@ form_conf_groups(swtpg_handle* h)
 swtpg_status
 reset_state(swtpg_handle* h)
 {
-  // Fresh zeroed ChanState (wibeth/tpg/ProcessingInfo.hpp:23-40) + per-channel RS memory factor (setState :131)
+  // Fresh zeroed ChanState (wibeth/tpg/ProcessingInfo.hpp:23-40) + per-channel RS memory factor (setState :131) + per-channel
+  // hit threshold: the link's table, else its configuration's threshold, so that every link has a valid row
   std::vector<uint32_t> st(size_t(h->n_groups) * kStateWordsPerGroup, 0u);
   for (uint32_t g = 0; g < h->n_groups; ++g) {
     const uint32_t link = g / h->groups_per_link, sub = g % h->groups_per_link;
+    const std::vector<uint16_t>& table = h->link_thresholds[link];
     for (uint32_t lane = 0; lane < 32; ++lane) {
       uint32_t lo = h->link_rs_factor[link], hi = lo;
       if (h->h_rs_factor && h->rs_table_link[link]) {
@@ -416,6 +418,12 @@ reset_state(swtpg_handle* h)
         hi = f[1];
       }
       st[size_t(g) * kStateWordsPerGroup + SV_RS_FACTOR * 32 + lane] = lo | (hi << 16);
+      lo = hi = h->confs[h->link_conf[link]].threshold;
+      if (!table.empty()) {
+        lo = table[sub * 64 + 2 * lane];
+        hi = table[sub * 64 + 2 * lane + 1];
+      }
+      st[size_t(g) * kStateWordsPerGroup + SV_THRESHOLD * 32 + lane] = lo | (hi << 16);
     }
   }
   SW_CUDA(h, cudaMemcpyAsync(h->d_state, st.data(), st.size() * 4, cudaMemcpyHostToDevice, h->stream));
@@ -611,6 +619,15 @@ classify_config(int32_t format, const swtpg_link_config& in, TpgConf* out, const
   return SWTPG_OK;
 }
 
+// Whether a link running `algorithm` may have a per-channel threshold table: the algorithms whose threshold is in ADC counts. FIR +
+// IQR and WIB2 AbsRS multiply it by an IQR sigma on 4 x int64 lanes that carry between neighbouring channels (iqr_threshold_exact),
+// where a per-channel multiplier has no reference meaning.
+bool
+threshold_table_allowed(int32_t format, int32_t algorithm)
+{
+  return algorithm != SWTPG_ALGO_FIR_IQR && !(format == SWTPG_FORMAT_WIB2 && algorithm == SWTPG_ALGO_ABS_RS);
+}
+
 // Whether links of configurations a and b can run in one launch: they agree in every field their algorithm reads (the kernel
 // parameters the policies of launch() consume). The policy flags follow from those fields. rs_memory_factor is per-link state
 // (SV_RS_FACTOR rows), not a kernel parameter, so it never splits a group.
@@ -764,6 +781,7 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
   h->conf_links.assign(1, cfg->n_links);
   h->link_conf.assign(cfg->n_links, 0);
   h->link_rs_factor.assign(cfg->n_links, cfg->rs_memory_factor);
+  h->link_thresholds.assign(cfg->n_links, {});
   h->rs_table_link.assign(cfg->n_links, 0);
   // TP buffer: explicit, else samples/128 per batch clamped to [64 Ki, 16 Mi] records (physical TP rates are orders of
   // magnitude below one per 128 samples; the high-occupancy stress configuration sets tp_capacity itself).
@@ -923,6 +941,8 @@ swtpg_set_link_config(swtpg_handle* h, uint32_t link, const swtpg_link_config* c
     rs_factor = c->rs_memory_factor;
   }
   std::lock_guard<std::mutex> lk(h->engine_mu); // links' conf() calls may arrive from several threads
+  if (!h->link_thresholds[link].empty() && !threshold_table_allowed(h->cfg.format, conf.algorithm))
+    return fail(h, SWTPG_ERR_UNSUPPORTED, "the link has a per-channel threshold table, which its new algorithm cannot use (clear it first)");
   const uint32_t old = h->link_conf[link];
   --h->conf_links[old];
   auto in_use = [&](uint32_t i) { return i == 0 || h->conf_links[i] != 0; }; // the handle's own always counts
@@ -947,6 +967,29 @@ swtpg_set_link_config(swtpg_handle* h, uint32_t link, const swtpg_link_config* c
   h->link_conf[link] = uint8_t(at);
   h->link_rs_factor[link] = rs_factor;
   h->conf_groups_stale = true;
+  return SWTPG_OK;
+}
+
+swtpg_status
+swtpg_set_link_thresholds(swtpg_handle* h, uint32_t link, const uint16_t* by_channel)
+{
+  if (!h)
+    return fail(nullptr, SWTPG_ERR_INVALID_ARG, "handle is NULL");
+  if (h->started)
+    return fail(h, SWTPG_ERR_STATE, "a link's thresholds can only change while the handle is stopped");
+  if (link >= h->cfg.n_links)
+    return fail(h, SWTPG_ERR_INVALID_ARG, "link out of range");
+  std::lock_guard<std::mutex> lk(h->engine_mu); // links' conf() calls may arrive from several threads
+  if (!by_channel) {
+    h->link_thresholds[link].clear();
+    return SWTPG_OK;
+  }
+  for (uint32_t c = 0; c < h->channels; ++c)
+    if (by_channel[c] > 32767u)
+      return fail(h, SWTPG_ERR_INVALID_ARG, "a per-channel threshold is above 32767");
+  if (!threshold_table_allowed(h->cfg.format, h->confs[h->link_conf[link]].algorithm))
+    return fail(h, SWTPG_ERR_UNSUPPORTED, "per-channel thresholds exist for SimpleThreshold and the WIBEth running sums only");
+  h->link_thresholds[link].assign(by_channel, by_channel + h->channels);
   return SWTPG_OK;
 }
 

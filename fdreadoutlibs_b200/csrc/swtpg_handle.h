@@ -58,6 +58,9 @@ struct swtpg_handle
   std::vector<uint32_t> conf_links;    // links using each entry of confs; an entry other than 0 with none is free
   std::vector<uint8_t> link_conf;      // [n_links]
   std::vector<uint16_t> link_rs_factor; // [n_links] rs_memory_factor of each link's configuration
+  // [n_links] per-channel hit thresholds of swtpg_set_link_thresholds, by frame channel; empty = the configuration's threshold.
+  // Only links whose algorithm compares ADC counts have one (threshold_table_allowed); swtpg_start writes the SV_THRESHOLD rows.
+  std::vector<std::vector<uint16_t>> link_thresholds;
   // Configuration groups: one per entry of confs in use, formed by swtpg_start when a link's configuration has changed, and
   // frozen while the handle is started (the streaming engine's threads read them without a lock, so swtpg_set_link_config
   // refuses to run then).

@@ -67,7 +67,9 @@ enum StateVar
   SV_ACC_RS,
   SV_RS_FACTOR,
   SV_RING0, // .. SV_RING0 + 7
-  SV_COUNT = SV_RING0 + 8
+  SV_THRESHOLD = SV_RING0 + 8, // u16x2 hit threshold by lane of the ADC-threshold algorithms (swtpg_set_link_thresholds), written by
+                               // swtpg_start; FIR + IQR and WIB2 AbsRS read KernelParams::threshold instead
+  SV_COUNT
 };
 constexpr uint32_t kStateWordsPerGroup = SV_COUNT * 32;
 constexpr uint32_t kFlagInitialized = 1u;
@@ -204,6 +206,7 @@ struct ChanRegs
   int q25, q75, a25, a75;
   int rs, med_rs, acc_rs, rs_factor;
   int ring[8];
+  int threshold; // SV_THRESHOLD as int16, like the reference's signed compare against (int16)threshold
 };
 
 template<int ALGO, bool WIB2>
@@ -230,6 +233,8 @@ struct ScalarAlgo
 #pragma unroll
       for (int j = 0; j < 8; ++j)
         r.ring[j] = g(SV_RING0 + j);
+      if constexpr (ALGO != SWTPG_ALGO_FIR_IQR && !(WIB2 && ALGO == SWTPG_ALGO_ABS_RS)) // these compare against an IQR sigma
+        r.threshold = g(SV_THRESHOLD);
     }
     kphase = (flags >> 8) & 7u;
   }
@@ -286,7 +291,6 @@ struct ScalarAlgo
   __device__ __forceinline__ void tick(uint32_t S, const TickCtx& ctx, int t, uint32_t lane, uint32_t& ped_out, uint32_t& wav_out)
   {
     const KernelParams& p = *ctx.p;
-    const int thr = int(int16_t(uint16_t(p.threshold)));
     int ped[2], wav[2];
     if constexpr (ALGO == SWTPG_ALGO_FIR_IQR) {
       // wib2/tpg/ProcessAVX2FIR.hpp:103-283
@@ -405,7 +409,7 @@ struct ScalarAlgo
           r.rs = rs;
           level = rs;
         }
-        const bool over = level > thr;
+        const bool over = level > r.threshold; // the channel's own threshold (SV_THRESHOLD)
         const bool left = r.prev && !over;
         if constexpr (WIB2) { // wib2/tpg/ProcessAVX2.hpp:104-121
           r.charge = sat16(int(int16_t(r.charge)) + ((over ? x : 0) >> p.tap_exponent)) & 0xFFFF;
@@ -503,10 +507,13 @@ struct PackedSimpleT
     cLL = L * 0x00010001u;
     c2L = 2u * L * 0x00010001u;
     kM1 = p.all_ones;
-    uint32_t th = p.threshold > 16383u ? 16383u : p.threshold; // s' <= 16383: any larger threshold is never exceeded
-    th += 1u;
-    thr1 = th | (th << 16);
     shift = shmask = 0;
+  }
+  // thr1 of a lane's two channels from their SV_THRESHOLD row (0..32767 per half): each half clamped to `max` first, where any
+  // larger threshold is never exceeded, then + 1. Once per work item, so the tick loop is the same as with one threshold.
+  static __device__ __forceinline__ uint32_t thr1_of(uint32_t row, uint32_t max)
+  {
+    return add2(minu2(row, max * 0x00010001u), 0x00010001u);
   }
   // Register form of the accumulator: (acc - 1) as the bit pattern of an fp16x2 subnormal (value * 2^-24, sign-magnitude).
   static __device__ __forceinline__ uint32_t acc_to_reg(uint32_t v)
@@ -535,6 +542,7 @@ struct PackedSimpleT
     Tn = neg2(st[SV_TOVER * 32 + lane]);
     PK1 = add2(st[SV_PEAK_ADC * 32 + lane], 0x00010001u);
     PTn = neg2(st[SV_PEAK_TIME * 32 + lane]);
+    thr1 = thr1_of(st[SV_THRESHOLD * 32 + lane], 16383u); // s' <= 16383
     dvalid = false;
     dwhen = 0u;
 #pragma unroll
@@ -827,15 +835,13 @@ struct PackedRsWibEth : PackedSimpleWibEth
   __device__ __forceinline__ void configure(const KernelParams& p)
   {
     PackedSimpleWibEth::configure(p);
-    // RS - median_RS is in [-6554, 6554]: a larger threshold is never exceeded (and stays inside the comparator's range)
-    uint32_t th = p.threshold > 6555u ? 6555u : p.threshold;
-    th += 1u;
-    thr1 = th | (th << 16);
     scale = p.rs_scale;
   }
   __device__ __forceinline__ void load(const uint32_t* st, uint32_t lane, uint32_t flags)
   {
     PackedSimpleWibEth::load(st, lane, flags);
+    // RS - median_RS is in [-6554, 6554]: a larger threshold is never exceeded (and stays inside the comparator's range)
+    thr1 = thr1_of(st[SV_THRESHOLD * 32 + lane], 6555u);
     RS1 = add2(st[SV_RS * 32 + lane], 0x00010001u);
     MRq = add2(~st[SV_MED_RS * 32 + lane], 0x00020002u);
     AR = acc_to_reg(st[SV_ACC_RS * 32 + lane]);

@@ -149,6 +149,34 @@ TpgEngine::set_link_memory_factor(uint32_t link, const uint16_t* by_channel, uin
   check(m_h, swtpg_set_link_rs_memory_factor(m_h, link, by_channel), "swtpg_set_link_rs_memory_factor");
 }
 
+void
+TpgEngine::set_link_thresholds(uint32_t link, const uint16_t* by_channel, uint32_t n_channels)
+{
+  const uint32_t channels = m_cfg.format == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_CHANNELS : SWTPG_WIBETH_CHANNELS;
+  if (by_channel && n_channels != channels)
+    throw std::invalid_argument("TpgEngine::set_link_thresholds: one threshold per frame channel of the link");
+  check(m_h, swtpg_set_link_thresholds(m_h, link, by_channel), "swtpg_set_link_thresholds");
+}
+
+// The per-frame-channel table of RawDataProcessorConf::tpg_plane_threshold: channel c of the link (crate, slot, link) takes the
+// threshold of its plane, or tpg_threshold where that is -1. Empty when no plane has its own.
+static std::vector<uint16_t>
+plane_threshold_table(const RawDataProcessorConf& config, const ChannelMap& map, uint32_t channels)
+{
+  std::vector<uint16_t> table;
+  const auto& plane = config.tpg_plane_threshold;
+  if (plane[0] < 0 && plane[1] < 0 && plane[2] < 0)
+    return table;
+  for (int32_t t : plane)
+    if (t > 32767)
+      throw std::invalid_argument("tpg_plane_threshold: above 32767");
+  for (uint32_t c = 0; c < channels; ++c) {
+    const int32_t t = plane[get_plane_from_offline_channel(map(config.crate_id, config.slot_id, config.link_id, c))];
+    table.push_back(t >= 0 ? uint16_t(t) : config.tpg_threshold);
+  }
+  return table;
+}
+
 bool
 TpgEngine::submit(uint32_t link, const void* unit, size_t bytes, uint64_t wait_us)
 {
@@ -299,6 +327,10 @@ WIBEthFrameProcessor::conf(const RawDataProcessorConf& config)
     a.rs_scale_factor = m_tpg_rs_scale_factor;
     m_wibeth_frame_handler->link = m_engine->attach(this);
     m_engine->configure(m_wibeth_frame_handler->link, a);
+    // the table must be in place before start(), so it comes from the configured ids rather than the first frame's header (a link
+    // whose frames carry other ids is reported as a LinkMisconfiguration)
+    const std::vector<uint16_t> table = plane_threshold_table(config, m_channel_map, SWTPG_WIBETH_CHANNELS);
+    m_engine->set_link_thresholds(m_wibeth_frame_handler->link, table.empty() ? nullptr : table.data(), uint32_t(table.size()));
     inherited::add_postprocess_task([this](constframeptr fp) { find_hits(fp, m_wibeth_frame_handler.get()); });
   }
   inherited::conf(config);
@@ -532,10 +564,14 @@ WIB2FrameProcessor::conf(const RawDataProcessorConf& config)
   if (config.enable_tpg) {
     m_tpg_enabled = true;
     m_channel_map = make_map(config.channel_map_name);
+    const std::vector<uint16_t> table = plane_threshold_table(config, m_channel_map, SWTPG_WIB2_CHANNELS);
+    if (!table.empty() && a.algorithm != SWTPG_ALGO_SIMPLE_THRESHOLD) // FIR + IQR and AbsRS multiply the threshold by an IQR sigma
+      throw std::invalid_argument("tpg_plane_threshold: WIB2 supports per-plane thresholds with SimpleThreshold only");
     a.threshold = config.tpg_threshold;
     a.frugal_acc_limit = 10;
     m_handler->link = m_engine->attach(this);
     m_engine->configure(m_handler->link, a);
+    m_engine->set_link_thresholds(m_handler->link, table.empty() ? nullptr : table.data(), uint32_t(table.size()));
     inherited::add_postprocess_task([this](constframeptr fp) { find_hits(fp, m_handler.get()); });
   }
   inherited::conf(config);
@@ -832,6 +868,7 @@ struct swtpg_host_link_conf
   float tpg_rs_memory_factor, tpg_rs_scale_factor;
   uint16_t tpg_threshold;
   int16_t tpg_frugal_streaming_accumulator_limit;
+  int32_t tpg_plane_threshold[3]; // -1 = tpg_threshold
 };
 
 struct swtpg_host_tp
@@ -903,6 +940,7 @@ host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links)
         rc.tpg_rs_memory_factor = links[l].tpg_rs_memory_factor;
         rc.tpg_rs_scale_factor = links[l].tpg_rs_scale_factor;
         rc.tpg_frugal_streaming_accumulator_limit = links[l].tpg_frugal_streaming_accumulator_limit;
+        std::copy(links[l].tpg_plane_threshold, links[l].tpg_plane_threshold + 3, rc.tpg_plane_threshold.begin());
       }
       swtpg_host* hp = h.get();
       auto sink = [hp, l](TriggerPrimitiveTypeAdapter&& tp) {

@@ -121,6 +121,10 @@ struct RawDataProcessorConf
   std::string channel_map_name = "linear";
   bool emulator_mode = false;
   bool correct_channel_lookup = false; // false: index the position-ordered LUT with the frame channel, as production does (H2)
+  // Not a reference field: hit threshold per plane, indexed by get_plane_from_offline_channel (0 = collection); -1 = tpg_threshold.
+  // conf() resolves it into a per-frame-channel table through the channel map and the configured crate / slot / link ids
+  // (swtpg_set_link_thresholds). SimpleThreshold and the WIBEth running sums only.
+  std::array<int32_t, 3> tpg_plane_threshold{ -1, -1, -1 };
   // Back-pressure from the GPU pipeline: false = drop the frame and count it (what a full queue does to the reference's
   // try_send); true = wait for a staging slot (file replay / emulators, where losing data is worse than stalling).
   bool block_on_backpressure = false;
@@ -235,6 +239,9 @@ public:
   void stop();                                 // flush + drain; the last processor to stop ends the run
   // per-position RS memory factor of one link, by FRAME channel (src/wibeth/WIBEthFrameProcessor.cpp:437-456 + setState)
   void set_link_memory_factor(uint32_t link, const uint16_t* by_channel, uint32_t n_channels);
+  // per-channel hit thresholds of one link, by FRAME channel (swtpg_set_link_thresholds); nullptr = the link's tpg_threshold.
+  // Before start(), like configure().
+  void set_link_thresholds(uint32_t link, const uint16_t* by_channel, uint32_t n_channels);
   // false = back-pressure (the link's ring is full). wait_us > 0: sleep up to that long for room first (swtpg_submit_wait)
   bool submit(uint32_t link, const void* unit, size_t bytes, uint64_t wait_us = 0);
   // Zero-copy ingest: the latency buffer(s) the constframeptrs point into (swtpg_register_buffer). After conf().

@@ -23,7 +23,8 @@ class HostConf(C.Structure):
 
 class HostLinkConf(C.Structure):
     _fields_ = [("tpg_algorithm", C.c_char * 32), ("tpg_rs_memory_factor", C.c_float), ("tpg_rs_scale_factor", C.c_float),
-                ("tpg_threshold", C.c_uint16), ("tpg_frugal_streaming_accumulator_limit", C.c_int16)]
+                ("tpg_threshold", C.c_uint16), ("tpg_frugal_streaming_accumulator_limit", C.c_int16),
+                ("tpg_plane_threshold", C.c_int32 * 3)]
 
 
 HOST_TP_DTYPE = np.dtype([("time_start", "<u8"), ("time_peak", "<u8"), ("time_over_threshold", "<u8"), ("channel", "<u4"),
@@ -122,7 +123,8 @@ class FrameProcessors:
                  sink_capacity: int = 0, block_on_backpressure: bool = True, device: int = 0, count_only_sink: bool = False,
                  n_slots: int = 4, link_confs=None):
         """link_confs: optional list of n_links dicts, each overriding algorithm, threshold, rs_memory_factor, rs_scale_factor
-        and acc_limit for its link's conf(); the keys it leaves out take the arguments above."""
+        and acc_limit for its link's conf(); the keys it leaves out take the arguments above. A dict may also set
+        plane_threshold: three thresholds by plane (0 = collection), -1 = the link's threshold (tpg_plane_threshold)."""
         c = HostConf()
         c.device, c.format, c.n_links, c.superchunk_units = device, 1 if fmt == "wib2" else 0, n_links, superchunk_units
         c.tpg_algorithm = algorithm.encode()
@@ -151,6 +153,8 @@ class FrameProcessors:
                 links[l].tpg_rs_memory_factor = lc.get("rs_memory_factor", rs_memory_factor)
                 links[l].tpg_rs_scale_factor = lc.get("rs_scale_factor", rs_scale_factor)
                 links[l].tpg_frugal_streaming_accumulator_limit = lc.get("acc_limit", acc_limit)
+                for p, t in enumerate(lc.get("plane_threshold", (-1, -1, -1))):
+                    links[l].tpg_plane_threshold[p] = t
             self.h = self.lib.swtpg_host_create_links(C.byref(c), links)
         if not self.h:
             raise HostError(self.lib.swtpg_host_last_error().decode())

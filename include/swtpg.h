@@ -189,6 +189,20 @@ typedef struct swtpg_link_config
  * of swtpg_set_*rs_memory_factor takes precedence over the link's rs_memory_factor, as over the handle's. */
 swtpg_status swtpg_set_link_config(swtpg_handle* h, uint32_t link, const swtpg_link_config* c);
 
+/* Per-channel thresholds of ONE link, by frame channel: by_channel[SWTPG_*_CHANNELS], each 0..32767 (ADC counts above the
+ * pedestal, or above the RS median). NULL = back to the threshold of the link's configuration. An extension of the reference,
+ * which applies one tpg_threshold to every channel of a frame processor: induction and collection planes, or a hot channel,
+ * can have their own without a configuration per threshold (and without masking the channel).
+ *   - Only while the handle is not started (SWTPG_ERR_STATE otherwise); takes effect at the next swtpg_start, like
+ *     swtpg_set_link_config. The table stays until NULL or swtpg_destroy: it survives swtpg_stop / swtpg_start and later
+ *     swtpg_set_link_config calls, and takes precedence over the threshold of the link's configuration.
+ *   - SWTPG_ERR_INVALID_ARG for a NULL handle, link >= n_links or an entry above 32767.
+ *   - SWTPG_ERR_UNSUPPORTED for a table on a link whose algorithm is FIR_IQR or WIB2 AbsRS: there the threshold multiplies an
+ *     IQR sigma. swtpg_set_link_config refuses the same way to move a link that has a table to one of those algorithms
+ *     (a NULL that returns it to such a handle configuration included). A refused call changes nothing; NULL is always accepted.
+ *   - Tables do not split configuration groups: a link's thresholds are per-channel state, like its RS memory factors. */
+swtpg_status swtpg_set_link_thresholds(swtpg_handle* h, uint32_t link, const uint16_t* by_channel);
+
 /*
  * Batch entry points. `frames` is link-major: unit u of link l starts at ((l * units_stride) + u) * unit_bytes.
  * n_units[l] <= units_stride <= cfg.max_units valid units for link l (ragged batches allowed; NULL = all links
