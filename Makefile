@@ -29,12 +29,16 @@ $(OBJ)/swtpg_stream.o: $(CSRC)/swtpg_stream.cu $(CSRC)/swtpg_handle.h include/sw
 $(OBJ)/swtpg_sort.o: $(CSRC)/swtpg_sort.cu $(CSRC)/swtpg_handle.h include/swtpg.h
 	@mkdir -p $(OBJ)
 	$(NVCC) $(NVFLAGS) -c -o $@ $(CSRC)/swtpg_sort.cu 2> build_ptxas_sort.log || (cat build_ptxas_sort.log; exit 1)
+# per-channel ADC statistics (SWTPG_FLAG_ADC_STATS)
+$(OBJ)/swtpg_stats.o: $(CSRC)/swtpg_stats.cu $(CSRC)/swtpg_device.cuh $(CSRC)/swtpg_handle.h include/swtpg.h
+	@mkdir -p $(OBJ)
+	$(NVCC) $(NVFLAGS) -c -o $@ $(CSRC)/swtpg_stats.cu 2> build_ptxas_stats.log || (cat build_ptxas_stats.log; exit 1)
 # host-only pieces: staging copy, TP sort / merge, FIR tap design
 $(OBJ)/swtpg_hostutil.o: $(CSRC)/swtpg_hostutil.cpp include/swtpg.h
 	@mkdir -p $(OBJ)
 	g++ -O2 -std=c++17 -Wall -fPIC -c -o $@ $(CSRC)/swtpg_hostutil.cpp
 
-$(LIB): $(OBJ)/swtpg_capi.o $(OBJ)/swtpg_stream.o $(OBJ)/swtpg_sort.o $(OBJ)/swtpg_hostutil.o
+$(LIB): $(OBJ)/swtpg_capi.o $(OBJ)/swtpg_stream.o $(OBJ)/swtpg_sort.o $(OBJ)/swtpg_stats.o $(OBJ)/swtpg_hostutil.o
 	$(NVCC) $(ARCH) -shared -o $@ $^ -lpthread
 
 $(GENLIB): $(CSRC)/framegen_capi.cu $(CSRC)/framegen.h include/swtpg_framegen.h include/swtpg.h
@@ -57,6 +61,6 @@ oracle:
 	$(MAKE) -C oracle all
 
 clean:
-	rm -rf $(LIB) $(GENLIB) $(HOST) $(OBJ) build_ptxas.log build_ptxas_stream.log build_ptxas_sort.log
+	rm -rf $(LIB) $(GENLIB) $(HOST) $(OBJ) build_ptxas.log build_ptxas_stream.log build_ptxas_sort.log build_ptxas_stats.log
 	$(MAKE) -C oracle clean
 .PHONY: all lib host apps oracle clean

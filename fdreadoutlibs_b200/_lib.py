@@ -58,6 +58,17 @@ class SwtpgLinkConfig(C.Structure):
     ]
 
 
+class SwtpgAdcStats(C.Structure):
+    _fields_ = [
+        ("samples", C.c_uint64),
+        ("sum", C.c_uint64),
+        ("sum_sq", C.c_uint64),
+        ("min", C.c_uint16),
+        ("max", C.c_uint16),
+        ("reserved", C.c_uint32),
+    ]
+
+
 class SwtpgCounters(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in (
         "units_processed", "samples_processed", "tps_emitted", "tps_dropped_overflow", "batches", "submit_busy",
@@ -95,6 +106,7 @@ EXPORTS = {
     "swtpg_stream_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
     "swtpg_sync": (C.c_int, [C.c_void_p]),
     "swtpg_dump_state": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p]),
+    "swtpg_read_adc_stats": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int]),
     "swtpg_get_counters": (C.c_int, [C.c_void_p, C.POINTER(SwtpgCounters)]),
     "swtpg_sort_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "swtpg_alloc_pinned": (C.c_void_p, [C.c_size_t, C.c_int]),

@@ -23,6 +23,7 @@ ALGORITHMS = {
 }
 FORMATS = {"wibeth": FORMAT_WIBETH, "wib2": FORMAT_WIB2}
 FLAG_SORTED_TPS = 1  # SWTPG_FLAG_SORTED_TPS
+FLAG_ADC_STATS = 2  # SWTPG_FLAG_ADC_STATS
 
 
 class SwtpgError(RuntimeError):
@@ -53,9 +54,10 @@ class TPGenerator:
     def __init__(self, n_links: int, max_units: int, *, fmt: str = "wibeth", algorithm: str = "SimpleThreshold", threshold: int = 60,
                  acc_limit: int = 10, rs_memory_factor: int = 8, rs_scale_factor: int = 5, fir_taps: Optional[Sequence[int]] = None,
                  tap_exponent: int = 6, tp_capacity: int = 0, n_slots: int = 0, device: int = 0, wib2_adc_offset: int = 0,
-                 dispatch_timeout_us: int = 0, sorted_tps: bool = False):
+                 dispatch_timeout_us: int = 0, sorted_tps: bool = False, adc_stats: bool = False):
         """sorted_tps: SWTPG_FLAG_SORTED_TPS — every batch's TP list comes back ordered by (time_start, link, channel), ordered on
-        the device (include/swtpg.h)."""
+        the device (include/swtpg.h). adc_stats: SWTPG_FLAG_ADC_STATS — per-channel ADC statistics of every batch, read by
+        read_adc_stats()."""
         if algorithm not in ALGORITHMS:
             raise TPGAlgorithmInexistent(algorithm)
         cfg = SwtpgConfig()
@@ -77,7 +79,7 @@ class TPGenerator:
         cfg.tap_exponent = tap_exponent
         cfg.wib2_adc_offset = wib2_adc_offset
         cfg.dispatch_timeout_us = dispatch_timeout_us
-        cfg.flags = FLAG_SORTED_TPS if sorted_tps else 0
+        cfg.flags = (FLAG_SORTED_TPS if sorted_tps else 0) | (FLAG_ADC_STATS if adc_stats else 0)
         self.cfg = cfg
         self.fmt = fmt
         self.n_links = n_links
@@ -290,6 +292,15 @@ class TPGenerator:
     def dump_state(self, link: int) -> np.ndarray:
         out = np.zeros(self.channels, dtype=F.STATE_DTYPE)
         self._check(lib.swtpg_dump_state(self._h, link, out.ctypes.data))
+        return out
+
+    def read_adc_stats(self, link0: int = 0, n_links: Optional[int] = None, reset: bool = False) -> np.ndarray:
+        """swtpg_read_adc_stats: the current window of links [link0, link0 + n_links) (default: to the last link) as an
+        (n_links, channels) ADC_STATS_DTYPE array, by frame channel. reset=True starts a new window of those links."""
+        if n_links is None:
+            n_links = max(0, self.n_links - link0)
+        out = np.zeros((n_links, self.channels), dtype=F.ADC_STATS_DTYPE)
+        self._check(lib.swtpg_read_adc_stats(self._h, link0, n_links, out.ctypes.data, 1 if reset else 0))
         return out
 
     def sort_stats(self) -> dict:

@@ -28,6 +28,7 @@ static_assert(sizeof(swtpg_config) == 72, "swtpg_config layout changed: bump SWT
 static_assert(sizeof(swtpg_channel_state) == 48, "swtpg_channel_state layout changed");
 static_assert(sizeof(swtpg_counters) == 80, "swtpg_counters layout changed");
 static_assert(sizeof(swtpg_link_config) == 36, "swtpg_link_config layout changed");
+static_assert(sizeof(swtpg_adc_stats) == 32, "swtpg_adc_stats layout changed");
 
 namespace {
 thread_local std::string g_create_error;
@@ -433,6 +434,19 @@ reset_state(swtpg_handle* h)
   return SWTPG_OK;
 }
 
+// swtpg_start: every window starts empty, after the statistics work of the previous run (reset_state then waits for the stream).
+swtpg_status
+reset_adc_stats(swtpg_handle* h)
+{
+  std::lock_guard<std::mutex> lk(h->stats_mu);
+  if (h->stats_stream && h->stats_stream != h->stream)
+    SW_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_stats, 0));
+  SW_CUDA(h, cudaMemsetAsync(h->d_adc_stats, 0, size_t(h->cfg.n_links) * h->channels * sizeof(swtpg_adc_stats), h->stream));
+  SW_CUDA(h, cudaEventRecord(h->ev_stats, h->stream));
+  h->stats_stream = h->stream;
+  return SWTPG_OK;
+}
+
 // Rewrites the SV_RS_FACTOR rows of links [link0, link0 + n) from h->h_rs_factor (or each link's configured factor): ONE strided
 // asynchronous copy on the compute stream, i.e. ordered before every kernel launched after this call and after every kernel
 // launched before it. The source is pageable, so the runtime has staged it when the call returns.
@@ -504,6 +518,8 @@ enqueue_batch(swtpg_handle* h, const void* d_frames, const uint32_t* n_units, ui
                     : launch_groups<false>(h, d_frames, d_nu, stride, h->d_tps, h->d_count, ped, wav, s));
     SW_CUDA(h, cudaEventRecord(h->ev1, s));
     h->timed = true;
+    if (h->d_adc_stats)
+      SW_CUDA(h, swtpg_internal::launch_adc_stats(h, d_frames, d_nu, stride, s));
   }
   h->last_stream = s;
   h->counters.units_processed += units;
@@ -743,7 +759,7 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
     return fail(nullptr, cs, why);
   if (cfg->wib2_adc_offset % 4 != 0 || cfg->wib2_adc_offset > SWTPG_WIB2_FRAME_BYTES - 448)
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "wib2_adc_offset must be a multiple of 4 and leave room for the 448-byte ADC block");
-  if (cfg->flags & ~SWTPG_FLAG_SORTED_TPS)
+  if (cfg->flags & ~(SWTPG_FLAG_SORTED_TPS | SWTPG_FLAG_ADC_STATS))
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "unknown bits in swtpg_config.flags");
 
   int ndev = 0;
@@ -808,6 +824,14 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
   }
   if (cfg->flags & SWTPG_FLAG_SORTED_TPS)
     h->sorter = swtpg_internal::sorter_create();
+  if (cfg->flags & SWTPG_FLAG_ADC_STATS) {
+    const size_t bytes = size_t(cfg->n_links) * h->channels * sizeof(swtpg_adc_stats);
+    SW_CUDA(hp, cudaMalloc(&h->d_adc_stats, bytes));
+    SW_CUDA(hp, cudaMemset(h->d_adc_stats, 0, bytes));
+    SW_CUDA(hp, cudaMallocHost(&h->h_adc_stats, bytes));
+    SW_CUDA(hp, cudaEventCreateWithFlags(&h->ev_stats, cudaEventDisableTiming));
+    SW_CUDA(hp, cudaEventCreateWithFlags(&h->ev_stats_read, cudaEventDisableTiming));
+  }
   *out = h.release();
   return SWTPG_OK;
 }
@@ -847,6 +871,10 @@ swtpg_destroy(swtpg_handle* h)
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->sorter) swtpg_internal::sorter_destroy(h->sorter);
+  if (h->d_adc_stats) cudaFree(h->d_adc_stats);
+  if (h->h_adc_stats) cudaFreeHost(h->h_adc_stats);
+  if (h->ev_stats) cudaEventDestroy(h->ev_stats);
+  if (h->ev_stats_read) cudaEventDestroy(h->ev_stats_read);
   delete[] h->h_rs_factor;
   delete h;
 }
@@ -859,6 +887,8 @@ swtpg_start(swtpg_handle* h)
   SW_CUDA(h, cudaSetDevice(h->cfg.device));
   swtpg_status s = SWTPG_OK;
   if (h->conf_groups_stale && (s = form_conf_groups(h)) != SWTPG_OK)
+    return s;
+  if (h->d_adc_stats && (s = reset_adc_stats(h)) != SWTPG_OK)
     return s;
   s = reset_state(h);
   if (s != SWTPG_OK)
@@ -1223,6 +1253,50 @@ swtpg_dump_state(swtpg_handle* h, uint32_t link, swtpg_channel_state* out)
     o.initialized = uint16_t(fl[g] & kFlagInitialized);
     for (int j = 0; j < 8; ++j)
       o.prev_samp[j] = int16_t(get(SV_RING0 + j));
+  }
+  return SWTPG_OK;
+}
+
+swtpg_status
+swtpg_read_adc_stats(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_adc_stats* out, int reset)
+{
+  if (!h)
+    return fail(nullptr, SWTPG_ERR_INVALID_ARG, "handle is NULL");
+  if (!out)
+    return fail(h, SWTPG_ERR_INVALID_ARG, "out is NULL");
+  if (!h->d_adc_stats)
+    return fail(h, SWTPG_ERR_STATE, "the handle was created without SWTPG_FLAG_ADC_STATS");
+  if (uint64_t(link0) + n_links > h->cfg.n_links)
+    return fail(h, SWTPG_ERR_INVALID_ARG, "link0 + n_links exceeds cfg.n_links");
+  if (n_links == 0)
+    return SWTPG_OK;
+  SW_CUDA(h, cudaSetDevice(h->cfg.device));
+  std::lock_guard<std::mutex> rd(h->read_mu);
+  const size_t first = size_t(link0) * h->channels, n = size_t(n_links) * h->channels;
+  {
+    // Copy and reset are enqueued back to back on the stream of the last batch: a batch enqueued meanwhile falls after both.
+    std::lock_guard<std::mutex> lk(h->stats_mu);
+    const cudaStream_t s = h->stats_stream ? h->stats_stream : h->stream;
+    SW_CUDA(h, cudaMemcpyAsync(h->h_adc_stats + first, h->d_adc_stats + first, n * sizeof(swtpg_adc_stats), cudaMemcpyDeviceToHost, s));
+    if (reset) {
+      SW_CUDA(h, cudaMemsetAsync(h->d_adc_stats + first, 0, n * sizeof(swtpg_adc_stats), s));
+      SW_CUDA(h, cudaEventRecord(h->ev_stats, s));
+      h->stats_stream = s;
+    }
+    SW_CUDA(h, cudaEventRecord(h->ev_stats_read, s));
+  }
+  SW_CUDA(h, cudaEventSynchronize(h->ev_stats_read));
+  for (size_t i = 0; i < n; ++i) {
+    const swtpg_adc_stats& a = h->h_adc_stats[first + i];
+    uint32_t ext[2];
+    memcpy(ext, &a.min, sizeof ext); // {16383 - min, max} (swtpg_handle::d_adc_stats)
+    swtpg_adc_stats& o = out[i];
+    o.samples = a.samples;
+    o.sum = a.sum;
+    o.sum_sq = a.sum_sq;
+    o.min = a.samples ? uint16_t(0x3FFFu - ext[0]) : 0;
+    o.max = a.samples ? uint16_t(ext[1]) : 0;
+    o.reserved = 0;
   }
   return SWTPG_OK;
 }

@@ -2,6 +2,7 @@
 //   swtpg_capi.cu    create / destroy / start / stop, the batch entry points and the kernel launch table
 //   swtpg_stream.cu  the streaming path (swtpg_submit ... swtpg_poll): per-link rings, dispatcher and completion threads,
 //                    the gather kernel that pulls frames out of pinned host memory
+//   swtpg_stats.cu   the per-channel ADC statistics kernel (SWTPG_FLAG_ADC_STATS)
 // Not installed; nothing outside csrc/ includes it.
 #pragma once
 
@@ -96,6 +97,17 @@ struct swtpg_handle
   std::vector<uint8_t> rs_table_link; // [n_links] 1 = the link's rows of h_rs_factor were set (else its configuration's factor)
   swtpg_internal::TpSorter* sorter = nullptr; // SWTPG_FLAG_SORTED_TPS: device-side ordering of TP lists (swtpg_sort.cu)
 
+  // SWTPG_FLAG_ADC_STATS (all null without it). d_adc_stats[n_links][channels] holds the current window of every channel in the
+  // layout of swtpg_adc_stats, except its last 8 bytes: {16383 - min, max} as two 32-bit words, so that zeroed memory is an empty
+  // window and both merge by atomicMax. Every statistics kernel and every read runs in one order: each waits for ev_stats, which
+  // is recorded after the last of them on stats_stream, when it runs on another stream. stats_mu guards those two and keeps a
+  // read's copy and reset together; read_mu serialises reads (h_adc_stats, ev_stats_read).
+  swtpg_adc_stats* d_adc_stats = nullptr;
+  swtpg_adc_stats* h_adc_stats = nullptr; // pinned, same size
+  cudaEvent_t ev_stats = nullptr, ev_stats_read = nullptr;
+  cudaStream_t stats_stream = nullptr;
+  std::mutex stats_mu, read_mu;
+
   // streaming path (swtpg_stream.cu), created on the first swtpg_submit / swtpg_register_buffer
   std::mutex engine_mu;
   std::atomic<swtpg_internal::StreamEngine*> engine{ nullptr };
@@ -160,6 +172,10 @@ fail(swtpg_handle* h, swtpg_status s, const char* msg)
 // ([n_links][units_stride][unit_bytes], d_nunits = per-link valid units or nullptr) on stream `s`. TPs go to d_tps / d_count.
 cudaError_t launch_batch_kernel(swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t units_stride, swtpg_tp* d_tps,
                                 unsigned* d_count, cudaStream_t s);
+
+// swtpg_stats.cu: adds one batch, laid out as for launch_batch_kernel, to the per-channel ADC statistics (SWTPG_FLAG_ADC_STATS) on
+// stream `s`, after the statistics work of earlier batches and reads whatever stream that ran on.
+cudaError_t launch_adc_stats(swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t units_stride, cudaStream_t s);
 
 // swtpg_sort.cu: device-side ordering of a batch's TP list (SWTPG_FLAG_SORTED_TPS)
 TpSorter* sorter_create();

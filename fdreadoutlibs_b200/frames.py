@@ -52,6 +52,13 @@ STATE_DTYPE = np.dtype(
 )
 assert STATE_DTYPE.itemsize == 48
 
+# swtpg_adc_stats of include/swtpg.h: one channel over one window of swtpg_read_adc_stats
+ADC_STATS_DTYPE = np.dtype(
+    [("samples", "<u8"), ("sum", "<u8"), ("sum_sq", "<u8"), ("min", "<u2"), ("max", "<u2"), ("reserved", "<u4")],
+    align=True,
+)
+assert ADC_STATS_DTYPE.itemsize == 32
+
 # Lane l of AVX2 register r holds frame channel 16r + LANE_PERM[l] (unittest/WIBEthFrameExpansion_test.cxx:111,124).
 LANE_PERM = np.array([0, 1, 2, 3, 4, 5, 6, 7, 15, 8, 9, 10, 11, 12, 13, 14], dtype=np.int64)
 

@@ -3,6 +3,7 @@
 #include "swtpg_host.hpp"
 
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <ctime>
 #include <thread>
@@ -147,6 +148,15 @@ TpgEngine::set_link_memory_factor(uint32_t link, const uint16_t* by_channel, uin
 {
   // one small asynchronous copy for this link's rows, ordered on the compute stream; no engine-wide lock, no other link waits
   check(m_h, swtpg_set_link_rs_memory_factor(m_h, link, by_channel), "swtpg_set_link_rs_memory_factor");
+}
+
+void
+TpgEngine::read_adc_stats(uint32_t link, swtpg_adc_stats* out, uint32_t n_channels, bool reset)
+{
+  const uint32_t channels = m_cfg.format == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_CHANNELS : SWTPG_WIBETH_CHANNELS;
+  if (n_channels != channels)
+    throw std::invalid_argument("TpgEngine::read_adc_stats: one entry per frame channel of the link");
+  check(m_h, swtpg_read_adc_stats(m_h, link, 1, out, reset ? 1 : 0), "swtpg_read_adc_stats");
 }
 
 void
@@ -450,6 +460,37 @@ WIBEthFrameProcessor::timestamp_check(frameptr fp)
   m_last_processed_daq_ts = m_current_ts;
 }
 
+namespace {
+ChannelAdcStats
+channel_adc_stats(uint32_t offline_channel, const swtpg_adc_stats& a)
+{
+  ChannelAdcStats o;
+  o.offline_channel = offline_channel;
+  o.samples = a.samples;
+  if (a.samples) {
+    // variance = (n sum_sq - sum^2) / n^2, the numerator exact in 128 bits
+    const unsigned __int128 n = a.samples, num = n * a.sum_sq - (unsigned __int128)a.sum * a.sum;
+    o.mean = double(a.sum) / double(a.samples);
+    o.rms = std::sqrt(double(num) / (double(a.samples) * double(a.samples)));
+    o.min = a.min;
+    o.max = a.max;
+  }
+  return o;
+}
+} // namespace
+
+void
+WIBEthFrameProcessor::get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset)
+{
+  out.clear();
+  if (!m_maps_ready.load(std::memory_order_acquire))
+    return;
+  swtpg_adc_stats s[64];
+  m_engine->read_adc_stats(m_wibeth_frame_handler->link, s, 64, reset);
+  for (uint32_t c = 0; c < 64; ++c)
+    out.push_back(channel_adc_stats(m_offline_of_channel[c], s[c]));
+}
+
 void
 WIBEthFrameProcessor::find_hits(constframeptr fp, WIBEthFrameHandler* frame_handler)
 {
@@ -658,6 +699,18 @@ WIB2FrameProcessor::timestamp_check(frameptr fp)
   }
   m_previous_ts = m_current_ts;
   m_last_processed_daq_ts = m_current_ts;
+}
+
+void
+WIB2FrameProcessor::get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset)
+{
+  out.clear();
+  if (!m_maps_ready.load(std::memory_order_acquire))
+    return;
+  swtpg_adc_stats s[256];
+  m_engine->read_adc_stats(m_handler->link, s, 256, reset);
+  for (uint32_t c = 0; c < 256; ++c)
+    out.push_back(channel_adc_stats(m_register_channels[c], s[c]));
 }
 
 void
@@ -905,11 +958,12 @@ swtpg_host_last_error(void)
 }
 
 static swtpg_host*
-host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links)
+host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_t flags = SWTPG_FLAG_NONE)
 {
   try {
     auto h = std::make_unique<swtpg_host>();
-    h->engine = std::make_shared<TpgEngine>(c->device, swtpg_format(c->format), c->n_links, c->superchunk_units, c->n_slots ? c->n_slots : 4u);
+    h->engine = std::make_shared<TpgEngine>(c->device, swtpg_format(c->format), c->n_links, c->superchunk_units, c->n_slots ? c->n_slots : 4u,
+                                            0u, flags);
     h->sink_capacity = c->sink_capacity;
     h->count_only = c->count_only_sink != 0;
     h->queues.resize(c->n_links);
@@ -984,6 +1038,13 @@ swtpg_host*
 swtpg_host_create_links(const swtpg_host_conf* c, const swtpg_host_link_conf* links)
 {
   return host_create(c, links);
+}
+
+// The same with SWTPG_FLAG_* for the engine's handle (SWTPG_FLAG_ADC_STATS: the processors' get_adc_stats); links may be NULL.
+swtpg_host*
+swtpg_host_create_flags(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_t flags)
+{
+  return host_create(c, links, flags);
 }
 
 void
@@ -1245,6 +1306,26 @@ swtpg_host_register_buffer(swtpg_host* h, void* base, size_t bytes, int on)
     return -1;
   }
   return 0;
+}
+
+// ChannelAdcStats of a link's processor: out[cap] (64 WIBEth / 256 WIB2 entries, none before the first frame); the entry count, -1 on error
+static_assert(sizeof(ChannelAdcStats) == 40, "hostshim.HOST_ADC_STATS_DTYPE mirrors ChannelAdcStats");
+int
+swtpg_host_adc_stats(swtpg_host* h, uint32_t link, int reset, ChannelAdcStats* out, uint32_t cap)
+{
+  try {
+    std::vector<ChannelAdcStats> v;
+    if (!h->eth.empty())
+      h->eth.at(link)->get_adc_stats(v, reset != 0);
+    else
+      h->wib2.at(link)->get_adc_stats(v, reset != 0);
+    const size_t n = std::min<size_t>(v.size(), cap);
+    std::copy(v.begin(), v.begin() + n, out);
+    return int(n);
+  } catch (const std::exception& e) {
+    g_host_error = e.what();
+    return -1;
+  }
 }
 
 // position -> offline channel map of a link (after its first frame)

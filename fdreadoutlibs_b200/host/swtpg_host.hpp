@@ -219,6 +219,16 @@ private:
   std::vector<std::function<void(const ReadoutType*)>> m_post;
 };
 
+// Not a reference type: ADC statistics of one channel of a link over one window of swtpg_read_adc_stats, reported under the
+// offline channel that channel's TPs carry. rms = sqrt(sum_sq / samples - mean^2); all zero when samples == 0.
+struct ChannelAdcStats
+{
+  uint32_t offline_channel = 0;
+  uint64_t samples = 0;
+  double mean = 0, rms = 0;
+  uint16_t min = 0, max = 0;
+};
+
 // ---- the GPU pipeline shared by the links of one device -------------------------------------------------------------------
 class FrameProcessorBase;
 // One swtpg_handle per GPU; every frame processor attached to it owns one link index. Any link's post-processing thread
@@ -242,6 +252,8 @@ public:
   // per-channel hit thresholds of one link, by FRAME channel (swtpg_set_link_thresholds); nullptr = the link's tpg_threshold.
   // Before start(), like configure().
   void set_link_thresholds(uint32_t link, const uint16_t* by_channel, uint32_t n_channels);
+  // swtpg_read_adc_stats of one link: out[n_channels] by frame channel (an engine created with SWTPG_FLAG_ADC_STATS). After conf().
+  void read_adc_stats(uint32_t link, swtpg_adc_stats* out, uint32_t n_channels, bool reset);
   // false = back-pressure (the link's ring is full). wait_us > 0: sleep up to that long for room first (swtpg_submit_wait)
   bool submit(uint32_t link, const void* unit, size_t bytes, uint64_t wait_us = 0);
   // Zero-copy ingest: the latency buffer(s) the constframeptrs point into (swtpg_register_buffer). After conf().
@@ -303,6 +315,9 @@ public:
   void start() override;                                        // (:111-144)
   void stop() override;                                         // (:146-154)
   void get_info(RawDataProcessorInfo& info);                    // (:237-292)
+  // Not in the reference: the ADC statistics of this link's channels since the last reset (engine flag SWTPG_FLAG_ADC_STATS), by
+  // the offline channel its TPs carry, masked channels included. Empty until the first frame has built the channel map.
+  void get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset);
 
   void sequence_check(frameptr fp);                             // (:298-353)
   void timestamp_check(frameptr fp);                            // (:359-405)
@@ -369,6 +384,7 @@ public:
   void start() override;
   void stop() override;
   void get_info(RawDataProcessorInfo& info);
+  void get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset); // as WIBEthFrameProcessor::get_adc_stats
   void timestamp_check(frameptr fp);                                  // (:293-340)
   void find_hits(constframeptr fp, WIB2FrameHandler* frame_handler);  // (:345-396)
   void process_swtpg_hits(const swtpg_tp* tps, size_t n) override;    // (:398-479)

@@ -32,6 +32,12 @@ HOST_TP_DTYPE = np.dtype([("time_start", "<u8"), ("time_peak", "<u8"), ("time_ov
                           ("version", "<u2"), ("flag", "<u2")], align=True)
 
 
+# ChannelAdcStats of swtpg_host.hpp
+HOST_ADC_STATS_DTYPE = np.dtype([("offline_channel", "<u4"), ("samples", "<u8"), ("mean", "<f8"), ("rms", "<f8"), ("min", "<u2"),
+                                 ("max", "<u2")], align=True)
+assert HOST_ADC_STATS_DTYPE.itemsize == 40
+
+
 class HostInfo(C.Structure):
     _fields_ = [("num_seq_id_errors", C.c_uint64), ("min_seq_id_jump", C.c_int32), ("max_seq_id_jump", C.c_int32),
                 ("num_ts_errors", C.c_uint64), ("rate_tp_hits", C.c_double), ("num_tps_sent", C.c_uint64),
@@ -57,7 +63,8 @@ EXPORTS = ["swtpg_host_tpsets_create", "swtpg_host_tpsets_destroy", "swtpg_host_
            "swtpg_host_tpsets_cutoff", "swtpg_host_tpsets_count", "swtpg_host_tpsets_get", "swtpg_host_tpsets_info",
            "swtpg_host_push_parallel", "swtpg_host_push_feeders", "swtpg_host_tp_count", "swtpg_host_counters", "swtpg_host_stream_timing", "swtpg_host_last_error", "swtpg_host_create", "swtpg_host_create_links", "swtpg_host_destroy", "swtpg_host_start", "swtpg_host_stop", "swtpg_host_push",
            "swtpg_host_take_tps", "swtpg_host_get_info", "swtpg_host_error_count", "swtpg_host_misconfigurations",
-           "swtpg_host_last_daq_time", "swtpg_host_register_channel_map", "swtpg_host_register_buffer"]
+           "swtpg_host_last_daq_time", "swtpg_host_register_channel_map", "swtpg_host_register_buffer", "swtpg_host_adc_stats",
+           "swtpg_host_create_flags"]
 
 _lib = None
 
@@ -93,6 +100,9 @@ def host_lib():
         lib.swtpg_host_last_daq_time.argtypes = [C.c_void_p, C.c_uint32]
         lib.swtpg_host_register_channel_map.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
         lib.swtpg_host_register_buffer.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int]
+        lib.swtpg_host_create_flags.restype = C.c_void_p
+        lib.swtpg_host_create_flags.argtypes = [C.POINTER(HostConf), C.POINTER(HostLinkConf), C.c_uint32]
+        lib.swtpg_host_adc_stats.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p, C.c_uint32]
         lib.swtpg_host_tpsets_create.restype = C.c_void_p
         lib.swtpg_host_tpsets_create.argtypes = [C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32, C.c_uint32]
         lib.swtpg_host_tpsets_destroy.argtypes = [C.c_void_p]
@@ -121,10 +131,11 @@ class FrameProcessors:
                  crate_id: int = 1, slot_id: int = 0, first_link_id: int = 0, enable_tpg: bool = True, emulator_mode: bool = False,
                  correct_channel_lookup: bool = False, reversed_map: bool = False, collection_simple_threshold: bool = False,
                  sink_capacity: int = 0, block_on_backpressure: bool = True, device: int = 0, count_only_sink: bool = False,
-                 n_slots: int = 4, link_confs=None):
+                 n_slots: int = 4, link_confs=None, adc_stats: bool = False):
         """link_confs: optional list of n_links dicts, each overriding algorithm, threshold, rs_memory_factor, rs_scale_factor
         and acc_limit for its link's conf(); the keys it leaves out take the arguments above. A dict may also set
-        plane_threshold: three thresholds by plane (0 = collection), -1 = the link's threshold (tpg_plane_threshold)."""
+        plane_threshold: three thresholds by plane (0 = collection), -1 = the link's threshold (tpg_plane_threshold).
+        adc_stats: the engine's handle accumulates per-channel ADC statistics (SWTPG_FLAG_ADC_STATS), read by adc_stats()."""
         c = HostConf()
         c.device, c.format, c.n_links, c.superchunk_units = device, 1 if fmt == "wib2" else 0, n_links, superchunk_units
         c.tpg_algorithm = algorithm.encode()
@@ -142,7 +153,10 @@ class FrameProcessors:
         c.n_slots = n_slots
         self.lib = host_lib()
         self.n_links = n_links
-        if link_confs is None:
+        if adc_stats:
+            assert link_confs is None
+            self.h = self.lib.swtpg_host_create_flags(C.byref(c), None, 2)  # SWTPG_FLAG_ADC_STATS
+        elif link_confs is None:
             self.h = self.lib.swtpg_host_create(C.byref(c))
         else:
             assert len(link_confs) == n_links
@@ -186,6 +200,15 @@ class FrameProcessors:
         st = FeedStats()
         self._check(self.lib.swtpg_host_push_feeders(self.h, payloads.ctypes.data, payloads.shape[1], n_threads, burst, pace, passes, C.byref(st)))
         return {"wall_s": st.wall_s, "feeder_cpu_s": st.feeder_cpu_s, "payloads": int(st.payloads), "late_bursts": int(st.late_bursts)}
+
+    def adc_stats(self, link: int, reset: bool = False) -> np.ndarray:
+        """The processor's get_adc_stats: HOST_ADC_STATS_DTYPE entries by the offline channel its TPs carry (empty before its
+        first frame). reset=True starts a new window of the link."""
+        out = np.zeros(256, dtype=HOST_ADC_STATS_DTYPE)
+        n = self.lib.swtpg_host_adc_stats(self.h, link, 1 if reset else 0, out.ctypes.data, out.size)
+        if n < 0:
+            raise HostError(self.lib.swtpg_host_last_error().decode())
+        return out[:n].copy()
 
     def counters(self) -> dict:
         """swtpg_get_counters of the engine behind the processors."""

@@ -109,6 +109,9 @@ typedef struct swtpg_config
  * radix sort of packed keys in HBM), identical to what swtpg_sort_tps makes of the unordered list. Lists of one handle can
  * then be merged across GPUs with swtpg_merge_sorted without a host sort. */
 #define SWTPG_FLAG_SORTED_TPS 1u
+/* Per-channel ADC statistics of every link (swtpg_read_adc_stats): one extra read of every batch on the device, after its TPG kernel
+ * and on the same stream. Without the flag nothing is allocated or launched for them. */
+#define SWTPG_FLAG_ADC_STATS 2u
 
 /* Per-channel carried state, by frame channel: ChanState of wibeth/tpg/ProcessingInfo.hpp:20-66 and
  * wib2/tpg/ProcessingInfo.hpp:20-68. Used for parity dumps only. */
@@ -289,6 +292,28 @@ swtpg_status swtpg_stream_timing(swtpg_handle* h, double* gather_ms, double* ker
 
 /* Carried state of one link, by frame channel (ChanState parity). out has SWTPG_*_CHANNELS entries. */
 swtpg_status swtpg_dump_state(swtpg_handle* h, uint32_t link, swtpg_channel_state* out);
+
+/* Statistics of the raw ADC values of one channel (frame channel, as swtpg_tp.channel) over one window. 32 bytes.
+ * pedestal = sum / samples, RMS noise = sqrt(sum_sq / samples - pedestal^2). An extension of the reference, whose opmon reports
+ * only the TP rate per channel: the noise that a per-channel threshold (swtpg_set_link_thresholds) is usually a multiple of,
+ * and saturated (max 16383) or dead (min == max) channels. */
+typedef struct swtpg_adc_stats
+{
+  uint64_t samples;      /* samples of this channel in the window */
+  uint64_t sum;          /* sum of the raw 14-bit ADC values */
+  uint64_t sum_sq;       /* sum of their squares: exact while samples < 2^36 (9.7 h of one channel's data) */
+  uint16_t min, max;     /* raw ADC extremes; both 0 when samples == 0 */
+  uint32_t reserved;
+} swtpg_adc_stats;
+/* out[n_links][SWTPG_*_CHANNELS] for links link0 .. link0 + n_links - 1 (handles created with SWTPG_FLAG_ADC_STATS). Every sample of
+ * every valid unit (u < n_units[l]) of every batch, from every batch entry point and the streaming path, is counted once.
+ *   - A window holds exactly the batches enqueued before the read that ends it: the read is ordered like a batch, on the stream of
+ *     the last batch, and waits only for that work. reset != 0 starts the next window of these links at that point, so every batch
+ *     falls into exactly one window, also while the streaming path dispatches batches or other threads read other links.
+ *   - swtpg_start zeroes every window; after swtpg_stop they stay readable; before the first batch they read as zeros.
+ *   - SWTPG_ERR_STATE on a handle created without the flag; SWTPG_ERR_INVALID_ARG for a NULL handle or out, or for
+ *     link0 + n_links > cfg.n_links. */
+swtpg_status swtpg_read_adc_stats(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_adc_stats* out, int reset);
 swtpg_status swtpg_get_counters(swtpg_handle* h, swtpg_counters* out);
 /* SWTPG_FLAG_SORTED_TPS bookkeeping: device time (CUDA events, includes the 16-byte read-back of the key range) of the last
  * ordered list and of all lists since swtpg_create, how many lists were ordered on the device, and how many of them the host
