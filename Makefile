@@ -19,7 +19,7 @@ lib: $(LIB) $(GENLIB)
 # the fused kernels + launch table (slow to compile: every policy x kernel form is instantiated here)
 $(OBJ)/swtpg_capi.o: $(CSRC)/swtpg_capi.cu $(CSRC)/swtpg_kernels.cuh $(CSRC)/swtpg_device.cuh $(CSRC)/swtpg_handle.h include/swtpg.h
 	@mkdir -p $(OBJ)
-	$(NVCC) $(NVFLAGS) $(KFLAGS) -c -o $@ $(CSRC)/swtpg_capi.cu 2> build_ptxas.log || (cat build_ptxas.log; exit 1)
+	$(NVCC) $(NVFLAGS) -c -o $@ $(CSRC)/swtpg_capi.cu 2> build_ptxas.log || (cat build_ptxas.log; exit 1)
 	@grep -E "error|warning: v" build_ptxas.log || true
 # the streaming engine + gather kernels
 $(OBJ)/swtpg_stream.o: $(CSRC)/swtpg_stream.cu $(CSRC)/swtpg_handle.h include/swtpg.h

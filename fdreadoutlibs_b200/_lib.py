@@ -10,8 +10,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# SWTPG_LIB: tuning aid — load an alternative build of the SAME library (e.g. compiled with other kernel macros)
-LIB_PATH = os.environ.get("SWTPG_LIB") or os.path.join(_HERE, "libswtpg_b200.so")
+LIB_PATH = os.path.join(_HERE, "libswtpg_b200.so")
 
 SWTPG_OK, SWTPG_ERR_INVALID_ARG, SWTPG_ERR_CUDA, SWTPG_ERR_BUSY, SWTPG_ERR_OVERFLOW, SWTPG_ERR_STATE, SWTPG_ERR_UNSUPPORTED = range(7)
 FORMAT_WIBETH, FORMAT_WIB2 = 0, 1

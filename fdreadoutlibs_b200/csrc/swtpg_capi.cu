@@ -43,139 +43,108 @@ swtpg_internal::set_create_error(const char* msg)
 namespace {
 
 // ---- kernel launch table ------------------------------------------------------------------------------------------
-// Geometry of the WIBEth kernel: WARPS links per CTA, per-warp ring of NSTAGE stages of CHUNK ticks (112 B each).
-template<int WARPS, int NSTAGE, int CHUNK, int MIN_CTAS = 1>
-struct Geo
-{
-  static constexpr int warps = WARPS, stages = NSTAGE, chunk = CHUNK, min_ctas = MIN_CTAS;
-  static constexpr size_t smem = WibEthSmem<WARPS, NSTAGE, CHUNK>::total;
-};
-// Default: one link-warp per CTA with a ring of 2 stages x 32 ticks (7 KB) + 2.5 KB hit staging. Measured best of the
-// geometries below on B200 (profiles/r01_geometry_sweep.txt): the kernel is issue-bound, so deeper rings do not help, and
-// single-warp CTAs let the block scheduler spread the 20 resident warps per SM evenly over the four sub-partitions.
-#ifndef SWTPG_GEO_STAGES
-#define SWTPG_GEO_STAGES 2
-#define SWTPG_GEO_CHUNK 32
-#endif
-#ifndef SWTPG_GEO_MINCTAS
-#define SWTPG_GEO_MINCTAS 1
-#endif
-using GeoDefault = Geo<1, SWTPG_GEO_STAGES, SWTPG_GEO_CHUNK, SWTPG_GEO_MINCTAS>;
-
-#ifndef SWTPG_AUTO_SLICE_GEOM
-#define SWTPG_AUTO_SLICE_GEOM 1 // sliced launches: equal slices (0) or halving ones (1)
-#endif
-
-// WARPS_PER_SM: 0 = the policy's own measured optimum (Algo::kWarpsPerSm). SLICE_WHOLE_ROUNDS: hand the links out in slices
-// even when their number is a whole multiple of the persistent warps.
-template<class Algo, bool DUMP, class G, int WARPS_PER_SM = 0, bool SLICE_WHOLE_ROUNDS = false>
+// CTAs of persistent kernel K the whole GPU holds at once (SMs x resident CTAs per SM, the latter capped at `cap` if cap > 0),
+// and the SM count. Queried once per kernel and device.
+template<auto K>
 cudaError_t
-launch_wibeth_geo(const KernelParams& kp, cudaStream_t s)
+residency(int threads, size_t smem, int cap, unsigned* resident, unsigned* sms)
 {
-  auto k = wibeth_kernel<Algo, G::warps, G::stages, G::chunk, DUMP, G::min_ctas>;
-  // Persistent grid: as many CTAs as the device holds at once (SMs x resident CTAs per SM); warps walk the links.
-  static int resident[64]; // per instantiation and device: CTAs the whole GPU can hold, 0 = not queried yet
-  static int sm_count[64];
+  static int res[64], sm[64]; // 0 = not queried yet
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess)
     return e;
   if (dev < 0 || dev >= 64)
     return cudaErrorInvalidDevice;
-  if (resident[dev] == 0) {
-    e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, int(G::smem));
+  if (res[dev] == 0) {
+    e = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess)
       return e;
-    int per_sm = 0, sms = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, G::warps * 32, G::smem);
+    int per_sm = 0, n = 0;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, K, threads, smem);
     if (e != cudaSuccess)
       return e;
-    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    e = cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
     if (e != cudaSuccess)
       return e;
-    if (const char* cap = getenv("SWTPG_CTAS_PER_SM")) // tuning aid
-      per_sm = std::min(per_sm, std::max(1, atoi(cap)));
-    sm_count[dev] = std::max(1, sms);
-    resident[dev] = std::max(1, per_sm * sms);
+    if (cap > 0) // the policy's measured optimum, if the device holds that many
+      per_sm = std::min(per_sm, cap);
+    sm[dev] = std::max(1, n);
+    res[dev] = std::max(1, per_sm * n);
   }
+  *resident = unsigned(res[dev]);
+  *sms = unsigned(sm[dev]);
+  return cudaSuccess;
+}
+
+// Geometry of the WIBEth kernel: one link-warp per CTA with a ring of 2 stages x 32 ticks (7 KB) + 2.5 KB hit staging. Measured
+// best on B200 (profiles/r01_geometry_sweep.txt): the kernel is issue-bound, so deeper rings do not help, and single-warp CTAs
+// let the block scheduler spread the 20 resident warps per SM evenly over the four sub-partitions.
+constexpr int kGeoStages = 2, kGeoChunk = 32;
+
+// WARPS_PER_SM: 0 = the policy's own measured optimum (Algo::kWarpsPerSm). SLICE_WHOLE_ROUNDS: hand the links out in slices
+// even when their number is a whole multiple of the persistent warps.
+template<class Algo, bool DUMP, int WARPS_PER_SM = 0, bool SLICE_WHOLE_ROUNDS = false>
+cudaError_t
+launch_wibeth_geo(const KernelParams& kp, cudaStream_t s)
+{
+  constexpr auto k = wibeth_kernel<Algo, 1, kGeoStages, kGeoChunk, DUMP, 1>;
+  constexpr size_t smem = WibEthSmem<1, kGeoStages, kGeoChunk>::total;
+  // Persistent grid: at most as many CTAs as the device holds at once; warps walk the links.
+  unsigned resident = 0, sms = 0;
+  const cudaError_t e = residency<k>(32, smem, 0, &resident, &sms);
+  if (e != cudaSuccess)
+    return e;
   // Persistent warps claim links dynamically (wibeth_kernel), so the grid only has to load every SM sub-partition alike:
   // a multiple of 4 single-warp CTAs per SM (20 on B200: 5 warps per sub-partition; a 21st warp would make one
   // sub-partition of every SM 20 % slower than its neighbours — profiles/README.md).
-  const unsigned per_sm = unsigned(resident[dev]) / unsigned(sm_count[dev]);
-  unsigned even = G::warps == 1 && per_sm >= 4 ? per_sm / 4 * 4 : per_sm;
+  const unsigned per_sm = resident / sms;
+  unsigned even = per_sm >= 4 ? per_sm / 4 * 4 : per_sm;
   constexpr int kWarpsPerSm = WARPS_PER_SM > 0 ? WARPS_PER_SM : Algo::kWarpsPerSm;
-  if (G::warps == 1 && kWarpsPerSm > 0) // the measured optimum, if the device holds that many
+  if (kWarpsPerSm > 0) // the measured optimum, if the device holds that many
     even = std::min<unsigned>(even, unsigned(kWarpsPerSm));
-  unsigned warps = std::min<unsigned>(kp.n_links, even * unsigned(sm_count[dev]) * G::warps);
-  static const int warps_override = [] { const char* e = getenv("SWTPG_WARPS"); return e ? atoi(e) : 0; }(); // tuning aid
-  if (warps_override > 0)
-    warps = std::min<unsigned>(unsigned(warps_override), kp.n_links);
-  const unsigned grid = std::min<unsigned>((warps + G::warps - 1) / G::warps, unsigned(resident[dev]));
+  const unsigned grid = std::min<unsigned>(std::min<unsigned>(kp.n_links, even * sms), resident);
   // More links than persistent warps = several rounds of links per warp, and whatever the last round leaves idle is lost (round 2,
   // straight-line SimpleThreshold policy: 6000 links on 4144 warps 64.9 % of the HBM peak, 8288 = two full rounds 73.0 %). Handing
-  // the links out in 4 slices makes the rounds short, at the price of the extra state round trips (about 3 % per launch):
-  //   * HALVING slices (n/2, n/4, n/8, n/8 units): what the launch's last round leaves idle is at most one LAST slice, so small
-  //     last slices shorten the tail without more round trips per link than four equal ones (pipelined SimpleThreshold policy at
-  //     20 warps per SM, 5920 links: whole links 68.9 %, equal slices 70.8 %, halving 73.1 %; 6000 links 71.0 -> 73.3 %; AbsRS + 2.5 %;
-  //     profiles/r02_halving_slices_probe.txt). The straight-line policy at 28 warps per SM is the one case that loses with them.
+  // the links out in 4 HALVING slices (n/2, n/4, n/8, n/8 units) makes the rounds short, at the price of the extra state round
+  // trips (about 3 % per launch): what the launch's last round leaves idle is at most one LAST slice, so small last slices shorten
+  // the tail without more round trips per link than four equal ones (pipelined SimpleThreshold policy at 20 warps per SM, 5920
+  // links: whole links 68.9 %, equal slices 70.8 %, halving 73.1 %; 6000 links 71.0 -> 73.3 %; AbsRS + 2.5 %;
+  // profiles/r02_halving_slices_probe.txt).
   //   * For most policies a link count that is a whole number of rounds keeps whole links (straight-line form, 8288 links: 73.0 %
   //     against 70.8 % sliced); the pipelined SimpleThreshold policy gains from slices even then (SLICE_WHOLE_ROUNDS).
   // A launch that cannot fill the GPU keeps whole links: time is sequential per link, slices could only wait for each other.
   KernelParams kq = kp;
   unsigned parts = 1;
-  const unsigned persistent = grid * unsigned(G::warps);
-  if (kp.n_links > persistent && (SLICE_WHOLE_ROUNDS || kp.n_links % persistent != 0))
+  if (kp.n_links > grid && (SLICE_WHOLE_ROUNDS || kp.n_links % grid != 0))
     parts = std::max(1u, std::min(4u, kp.units_stride / 16u));
-  static const int parts_override = [] { const char* e = getenv("SWTPG_PARTS"); return e ? atoi(e) : 0; }(); // tuning aid
+  // Test hook: SWTPG_PARTS=n hands every launch out in n slices (at most 8), so that the GPU suite can run its cases with every
+  // link sliced (tests/test_gpu_parity.py::test_links_handed_out_in_slices).
+  static const int parts_override = [] { const char* e = getenv("SWTPG_PARTS"); return e ? atoi(e) : 0; }();
   if (parts_override > 0)
     parts = std::min(unsigned(parts_override), 8u);
   kq.parts_log2 = 0;
   while ((2u << kq.parts_log2) <= parts) // the largest power of two not above it
     ++kq.parts_log2;
-  static const int geom = [] { const char* e = getenv("SWTPG_SLICE_GEOM"); return e ? atoi(e) : SWTPG_AUTO_SLICE_GEOM; }(); // tuning aid
-  kq.slice_geom = geom != 0 ? 1u : 0u;
-  k<<<grid, G::warps * 32, G::smem, s>>>(kq);
+  kq.slice_geom = 1u; // halving slices
+  k<<<grid, 32, smem, s>>>(kq);
   return cudaGetLastError();
 }
 
-// CTA form of the WIBEth kernel (wibeth_quad_kernel): 4 consumer warps + 1 producer warp per quad of links.
+// CTA form of the WIBEth kernel (wibeth_quad_kernel): 4 consumer warps + 1 producer warp per quad of links, ring of 2 x 32 ticks.
 template<class Algo, bool DUMP>
 cudaError_t
 launch_wibeth_quad(const KernelParams& kp, cudaStream_t s)
 {
-#ifndef SWTPG_QUAD_STAGES
-#define SWTPG_QUAD_STAGES 2
-#define SWTPG_QUAD_CHUNK 32
-#endif
-  constexpr int kStages = SWTPG_QUAD_STAGES, kChunk = SWTPG_QUAD_CHUNK;
-  auto k = wibeth_quad_kernel<Algo, kStages, kChunk, DUMP>;
+  constexpr int kStages = 2, kChunk = 32;
+  constexpr auto k = wibeth_quad_kernel<Algo, kStages, kChunk, DUMP>;
   constexpr size_t smem = WibEthQuadSmem<kStages, kChunk>::total;
-  static int resident[64];
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
+  unsigned resident = 0, sms = 0;
+  const cudaError_t e = residency<k>((kQuad + 1) * 32, smem, Algo::kQuadCtasPerSm, &resident, &sms);
   if (e != cudaSuccess)
     return e;
-  if (dev < 0 || dev >= 64)
-    return cudaErrorInvalidDevice;
-  if (resident[dev] == 0) {
-    e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-    if (e != cudaSuccess)
-      return e;
-    int per_sm = 0, sms = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, (kQuad + 1) * 32, smem);
-    if (e != cudaSuccess)
-      return e;
-    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (e != cudaSuccess)
-      return e;
-    if (const char* cap = getenv("SWTPG_CTAS_PER_SM")) // tuning aid
-      per_sm = std::min(per_sm, std::max(1, atoi(cap)));
-    else if (Algo::kQuadCtasPerSm > 0) // the policy's measured optimum, if the device holds that many
-      per_sm = std::min(per_sm, Algo::kQuadCtasPerSm);
-    resident[dev] = std::max(1, per_sm * sms);
-  }
   const unsigned quads = (kp.n_links + kQuad - 1) / kQuad;
-  const unsigned grid = std::min<unsigned>(quads, unsigned(resident[dev])); // persistent CTAs claim quads dynamically
+  const unsigned grid = std::min<unsigned>(quads, resident); // persistent CTAs claim quads dynamically
   k<<<grid, (kQuad + 1) * 32, smem, s>>>(kp);
   return cudaGetLastError();
 }
@@ -183,9 +152,9 @@ launch_wibeth_quad(const KernelParams& kp, cudaStream_t s)
 // Which form of the WIBEth kernel a policy runs is a measured choice (profiles/r01_quad_vs_warp.txt): the CTA form is 14 % faster
 // for FIR + IQR (ptxas needs 64 registers instead of 109 for it, so 20 consumer warps fit an SM), the one-warp-per-CTA form
 // 2-5 % faster for SimpleThreshold and the running sums (the quad's lock-step costs more than the producer bookkeeping it
-// saves). SWTPG_WIBETH_KERNEL=warp forces the latter.
-// WIBEth SimpleThreshold, the production algorithm: which form of its policy runs, on which ring and with how many persistent
-// warps is a measured choice (profiles/r02_simple_pipeline_sweep.txt, profiles/r02_halving_slices_probe.txt).
+// saves).
+// WIBEth SimpleThreshold, the production algorithm: which form of its policy runs and with how many persistent warps is a
+// measured choice (profiles/r02_simple_pipeline_sweep.txt, profiles/r02_halving_slices_probe.txt).
 //   * The software-pipelined form (prefetch of the next group's rows + deferred quiet test, PackedSimpleT<true>, 92 registers) on
 //     the 2 x 32-tick ring runs every launch since its dependent chain lost an instruction (the accumulator reset as one IMAD):
 //     with 20 warps per SM and halving slices it beats the straight-line form with 28 at every link count — 5920 links 73.1 %
@@ -194,54 +163,41 @@ launch_wibeth_quad(const KernelParams& kp, cudaStream_t s)
 //   * Below one link per warp of the 20-per-SM grid (2960 links on B200: a 750-link shard of an 8-GPU module, the streaming
 //     path's 240 links, one APA) a launch is bound by what ONE warp does per tick and keeps at most 16 warps per SM (measured
 //     optimum of the round-2 sweep); beyond that 20 warps per SM and slices even for whole rounds.
-// SWTPG_SIMPLE_PIPE (tuning aid): 1 = the pipelined form with the policy's own 16 warps per SM, 0 = the straight-line form on the
-// default ring (20 warps per SM), 2 = the straight-line form on the 2 x 16-tick ring with 28 warps per SM (round 2's full-load form).
 template<bool DUMP>
 cudaError_t
 launch_wibeth_simple(const KernelParams& kp, cudaStream_t s)
 {
-  static const int forced = [] { const char* e = getenv("SWTPG_SIMPLE_PIPE"); return e ? atoi(e) : -1; }();
-  if (forced == 0)
-    return launch_wibeth_geo<PackedSimpleWibEth, DUMP, GeoDefault>(kp, s);
-  if (forced == 1)
-    return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, GeoDefault>(kp, s);
-  if (forced == 2)
-    return launch_wibeth_geo<PackedSimpleWibEth, DUMP, Geo<1, 2, 16>, 28>(kp, s);
   int sms = 148, dev = 0;
   if (cudaGetDevice(&dev) == cudaSuccess)
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   constexpr int kFullWarpsPerSm = 20;
   if (kp.n_links >= unsigned(kFullWarpsPerSm * sms)) // 2960 links: 66.5 % with 20 warps per SM against 64.2 % with 16; 2500: 56.7 / 58.2 %
-    return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, GeoDefault, kFullWarpsPerSm, true>(kp, s);
-  return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, GeoDefault>(kp, s);
+    return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, kFullWarpsPerSm, true>(kp, s);
+  return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP>(kp, s);
 }
 
 template<class Algo, bool DUMP>
 cudaError_t
 launch_wibeth(const KernelParams& kp, cudaStream_t s)
 {
-  if constexpr (std::is_same<Algo, PackedSimpleWibEth>::value && Algo::kQuadCtasPerSm == 0)
+  if constexpr (std::is_same<Algo, PackedSimpleWibEth>::value) {
     return launch_wibeth_simple<DUMP>(kp, s);
-  if constexpr (Algo::kQuadCtasPerSm > 0) {
-    static const bool warp_form = [] {
-      const char* e = getenv("SWTPG_WIBETH_KERNEL");
-      return e && std::string(e) == "warp";
-    }();
-    if (!warp_form)
-      return launch_wibeth_quad<Algo, DUMP>(kp, s);
+  } else if constexpr (Algo::kQuadCtasPerSm > 0) {
+    return launch_wibeth_quad<Algo, DUMP>(kp, s);
+  } else {
+    // The running sums (AbsRS, StandardRS; one-warp-per-CTA form): a launch of more than one round of a 20-per-SM grid runs 20
+    // warps per SM with halving slices, whole rounds included — AbsRS 28.7 -> 30.4 % of the HBM peak at 5920 links (its own
+    // optimum of 16 warps per SM holds for whole links: 20 unsliced 26.9 %), StandardRS 35.4 -> 36.7 %
+    // (profiles/r02_warps_crossover_probe.txt).
+    if constexpr (std::is_same<Algo, PackedRsWibEth<false>>::value || std::is_same<Algo, PackedRsWibEth<true>>::value) {
+      int sms = 148, dev = 0;
+      if (cudaGetDevice(&dev) == cudaSuccess)
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+      if (kp.n_links > unsigned(20 * sms))
+        return launch_wibeth_geo<Algo, DUMP, 20, true>(kp, s);
+    }
+    return launch_wibeth_geo<Algo, DUMP>(kp, s);
   }
-  // The running sums (AbsRS, StandardRS; one-warp-per-CTA form): a launch of more than one round of a 20-per-SM grid runs 20
-  // warps per SM with halving slices, whole rounds included — AbsRS 28.7 -> 30.4 % of the HBM peak at 5920 links (its own
-  // optimum of 16 warps per SM holds for whole links: 20 unsliced 26.9 %), StandardRS 35.4 -> 36.7 %
-  // (profiles/r02_warps_crossover_probe.txt).
-  if constexpr (std::is_same<Algo, PackedRsWibEth<false>>::value || std::is_same<Algo, PackedRsWibEth<true>>::value) {
-    int sms = 148, dev = 0;
-    if (cudaGetDevice(&dev) == cudaSuccess)
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (kp.n_links > unsigned(20 * sms))
-      return launch_wibeth_geo<Algo, DUMP, GeoDefault, 20, true>(kp, s);
-  }
-  return launch_wibeth_geo<Algo, DUMP, GeoDefault>(kp, s);
 }
 
 // WIB2: one CTA (4 consumer warps + 1 producer warp) per link at a time, ring of 4 superchunks; persistent over links.
@@ -249,33 +205,14 @@ template<class Algo, bool DUMP>
 cudaError_t
 launch_wib2(const KernelParams& kp, cudaStream_t s)
 {
-#ifndef SWTPG_WIB2_STAGES
-#define SWTPG_WIB2_STAGES 4
-#endif
-  constexpr int kStages = SWTPG_WIB2_STAGES;
-  auto k = wib2_kernel<Algo, kStages, DUMP>;
+  constexpr int kStages = 4;
+  constexpr auto k = wib2_kernel<Algo, kStages, DUMP>;
   constexpr size_t smem = Wib2Smem<kStages>::total;
-  static int resident[64];
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
+  unsigned resident = 0, sms = 0;
+  const cudaError_t e = residency<k>((kWib2Warps + 1) * 32, smem, 0, &resident, &sms);
   if (e != cudaSuccess)
     return e;
-  if (dev < 0 || dev >= 64)
-    return cudaErrorInvalidDevice;
-  if (resident[dev] == 0) {
-    e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-    if (e != cudaSuccess)
-      return e;
-    int per_sm = 0, sms = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, (kWib2Warps + 1) * 32, smem);
-    if (e != cudaSuccess)
-      return e;
-    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (e != cudaSuccess)
-      return e;
-    resident[dev] = std::max(1, per_sm * sms);
-  }
-  const unsigned grid = std::min<unsigned>(kp.n_links, unsigned(resident[dev])); // persistent CTAs claim links dynamically
+  const unsigned grid = std::min<unsigned>(kp.n_links, resident); // persistent CTAs claim links dynamically
   k<<<grid, (kWib2Warps + 1) * 32, smem, s>>>(kp); // 4 consumer warps + the producer warp
   return cudaGetLastError();
 }
@@ -347,8 +284,7 @@ make_params(const swtpg_handle* h, const ConfGroup& g, const void* d_frames, con
   for (int i = 0; i < 8; ++i)
     kp.taps[i] = c.fir_taps[i];
   kp.wib2_adc_offset = h->cfg.wib2_adc_offset;
-  static const bool force_exact = [] { const char* e = getenv("SWTPG_FIR_FORCE_EXACT"); return e && atoi(e) != 0; }();
-  kp.debug_flags = (force_exact || c.fir_force_exact) ? 1u : 0u;
+  kp.debug_flags = c.fir_force_exact ? 1u : 0u;
   kp.all_ones = 0xFFFFFFFFu;
   kp.one = 1u;
   return kp;
@@ -591,13 +527,12 @@ classify_config(int32_t format, const swtpg_link_config& in, TpgConf* out, const
     swtpg_firwin_int(7, 0.1, 1 << c.tap_exponent, c.fir_taps);
     c.fir_taps[7] = 0;
   }
-  const bool scalar_forced = getenv("SWTPG_FORCE_SCALAR") != nullptr;
   // Packed fast path validity (see PackedSimpleWibEth)
   c.fast_simple = c.algorithm == SWTPG_ALGO_SIMPLE_THRESHOLD && c.threshold <= 32767 &&
-                  (wib2 || (c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000)) && !scalar_forced;
+                  (wib2 || (c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000));
 
   c.fast_rs = !wib2 && (c.algorithm == SWTPG_ALGO_ABS_RS || c.algorithm == SWTPG_ALGO_STANDARD_RS) && c.threshold <= 32767 &&
-              c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000 && !scalar_forced;
+              c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000;
   // WIB2 AbsRS fast path validity (see PackedRsIqrWib2); threshold >= 1 is enforced above for the algorithm as such
   if (wib2 && c.algorithm == SWTPG_ALGO_ABS_RS && c.threshold >= 1) {
     const uint32_t e = c.tap_exponent, mult = 1u << e;
@@ -605,7 +540,7 @@ classify_config(int32_t format, const swtpg_link_config& in, TpgConf* out, const
     // thresholds sigma * threshold are compared by the bf16 comparator (valid up to 32640) and built by a packed multiply-add
     // (no carry between the halves while (sigmaMax + 3) * threshold < 2^16); outside that range every group takes the
     // exact-threshold tier (plain signed compares on the 64-bit-lane product, like the reference's _mm256_cmpgt_epi16)
-    const bool packed_ok = e >= 1 && e <= 10 && !scalar_forced;
+    const bool packed_ok = e >= 1 && e <= 10;
     const bool range_ok = (sigma_max + 3) * c.threshold < 65536 && sigma_max * c.threshold <= 32640;
     c.fast_rs_wib2 = packed_ok;
     c.fir_force_exact = packed_ok && !range_ok;
@@ -624,7 +559,7 @@ classify_config(int32_t format, const swtpg_link_config& in, TpgConf* out, const
     // reference's _mm256_cmpgt_epi16 sees the product as a NEGATIVE int16 once a channel's IQR is large enough, so such
     // configurations run the same packed trackers and filter with the exact-threshold tier forced on for every group.
     const uint64_t K = uint64_t(mult) * c.threshold;
-    const bool packed_ok = c.algorithm == SWTPG_ALGO_FIR_IQR && e >= 1 && e <= 10 && !scalar_forced;
+    const bool packed_ok = c.algorithm == SWTPG_ALGO_FIR_IQR && e >= 1 && e <= 10;
     const bool range_ok = (sigma_max + 3) * K < 65536 && sigma_max * K <= 32640;
     c.fast_fir = packed_ok && taps_ok;      // binomial cascade
     c.fast_fir_any = packed_ok && !taps_ok; // any other taps[0..6]: packed multiply-add chain (PackedFirIqrAnyTaps)

@@ -12,13 +12,6 @@
 
 #include "../../include/swtpg.h"
 
-#ifndef SWTPG_HIT_CAP
-#define SWTPG_HIT_CAP 160
-#endif
-#ifndef SWTPG_EXTRACT_IMAD
-#define SWTPG_EXTRACT_IMAD 0
-#endif
-
 namespace swtpg {
 
 // ---- packed 16x2 primitives ------------------------------------------------------------------------------------
@@ -125,14 +118,6 @@ ne2_abs_one(uint32_t a, uint32_t b)
   asm("{.reg .b32 t; abs.f16x2 t, %1; set.ne.f16x2.f16x2 %0, t, %2;}" : "=r"(r) : "r"(a), "r"(b));
   return r;
 }
-// Per half: 1.0 (0x3C00) where a == b as fp16, else 0.0 (HSET2.BF.EQ).
-__device__ __forceinline__ uint32_t
-eq2_one(uint32_t a, uint32_t b)
-{
-  uint32_t r;
-  asm("set.eq.f16x2.f16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
-  return r;
-}
 // Per-half "a > b" as 0xFFFF / 0x0000 for 0 <= a <= 32767 and 0 <= b <= 32640, computed by the bf16 comparator on the bit
 // patterns (HSET2.BF16_V2.GTU): non-negative bf16 values order like their patterns up to +inf = 0x7F80 = 32640; patterns
 // above that are NaNs, for which the "or unordered" flavour answers true — and a > 32640 >= b is indeed true.
@@ -216,6 +201,8 @@ elect_one()
   asm volatile("{\n.reg .pred P;\nelect.sync _|P, 0xFFFFFFFF;\nselp.u32 %0, 1, 0, P;\n}" : "=r"(pred));
   return pred != 0;
 }
+// Also the producer warps' wait on their `empty` barriers: try_wait parks the thread in hardware, so this loop is as fast as a
+// suspend-time hint and faster than a nanosleep back-off (measured, profiles/r02_producer_wait.txt).
 __device__ __forceinline__ void
 mbar_wait(uint64_t* bar, uint32_t parity)
 {
@@ -229,50 +216,6 @@ mbar_wait(uint64_t* bar, uint32_t parity)
                "}" ::"r"(smem_u32(bar)),
                "r"(parity)
                : "memory");
-}
-
-// Wait of a PRODUCER warp's lane on an `empty` barrier. A producer has nothing to do until its consumers release a stage
-// (microseconds), and a spinning try_wait loop issues SYNCS + BRA + YIELD every ~15 cycles on a sub-partition that the
-// consumer warps need (measured round 1: 30 % of all issued warp-instructions of the CTA-form kernels were this loop).
-//   SWTPG_PRODUCER_WAIT = 0  spin (round-1 behaviour)
-//                       = 1  try_wait with a suspend-time hint: the hardware parks the thread until the phase completes
-//                       = 2  test_wait + nanosleep back-off
-#ifndef SWTPG_PRODUCER_WAIT
-#define SWTPG_PRODUCER_WAIT 0
-#endif
-#ifndef SWTPG_PRODUCER_SLEEP_NS
-#define SWTPG_PRODUCER_SLEEP_NS 200
-#endif
-__device__ __forceinline__ bool
-mbar_test(uint64_t* bar, uint32_t parity)
-{
-  uint32_t ok;
-  asm volatile("{\n.reg .pred p;\nmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-               : "=r"(ok)
-               : "r"(smem_u32(bar)), "r"(parity)
-               : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void
-mbar_wait_producer(uint64_t* bar, uint32_t parity)
-{
-#if SWTPG_PRODUCER_WAIT == 1
-  asm volatile("{\n"
-               ".reg .pred p;\n"
-               "WAIT_%=:\n"
-               "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-               "@p bra DONE_%=;\n"
-               "bra WAIT_%=;\n"
-               "DONE_%=:\n"
-               "}" ::"r"(smem_u32(bar)),
-               "r"(parity), "r"(1000000u)
-               : "memory");
-#elif SWTPG_PRODUCER_WAIT == 2
-  while (!mbar_test(bar, parity))
-    __nanosleep(SWTPG_PRODUCER_SLEEP_NS);
-#else
-  mbar_wait(bar, parity);
-#endif
 }
 
 // ---- 14-bit pair extraction ---------------------------------------------------------------------------------------
@@ -296,18 +239,7 @@ __device__ __forceinline__ uint32_t
 extract_pair(const uint32_t* row, const PairPos& pp)
 {
   const uint32_t x = __funnelshift_r(row[pp.w0], row[pp.w1], pp.sh); // 28 payload bits + 4 junk bits on top
-#if SWTPG_EXTRACT_IMAD == 2
-  // z = f0 + f1*2^14 (28 bits); z + (z >> 14) * (2^16 - 2^14) = f0 + f1*2^16: LOP3 + SHF (ALU pipe) + IMAD (FMA pipe)
-  const uint32_t z = x & 0x0FFFFFFFu;
-  return (z >> 14) * 0xC000u + z;
-#elif SWTPG_EXTRACT_IMAD
-  // Same result with one ALU-pipe op fewer (the ALU pipe is the kernel's bottleneck, profiles/r01_*): z = f0 + f1*2^14;
-  // f1 = z >> 14 as a high multiply (IMAD.HI, FMA pipe), then z + f1*(2^16 - 2^14) = f0 + f1*2^16 (IMAD, FMA pipe).
-  const uint32_t z = x & 0x0FFFFFFFu;
-  return __umulhi(z, 1u << 18) * 0xC000u + z;
-#else
   return (x & 0x3FFFu) | ((x << 2) & 0x3FFF0000u);                   // -> u16x2 {adc(2l), adc(2l+1)}
-#endif
 }
 
 // The same pair with 0x4000 subtracted from each half (bits 14 and 15 forced to one: S - 16384 in two's complement), at the same
@@ -380,7 +312,7 @@ constexpr uint32_t kHitUnitBits = 18; // units per batch must stay below 2^18 (c
 
 struct HitStage
 {
-  static constexpr uint32_t kCap = SWTPG_HIT_CAP;     // pair records; a 4-tick group parks at most one per lane and tick = 128,
+  static constexpr uint32_t kCap = 160;               // pair records; a 4-tick group parks at most one per lane and tick = 128,
   static constexpr uint32_t kFlushAbove = kCap - 128; // so checking once per group with <= kCap-128 parked never overflows
   uint4* buf;                                 // warp-private, kCap entries
   uint32_t* aux;                              // warp-private, kCap entries (peak_time pairs)
@@ -393,18 +325,14 @@ struct HitStage
   // Any subset of lanes may call. charge_left = charge & left (per half), the other words are the packed state registers.
   __device__ __forceinline__ void push(uint32_t m, uint32_t charge_left, uint32_t tover, uint32_t peak, uint32_t ptime) const
   {
-#if !defined(SWTPG_EXPERIMENT_NO_PUSH) // timing experiment only (no TPs come out)
     const uint32_t slot = atomicAdd(cnt, 1u);
     buf[slot] = make_uint4(m, charge_left, tover, peak);
     aux[slot] = ptime;
-#endif
   }
   __device__ __forceinline__ void push(uint32_t m, uint32_t charge_left, uint32_t tover) const // finders without peak tracking
   {
-#if !defined(SWTPG_EXPERIMENT_NO_PUSH)
     const uint32_t slot = atomicAdd(cnt, 1u);
     buf[slot] = make_uint4(m, charge_left, tover, 0u);
-#endif
   }
   // Warp-uniform (every lane reads the same word); the warp is converged at both call sites.
   __device__ __forceinline__ uint32_t count() const { return *reinterpret_cast<volatile uint32_t*>(cnt); }

@@ -16,36 +16,6 @@
 
 #include <type_traits>
 
-#ifndef SWTPG_STEP_NEGL
-#define SWTPG_STEP_NEGL 1 // integer frugal step of SimpleThreshold / the running sums: accumulator reset as ONE IMAD with -L (0: c - L * D)
-#endif
-#ifndef SWTPG_SLICE_FENCES
-#define SWTPG_SLICE_FENCES 2 // sliced hand-out: 2 = every lane fences before lane 0's release store; 1 = the release alone
-#endif
-#ifndef SWTPG_GROUP_UNROLL
-#define SWTPG_GROUP_UNROLL 4
-#endif
-#ifndef SWTPG_FIR_GROUP_UNROLL
-#define SWTPG_FIR_GROUP_UNROLL 2
-#endif
-#ifndef SWTPG_QUAD_SIMPLE
-#define SWTPG_QUAD_SIMPLE 0
-#endif
-#ifndef SWTPG_ELECT
-#define SWTPG_ELECT 1
-#endif
-#ifndef SWTPG_RS_GROUP_UNROLL
-#define SWTPG_RS_GROUP_UNROLL 2
-#endif
-#ifndef SWTPG_FLOAT_ACC
-#define SWTPG_FLOAT_ACC 1
-#endif
-// Frugal accumulator of the SimpleThreshold / running-sum pedestal: 0 = fp16x2 subnormal (round 1), 1 = biased integer, seven
-// instructions per tick, 2 = biased integer with the step taken off the median's dependent chain (eight instructions, shorter chain)
-#ifndef SWTPG_SIMPLE_INT
-#define SWTPG_SIMPLE_INT 1
-#endif
-
 namespace swtpg {
 
 // ---- HBM-resident per-group state (struct of arrays: [group][var][lane], u32 = two packed channels) -------------
@@ -88,7 +58,9 @@ struct KernelParams
   uint32_t* link_cursor;   // [2] {links claimed beyond each warp's first, warps finished}; zero between launches (WIBEth kernel)
   uint32_t* link_done;     // [links of the handle] slices of the link finished in THIS launch; zero between launches (wibeth_kernel, sliced)
   uint32_t parts_log2;     // wibeth_kernel: a link's units are handed out in 2^parts_log2 consecutive slices (0 = whole links)
-  uint32_t slice_geom;     // ... of equal length (0) or halving: n/2, n/4, ..., and the rest (1)
+  uint32_t slice_geom;     // ... of equal length (0) or halving: n/2, n/4, ..., and the rest (1). The host always asks for halving
+                           // slices; the equal-slice arm stays because removing it changed the compiled tick loop of every
+                           // wibeth_kernel and measured slower on B200 (AbsRS 2.6 %, SimpleThreshold 0.8 %)
   TpSink sink;
   int16_t* pedestal_out;   // debug dumps [link][unit][tick][channel] or nullptr
   int16_t* waveform_out;
@@ -101,7 +73,7 @@ struct KernelParams
   int32_t tap_exponent;
   int32_t taps[8];
   uint32_t wib2_adc_offset;
-  uint32_t debug_flags;    // bit 0: PackedFirIqr always takes its exact-threshold tier (test aid, SWTPG_FIR_FORCE_EXACT=1)
+  uint32_t debug_flags;    // bit 0: PackedFirIqr always takes its exact-threshold tier (configurations outside the comparator's range)
   uint32_t all_ones;       // 0xFFFFFFFF: a constant the compiler cannot fold, so that it stays in ONE register (VIADDMNMX takes a
                            // single immediate; ptxas otherwise re-materialises the -1 operand with a move in front of every use)
   uint32_t one;            // 1: multiplier of the adds that are to run on the FMA pipe as IMAD (see fma_add below)
@@ -460,12 +432,11 @@ struct ScalarAlgo
 //                             clamp(Sb + Mq, 0, 2) = sign(s - m) + 1 is a single VIADDMNMX.S16x2.RELU, and Mq stays in
 //                             [2, 16385]: it never passes through 0x0000 / 0xFFFF, so its +-1 steps are ONE 32-bit
 //                             three-input add (IADD3) — no carry or borrow can cross the halves;
-//   A   = accumulator - 1     as the bit pattern of an fp16x2 subnormal (value * 2^-24, sign-magnitude: exact integer
-//                             arithmetic for |v| <= 1023 on the FMA pipe);
+//   A   = accumulator + L     a small non-negative integer per half ([0, 2L]), so that sums with the sign code are plain
+//                             32-bit adds (see pedestal_step);
 //   PK1 = peak_adc + 1        compared against sp1;   thr1 = threshold + 1 likewise;   Tn = -tover, PTn = -peak_time.
-// The recurrence median(t) -> median(t+1) is the critical path of a link (time is sequential per channel): VIADDMNMX ->
-// HADD2 -> HFMA2.SAT -> IADD3, four dependent instructions per tick (round 1: five). Everything else is taken off that
-// path by a two-stage software pipeline inside group(): the raw words of the NEXT group's rows are loaded before this
+// The recurrence median(t) -> median(t+1) is the critical path of a link (time is sequential per channel). Everything else
+// is taken off that path by a two-stage software pipeline inside group(): the raw words of the NEXT group's rows are loaded before this
 // group's arithmetic starts (prefetch across the quiet-test branch), and the quiet test / hit bookkeeping of a group is
 // DEFERRED by one group, so that it is scheduled in the shadow of the next group's pedestal chain.
 // =====================================================================================================================
@@ -476,17 +447,18 @@ struct ScalarAlgo
 template<bool PIPE>
 struct PackedSimpleT
 {
-  static constexpr int kGroupUnroll = SWTPG_GROUP_UNROLL;
+  static constexpr int kGroupUnroll = 4;
   // persistent warps per SM, measured: 5 per sub-partition for the straight-line form (profiles/r01_warps_sweep.txt), 4 for the
   // pipelined one below one round of links (92 registers; profiles/r02_simple_pipeline_sweep.txt); from 2960 links on the host
   // asks for 20 (profiles/r02_pipelined_full_load_probe.txt, r02_warps_crossover_probe.txt)
   static constexpr int kWarpsPerSm = PIPE ? 16 : 20;
-  static constexpr int kQuadCtasPerSm = SWTPG_QUAD_SIMPLE; // 0: one warp per CTA (measured faster for this policy)
+  static constexpr int kQuadCtasPerSm = 0; // one warp per CTA: the CTA form measured slower for this policy (65.4 % against
+                                           // 68.2 % of the HBM peak at 5920 links, profiles/r02_quad_form_probe.txt)
   static constexpr int kWib2MinCtas = 5;
   static constexpr bool kWib2Fields = false; // which process_swtpg_hits derives the TP fields (and whether the peak is tracked)
   uint32_t Mq, A, prev, C, Tn, PK1, PTn;
-  uint32_t cUp, cDn, thr1;
-  uint32_t cL, cLn, c2L, cL1, cLL, kM1; // integer accumulator form: L, -L, (2L, 2L), L + 1, (L, L); 0xFFFFFFFF in a register
+  uint32_t cUp, cDn, thr1; // fp16 constants of the running sums' RS tracker (PackedRsWibEth::frugal)
+  uint32_t cLn, c2L, cLL, kM1; // -L, (2L, 2L), (L, L); 0xFFFFFFFF in a register
   uint32_t shift, shmask; // WIB2 flavour only
   uint32_t raw[8];        // software pipeline: words of the next group's four rows ...
   uint32_t dsp[4], dwhen; // ... and the deferred group: its four s' + 1 and (unit << 6 | first tick); dvalid below
@@ -501,9 +473,7 @@ struct PackedSimpleT
     const uint32_t dn = 0x8000u | L;       // -L: addend of the "acc - L" / "-acc - L" saturating tests (sign-magnitude)
     cUp = up | (up << 16);
     cDn = dn | (dn << 16);
-    cL = L;
     cLn = p.acc_limit_neg;
-    cL1 = L + 1u;
     cLL = L * 0x00010001u;
     c2L = 2u * L * 0x00010001u;
     kM1 = p.all_ones;
@@ -515,7 +485,8 @@ struct PackedSimpleT
   {
     return add2(minu2(row, max * 0x00010001u), 0x00010001u);
   }
-  // Register form of the accumulator: (acc - 1) as the bit pattern of an fp16x2 subnormal (value * 2^-24, sign-magnitude).
+  // Register form of the running sums' RS accumulator (PackedRsWibEth): (acc - 1) as the bit pattern of an fp16x2 subnormal
+  // (value * 2^-24, sign-magnitude).
   static __device__ __forceinline__ uint32_t acc_to_reg(uint32_t v)
   {
     v = add2(v, 0xFFFFFFFFu);
@@ -532,11 +503,7 @@ struct PackedSimpleT
   __device__ __forceinline__ void load(const uint32_t* st, uint32_t lane, uint32_t)
   {
     Mq = add2(~st[SV_MEDIAN * 32 + lane], 0x40024002u); // ~m = -m - 1
-#if SWTPG_SIMPLE_INT
     A = add2(st[SV_ACCUM * 32 + lane], cLL);            // acc + L in [0, 2L]
-#else
-    A = acc_to_reg(st[SV_ACCUM * 32 + lane]);
-#endif
     prev = st[SV_PREV * 32 + lane];
     C = st[SV_CHARGE * 32 + lane];
     Tn = neg2(st[SV_TOVER * 32 + lane]);
@@ -553,11 +520,7 @@ struct PackedSimpleT
   __device__ __forceinline__ void store(uint32_t* st, uint32_t lane, uint32_t) const
   {
     st[SV_MEDIAN * 32 + lane] = median();
-#if SWTPG_SIMPLE_INT
     st[SV_ACCUM * 32 + lane] = add2(A, neg2(cLL));
-#else
-    st[SV_ACCUM * 32 + lane] = acc_from_reg(A);
-#endif
     st[SV_PREV * 32 + lane] = prev;
     st[SV_CHARGE * 32 + lane] = C;
     st[SV_TOVER * 32 + lane] = neg2(Tn);
@@ -574,48 +537,24 @@ struct PackedSimpleT
   }
 
   // frugal streaming median (wibeth/tpg/UtilsAVX2.hpp:38-73) + pedestal subtraction (ProcessAVX2.hpp:85): Sb -> s' + 1.
-  // The accumulator lives as an fp16x2 subnormal stored minus one, so that adding sign+1 lands on the new value; both step
-  // flags come out of the FMA pipe as the integer bit patterns 0 / 1 (saturating fp16 FMAs of +-acc - L), and the median
-  // takes them in one 32-bit add. The ALU pipe does the sign, one compare and that add.
-  //
-  // Integer form (SWTPG_SIMPLE_INT, round 2): the accumulator biased by +L is a small non-negative number per half, like the
-  // sign code, so their sum is a plain 32-bit add (either pipe); one clamp takes out the two step values, the difference is
-  // the step D in {-1, 0, +1} per half held as ONE 32-bit integer (the low half may borrow from the high one — harmless, only
-  // linear 32-bit operations consume it and their results have non-negative halves again), and the accumulator returns to L
-  // where it stepped through one IMAD. Two instructions on the ALU pipe, two (one without the final add) on the FMA pipe, three
-  // that issue on either; the fp16 form has 2 / 5 / 1.
+  // The accumulator biased by +L is a small non-negative number per half, like the sign code, so their sum is a plain 32-bit
+  // add (either pipe); one clamp takes out the two step values, the difference is the step D in {-1, 0, +1} per half held as
+  // ONE 32-bit integer (the low half may borrow from the high one — harmless, only linear 32-bit operations consume it and their
+  // results have non-negative halves again), and the accumulator returns to L where it stepped through one IMAD. Two
+  // instructions on the ALU pipe, two (one without the final add) on the FMA pipe, three that issue on either; the fp16-subnormal
+  // accumulator of round 1 had 2 / 5 / 1 and measured slower (profiles/r02_integer_accumulators.txt).
   __device__ __forceinline__ uint32_t pedestal_step(uint32_t Sb)
   {
     const uint32_t sg1 = addclamp2(Sb, Mq, 0x00020002u);        // sign(s - m) + 1 in {0,1,2}
-#if SWTPG_SIMPLE_INT
     const uint32_t U = A + sg1;                                 // acc' + L + 1 in [0, 2L + 2]
     const uint32_t c = addclamp2(U, kM1, c2L);                  // clamp(acc' + L, 0, 2L)
-#if SWTPG_SIMPLE_INT == 2
-    const uint32_t W = Mq - U + 0x00010001u;                    // in the shadow of the clamp
-    const uint32_t V = cLL - cL * U;                            // L - L U
-    Mq = W + c;                                                 // m += U - 1 - c
-    A = cL1 * c + V;                                            // c - L (U - 1 - c)
-#else
     const uint32_t D = U - c - 0x00010001u;                     // the step
-#if SWTPG_STEP_NEGL
     A = cLn * D + c;                                            // back to L where it stepped: c - L D as ONE IMAD with -L from the
                                                                 // constant bank (written c - L * D ptxas negates D first: 62
-                                                                // instead of 59 instructions per quiet 4-tick group)
-#else
-    A = c - cL * D;
-#endif
+                                                                // instead of 59 instructions per quiet 4-tick group, 2-5 % slower
+                                                                // for the chain-bound forms, profiles/r02_step_form_probe.txt)
     Mq -= D;                                                    // (steering these adds to the FMA pipe measured 1 % slower here)
-#endif
     return add2(Sb, Mq);                                        // s' + 1 with the UPDATED median
-#else
-    const uint32_t T = hadd2_bits(A, sg1);                      // acc after this sample, in [-(L+1), L+1]
-    const uint32_t up1 = hfma2_sat_bits(T, 0x3C003C00u, cDn);   // sat(acc - L)  -> bit pattern 1: acc == L+1
-    const uint32_t dn1 = hfma2_sat_bits(T, 0xBC00BC00u, cDn);   // sat(-acc - L) -> bit pattern 1: acc == -(L+1)
-    const uint32_t keep = ne2_abs_one(T, cUp);                  // 1.0 unless |acc| == L+1
-    A = hfma2_bits(keep, T, 0x80018001u);                       // (stepped ? 0 : acc) - 1
-    Mq = Mq + dn1 - up1;                                        // m += up - down: one IADD3, halves cannot interact (see above)
-    return add2(Sb, Mq);                                        // s' + 1 with the UPDATED median
-#endif
   }
   __device__ __forceinline__ uint32_t over_mask(uint32_t sp1) const { return gt2_mask_nonneg(sp1, thr1); } // (:97-98)
 
@@ -736,7 +675,7 @@ using PackedSimpleWibEthPipe = PackedSimpleT<true>;
 // WIB2 SimpleThreshold (wib2/tpg/ProcessAVX2.hpp:24-200). Same pedestal recurrence with the limit fixed at 10 (:79); charge
 // accumulates (over ? s' : 0) >> tap_exponent with signed saturation (:110-112), no peak tracking, hit block = {chan, t,
 // charge, tover}. Validity: 0 <= threshold <= 32767. Straight-line groups only: the CTA form caps the registers for five CTAs
-// per SM, and the pipelined form measured 7 % slower there (gpurun_out/r02_probe3.txt).
+// per SM, and the pipelined form measured 7 % slower there (profiles/r02_simple_pipeline_sweep.txt).
 // =====================================================================================================================
 struct PackedSimpleWib2 : PackedSimpleWibEth
 {
@@ -823,7 +762,7 @@ struct PackedSimpleWib2 : PackedSimpleWibEth
 template<bool STANDARD>
 struct PackedRsWibEth : PackedSimpleWibEth
 {
-  static constexpr int kGroupUnroll = SWTPG_RS_GROUP_UNROLL;
+  static constexpr int kGroupUnroll = 2;
   static constexpr int kWarpsPerSm = STANDARD ? 20 : 16; // AbsRS: 4 warps per sub-partition beat 5 by 3 % (same sweep)
   uint32_t RS1, MRq, AR;     // RS + 1 (carried value, after median subtraction); 1 - median_RS; (acc_RS - 1) as fp16 subnormal
   int f_lo, f_hi, nf_lo, nf_hi, scale;
@@ -965,16 +904,11 @@ struct PackedRsWibEth : PackedSimpleWibEth
 //     6 packed adds per tick instead of 7 multiply-adds on a rotating ring, and every add wraps mod 2^16 exactly like the
 //     reference's mullo/add chain (ring homomorphism). The carried state stays the reference's ring: it is converted to
 //     cascade registers when a link is loaded and back when it is stored, which also removes the ring phase from the loop;
-//   * accumulators are fp16x2 subnormals and the median lives as 16385 - median against the biased sample Sb = S - 16384,
-//     with the four-instruction step of PackedSimpleT;
-//   * the kernel is bound by the ALU pipe (LOP3 / SHF / VIADD.16x2 / VIADDMNMX / IADD3: 16 lanes per sub-partition, half the
-//     issue rate), while the fp16 pipe (HFMA2 / HADD2 / HSET2) idles at 40 % — measured, profiles/r02_wibeth_fir_*. So every
-//     tracker keeps its ALU work to the sign test and one three-input add: the step flags come out of the fp16 pipe as the
-//     integer bit patterns 0 / 1 (saturating FMAs of +-acc - L), the quartile enables (sample below / above the OLD median,
-//     :119-121) multiply into the accumulator's FMA, and q25 lives as 16385 - q25, q75 as q75 + 2 — both inside [2, 16405] for
-//     every input, so their +-1 steps cannot carry between the halves. (Merging the two quartile trackers into one step on
-//     per-half selected operands — they never move in the same tick — saves 6 instructions per tick but ADDS three to the
-//     ALU pipe, the selects and write-backs being LOP3s: measured, no gain, not kept.)
+//   * the three trackers keep integer accumulators biased to small non-negative numbers, and the median, q25 and q75 live as
+//     16385 - value against the biased sample Sb = S - 16384 — inside [2, 16405] for every input, so their +-1 steps cannot
+//     carry between the halves (track() lists the instructions). They replaced fp16x2-subnormal accumulators whose step flags
+//     came out of the fp16 pipe, with the two quartile trackers merged into one step or kept separate: both forms measured
+//     slower (profiles/r02_integer_accumulators.txt);
 //   * sigma is only needed where the threshold is: the quiet test works with a lower bound of the group's sigmas taken from the
 //     quartiles after its last tick (sigma moves by at most one per tick, because at most one quartile moves), and the per-tick
 //     values are formed from the saved quartile registers only in a group that turns out busy;
@@ -984,23 +918,12 @@ struct PackedRsWibEth : PackedSimpleWibEth
 // =====================================================================================================================
 struct PackedFirIqr
 {
-  static constexpr int kGroupUnroll = SWTPG_FIR_GROUP_UNROLL;
+  static constexpr int kGroupUnroll = 2;
   static constexpr int kWarpsPerSm = 12; // 3 warps per sub-partition: 3 % faster than the 16 its 128 registers allow (same sweep)
   static constexpr int kWib2MinCtas = 5;
   static constexpr int kQuadCtasPerSm = 4; // CTA form, 16 consumer warps per SM (measured: 4 CTAs 29.8 %, 5 CTAs 27.8 %, profiles/r02_fir_forms.txt)
                                            // (64 registers instead of 109; profiles/r01_quad_vs_warp.txt)
-#ifndef SWTPG_FIR_INT
-#define SWTPG_FIR_INT 1 // 1: integer accumulators (round 2, see track()); 0: the fp16-subnormal forms of round 1 below
-#endif
-#ifndef SWTPG_FIR_U3
-#define SWTPG_FIR_U3 0 // integer form: the two three-input adds as one IADD3 each (ALU pipe, 0) or as two IMADs each (FMA pipe, 1)
-#endif
-#ifndef SWTPG_FIR_MERGED
-#define SWTPG_FIR_MERGED 1 // fp16 forms only. 1: the two quartile trackers share one step on per-half selected operands; 0: two separate steps
-#endif
-  // 16385 - median, 16385 - q25 in every form. Integer form: Q75p = 16385 - q75, A = acc + 10, A25 = acc25 + 10, A75 = acc75 + 11.
-  // fp16 forms: Q75p = q75 + 2, A = acc - 1 and the quartile accumulators as fp16x2 subnormal bit patterns
-  // (merged form acc25 - 1 and -acc75 - 1, separate form acc25 and acc75)
+  // Mq = 16385 - median, Q25n = 16385 - q25, Q75p = 16385 - q75, A = acc + 10, A25 = acc25 + 10, A75 = acc75 + 11.
   uint32_t Mq, A, Q25n, A25, Q75p, A75;
   uint32_t kM1, kP1; // 0xFFFFFFFF and 1 in registers the compiler cannot see through (KernelParams::all_ones, one)
   uint32_t d1, d2, d3, d4, d5, d6, o1, o2; // cascade: d_j = previous input of stage j, o1/o2 = previous two outputs
@@ -1012,12 +935,11 @@ struct PackedFirIqr
   __device__ __forceinline__ void begin_chunk(const uint32_t*, const PairPos&) {}
   template<bool WIB2_UNITS = false>
   __device__ __forceinline__ void finish_link(const TickCtx&) {}
-  static constexpr uint32_t kTiny = 0x00010001u;    // 2^-24 per half
-  static constexpr uint32_t kNegTiny = 0x80018001u;
-  static constexpr uint32_t kUp = 0x000B000Bu;      // (L+1) * 2^-24, L = 10
-  static constexpr uint32_t kDnEq = 0x800B800Bu;    // -(L+1)
+  // fp16-subnormal constants of PackedRsIqrWib2's RS tracker (L = 10)
+  static constexpr uint32_t kNegTiny = 0x80018001u; // -2^-24 per half
+  static constexpr uint32_t kUp = 0x000B000Bu;      // (L+1) * 2^-24
   static constexpr uint32_t kNegL = 0x800A800Au;    // -L
-  static constexpr uint32_t kOne = 0x3C003C00u, kNegOne = 0xBC00BC00u;
+  static constexpr uint32_t kNegOne = 0xBC00BC00u;
 
   template<bool WIB2_UNITS>
   static __device__ __forceinline__ void flush(const HitStage& h, const TpSink& k, const uint8_t* link_base, uint32_t link, uint32_t lane,
@@ -1042,7 +964,7 @@ struct PackedFirIqr
     kP1 = p.one;
   }
   static __device__ __forceinline__ uint32_t to_sm(uint32_t v)
-  { // two's complement s16x2 -> sign-magnitude (= bit pattern of value * 2^-24 as fp16), |v| <= 1023
+  { // two's complement s16x2 -> sign-magnitude (= bit pattern of value * 2^-24 as fp16), |v| <= 1023; PackedRsIqrWib2's RS tracker
     const uint32_t neg = (v & 0x80008000u) >> 15, m = neg * 0xFFFFu;
     return (add2(v ^ m, neg) & 0x7FFF7FFFu) | (m & 0x80008000u);
   }
@@ -1063,22 +985,10 @@ struct PackedFirIqr
   {
     Mq = add2(~st[SV_MEDIAN * 32 + lane], 0x40024002u);       // ~m = -m - 1
     Q25n = add2(~st[SV_Q25 * 32 + lane], 0x40024002u);
-#if SWTPG_FIR_INT
     A = add2(st[SV_ACCUM * 32 + lane], 0x000A000Au);
     Q75p = add2(~st[SV_Q75 * 32 + lane], 0x40024002u);
     A25 = add2(st[SV_A25 * 32 + lane], 0x000A000Au);
     A75 = add2(st[SV_A75 * 32 + lane], 0x000B000Bu);
-#else
-    A = to_sm(add2(st[SV_ACCUM * 32 + lane], 0xFFFFFFFFu));
-    Q75p = add2(st[SV_Q75 * 32 + lane], 0x00020002u);
-#if SWTPG_FIR_MERGED
-    A25 = to_sm(add2(st[SV_A25 * 32 + lane], 0xFFFFFFFFu));
-    A75 = to_sm(~st[SV_A75 * 32 + lane]);                      // ~a = -a - 1
-#else
-    A25 = to_sm(st[SV_A25 * 32 + lane]);
-    A75 = to_sm(st[SV_A75 * 32 + lane]);
-#endif
-#endif
     prev = st[SV_PREV * 32 + lane];
     C = st[SV_CHARGE * 32 + lane];
     Tn = neg2(st[SV_TOVER * 32 + lane]);
@@ -1087,22 +997,10 @@ struct PackedFirIqr
   {
     st[SV_MEDIAN * 32 + lane] = median();
     st[SV_Q25 * 32 + lane] = add2(~Q25n, 0x40024002u);
-#if SWTPG_FIR_INT
     st[SV_ACCUM * 32 + lane] = add2(A, 0xFFF6FFF6u);
     st[SV_Q75 * 32 + lane] = add2(~Q75p, 0x40024002u);
     st[SV_A25 * 32 + lane] = add2(A25, 0xFFF6FFF6u);
     st[SV_A75 * 32 + lane] = add2(A75, 0xFFF5FFF5u);
-#else
-    st[SV_ACCUM * 32 + lane] = add2(from_sm(A), 0x00010001u);
-    st[SV_Q75 * 32 + lane] = add2(Q75p, 0xFFFEFFFEu);
-#if SWTPG_FIR_MERGED
-    st[SV_A25 * 32 + lane] = add2(from_sm(A25), 0x00010001u);
-    st[SV_A75 * 32 + lane] = ~from_sm(A75);
-#else
-    st[SV_A25 * 32 + lane] = from_sm(A25);
-    st[SV_A75 * 32 + lane] = from_sm(A75);
-#endif
-#endif
     st[SV_PREV * 32 + lane] = prev;
     st[SV_CHARGE * 32 + lane] = C;
     st[SV_TOVER * 32 + lane] = neg2(Tn);
@@ -1151,30 +1049,13 @@ struct PackedFirIqr
   {
     Mq = add2(~Sb, 0x00020002u);               // 16385 - ped = 1 - Sb
     Q25n = add2(~Sb, 0x00160016u);             // 16385 - (ped - 20)
-#if SWTPG_FIR_INT
     Q75p = add2(~Sb, 0xFFEEFFEEu);             // 16385 - (ped + 20)
-#else
-    Q75p = add2(Sb, 0x40164016u);              // (ped + 20) + 2
-#endif
   }
 
-  // One frugal quartile step on the halves `en` (1.0 / 0.0 per half); c = sign(...) + 1 in {0,1,2} as the sign test delivers it.
-  // Returns the step as two bit patterns 0 / 1 (up, down); the caller adds them to its register with the sign its form needs.
-  static __device__ __forceinline__ void quartile_acc(uint32_t& Aq, uint32_t sgn, uint32_t en, uint32_t& up, uint32_t& dn)
-  {
-    const uint32_t T = hfma2_bits(en, sgn, Aq);                       // acc (+= sign on the enabled halves)
-    up = hfma2_sat_bits(T, kOne, kNegL);                              // bit pattern 1 where acc reached  L+1
-    dn = hfma2_sat_bits(T, kNegOne, kNegL);                           // ...                             -(L+1)
-    Aq = hfma2_bits(ne2_abs_one(T, kUp), T, 0u);                      // reset where stepped
-  }
-  // The three frugal trackers of one tick (Sb = raw - 16384). Returns 16385 - median (integer form) or s' + 1 = raw - median + 1
-  // (fp16 forms), updated median: see sp1_of / clamped_sample.
-  // fp16 forms — ALU pipe: three sign tests, one complement, three IADD3, the final add. Everything else runs on the fp16 pipe.
-  //
-  // Integer form (SWTPG_FIR_INT, round 2). A frugal accumulator stays in [-10, 10] between ticks, so biased by +10 it is a small
-  // NON-NEGATIVE number in each half, and so are the sign codes {0,1,2}: sums of such values are plain 32-bit adds (IADD3 issues on
-  // either pipe at twice the rate of the packed-16x2 and fp16x2 instructions) because nothing carries between the halves. One
-  // tracker step is
+  // The three frugal trackers of one tick (Sb = raw - 16384). Returns 16385 - median, updated: see sp1_of / clamped_sample.
+  // A frugal accumulator stays in [-10, 10] between ticks, so biased by +10 it is a small NON-NEGATIVE number in each half, and so
+  // are the sign codes {0,1,2}: sums of such values are plain 32-bit adds (IADD3 issues on either pipe at twice the rate of the
+  // packed-16x2 and fp16x2 instructions) because nothing carries between the halves. One tracker step is
   //     U = B + sign + 1                      acc' + 11 in [0, 22]                                         IADD3
   //     c = clamp(U - 1, 0, 20)               acc' + 10 without the two step values                        VIADDMNMX.RELU
   //     D = U - 1 - c                         the step, -1 / 0 / +1 per half, as ONE 32-bit integer        IADD3
@@ -1186,15 +1067,15 @@ struct PackedFirIqr
   // median) cost no select: the clamp's upper bound is 2 on the enabled halves and 0 elsewhere, which turns the sign code into 0
   // there, and the missing +1 comes from n1 (q25, "+10" form) or is taken back out by g1 (q75, "+11" form).
   // Per tick: 8 ALU-pipe instructions (sign tests, clamps, enables), 3-4 on the FMA pipe, 10 adds that go to whichever is free
-  // — against 13 / 8 / 2 for the merged fp16 form and 9 / 14 / 3 for the separate one.
+  // — against 13 / 8 / 2 for the fp16-subnormal form with merged quartile trackers and 9 / 14 / 3 with separate ones. The
+  // three-input adds stay IADD3s: as two IMADs each on the FMA pipe they gained nothing (profiles/r02_fma_steering_probe.txt, u3).
   __device__ __forceinline__ uint32_t track(uint32_t Sb)
   {
     const uint32_t sg1 = addclamp2(Sb, Mq, 0x00020002u);              // sign(raw - median) + 1, OLD median   (:108-117)
-#if SWTPG_FIR_INT
     // q25 on the halves below the OLD median (:119)
     const uint32_t n1 = min2(sg1, 0x00010001u);                       // 0 where below, 1 elsewhere
     const uint32_t s25 = addclamp2(Sb, Q25n, n1 * (kM1 + kM1) + 0x00020002u); // bound 2 - 2 n1 (IMAD): sign(raw - q25) + 1 where enabled, else 0
-    const uint32_t U25 = SWTPG_FIR_U3 ? fma_add(n1, fma_add(s25, A25, kP1), kP1) : A25 + s25 + n1; // acc25' + 11
+    const uint32_t U25 = A25 + s25 + n1;                              // acc25' + 11
     const uint32_t c25 = addclamp2(U25, kM1, 0x00140014u);
     const uint32_t D25 = U25 - c25 - 0x00010001u;
     A25 = c25 - 10u * D25;
@@ -1202,7 +1083,7 @@ struct PackedFirIqr
     // q75 on the halves above it (:121)
     const uint32_t g1 = __viaddmax_s16x2_relu(sg1, kM1, 0u);          // 1 where above, 0 elsewhere
     const uint32_t s75 = addclamp2(Sb, Q75p, fma_add(g1, g1, kP1));  // bound 2 g1: sign(raw - q75) + 1 where enabled, else 0
-    const uint32_t U75 = SWTPG_FIR_U3 ? fma_sub(fma_add(s75, A75, kP1), g1, kM1) : A75 + s75 - g1; // acc75' + 11
+    const uint32_t U75 = A75 + s75 - g1;                              // acc75' + 11
     const uint32_t c75 = addclamp2(U75, kM1, 0x00140014u);
     const uint32_t D75 = U75 - c75 - 0x00010001u;
     A75 = U75 - 11u * D75;
@@ -1214,70 +1095,22 @@ struct PackedFirIqr
     A = cm - 10u * D;
     Mq = fma_sub(Mq, D, kM1);
     return Mq;
-#else
-    const uint32_t ltf = eq2_one(sg1, 0u), gtf = eq2_one(sg1, 0x00020002u);
-#if SWTPG_FIR_MERGED
-    // q25 moves only on the halves below the OLD median and q75 only on the halves above it (:119-121): per half at most one of
-    // them does anything, so ONE frugal step runs on per-half SELECTED operands — (Sb, 16385 - q25, acc25) below, (~raw, q75 + 2,
-    // -acc75) elsewhere: with the sample and the accumulator negated the q75 tracker obeys the same "register += down - up"
-    // rule as the q25 one — and is written back through the two masks; where the sample equals the median it is dropped.
-    (void)ltf;
-    (void)gtf;
-    const uint32_t lt = eq2_mask(sg1, 0u), gt = eq2_mask(sg1, 0x00020002u);
-    const uint32_t a = (lt & Sb) | (~lt & (~Sb | 0xC000C000u));       // raw - 16384 below; ~raw = -raw - 1 elsewhere (one LOP3)
-    const uint32_t Qs = (lt & Q25n) | (~lt & Q75p), As = (lt & A25) | (~lt & A75);
-    const uint32_t Tq = hadd2_bits(As, addclamp2(a, Qs, 0x00020002u)); // acc25 | -acc75 after this sample
-    const uint32_t uq = hfma2_sat_bits(Tq, kOne, kNegL), dq = hfma2_sat_bits(Tq, kNegOne, kNegL);
-    const uint32_t An = hfma2_bits(ne2_abs_one(Tq, kUp), Tq, kNegTiny); // (stepped ? 0 : acc) - 1
-    const uint32_t Qn = Qs + dq - uq;
-    Q25n = (lt & Qn) | (~lt & Q25n);
-    A25 = (lt & An) | (~lt & A25);
-    Q75p = (gt & Qn) | (~gt & Q75p);
-    A75 = (gt & An) | (~gt & A75);
-#else
-    uint32_t up, dn;
-    // q25 on the halves below the median (:119): sign(raw - q25) from Sb + (16385 - q25)
-    quartile_acc(A25, hadd2_bits(addclamp2(Sb, Q25n, 0x00020002u), kNegTiny), ltf, up, dn);
-    Q25n = Q25n + dn - up;                                            // 16385 - q25 steps down when q25 steps up
-    // q75 on the halves above (:121): 1 - (sign(q75 - raw) + 1) from ~raw + (q75 + 2), ~raw = -raw - 1 = ~Sb | 0xC000 per half
-    quartile_acc(A75, hfma2_bits(addclamp2(~Sb | 0xC000C000u, Q75p, 0x00020002u), kNegOne, kTiny), gtf, up, dn);
-    Q75p = Q75p + up - dn;
-#endif
-    // median (:125), as PackedSimpleT::pedestal_step with L = 10
-    const uint32_t T = hadd2_bits(A, sg1);
-    const uint32_t up1 = hfma2_sat_bits(T, kOne, kNegL), dn1 = hfma2_sat_bits(T, kNegOne, kNegL);
-    A = hfma2_bits(ne2_abs_one(T, kUp), T, kNegTiny);
-    Mq = Mq + dn1 - up1;
-    return add2(Sb, Mq);
-#endif
   }
   // min(q75 - q25, sigmaMax) + 3 (:131-134) from a pair of quartile registers (Q75p, Q25n)
   __device__ __forceinline__ uint32_t sig3_of(uint32_t q75p, uint32_t q25n) const
   {
-#if SWTPG_FIR_INT
     return addmin2(add2(~q75p, 0x00040004u), q25n, sig3max);          // -(16385 - q75) + 3 = ~Q75p + 4 per half
-#else
-    return addmin2(add2(q75p, 0xC000C000u), q25n, sig3max);
-#endif
   }
   // One tick: returns the filter output of this tick.
   // s' + 1 = raw - median + 1 from what track() returns
   static __device__ __forceinline__ uint32_t sp1_of(uint32_t Sb, uint32_t tr)
   {
-#if SWTPG_FIR_INT
     return add2(Sb, tr);
-#else
-    return tr;
-#endif
   }
   // min(raw - median, adcMax) (:128,142) from what track() returns
   __device__ __forceinline__ uint32_t clamped_sample(uint32_t Sb, uint32_t tr) const
   {
-#if SWTPG_FIR_INT
     return addmin2(Sb, fma_add(tr, 0xFFFEFFFFu, kP1), xmax);         // tr = 16385 - median >= 2: the -1 is a plain 32-bit add
-#else
-    return addmin2(tr, 0xFFFFFFFFu, xmax);                            // tr = raw - median + 1
-#endif
   }
   __device__ __forceinline__ uint32_t tick(uint32_t Sb)
   {
@@ -1745,7 +1578,7 @@ wibeth_kernel(const KernelParams p)
         pr_start(item);
       } while (pr_left == 0);
     }
-    if (SWTPG_ELECT ? elect_one() : lane == 0) {
+    if (elect_one()) {
       mbar_arrive_expect_tx(&bars[pr_slot], kChunkBytes);
       bulk_g2s(stages + pr_slot * kChunkBytes, pr_src, kChunkBytes, &bars[pr_slot]);
     }
@@ -1850,10 +1683,8 @@ wibeth_kernel(const KernelParams p)
     if (lane == 0)
       p.group_flags[link] = kFlagInitialized | (k_end << 8);
     if (p.parts_log2 != 0u) { // publish the state to the warp that runs the link's next slice; the last slice re-arms the counter
-#if SWTPG_SLICE_FENCES == 2
-      __threadfence();
-#endif
-      __syncwarp(); // orders the lanes' stores before lane 0's release, which is cumulative
+      __threadfence(); // every lane's (the release alone measured the same, profiles/r02_step_form_probe.txt)
+      __syncwarp();    // orders the lanes' stores before lane 0's release, which is cumulative
       if (lane == 0) {
         const uint32_t done = part + 1u == (1u << p.parts_log2) ? 0u : slices_before(link, part, u0) + 1u;
         asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p.link_done + link), "r"(done) : "memory");
@@ -1939,7 +1770,7 @@ wibeth_quad_kernel(const KernelParams p)
     uint32_t slot = 0, round = 0, pushed = 0;
     auto wait_slot = [&]() { // all four consumers released the stage's previous contents
       if (round != 0)
-        mbar_wait_producer(&empty[slot], (round - 1u) & 1u);
+        mbar_wait(&empty[slot], (round - 1u) & 1u);
     };
     uint32_t first_link = blockIdx.x * kQuad; // the CTA's first quad (work items); every further one is claimed from the cursor
     for (bool first = true;;) {
@@ -2166,7 +1997,7 @@ wib2_kernel(const KernelParams p)
     uint32_t slot = 0, round = 0, pushed = 0;
     auto wait_slot = [&]() { // all four consumers released the stage's previous contents
       if (round != 0)
-        mbar_wait_producer(&empty[slot], (round - 1u) & 1u);
+        mbar_wait(&empty[slot], (round - 1u) & 1u);
     };
     uint32_t item = blockIdx.x; // the CTA's first work item; every further one is claimed from the cursor (as in wibeth_kernel)
     for (bool first = true;; first = false) {

@@ -13,7 +13,7 @@
 // others back, and flush is just "dispatch now" — safe against concurrent submits because the dispatcher only ever takes
 // whole units below a `head` it has read with acquire semantics.
 //
-// The host-to-device transfer is ONE kernel per batch (gather_units_*): SM-issued copies read every unit where it lies in
+// The host-to-device transfer is ONE kernel per batch (gather_units_tma): SM-issued copies read every unit where it lies in
 // pinned, mapped host memory through a per-unit pointer table and lay the batch out link-major in HBM for the fused TPG
 // kernel. No per-link cudaMemcpyAsync calls (round 1 issued one per link and run), no staging pass for registered buffers.
 #include "swtpg_handle.h"
@@ -87,32 +87,6 @@ gather_units_tma(const GatherItem* __restrict__ items, uint32_t n, uint8_t* __re
   asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
 }
 
-// LSU form: one warp per unit, 16-byte loads with UNROLL of them in flight per lane, then the stores.
-template<int UNROLL>
-__global__ void __launch_bounds__(256)
-gather_units_lsu(const GatherItem* __restrict__ items, uint32_t n, uint8_t* __restrict__ dst, uint32_t vecs)
-{
-  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31u, warps = (gridDim.x * blockDim.x) >> 5;
-  for (uint32_t i = warp; i < n; i += warps) {
-    const GatherItem it = items[i];
-    const uint4* s = reinterpret_cast<const uint4*>(it.src);
-    uint4* d = reinterpret_cast<uint4*>(dst + it.dst_off);
-    for (uint32_t j0 = lane; j0 < vecs; j0 += 32u * UNROLL) {
-      uint4 v[UNROLL];
-#pragma unroll
-      for (int u = 0; u < UNROLL; ++u)
-        if (j0 + 32u * u < vecs)
-          asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                       : "=r"(v[u].x), "=r"(v[u].y), "=r"(v[u].z), "=r"(v[u].w)
-                       : "l"(s + j0 + 32u * u));
-#pragma unroll
-      for (int u = 0; u < UNROLL; ++u)
-        if (j0 + 32u * u < vecs)
-          d[j0 + 32u * u] = v[u];
-    }
-  }
-}
-
 // ---- engine -----------------------------------------------------------------------------------------------------------
 using Clock = std::chrono::steady_clock;
 
@@ -146,7 +120,7 @@ struct Batch
   uint32_t n_items = 0;
   cudaStream_t stream = nullptr;
   cudaEvent_t ev_gather = nullptr, ev_kernel = nullptr, ev_count = nullptr, ev_tps = nullptr;
-  cudaEvent_t ev_up = nullptr;                  // pointer table and lengths are on the device (serial gather stream only)
+  cudaEvent_t ev_up = nullptr;                  // pointer table and lengths are on the device (the gather stream waits for it)
   cudaEvent_t ev_g0 = nullptr, ev_k0 = nullptr; // timing: start of the gather / of the TPG kernel (device clocks, swtpg_stream_timing)
   cudaEvent_t ev_stats = nullptr;               // the ADC statistics kernel has read d_frames (SWTPG_FLAG_ADC_STATS only)
   uint32_t n_ready = 0, n_taken = 0;
@@ -189,8 +163,7 @@ struct StreamEngine
   std::mutex poll_mu; // one poller at a time
   std::chrono::microseconds timeout{ 5000 };
 
-  int gather_mode = 0, gather_ctas = 64; // 0 = TMA ring, 1 = LSU
-  cudaStream_t gather_stream = nullptr;  // the gathers of all batches run one after the other on this stream (null: each on its batch's)
+  cudaStream_t gather_stream = nullptr; // the gathers of all batches run one after the other on this stream
 
   void kick()
   {
@@ -210,7 +183,7 @@ struct StreamEngine
     cv_flush.notify_all();
     cv_space.notify_all();
   }
-  cudaError_t launch_gather(Batch& b, cudaStream_t gs);
+  cudaError_t launch_gather(Batch& b);
   cudaError_t enqueue(Batch& b);
   void dispatcher_main();
   void releaser_main();
@@ -220,6 +193,7 @@ struct StreamEngine
 namespace {
 
 constexpr int kGatherStages = 8;
+constexpr unsigned kGatherCtas = 64;
 
 void
 free_batch(Batch& b)
@@ -244,27 +218,16 @@ free_batch(Batch& b)
   if (b.stream) cudaStreamDestroy(b.stream);
 }
 
-int
-env_int(const char* name, int dflt)
-{
-  const char* e = getenv(name);
-  return e && *e ? atoi(e) : dflt;
-}
-
 } // namespace
 
 cudaError_t
-StreamEngine::launch_gather(Batch& b, cudaStream_t gs)
+StreamEngine::launch_gather(Batch& b)
 {
   if (b.n_items == 0)
     return cudaSuccess;
-  const unsigned grid = std::min<unsigned>(unsigned(gather_ctas), b.n_items);
-  if (gather_mode == 0) {
-    const size_t smem = size_t(kGatherStages) * unit_bytes + kGatherStages * 8;
-    gather_units_tma<kGatherStages><<<grid, 32, smem, gs>>>(b.d_items, b.n_items, b.d_frames, unit_bytes);
-  } else {
-    gather_units_lsu<8><<<grid, 256, 0, gs>>>(b.d_items, b.n_items, b.d_frames, unit_bytes / 16);
-  }
+  const unsigned grid = std::min<unsigned>(kGatherCtas, b.n_items);
+  const size_t smem = size_t(kGatherStages) * unit_bytes + kGatherStages * 8;
+  gather_units_tma<kGatherStages><<<grid, 32, smem, gather_stream>>>(b.d_items, b.n_items, b.d_frames, unit_bytes);
   return cudaGetLastError();
 }
 
@@ -280,16 +243,12 @@ StreamEngine::enqueue(Batch& b)
   return e
   TRY(cudaMemcpyAsync(b.d_items, b.h_items, size_t(b.n_items) * sizeof(GatherItem), cudaMemcpyHostToDevice, b.stream));
   TRY(cudaMemcpyAsync(b.d_nunits, b.h_nunits, size_t(n_links) * 4, cudaMemcpyHostToDevice, b.stream));
-  cudaStream_t gs = gather_stream ? gather_stream : b.stream;
-  if (gather_stream) {
-    TRY(cudaEventRecord(b.ev_up, b.stream));
-    TRY(cudaStreamWaitEvent(gs, b.ev_up, 0));
-  }
-  TRY(cudaEventRecord(b.ev_g0, gs));
-  TRY(launch_gather(b, gs));
-  TRY(cudaEventRecord(b.ev_gather, gs));
-  if (gather_stream)
-    TRY(cudaStreamWaitEvent(b.stream, b.ev_gather, 0));
+  TRY(cudaEventRecord(b.ev_up, b.stream));
+  TRY(cudaStreamWaitEvent(gather_stream, b.ev_up, 0));
+  TRY(cudaEventRecord(b.ev_g0, gather_stream));
+  TRY(launch_gather(b));
+  TRY(cudaEventRecord(b.ev_gather, gather_stream));
+  TRY(cudaStreamWaitEvent(b.stream, b.ev_gather, 0));
   TRY(cudaMemsetAsync(b.d_count, 0, sizeof(unsigned), b.stream));
   TRY(cudaStreamWaitEvent(h->stream, b.ev_gather, 0));
   TRY(cudaEventRecord(b.ev_k0, h->stream));
@@ -532,24 +491,18 @@ engine_create(swtpg_handle* h, StreamEngine** out)
   e->timeout = std::chrono::microseconds(h->cfg.dispatch_timeout_us ? h->cfg.dispatch_timeout_us : 5000u);
   e->links.reset(new LinkQ[e->n_links]);
   e->ring_ptr.reset(new const uint8_t*[size_t(e->n_links) * e->R]());
-  e->gather_mode = env_int("SWTPG_GATHER_MODE", 0);
-  e->gather_ctas = std::max(1, env_int("SWTPG_GATHER_CTAS", 64));
-  // One gather stream for all batches: their gathers run one after the other. Side by side (each on its batch's stream,
-  // SWTPG_GATHER_SERIAL=0) they share the host link worse than they use it one at a time: 45.4-46.8 against 48.2-48.8 GB/s at 240
-  // links with 3-6 slots (profiles/r02_gather_serial_probe.txt).
-  if (env_int("SWTPG_GATHER_SERIAL", 1) != 0)
-    SW_CUDA(h, cudaStreamCreateWithFlags(&e->gather_stream, cudaStreamNonBlocking));
-  if (e->gather_mode == 0) {
-    const size_t smem = size_t(kGatherStages) * e->unit_bytes + kGatherStages * 8;
-    SW_CUDA(h, cudaFuncSetAttribute(gather_units_tma<kGatherStages>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  }
+  // One gather stream for all batches: their gathers run one after the other. Side by side (each on its batch's stream) they
+  // share the host link worse than they use it one at a time: 45.4-46.8 against 48.2-48.8 GB/s at 240 links with 3-6 slots
+  // (profiles/r02_gather_serial_probe.txt).
+  SW_CUDA(h, cudaStreamCreateWithFlags(&e->gather_stream, cudaStreamNonBlocking));
+  const size_t smem = size_t(kGatherStages) * e->unit_bytes + kGatherStages * 8;
+  SW_CUDA(h, cudaFuncSetAttribute(gather_units_tma<kGatherStages>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   const size_t fbytes = size_t(e->n_links) * e->M * e->unit_bytes;
   const size_t n_items = size_t(e->n_links) * e->M;
   auto cleanup = [&]() {
     for (auto& b : e->batches)
       free_batch(*b);
-    if (e->gather_stream)
-      cudaStreamDestroy(e->gather_stream);
+    cudaStreamDestroy(e->gather_stream);
   };
   for (uint32_t i = 0; i < h->cfg.n_slots; ++i) {
     e->batches.emplace_back(new Batch);
@@ -785,8 +738,7 @@ engine_destroy(swtpg_handle* h)
   for (const auto& r : e->ranges)
     if (r.ours && cudaHostUnregister(reinterpret_cast<void*>(r.lo)) != cudaSuccess)
       cudaGetLastError();
-  if (e->gather_stream)
-    cudaStreamDestroy(e->gather_stream);
+  cudaStreamDestroy(e->gather_stream);
   delete e;
 }
 

@@ -27,9 +27,9 @@ from util import assert_same_tps
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "fdreadoutlibs_b200", "csrc")
 
-# Tuning aids change the geometry a launch takes, so under any of them the regimes asserted below are not the ones that run.
-TUNING_AIDS = ("SWTPG_PARTS", "SWTPG_WARPS", "SWTPG_SIMPLE_PIPE", "SWTPG_CTAS_PER_SM", "SWTPG_WIBETH_KERNEL", "SWTPG_SLICE_GEOM",
-               "SWTPG_FORCE_SCALAR", "SWTPG_LIB")
+# SWTPG_PARTS (the forced-slicing test hook) changes the geometry a launch takes: under it the regimes asserted below are not the
+# ones that run.
+TUNING_AIDS = ("SWTPG_PARTS",)
 
 
 def gpu(test):
@@ -43,9 +43,10 @@ HIT_MIX = (0, 1, 2, 3, 4, 5, 7, 8, 9, 15, 16, 17, 31, 32, 33, 63, 64)  # unit co
 
 
 # ---- the launch rules, restated -------------------------------------------------------------------------------------------
-# swtpg_capi.cu:100-135 (launch_wibeth_geo), :197-241 (launch_wibeth_simple, launch_wibeth), and the policies' constants
-# kWarpsPerSm / kQuadCtasPerSm (swtpg_kernels.cuh:476, 816, 979-981, 1381). test_restated_rules_match_the_source pins the
-# source lines this depends on, so the table has to be updated together with the rules.
+# swtpg_capi.cu: launch_wibeth_geo, launch_wibeth_simple, launch_wibeth, and the policies' constants kWarpsPerSm /
+# kQuadCtasPerSm (swtpg_kernels.cuh: PackedSimpleT, PackedRsWibEth, ScalarAlgo, PackedFirIqr, PackedFirIqrAnyTaps).
+# test_restated_launch_rules_match_the_source pins the source lines this depends on, so the table has to be updated together
+# with the rules.
 FULL_WARPS_PER_SM = 20   # kFullWarpsPerSm, and the running sums' 20 warps per SM above one round
 QUAD_CTAS_PER_SM = 4     # PackedFirIqr / PackedFirIqrAnyTaps::kQuadCtasPerSm
 MAX_CTAS_PER_SM = 32     # what an sm_100 SM holds at most
@@ -73,7 +74,7 @@ def expected_geometry(policy: str, n_links: int, units_stride: int, sms: int, fi
 
 
 def halving_slices(n: int, slices: int):
-    """[u0, u1) of each slice of a link with n units (SWTPG_AUTO_SLICE_GEOM = 1; tests/test_slice_arithmetic.py pins it)."""
+    """[u0, u1) of each slice of a link with n units (wibeth_kernel's slice_of; tests/test_slice_arithmetic.py pins it)."""
     out = []
     for part in range(slices):
         u0 = n - ((n + (1 << part) - 1) >> part)
@@ -82,23 +83,32 @@ def halving_slices(n: int, slices: int):
     return out
 
 
-def test_restated_rules_match_the_source():
+def test_restated_launch_rules_match_the_source():
     """CPU: the source lines `expected_geometry` restates. If one of them changes, update the restatement (and the cases)."""
     capi = re.sub(r"\s+", " ", open(os.path.join(CSRC, "swtpg_capi.cu")).read())
     kern = re.sub(r"\s+", " ", open(os.path.join(CSRC, "swtpg_kernels.cuh")).read())
-    for line in ("#define SWTPG_AUTO_SLICE_GEOM 1",
-                 "unsigned even = G::warps == 1 && per_sm >= 4 ? per_sm / 4 * 4 : per_sm;",
+    for line in ("constexpr auto k = wibeth_kernel<Algo, 1, kGeoStages, kGeoChunk, DUMP, 1>;",
+                 "unsigned even = per_sm >= 4 ? per_sm / 4 * 4 : per_sm;",
                  "even = std::min<unsigned>(even, unsigned(kWarpsPerSm));",
-                 "if (kp.n_links > persistent && (SLICE_WHOLE_ROUNDS || kp.n_links % persistent != 0))",
+                 "const unsigned grid = std::min<unsigned>(std::min<unsigned>(kp.n_links, even * sms), resident);",
+                 "if (kp.n_links > grid && (SLICE_WHOLE_ROUNDS || kp.n_links % grid != 0))",
                  "parts = std::max(1u, std::min(4u, kp.units_stride / 16u));",
+                 "kq.slice_geom = 1u; // halving slices",
                  f"constexpr int kFullWarpsPerSm = {FULL_WARPS_PER_SM};",
                  "if (kp.n_links >= unsigned(kFullWarpsPerSm * sms))",
-                 "return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, GeoDefault, kFullWarpsPerSm, true>(kp, s);",
-                 "return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, GeoDefault>(kp, s); }",
-                 f"if (kp.n_links > unsigned({FULL_WARPS_PER_SM} * sms)) return launch_wibeth_geo<Algo, DUMP, GeoDefault, {FULL_WARPS_PER_SM}, true>(kp, s);"):
+                 "return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, kFullWarpsPerSm, true>(kp, s);",
+                 "return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP>(kp, s); }",
+                 "if constexpr (std::is_same<Algo, PackedSimpleWibEth>::value) { return launch_wibeth_simple<DUMP>(kp, s); } "
+                 "else if constexpr (Algo::kQuadCtasPerSm > 0) { return launch_wibeth_quad<Algo, DUMP>(kp, s); }",
+                 f"if (kp.n_links > unsigned({FULL_WARPS_PER_SM} * sms)) return launch_wibeth_geo<Algo, DUMP, {FULL_WARPS_PER_SM}, true>(kp, s);"):
         assert line in capi, f"swtpg_capi.cu no longer has `{line}`"
     for line in ("static constexpr int kWarpsPerSm = PIPE ? 16 : 20;", "static constexpr int kWarpsPerSm = STANDARD ? 20 : 16;",
-                 "static constexpr int kWarpsPerSm = 0;", "#define SWTPG_QUAD_SIMPLE 0"):
+                 "static constexpr int kWarpsPerSm = 0;",
+                 # PackedSimpleT runs the one-warp-per-CTA form
+                 "static constexpr int kWarpsPerSm = PIPE ? 16 : 20; static constexpr int kQuadCtasPerSm = 0;",
+                 # the halving slices halving_slices restates
+                 "u0 = n - ((n + (1u << part) - 1u) >> part); "
+                 "u1 = part + 1u == (1u << p.parts_log2) ? n : n - ((n + (2u << part) - 1u) >> (part + 1u));"):
         assert line in kern, f"swtpg_kernels.cuh no longer has `{line}`"
     assert kern.count(f"static constexpr int kQuadCtasPerSm = {QUAD_CTAS_PER_SM};") == 2  # PackedFirIqr, PackedFirIqrAnyTaps
     # the restatement itself at B200's 148 SMs, for the regimes the GPU cases rely on
