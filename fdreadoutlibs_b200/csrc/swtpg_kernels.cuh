@@ -904,11 +904,14 @@ struct PackedRsWibEth : PackedSimpleWibEth
 //     6 packed adds per tick instead of 7 multiply-adds on a rotating ring, and every add wraps mod 2^16 exactly like the
 //     reference's mullo/add chain (ring homomorphism). The carried state stays the reference's ring: it is converted to
 //     cascade registers when a link is loaded and back when it is stored, which also removes the ring phase from the loop;
-//   * the three trackers keep integer accumulators biased to small non-negative numbers, and the median, q25 and q75 live as
-//     16385 - value against the biased sample Sb = S - 16384 — inside [2, 16405] for every input, so their +-1 steps cannot
-//     carry between the halves (track() lists the instructions). They replaced fp16x2-subnormal accumulators whose step flags
-//     came out of the fp16 pipe, with the two quartile trackers merged into one step or kept separate: both forms measured
-//     slower (profiles/r02_integer_accumulators.txt);
+//   * the three trackers keep integer accumulators biased to small non-negative numbers, and the median and q25 live as
+//     16385 - value against the biased sample Sb = S - 16384, inside [2, 16405] for every input. q75 can start above the
+//     14-bit range (seeded at first sample + 20, up to 16403), so 16385 - q75 reaches -18 and a +-1 step of the low half
+//     between 0xFFFF and 0x0000 would carry into the odd channel's half: its low half lives as 49153 - q75 against
+//     Sb - 0x8000 instead, inside [32750, 49152] (the high half's carry out of bit 31 is lost, so it keeps 16385 - q75).
+//     None of the +-1 steps can then carry between the halves (track() lists the instructions). They replaced fp16x2-subnormal
+//     accumulators whose step flags came out of the fp16 pipe, with the two quartile trackers merged into one step or kept
+//     separate: both forms measured slower (profiles/r02_integer_accumulators.txt);
 //   * sigma is only needed where the threshold is: the quiet test works with a lower bound of the group's sigmas taken from the
 //     quartiles after its last tick (sigma moves by at most one per tick, because at most one quartile moves), and the per-tick
 //     values are formed from the saved quartile registers only in a group that turns out busy;
@@ -923,9 +926,11 @@ struct PackedFirIqr
   static constexpr int kWib2MinCtas = 5;
   static constexpr int kQuadCtasPerSm = 4; // CTA form, 16 consumer warps per SM (measured: 4 CTAs 29.8 %, 5 CTAs 27.8 %, profiles/r02_fir_forms.txt)
                                            // (64 registers instead of 109; profiles/r01_quad_vs_warp.txt)
-  // Mq = 16385 - median, Q25n = 16385 - q25, Q75p = 16385 - q75, A = acc + 10, A25 = acc25 + 10, A75 = acc75 + 11.
+  // Mq = 16385 - median, Q25n = 16385 - q25, Q75p = {49153 - q75 (low half), 16385 - q75 (high half)}, A = acc + 10,
+  // A25 = acc25 + 10, A75 = acc75 + 11.
   uint32_t Mq, A, Q25n, A25, Q75p, A75;
   uint32_t kM1, kP1; // 0xFFFFFFFF and 1 in registers the compiler cannot see through (KernelParams::all_ones, one)
+  static constexpr uint32_t kQ75Bias = 0x4002C002u; // ~q75 + {49154, 16386} = Q75p, and back
   uint32_t d1, d2, d3, d4, d5, d6, o1, o2; // cascade: d_j = previous input of stage j, o1/o2 = previous two outputs
   uint32_t prev, C, Tn;
   uint32_t xmax, sig3max, K, Kneg3, shift, shmask, thr_cfg, mult;
@@ -986,7 +991,7 @@ struct PackedFirIqr
     Mq = add2(~st[SV_MEDIAN * 32 + lane], 0x40024002u);       // ~m = -m - 1
     Q25n = add2(~st[SV_Q25 * 32 + lane], 0x40024002u);
     A = add2(st[SV_ACCUM * 32 + lane], 0x000A000Au);
-    Q75p = add2(~st[SV_Q75 * 32 + lane], 0x40024002u);
+    Q75p = add2(~st[SV_Q75 * 32 + lane], kQ75Bias);
     A25 = add2(st[SV_A25 * 32 + lane], 0x000A000Au);
     A75 = add2(st[SV_A75 * 32 + lane], 0x000B000Bu);
     prev = st[SV_PREV * 32 + lane];
@@ -998,7 +1003,7 @@ struct PackedFirIqr
     st[SV_MEDIAN * 32 + lane] = median();
     st[SV_Q25 * 32 + lane] = add2(~Q25n, 0x40024002u);
     st[SV_ACCUM * 32 + lane] = add2(A, 0xFFF6FFF6u);
-    st[SV_Q75 * 32 + lane] = add2(~Q75p, 0x40024002u);
+    st[SV_Q75 * 32 + lane] = add2(~Q75p, kQ75Bias);
     st[SV_A25 * 32 + lane] = add2(A25, 0xFFF6FFF6u);
     st[SV_A75 * 32 + lane] = add2(A75, 0xFFF5FFF5u);
     st[SV_PREV * 32 + lane] = prev;
@@ -1049,7 +1054,7 @@ struct PackedFirIqr
   {
     Mq = add2(~Sb, 0x00020002u);               // 16385 - ped = 1 - Sb
     Q25n = add2(~Sb, 0x00160016u);             // 16385 - (ped - 20)
-    Q75p = add2(~Sb, 0xFFEEFFEEu);             // 16385 - (ped + 20)
+    Q75p = add2(~Sb, 0xFFEE7FEEu);             // {49153, 16385} - (ped + 20)
   }
 
   // The three frugal trackers of one tick (Sb = raw - 16384). Returns 16385 - median, updated: see sp1_of / clamped_sample.
@@ -1063,10 +1068,12 @@ struct PackedFirIqr
   //     Q = Q - D                             16385 - quantile follows                                     IADD3
   // D is a "true integer" d_hi * 65536 + d_lo whose low half may be negative (its bit pattern then borrows from the high half);
   // that is harmless because only LINEAR 32-bit operations consume it and every result they produce has non-negative halves
-  // again, for which the 32-bit value and the packed value coincide. The quartile enables (:119-121: sample below / above the OLD
-  // median) cost no select: the clamp's upper bound is 2 on the enabled halves and 0 elsewhere, which turns the sign code into 0
-  // there, and the missing +1 comes from n1 (q25, "+10" form) or is taken back out by g1 (q75, "+11" form).
-  // Per tick: 8 ALU-pipe instructions (sign tests, clamps, enables), 3-4 on the FMA pipe, 10 adds that go to whichever is free
+  // again, for which the 32-bit value and the packed value coincide — provided Q's low half stays clear of 0xFFFF / 0x0000, which
+  // is why q75's low half has its own bias (Q75p) and meets the sample as Sb - 0x8000 (one more IMAD per tick). The quartile
+  // enables (:119-121: sample below / above the OLD median) cost no select: the clamp's upper bound is 2 on the enabled halves and
+  // 0 elsewhere, which turns the sign code into 0 there, and the missing +1 comes from n1 (q25, "+10" form) or is taken back out
+  // by g1 (q75, "+11" form).
+  // Per tick: 8 ALU-pipe instructions (sign tests, clamps, enables), 4-5 on the FMA pipe, 10 adds that go to whichever is free
   // — against 13 / 8 / 2 for the fp16-subnormal form with merged quartile trackers and 9 / 14 / 3 with separate ones. The
   // three-input adds stay IADD3s: as two IMADs each on the FMA pipe they gained nothing (profiles/r02_fma_steering_probe.txt, u3).
   __device__ __forceinline__ uint32_t track(uint32_t Sb)
@@ -1082,7 +1089,8 @@ struct PackedFirIqr
     Q25n = fma_sub(Q25n, D25, kM1);
     // q75 on the halves above it (:121)
     const uint32_t g1 = __viaddmax_s16x2_relu(sg1, kM1, 0u);          // 1 where above, 0 elsewhere
-    const uint32_t s75 = addclamp2(Sb, Q75p, fma_add(g1, g1, kP1));  // bound 2 g1: sign(raw - q75) + 1 where enabled, else 0
+    const uint32_t Sb75 = fma_add(Sb, 0xFFFF8000u, kP1);             // low half S - 49152 (0xC000 | S - 0x8000: no borrow)
+    const uint32_t s75 = addclamp2(Sb75, Q75p, fma_add(g1, g1, kP1)); // bound 2 g1: sign(raw - q75) + 1 where enabled, else 0
     const uint32_t U75 = A75 + s75 - g1;                              // acc75' + 11
     const uint32_t c75 = addclamp2(U75, kM1, 0x00140014u);
     const uint32_t D75 = U75 - c75 - 0x00010001u;
@@ -1099,7 +1107,7 @@ struct PackedFirIqr
   // min(q75 - q25, sigmaMax) + 3 (:131-134) from a pair of quartile registers (Q75p, Q25n)
   __device__ __forceinline__ uint32_t sig3_of(uint32_t q75p, uint32_t q25n) const
   {
-    return addmin2(add2(~q75p, 0x00040004u), q25n, sig3max);          // -(16385 - q75) + 3 = ~Q75p + 4 per half
+    return addmin2(add2(~q75p, 0x00048004u), q25n, sig3max);          // -(16385 - q75) + 3 = ~Q75p + {32772, 4}
   }
   // One tick: returns the filter output of this tick.
   // s' + 1 = raw - median + 1 from what track() returns
