@@ -16,12 +16,9 @@ from fdreadoutlibs_b200 import _lib
 from fdreadoutlibs_b200 import api as A
 from fdreadoutlibs_b200 import frames as F
 from fdreadoutlibs_b200 import hostshim as H
-from test_gpu_link_config import all_wibeth_policies
-from test_gpu_launch_geometry import ragged_units, sms
-from test_host_shim import linear_map
+from util import all_wibeth_policies, channels, create_status, linear_map, ragged_units, run_device, sms
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-gpu = pytest.mark.gpu
 
 
 # ---- CPU --------------------------------------------------------------------------------------------------------------------------
@@ -46,34 +43,14 @@ def test_read_adc_stats_without_handle():
     assert _lib.lib.swtpg_read_adc_stats(None, 0, 1, out.ctypes.data, 0) == _lib.SWTPG_ERR_INVALID_ARG
 
 
-def create_status(flags):
-    cfg = _lib.SwtpgConfig()
-    cfg.struct_size = C.sizeof(cfg)
-    cfg.n_links, cfg.max_units, cfg.threshold, cfg.frugal_acc_limit = 2, 4, 60, 10
-    cfg.flags = flags
-    h = C.c_void_p()
-    st = _lib.lib.swtpg_create(C.byref(cfg), C.byref(h))
-    if h:
-        _lib.lib.swtpg_destroy(h)
-    return st
-
-
 def test_create_accepts_the_flag_and_still_refuses_unknown_bits():
     """Flag bit 2 passes validation (no device here: SWTPG_ERR_CUDA; on a GPU: a handle); bit 4 is still unknown."""
-    assert create_status(A.FLAG_ADC_STATS) in (_lib.SWTPG_OK, _lib.SWTPG_ERR_CUDA)
-    assert create_status(A.FLAG_ADC_STATS | A.FLAG_SORTED_TPS) in (_lib.SWTPG_OK, _lib.SWTPG_ERR_CUDA)
-    assert create_status(4) == _lib.SWTPG_ERR_INVALID_ARG
+    assert create_status(flags=A.FLAG_ADC_STATS) in (_lib.SWTPG_OK, _lib.SWTPG_ERR_CUDA)
+    assert create_status(flags=A.FLAG_ADC_STATS | A.FLAG_SORTED_TPS) in (_lib.SWTPG_OK, _lib.SWTPG_ERR_CUDA)
+    assert create_status(flags=4) == _lib.SWTPG_ERR_INVALID_ARG
 
 
 # ---- expected values --------------------------------------------------------------------------------------------------------------
-def channels(fmt):
-    return F.WIB2_CHANNELS if fmt == "wib2" else F.WIBETH_CHANNELS
-
-
-def unit_bytes(fmt):
-    return F.WIB2_SUPERCHUNK_BYTES if fmt == "wib2" else F.WIBETH_FRAME_BYTES
-
-
 def adc_of(fmt, units, adc_offset=F.WIB2_ADC_OFFSET):
     """(samples, channels) raw ADC values of a link's units."""
     if len(units) == 0:
@@ -138,7 +115,7 @@ def ragged_batch(fmt, seed, n_links, stride, nu, **gen_kw):
 
 
 # ---- batch entry points -----------------------------------------------------------------------------------------------------------
-@gpu
+@pytest.mark.gpu
 @pytest.mark.parametrize("fmt,adc_offset", [("wibeth", 0), ("wib2", 0), ("wib2", 24)])
 def test_ragged_batches(fmt, adc_offset):
     """Three ragged batches (links of 0, 1 and units_stride units) through process_host and process_host_debug. WIB2 also runs
@@ -161,7 +138,7 @@ def test_ragged_batches(fmt, adc_offset):
         assert_stats(g.read_adc_stats(), want, f"{fmt} ragged batches")
 
 
-@gpu
+@pytest.mark.gpu
 def test_constant_noisy_and_saturated_channels():
     """Channels stuck at 0 and at 16383, a channel spanning the whole range, the rest Gaussian noise around a pedestal."""
     rng = np.random.default_rng(510)
@@ -180,7 +157,7 @@ def test_constant_noisy_and_saturated_channels():
     assert (got["min"][:, 6] == 16383).all() and (got["max"][:, 6] == 16383).all()
 
 
-@gpu
+@pytest.mark.gpu
 def test_sums_of_squares_beyond_32_bits():
     """One batch of 4096 saturated frames (every ADC bit set): a channel's sum of squares passes 2^32 within every work item."""
     n, stride = 2, 4096
@@ -196,7 +173,7 @@ def test_sums_of_squares_beyond_32_bits():
     assert (got["min"] == 16383).all() and (got["max"] == 16383).all()
 
 
-@gpu
+@pytest.mark.gpu
 def test_each_link_counted_once_with_several_configuration_groups():
     """A handle with every WIBEth policy (six configuration groups, six launches per batch) counts each link once: its statistics
     equal a uniform handle's over the same frames, and the numpy values."""
@@ -220,7 +197,7 @@ def test_each_link_counted_once_with_several_configuration_groups():
 
 
 # ---- windows ----------------------------------------------------------------------------------------------------------------------
-@gpu
+@pytest.mark.gpu
 def test_windows():
     n, stride = 12, 4
     frames = [ragged_batch("wibeth", 530 + k, n, stride, np.full(n, stride)) for k in range(4)]
@@ -266,7 +243,7 @@ def test_windows():
         assert e.value.status == _lib.SWTPG_ERR_STATE
 
 
-@gpu
+@pytest.mark.gpu
 def test_process_device_on_a_torch_stream():
     """A read straight after swtpg_process_device on a caller stream, with no host synchronisation, includes that batch; a reset
     read there ends the window exactly at that batch."""
@@ -291,7 +268,7 @@ def test_process_device_on_a_torch_stream():
 
 
 # ---- streaming path ---------------------------------------------------------------------------------------------------------------
-@gpu
+@pytest.mark.gpu
 def test_streaming_path_with_a_concurrent_reader():
     """Units of 24 links, half zero-copy from a registered buffer and half staged, while a second thread reads with reset in a
     loop. TPs are polled as batches complete (un-polled batches back-pressure the rings). After drain() and a final read the
@@ -332,7 +309,7 @@ def test_streaming_path_with_a_concurrent_reader():
 
 
 # ---- full load --------------------------------------------------------------------------------------------------------------------
-@gpu
+@pytest.mark.gpu
 def test_full_load():
     """20 links per SM, 64 frames each, generated on the device; the statistics of a seeded sample of 64 links match numpy."""
     import torch
@@ -357,30 +334,7 @@ def test_full_load():
 
 
 # ---- the flag changes nothing else ------------------------------------------------------------------------------------------------
-def run_mixed(adc_stats, n, stride, nus, p, link_kw):
-    import torch
-
-    buf = torch.empty(n * stride * F.WIBETH_FRAME_BYTES, dtype=torch.uint8, device="cuda")
-    tps = []
-    try:
-        with S.TPGenerator(n, stride, tp_capacity=1 << 24, adc_stats=adc_stats) as g:
-            for l, kw in link_kw.items():
-                g.set_link_config(l, **kw)
-            g.start()
-            for k, nu in enumerate(nus):
-                S.gen_wibeth_device(p, buf.data_ptr(), n, stride, unit0=k * stride)
-                torch.cuda.synchronize()
-                g.process_device(buf.data_ptr(), stride, n_units=nu)
-                tps.append(F.sort_tps(g.fetch_tps(cap=1 << 24)))
-            state = np.stack([g.dump_state(l) for l in range(0, n, 7)])
-            counters = g.counters()
-    finally:
-        del buf
-        torch.cuda.empty_cache()
-    return tps, state, counters
-
-
-@gpu
+@pytest.mark.gpu
 def test_flag_changes_nothing_else_at_production_geometry():
     """A mixed SimpleThreshold / AbsRS / StandardRS handle at 20 warps per SM, ragged then full: TP lists, carried state and
     counters are bit-identical with the flag off and on."""
@@ -390,15 +344,15 @@ def test_flag_changes_nothing_else_at_production_geometry():
     link_kw = {l: kinds[l % 3] for l in range(n)}
     nus = [ragged_units(570, n, stride, (0, 1, 16, 63, 64)), None]
     p = S.gen_params(570, 0.1)
-    off = run_mixed(False, n, stride, nus, p, link_kw)
-    on = run_mixed(True, n, stride, nus, p, link_kw)
+    off = run_device("wibeth", n, stride, nus, p, link_kw=link_kw, adc_stats=False)
+    on = run_device("wibeth", n, stride, nus, p, link_kw=link_kw, adc_stats=True)
     for a, b in zip(off[0], on[0]):
-        assert a.size > 10000 and np.array_equal(a, b)
+        assert a.size > 10000 and np.array_equal(F.sort_tps(a), F.sort_tps(b))
     assert np.array_equal(off[1], on[1])
     assert off[2] == on[2]
 
 
-@gpu
+@pytest.mark.gpu
 def test_flag_changes_nothing_else_on_the_streaming_path():
     n, n_units = 16, 24
     units = S.gen_wibeth_host(S.gen_params(580, 0.3), n, n_units)
@@ -423,10 +377,7 @@ def reversed_map(crate, slot, stream, chan):
     return ((crate * 8 + slot) * 64 + stream) * 64 + (63 - chan)
 
 
-PERM = [0, 1, 2, 3, 4, 5, 6, 7, 15, 8, 9, 10, 11, 12, 13, 14]
-
-
-@gpu
+@pytest.mark.gpu
 @pytest.mark.parametrize("reversed_", [False, True])
 @pytest.mark.parametrize("correct", [False, True])
 def test_frame_processors_report_by_offline_channel(reversed_, correct):
@@ -449,7 +400,7 @@ def test_frame_processors_report_by_offline_channel(reversed_, correct):
     for l in range(n_links):
         cr, sl, st = crate, slot, stream + l  # emulator mode writes the configured ids into every header
         offline = [m(cr, sl, st, c) if correct else int(maps[l][c]) for c in range(64)]
-        assert [m(cr, sl, st, 16 * (p // 16) + PERM[p % 16]) for p in range(64)] == maps[l].tolist()
+        assert [m(cr, sl, st, int(F.position_to_channel(p))) for p in range(64)] == maps[l].tolist()
         a = adc_of("wibeth", units[l]).astype(np.float64)
         g = got[l]
         assert g.size == 64 and g["offline_channel"].tolist() == offline

@@ -5,8 +5,6 @@ The reference has one tpg_threshold per frame processor. Channels are independen
 with a table is, channel by channel, the uniform oracle run with that channel's threshold (TableOracle). Every link the GPU ran
 is compared with it: TPs and carried state."""
 import ctypes as C
-import os
-from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 import pytest
@@ -15,20 +13,13 @@ import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import _lib
 from fdreadoutlibs_b200 import frames as F
 from fdreadoutlibs_b200 import hostshim as H
-from oracle import binding as B
-from test_gpu_launch_geometry import HIT_MIX, expected_geometry, ragged_units
-from test_gpu_link_config import HANDLE, assert_links_match, full_conf, gpu, host_batches, oracle_for
-from test_host_shim import linear_map
-from util import assert_same_tps
+from util import (HANDLE, HIT_MIX, assert_links_match, assert_same_tps, channels, check, dump_states, expected_geometry, full_conf, gpu,
+                  host_batches, linear_map, link_config, oracle_for, ragged_units, replay_batches, replay_oracles, run_device, run_host, sms)
 
 # (format, algorithm, handle keyword arguments) of every algorithm a table applies to
 IN_SCOPE = [("wibeth", "SimpleThreshold", {}), ("wibeth", "AbsRS", dict(rs_memory_factor=7, rs_scale_factor=2)),
             ("wibeth", "StandardRS", dict(rs_memory_factor=6)), ("wib2", "SimpleThreshold", {})]
 EDGES = (0, 1, 16383, 16384, 32767)  # never exceeded from 16383 (SimpleThreshold) or 6555 (running sums) on
-
-
-def channels(fmt):
-    return 256 if fmt == "wib2" else 64
 
 
 def table(seed, fmt, lo=15, hi=80, edges=EDGES, values=None):
@@ -67,43 +58,15 @@ class TableOracle:
         return out
 
 
+def table_oracles(fmt, handle, link_kw, tables):
+    """oracle_of(link) for links configured by link_kw, with the thresholds of tables {link: table}."""
+    return lambda l: TableOracle(fmt, full_conf(handle, link_kw.get(l, {})), l, tables.get(l))
+
+
 def test_set_link_thresholds_without_handle():
     t = np.zeros(64, dtype=np.uint16)
     assert _lib.lib.swtpg_set_link_thresholds(None, 0, t.ctypes.data) == _lib.SWTPG_ERR_INVALID_ARG
     assert _lib.lib.swtpg_set_link_thresholds(None, 0, None) == _lib.SWTPG_ERR_INVALID_ARG
-
-
-# ---- harness ----------------------------------------------------------------------------------------------------------------------
-def run_handle(fmt, handle, link_kw, batches, tables, **gkw):
-    """The batches through one handle (process_host): links configured by link_kw, thresholds by tables {link: table}, both set
-    before start. Returns (TPs of all batches, per-link state)."""
-    n_links, stride = batches[0][0].shape[:2]
-    with S.TPGenerator(n_links, stride, fmt=fmt, **handle, **gkw) as g:
-        for l, kw in link_kw.items():
-            g.set_link_config(l, **kw)
-        for l, t in tables.items():
-            g.set_link_thresholds(l, t)
-        g.start()
-        got = np.concatenate([g.process_host(u, n_units=nu, cap=1 << 22) for u, nu in batches])
-        states = np.stack([g.dump_state(l) for l in range(n_links)])
-    return got, states
-
-
-def oracles_for(fmt, handle, link_kw, tables, n_links):
-    return [TableOracle(fmt, full_conf(handle, link_kw.get(l, {})), l, tables.get(l)) for l in range(n_links)]
-
-
-def run_oracles(fmt, handle, link_kw, batches, tables):
-    oracles = oracles_for(fmt, handle, link_kw, tables, batches[0][0].shape[0])
-    want = np.concatenate([B.oracle_process_links(None, u, nu, oracles=oracles)[0] for u, nu in batches])
-    return want, np.stack([o.state() for o in oracles])
-
-
-def check(what, fmt, handle, link_kw, batches, tables, min_tps=1):
-    got, gstate = run_handle(fmt, handle, link_kw, batches, tables)
-    want, ostate = run_oracles(fmt, handle, link_kw, batches, tables)
-    assert_links_match(what, fmt, handle, link_kw, got, gstate, want, ostate, min_tps)
-    return got, gstate
 
 
 # ---- every policy against the oracle ----------------------------------------------------------------------------------------------
@@ -117,7 +80,8 @@ def test_packed_policies_with_tables(fmt, algorithm, kw):
     handle = dict(algorithm=algorithm, threshold=40, **kw)
     tables = {l: table(310 + l, fmt) for l in range(n) if l % 3}
     nus = [ragged_units(310 + k, n, stride, (0, 1, stride)) for k in range(3)]
-    check(f"{fmt} {algorithm}", fmt, handle, {}, host_batches(fmt, 310, 0.3, n, stride, nus), tables, min_tps=1000)
+    check(f"{fmt} {algorithm}", fmt, handle, host_batches(fmt, 310, 0.3, n, stride, nus), thresholds=tables,
+          oracle_of=table_oracles(fmt, handle, {}, tables), min_tps=1000)
 
 
 # acc_limit 0 or 1001 and a WIB2 threshold above 32767 are outside the packed policies' validity ranges: ScalarAlgo runs
@@ -134,7 +98,8 @@ def test_scalar_fallbacks_with_tables(fmt, algorithm, kw):
     handle = dict(algorithm=algorithm, **{"threshold": 40, **kw})
     tables = {l: table(320 + l, fmt) for l in range(n) if l % 3}
     nus = [ragged_units(320 + k, n, stride, (0, 1, stride)) for k in range(3)]
-    check(f"scalar {fmt} {algorithm}", fmt, handle, {}, host_batches(fmt, 320, 0.3, n, stride, nus), tables, min_tps=500)
+    check(f"scalar {fmt} {algorithm}", fmt, handle, host_batches(fmt, 320, 0.3, n, stride, nus), thresholds=tables,
+          oracle_of=table_oracles(fmt, handle, {}, tables), min_tps=500)
 
 
 @gpu
@@ -143,71 +108,23 @@ def test_all_equal_table_is_bit_identical_to_no_table(fmt, algorithm, kw):
     n, stride = (8, 8) if fmt == "wib2" else (16, 16)
     nus = [ragged_units(330 + k, n, stride, (0, 1, stride)) for k in range(2)]
     batches = host_batches(fmt, 330, 0.3, n, stride, nus)
-    want_tps, want_state = run_handle(fmt, dict(algorithm=algorithm, threshold=35, **kw), {}, batches, {})
-    got_tps, got_state = run_handle(fmt, dict(algorithm=algorithm, threshold=70, **kw), {}, batches,
-                                    {l: np.full(channels(fmt), 35, dtype=np.uint16) for l in range(n)})
+    want_tps, want_state = run_host(fmt, dict(algorithm=algorithm, threshold=35, **kw), batches)
+    got_tps, got_state = run_host(fmt, dict(algorithm=algorithm, threshold=70, **kw), batches,
+                                  thresholds={l: np.full(channels(fmt), 35, dtype=np.uint16) for l in range(n)})
     assert want_tps.size > 100
     assert_same_tps(got_tps, want_tps, "all-equal tables")
     assert (got_state == want_state).all()
 
 
 # ---- production geometry ----------------------------------------------------------------------------------------------------------
-def run_device(fmt, n, stride, nus, p, link_kw, tables, tp_capacity=1 << 24, **handle):
-    """Launches of one handle on device-generated frames (launch k reads units [k stride, (k+1) stride)): (TPs, per-link state)."""
-    import torch
-
-    unit_bytes = F.WIB2_SUPERCHUNK_BYTES if fmt == "wib2" else F.WIBETH_FRAME_BYTES
-    gen = S.gen_wib2_device if fmt == "wib2" else S.gen_wibeth_device
-    buf = torch.empty(n * stride * unit_bytes, dtype=torch.uint8, device="cuda")
-    got = []
-    try:
-        with S.TPGenerator(n, stride, fmt=fmt, tp_capacity=tp_capacity, **handle) as g:
-            for l, kw in link_kw.items():
-                g.set_link_config(l, **kw)
-            for l, t in tables.items():
-                g.set_link_thresholds(l, t)
-            g.start()
-            for k, nu in enumerate(nus):
-                gen(p, buf.data_ptr(), n, stride, unit0=k * stride)
-                torch.cuda.synchronize()
-                g.process_device(buf.data_ptr(), stride, n_units=nu)
-                got.append(g.fetch_tps(cap=tp_capacity))
-            gstate = np.stack([g.dump_state(l) for l in range(n)])
-            assert g.counters()["units_processed"] == sum(n * stride if nu is None else int(nu.sum()) for nu in nus)
-    finally:
-        del buf
-        torch.cuda.empty_cache()
-    return np.concatenate(got), gstate
-
-
-def run_device_oracles(fmt, n, stride, nus, p, handle, link_kw, tables):
-    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
-
-    def one(l):
-        o = TableOracle(fmt, full_conf(handle, link_kw.get(l, {})), l, tables.get(l))
-        parts = [np.zeros(0, dtype=F.TP_DTYPE)]
-        for k, nu in enumerate(nus):
-            m = stride if nu is None else int(nu[l])
-            if m:
-                parts.append(o.process(gen(p, 1, m, link0=l, unit0=k * stride, n_threads=1)[0], cap=1 << 18))
-        return np.concatenate(parts), o.state()
-
-    with ThreadPoolExecutor(os.cpu_count() or 1) as ex:
-        res = list(ex.map(one, range(n)))
-    return np.concatenate([r[0] for r in res]), np.stack([r[1] for r in res])
-
-
 @gpu
 def test_mixed_handle_at_production_geometry():
     """SimpleThreshold, AbsRS and StandardRS groups in one handle, each sized from the SM count into the 20-warps-per-SM sliced
     regime, links of the three interleaved; two thirds of the links have tables (drawn from a few, so that neighbouring links of
     a group differ). Ragged unit counts around every slice edge, then a full launch: state carried across slices and launches."""
-    import torch
-
-    sms = torch.cuda.get_device_properties(0).multi_processor_count
-    per = 20 * sms + 1
+    per = 20 * sms() + 1
     for algo in ("SimpleThreshold", "AbsRS", "StandardRS"):
-        assert expected_geometry(algo, per, 64, sms) == (20, 4)
+        assert expected_geometry(algo, per, 64, sms()) == (20, 4)
     n = 3 * per
     rng = np.random.default_rng(340)
     kinds = np.array([0] * per + [1] * per + [2] * per)
@@ -219,26 +136,26 @@ def test_mixed_handle_at_production_geometry():
     stride = 64
     nus = [ragged_units(340, n, stride, HIT_MIX), None]
     p = S.gen_params(340, 0.1)
-    got, gstate = run_device("wibeth", n, stride, nus, p, link_kw, tables)
-    want, ostate = run_device_oracles("wibeth", n, stride, nus, p, {}, link_kw, tables)
-    assert_links_match("mixed production geometry", "wibeth", {}, link_kw, got, gstate, want, ostate, min_tps=100000)
+    got, gstate, _ = run_device("wibeth", n, stride, nus, p, link_kw=link_kw, thresholds=tables)
+    want, ostate = replay_oracles("wibeth", n, stride, nus, p, table_oracles("wibeth", {}, link_kw, tables))
+    assert_links_match("mixed production geometry", "wibeth", {}, link_kw, np.concatenate(got), gstate, np.concatenate(want), ostate,
+                       min_tps=100000)
 
 
 @gpu
 def test_wib2_ctas_take_several_links_with_tables():
     """WIB2 SimpleThreshold with 20 x SMs links, so every persistent CTA takes several links; each of a link's four channel
     groups reads its own row of the link's table."""
-    import torch
-
-    n = 20 * torch.cuda.get_device_properties(0).multi_processor_count
+    n = 20 * sms()
     rng = np.random.default_rng(350)
     pool = [table(350 + i, "wib2", edges=(1, 32767), values=(25, 45, 65)) for i in range(5)]
     tables = {l: pool[int(rng.integers(len(pool)))] for l in range(n) if l % 4}
     nus = [ragged_units(350 + k, n, 16, (0, 1, 16)) for k in range(2)]
     p = S.gen_params(350, 0.3)
-    got, gstate = run_device("wib2", n, 16, nus, p, {}, tables, threshold=60)
-    want, ostate = run_device_oracles("wib2", n, 16, nus, p, dict(threshold=60), {}, tables)
-    assert_links_match("WIB2 several links per CTA", "wib2", dict(threshold=60), {}, got, gstate, want, ostate, min_tps=10000)
+    got, gstate, _ = run_device("wib2", n, 16, nus, p, thresholds=tables, threshold=60)
+    want, ostate = replay_oracles("wib2", n, 16, nus, p, table_oracles("wib2", dict(threshold=60), {}, tables))
+    assert_links_match("WIB2 several links per CTA", "wib2", dict(threshold=60), {}, np.concatenate(got), gstate, np.concatenate(want),
+                       ostate, min_tps=10000)
 
 
 # ---- streaming path -----------------------------------------------------------------------------------------------------------------
@@ -248,7 +165,7 @@ def test_streaming_path_with_tables():
     link_kw = {l: [dict(threshold=30), dict(algorithm="AbsRS", threshold=30)][l % 2] for l in range(n)}
     tables = {l: table(360 + l, "wibeth") for l in range(n) if l != 3}
     units = S.gen_wibeth_host(S.gen_params(360, 0.3), n, n_units)
-    want, _ = run_oracles("wibeth", {}, link_kw, [(units, None)], tables)
+    want, _ = replay_batches([(units, None)], table_oracles("wibeth", {}, link_kw, tables))
     with S.TPGenerator(n, 4, sorted_tps=True) as g:
         for l, kw in link_kw.items():
             g.set_link_config(l, **kw)
@@ -264,18 +181,13 @@ def test_streaming_path_with_tables():
 
 
 # ---- call rules -----------------------------------------------------------------------------------------------------------------------
-def raw_set(g, link, t):
+def raw_thresholds(g, link, t):
     a = None if t is None else np.ascontiguousarray(t, dtype=np.uint16)
     return _lib.lib.swtpg_set_link_thresholds(g._h, link, None if a is None else a.ctypes.data)
 
 
 def raw_config(g, link, **kw):
-    c = _lib.SwtpgLinkConfig()
-    c.struct_size = C.sizeof(c)
-    c.algorithm, c.threshold, c.frugal_acc_limit, c.rs_memory_factor, c.rs_scale_factor = 0, 60, 10, 8, 5
-    for k, v in kw.items():
-        setattr(c, k, v)
-    return _lib.lib.swtpg_set_link_config(g._h, link, C.byref(c))
+    return _lib.lib.swtpg_set_link_config(g._h, link, C.byref(link_config(**kw)))
 
 
 @gpu
@@ -283,32 +195,32 @@ def test_call_rules():
     n = 4
     t = table(370, "wibeth")
     with S.TPGenerator(n, 4) as g:
-        assert raw_set(g, n, t) == _lib.SWTPG_ERR_INVALID_ARG  # link out of range
-        assert raw_set(g, n, None) == _lib.SWTPG_ERR_INVALID_ARG
+        assert raw_thresholds(g, n, t) == _lib.SWTPG_ERR_INVALID_ARG  # link out of range
+        assert raw_thresholds(g, n, None) == _lib.SWTPG_ERR_INVALID_ARG
         bad = t.copy()
         bad[17] = 32768
-        assert raw_set(g, 0, bad) == _lib.SWTPG_ERR_INVALID_ARG  # above 32767
+        assert raw_thresholds(g, 0, bad) == _lib.SWTPG_ERR_INVALID_ARG  # above 32767
         assert raw_config(g, 1, algorithm=_lib.ALGO_FIR_IQR, threshold=5) == _lib.SWTPG_OK
-        assert raw_set(g, 1, t) == _lib.SWTPG_ERR_UNSUPPORTED  # FIR + IQR: the threshold multiplies a sigma
-        assert raw_set(g, 1, None) == _lib.SWTPG_OK            # clearing is always accepted
-        assert raw_set(g, 0, t) == _lib.SWTPG_OK
+        assert raw_thresholds(g, 1, t) == _lib.SWTPG_ERR_UNSUPPORTED  # FIR + IQR: the threshold multiplies a sigma
+        assert raw_thresholds(g, 1, None) == _lib.SWTPG_OK            # clearing is always accepted
+        assert raw_thresholds(g, 0, t) == _lib.SWTPG_OK
         assert raw_config(g, 0, algorithm=_lib.ALGO_FIR_IQR, threshold=5) == _lib.SWTPG_ERR_UNSUPPORTED  # a link with a table
         assert raw_config(g, 0, algorithm=_lib.ALGO_ABS_RS, threshold=5) == _lib.SWTPG_OK                # ... may change otherwise
         g.start()
-        assert raw_set(g, 2, t) == _lib.SWTPG_ERR_STATE
-        assert raw_set(g, 0, None) == _lib.SWTPG_ERR_STATE
+        assert raw_thresholds(g, 2, t) == _lib.SWTPG_ERR_STATE
+        assert raw_thresholds(g, 0, None) == _lib.SWTPG_ERR_STATE
         g.stop()
-        assert raw_set(g, 2, t) == _lib.SWTPG_OK
+        assert raw_thresholds(g, 2, t) == _lib.SWTPG_OK
     with S.TPGenerator(2, 4, algorithm="FIR", threshold=5) as g:
-        assert raw_set(g, 0, t) == _lib.SWTPG_ERR_UNSUPPORTED
+        assert raw_thresholds(g, 0, t) == _lib.SWTPG_ERR_UNSUPPORTED
         assert raw_config(g, 0, algorithm=_lib.ALGO_SIMPLE_THRESHOLD, threshold=30) == _lib.SWTPG_OK
-        assert raw_set(g, 0, t) == _lib.SWTPG_OK
+        assert raw_thresholds(g, 0, t) == _lib.SWTPG_OK
         assert _lib.lib.swtpg_set_link_config(g._h, 0, None) == _lib.SWTPG_ERR_UNSUPPORTED  # back to the handle's FIR + IQR
     t2 = table(371, "wib2")
     with S.TPGenerator(2, 4, fmt="wib2") as g:
         assert raw_config(g, 0, algorithm=_lib.ALGO_ABS_RS, threshold=20) == _lib.SWTPG_OK
-        assert raw_set(g, 0, t2) == _lib.SWTPG_ERR_UNSUPPORTED  # WIB2 AbsRS: sigma units too
-        assert raw_set(g, 1, t2) == _lib.SWTPG_OK
+        assert raw_thresholds(g, 0, t2) == _lib.SWTPG_ERR_UNSUPPORTED  # WIB2 AbsRS: sigma units too
+        assert raw_thresholds(g, 1, t2) == _lib.SWTPG_OK
         assert raw_config(g, 1, algorithm=_lib.ALGO_ABS_RS, threshold=20) == _lib.SWTPG_ERR_UNSUPPORTED
 
 
@@ -329,19 +241,19 @@ def test_tables_persist_and_refused_calls_change_nothing():
         # refused: a table above 32767 on link 4, link 1 with a table moved to FIR + IQR
         bad = t[4].copy()
         bad[0] = 40000
-        assert raw_set(g, 4, bad) == _lib.SWTPG_ERR_INVALID_ARG
+        assert raw_thresholds(g, 4, bad) == _lib.SWTPG_ERR_INVALID_ARG
         assert raw_config(g, 1, algorithm=_lib.ALGO_FIR_IQR, threshold=5) == _lib.SWTPG_ERR_UNSUPPORTED
         g.set_link_config(0, algorithm="AbsRS", threshold=25)  # the table stays and takes precedence over 25
         g.set_link_thresholds(2, None)                         # back to the configuration's 40
         g.start()
         run2 = g.process_host(batches[0][0])
-        state2 = np.stack([g.dump_state(l) for l in range(n)])
+        state2 = dump_states(g)
     first = {l: t[l] for l in (0, 1, 2, 3)}
-    want1, _ = run_oracles("wibeth", handle, {}, batches, first)
+    want1, _ = replay_batches(batches, table_oracles("wibeth", handle, {}, first))
     assert_same_tps(run1, want1, "first run")
     link_kw = {0: dict(algorithm="AbsRS", threshold=25)}
     second = {l: t[l] for l in (0, 1, 3)}
-    want2, ostate2 = run_oracles("wibeth", handle, link_kw, batches, second)
+    want2, ostate2 = replay_batches(batches, table_oracles("wibeth", handle, link_kw, second))
     assert_links_match("after stop / start", "wibeth", handle, link_kw, run2, state2, want2, ostate2, min_tps=100)
 
 

@@ -24,7 +24,7 @@ import pytest
 import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import frames as F
 from oracle import binding as B
-from util import assert_same_tps
+from util import assert_same_state, assert_same_tps, channels, dump_states, ticks_per_unit
 
 TS0 = 1 << 40
 ANY_TAPS = [-3, 7, 20, 31, 20, 7, -3]  # test_gpu_parity.py ANY_TAPS[1]: PackedFirIqrAnyTaps
@@ -46,14 +46,6 @@ WIB2 = [p for p, (f, _) in POLICIES.items() if f == "wib2"]
 ALL = ETH + WIB2
 QUARTILES = ["eth_fir", "eth_fir_any", "wib2_fir", "wib2_absrs"]  # the policies that run PackedFirIqr::track()
 WITH_ACC_LIMIT = ("eth_simple", "eth_absrs", "eth_stdrs")
-
-
-def ticks_per_unit(fmt):
-    return F.WIB2_SUPERCHUNK_FRAMES if fmt == "wib2" else F.WIBETH_TICKS
-
-
-def channels(fmt):
-    return F.WIB2_CHANNELS if fmt == "wib2" else F.WIBETH_CHANNELS
 
 
 # ---- builder ----------------------------------------------------------------------------------------------------------------
@@ -454,22 +446,6 @@ def oracle_run(name, policy):
     return dict(units=units, tps=tps, ped=np.stack(peds), wav=np.stack(wavs), final=finals[0], finals=np.stack(finals), states=states)
 
 
-def state_fields(policy):
-    fmt, cfg = POLICIES[policy]
-    f = ["pedestal", "accum", "prev_was_over", "hit_charge", "hit_tover", "initialized"]
-    if fmt == "wibeth" and cfg["algorithm"] != "FIR":
-        f += ["hit_peak_adc", "hit_peak_time"]
-    if cfg["algorithm"] in ("AbsRS", "StandardRS"):
-        f += ["rs", "pedestal_rs", "accum_rs"]
-    if fmt == "wibeth" and cfg["algorithm"] in ("AbsRS", "StandardRS"):
-        f += ["rs_memory_factor"]
-    if cfg["algorithm"] == "FIR" or policy == "wib2_absrs":
-        f += ["quantile25", "quantile75", "accum25", "accum75"]
-    if cfg["algorithm"] == "FIR":
-        f += ["prev_samp"]
-    return f
-
-
 def run_gpu(name, policy, step, sorted_tps=False):
     case = build(name, policy)
     want = oracle_run(name, policy)
@@ -482,7 +458,7 @@ def run_gpu(name, policy, step, sorted_tps=False):
             chunk = np.ascontiguousarray(units[:, u:u + step])
             t, p, w = g.process_host(chunk, units_stride=chunk.shape[1], debug=True, cap=1 << 21)
             got.append(t), gp.append(p), gw.append(w)
-        states = np.stack([g.dump_state(l) for l in range(n_links)])
+        states = dump_states(g)
     return got, np.concatenate(gp, axis=1), np.concatenate(gw, axis=1), states
 
 
@@ -491,12 +467,8 @@ def compare(name, policy, step):
     got, gp, gw, gstate = run_gpu(name, policy, step)
     what = f"{name} / {policy} / {step} units per batch"
     assert_same_tps(np.concatenate(got), np.concatenate(want["tps"]), what)
-    for f in state_fields(policy):
-        bad = gstate[f] != want["finals"][f]
-        if bad.any():
-            l, c = (int(i[0]) for i in np.nonzero(bad.reshape(bad.shape[0], bad.shape[1], -1).any(axis=2)))
-            pytest.fail(f"{what}: state field {f} differs on {int(bad.reshape(bad.shape[0], bad.shape[1], -1).any(axis=2).sum())} "
-                        f"channels, first link {l} channel {c}: GPU {gstate[f][l][c]}, oracle {want['finals'][f][l][c]}")
+    fmt, cfg = POLICIES[policy]
+    assert_same_state(gstate, want["finals"], fmt, cfg["algorithm"], what)
     for label, g, w in (("pedestal", gp, want["ped"]), ("waveform", gw, want["wav"])):
         bad = g != w
         if bad.any():

@@ -14,75 +14,23 @@ and replays the same launch sequence (one `Oracle` per link, in a thread pool: c
 import os
 import re
 import time
-from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 import pytest
 
 import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import frames as F
-from oracle import binding as B
-from util import assert_same_tps
+from util import (FULL_WARPS_PER_SM, HIT_MIX, MAX_CTAS_PER_SM, QUAD_CTAS_PER_SM, assert_same_state, assert_same_tps, configured_oracles,
+                  expected_geometry, gpu, halving_slices, ragged_units, replay_oracles, run_device, sms)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "fdreadoutlibs_b200", "csrc")
 
-# SWTPG_PARTS (the forced-slicing test hook) changes the geometry a launch takes: under it the regimes asserted below are not the
-# ones that run.
-TUNING_AIDS = ("SWTPG_PARTS",)
-
-
-def gpu(test):
-    skip = pytest.mark.skipif(any(v in os.environ for v in TUNING_AIDS), reason="a tuning aid is set: launches leave the default geometry")
-    return pytest.mark.gpu(skip(test))
-
-
 TS0 = 1 << 40  # the generator's first timestamp; a WIBEth unit spans 2048 clock ticks, a WIB2 superchunk 12 x 32
 WIDE_PULSES = dict(amp_min=3000, amp_max=15000, hw_min=6, hw_max=16, ped_base=300, ped_step=3, noise_q8=40 * 256)
-HIT_MIX = (0, 1, 2, 3, 4, 5, 7, 8, 9, 15, 16, 17, 31, 32, 33, 63, 64)  # unit counts around every slice edge of stride 64
 
 
-# ---- the launch rules, restated -------------------------------------------------------------------------------------------
-# swtpg_capi.cu: launch_wibeth_geo, launch_wibeth_simple, launch_wibeth, and the policies' constants kWarpsPerSm /
-# kQuadCtasPerSm (swtpg_kernels.cuh: PackedSimpleT, PackedRsWibEth, ScalarAlgo, PackedFirIqr, PackedFirIqrAnyTaps).
-# test_restated_launch_rules_match_the_source pins the source lines this depends on, so the table has to be updated together
-# with the rules.
-FULL_WARPS_PER_SM = 20   # kFullWarpsPerSm, and the running sums' 20 warps per SM above one round
-QUAD_CTAS_PER_SM = 4     # PackedFirIqr / PackedFirIqrAnyTaps::kQuadCtasPerSm
-MAX_CTAS_PER_SM = 32     # what an sm_100 SM holds at most
-
-
-def expected_geometry(policy: str, n_links: int, units_stride: int, sms: int, fits: int = MAX_CTAS_PER_SM):
-    """(persistent warps per SM, slices per link) of a WIBEth launch of the one-warp-per-CTA form. `fits`: single-warp CTAs of
-    the policy an SM holds (occupancy); every packed policy fits at least the 20 it asks for. policy: "SimpleThreshold"
-    (the pipelined form every packed launch runs), "AbsRS", "StandardRS", "scalar" (ScalarAlgo: as many warps as fit)."""
-    even = fits // 4 * 4 if fits >= 4 else fits  # a multiple of 4: every SM sub-partition loaded alike
-    if policy == "SimpleThreshold":  # PackedSimpleWibEthPipe: 16 per SM, from 20 * SMs links on 20 and slices for whole rounds
-        cap, whole_rounds = (FULL_WARPS_PER_SM, True) if n_links >= FULL_WARPS_PER_SM * sms else (16, False)
-    elif policy in ("AbsRS", "StandardRS"):  # PackedRsWibEth: 16 (AbsRS) / 20 (StandardRS), above one 20-per-SM round 20, sliced
-        cap, whole_rounds = (FULL_WARPS_PER_SM, True) if n_links > FULL_WARPS_PER_SM * sms else (16 if policy == "AbsRS" else 20, False)
-    elif policy == "scalar":
-        cap, whole_rounds = even, False
-    else:
-        raise ValueError(policy)
-    warps = min(even, cap)
-    persistent = min(n_links, warps * sms)
-    parts = 1
-    if n_links > persistent and (whole_rounds or n_links % persistent != 0):
-        parts = max(1, min(4, units_stride // 16))
-    return warps, 1 << (parts.bit_length() - 1)  # the largest power of two not above it
-
-
-def halving_slices(n: int, slices: int):
-    """[u0, u1) of each slice of a link with n units (wibeth_kernel's slice_of; tests/test_slice_arithmetic.py pins it)."""
-    out = []
-    for part in range(slices):
-        u0 = n - ((n + (1 << part) - 1) >> part)
-        u1 = n if part + 1 == slices else n - ((n + (2 << part) - 1) >> (part + 1))
-        out.append((u0, u1))
-    return out
-
-
+# ---- the launch rules util.py restates --------------------------------------------------------------------------------------
 def test_restated_launch_rules_match_the_source():
     """CPU: the source lines `expected_geometry` restates. If one of them changes, update the restatement (and the cases)."""
     capi = re.sub(r"\s+", " ", open(os.path.join(CSRC, "swtpg_capi.cu")).read())
@@ -130,38 +78,6 @@ def test_restated_launch_rules_match_the_source():
 
 
 # ---- harness --------------------------------------------------------------------------------------------------------------
-def sms() -> int:
-    import torch
-
-    return torch.cuda.get_device_properties(0).multi_processor_count
-
-
-BASE_FIELDS = ["pedestal", "accum", "prev_was_over", "hit_charge", "hit_tover", "initialized"]
-
-
-def state_fields(fmt: str, algorithm: str):
-    """The carried state each policy keeps (as test_gpu_parity.py's oracle tests compare it)."""
-    f = list(BASE_FIELDS)
-    if fmt == "wibeth" and algorithm != "FIR":
-        f += ["hit_peak_adc", "hit_peak_time"]
-    if fmt == "wibeth" and algorithm in ("AbsRS", "StandardRS"):
-        f += ["rs", "pedestal_rs", "accum_rs", "rs_memory_factor"]
-    if algorithm == "FIR":
-        f += ["quantile25", "quantile75", "accum25", "accum75", "prev_samp"]
-    return f
-
-
-def ragged_units(seed: int, n_links: int, stride: int, specials=()):
-    """Seeded per-link unit counts in [0, stride], with each of `specials` on a few links spread over the whole range."""
-    rng = np.random.default_rng(seed)
-    nu = rng.integers(0, stride + 1, n_links).astype(np.uint32)
-    specials = [s for s in specials if s <= stride]
-    at = rng.choice(n_links, size=min(n_links, 4 * len(specials)), replace=False)
-    for i, l in enumerate(at):
-        nu[l] = specials[i % len(specials)]
-    return nu
-
-
 def locate(tp, fmt: str, stride: int, nus, slices: int) -> str:
     """Launch, unit and slice a TP's start falls in (for the failure message)."""
     unit = (int(tp["time_start"]) - TS0) // (384 if fmt == "wib2" else 2048)
@@ -173,68 +89,18 @@ def locate(tp, fmt: str, stride: int, nus, slices: int) -> str:
     return f"launch {k}, unit {u} of {n}, slice {part} of {slices}"
 
 
-def run_gpu(fmt, n_links, stride, nus, p, tp_capacity, rs_factors=None, **handle_kw):
-    """Every launch of one handle on device-generated frames: (TP list of each launch, per-link state, counters [+ sort stats])."""
-    import torch
-
-    unit_bytes = F.WIB2_SUPERCHUNK_BYTES if fmt == "wib2" else F.WIBETH_FRAME_BYTES
-    gen = S.gen_wib2_device if fmt == "wib2" else S.gen_wibeth_device
-    buf = torch.empty(n_links * stride * unit_bytes, dtype=torch.uint8, device="cuda")
-    got = []
-    try:
-        with S.TPGenerator(n_links, stride, fmt=fmt, tp_capacity=tp_capacity, **handle_kw) as g:
-            if rs_factors is not None:
-                g.set_rs_memory_factor(rs_factors)
-            g.start()
-            for k, nu in enumerate(nus):
-                gen(p, buf.data_ptr(), n_links, stride, unit0=k * stride)
-                torch.cuda.synchronize()  # the generator runs on the legacy stream, the handle on its own
-                g.process_device(buf.data_ptr(), stride, n_units=nu)
-                got.append(g.fetch_tps(cap=tp_capacity))  # waits for the launch: the buffer is free to be rewritten
-            states = np.stack([g.dump_state(l) for l in range(n_links)])
-            info = g.counters()
-            if handle_kw.get("sorted_tps"):
-                info["sort"] = g.sort_stats()
-    finally:
-        del buf
-        torch.cuda.empty_cache()
-    return got, states, info
-
-
-def run_oracle(cfg, fmt, n_links, stride, nus, p, rs_factors=None, cap=1 << 18):
-    """The same launch sequence per link on the CPU: (TPs of each link, per-link state)."""
-    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
-
-    def one(l):
-        o = B.Oracle(cfg, link_id=l)
-        if rs_factors is not None:
-            o.set_memory_factor(rs_factors[l])
-        parts = []
-        for k, nu in enumerate(nus):
-            n = stride if nu is None else int(nu[l])
-            if n:
-                parts.append(o.process(gen(p, 1, n, link0=l, unit0=k * stride, n_threads=1)[0], cap=cap))
-        return np.concatenate(parts) if parts else np.zeros(0, dtype=F.TP_DTYPE), o.state()
-
-    with ThreadPoolExecutor(os.cpu_count() or 1) as ex:
-        res = list(ex.map(one, range(n_links)))
-    return [r[0] for r in res], np.stack([r[1] for r in res])
-
-
 def check_every_link(what, fmt, algorithm, n_links, stride, nus, seed, rate, thr, slices=1, tp_capacity=1 << 24, rs_factors=None,
                      gen_kw=None, oracle_cap=1 << 18, min_tps=1, **kw):
     """Runs the launches on the GPU and the oracle, then compares every link: TPs, carried state, units processed."""
     p = S.gen_params(seed, rate, **(gen_kw or {}))
+    handle = dict(algorithm=algorithm, threshold=thr, **kw)
     t0 = time.time()
-    got, gstate, info = run_gpu(fmt, n_links, stride, nus, p, tp_capacity, rs_factors, algorithm=algorithm, threshold=thr, **kw)
+    got, gstate, _ = run_device(fmt, n_links, stride, nus, p, rs_factors=rs_factors, tp_capacity=tp_capacity, **handle)
     t1 = time.time()
-    okw = {k: v for k, v in kw.items() if k in ("acc_limit", "rs_memory_factor", "rs_scale_factor", "fir_taps", "tap_exponent")}
-    cfg = B.make_config(fmt=fmt, algorithm=S.ALGORITHMS[algorithm], threshold=thr, **okw)
-    want, ostate = run_oracle(cfg, fmt, n_links, stride, nus, p, rs_factors, oracle_cap)
+    oracle_of = configured_oracles(fmt, handle, rs_tables=None if rs_factors is None else dict(enumerate(rs_factors)))
+    want, ostate = replay_oracles(fmt, n_links, stride, nus, p, oracle_of, cap=oracle_cap)
     t2 = time.time()
 
-    assert info["units_processed"] == sum(n_links * stride if nu is None else int(nu.sum()) for nu in nus), \
-        f"{what}: {info['units_processed']} units processed"
     allg = np.concatenate(got)
     assert allg.size >= min_tps, f"{what}: only {allg.size} TPs, the case does not exercise the hit path"
     assert allg.size == 0 or int(allg["link"].max()) < n_links
@@ -250,13 +116,7 @@ def check_every_link(what, fmt, algorithm, n_links, stride, nus, seed, rate, thr
             a, b = set(mine.tolist()), set(theirs.tolist())
             first = np.array([min((a ^ b), key=lambda r: (r[0], r[6], r[5]))], dtype=F.TP_DTYPE)[0]
         assert_same_tps(mine, theirs, f"{what}: link {l} ({locate(first, fmt, stride, nus, slices)})")
-    for f in state_fields(fmt, algorithm):
-        bad = (gstate[f] != ostate[f]).reshape(n_links, -1).any(axis=1)
-        if bad.any():
-            l = int(np.nonzero(bad)[0][0])
-            ch = int(np.nonzero((gstate[f][l] != ostate[f][l]).reshape(gstate.shape[1], -1).any(axis=1))[0][0])
-            pytest.fail(f"{what}: state field {f} differs on {int(bad.sum())} links, first link {l} channel {ch}: "
-                        f"GPU {gstate[f][l][ch]}, oracle {ostate[f][l][ch]}")
+    assert_same_state(gstate, ostate, fmt, algorithm, what)
     print(f"{what}: {n_links} links, {allg.size} TPs identical; GPU {t1 - t0:.1f} s, oracle {t2 - t1:.1f} s")
 
 
@@ -277,8 +137,8 @@ def test_full_load_device_ordered():
     input is the first launch of test_full_load_whole_rounds, checked there against the oracle link for link."""
     n = 40 * sms()
     p = S.gen_params(2, 0.02)
-    plain, _, _ = run_gpu("wibeth", n, 64, [None], p, 1 << 22, threshold=60)
-    ordered, _, info = run_gpu("wibeth", n, 64, [None], p, 1 << 22, threshold=60, sorted_tps=True)
+    plain, _, _ = run_device("wibeth", n, 64, [None], p, tp_capacity=1 << 22, threshold=60)
+    ordered, _, info = run_device("wibeth", n, 64, [None], p, tp_capacity=1 << 22, threshold=60, sorted_tps=True)
     want = S.sort_tps(plain[0])
     assert want.size > 100000 and int(want["link"].max()) >= 4096
     assert ordered[0].size == want.size and (ordered[0] == want).all()

@@ -7,25 +7,17 @@ it did before links had their own."""
 import ctypes as C
 import os
 import subprocess
-from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
-import pytest
 
 import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import _lib
-from fdreadoutlibs_b200 import frames as F
 from fdreadoutlibs_b200 import hostshim as H
-from oracle import binding as B
-from test_gpu_launch_geometry import TUNING_AIDS, expected_geometry, halving_slices, ragged_units, state_fields
-from test_host_shim import as_tuples, expected_host_tps
-from util import assert_same_tps
+from util import (HANDLE, all_wibeth_policies, as_tuples, assert_links_match, assert_same_tps, check, configured_oracles, dump_states,
+                  expected_geometry, expected_host_tps, gpu, halving_slices, host_batches, link_config, oracle_for, ragged_units,
+                  replay_batches, replay_oracles, run_device, run_host, sms)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-# what TPGenerator's own configuration defaults to
-HANDLE = dict(algorithm="SimpleThreshold", threshold=60, acc_limit=10, rs_memory_factor=8, rs_scale_factor=5, fir_taps=None, tap_exponent=6)
-TPG_KEYS = tuple(HANDLE)
 
 
 # ---- CPU --------------------------------------------------------------------------------------------------------------------
@@ -52,69 +44,6 @@ def test_set_link_config_without_handle():
     assert _lib.lib.swtpg_set_link_config(None, 0, None) == _lib.SWTPG_ERR_INVALID_ARG
 
 
-# ---- harness ----------------------------------------------------------------------------------------------------------------
-def gpu(test):
-    skip = pytest.mark.skipif(any(v in os.environ for v in TUNING_AIDS), reason="a tuning aid is set: launches leave the default geometry")
-    return pytest.mark.gpu(skip(test))
-
-
-def full_conf(handle, link_kw):
-    return {**HANDLE, **{k: v for k, v in handle.items() if k in TPG_KEYS}, **link_kw}
-
-
-def oracle_for(fmt, conf, link):
-    cfg = B.make_config(fmt=fmt, algorithm=S.ALGORITHMS[conf["algorithm"]], threshold=conf["threshold"], acc_limit=conf["acc_limit"],
-                        rs_memory_factor=conf["rs_memory_factor"], rs_scale_factor=conf["rs_scale_factor"], fir_taps=conf["fir_taps"],
-                        tap_exponent=conf["tap_exponent"])
-    return B.Oracle(cfg, link_id=link)
-
-
-def host_batches(fmt, seed, rate, n_links, stride, nus, gen_kw=None):
-    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
-    p = S.gen_params(seed, rate, **(gen_kw or {}))
-    return [(gen(p, n_links, stride, unit0=k * stride), nu) for k, nu in enumerate(nus)]
-
-
-def run_handle(fmt, handle, link_kw, batches, tables=None, **gkw):
-    """The batches through one handle (process_host) whose links are configured by link_kw {link: set_link_config kwargs};
-    tables {link: per-channel RS memory factors} are set after start. Returns (TPs of all batches, per-link state)."""
-    n_links, stride = batches[0][0].shape[:2]
-    with S.TPGenerator(n_links, stride, fmt=fmt, **handle, **gkw) as g:
-        for l, kw in link_kw.items():
-            g.set_link_config(l, **kw)
-        g.start()
-        for l, t in (tables or {}).items():
-            g.set_link_rs_memory_factor(l, t)
-        got = np.concatenate([g.process_host(u, n_units=nu, cap=1 << 22) for u, nu in batches])
-        states = np.stack([g.dump_state(l) for l in range(n_links)])
-    return got, states
-
-
-def run_oracles(fmt, handle, link_kw, batches, tables=None):
-    """The same batches per link on the CPU, each link with its own configuration (oracle_process_links with one Oracle per link)."""
-    n_links = batches[0][0].shape[0]
-    oracles = [oracle_for(fmt, full_conf(handle, link_kw.get(l, {})), l) for l in range(n_links)]
-    for l, t in (tables or {}).items():
-        oracles[l].set_memory_factor(t)
-    want = np.concatenate([B.oracle_process_links(None, u, nu, oracles=oracles)[0] for u, nu in batches])
-    return want, np.stack([o.state() for o in oracles])
-
-
-def assert_links_match(what, fmt, handle, link_kw, got, gstate, want, ostate, min_tps=1):
-    assert got.size >= min_tps, f"{what}: only {got.size} TPs"
-    assert_same_tps(got, want, what)
-    for l in range(gstate.shape[0]):
-        for f in state_fields(fmt, full_conf(handle, link_kw.get(l, {}))["algorithm"]):
-            assert (gstate[f][l] == ostate[f][l]).all(), f"{what}: link {l} state field {f} differs from the oracle"
-
-
-def check(what, fmt, handle, link_kw, batches, tables=None, min_tps=1):
-    got, gstate = run_handle(fmt, handle, link_kw, batches, tables)
-    want, ostate = run_oracles(fmt, handle, link_kw, batches, tables)
-    assert_links_match(what, fmt, handle, link_kw, got, gstate, want, ostate, min_tps)
-    return got, gstate
-
-
 # ---- per-link configurations against the oracle ---------------------------------------------------------------------------
 @gpu
 def test_wibeth_simple_thresholds_and_accumulator_limits():
@@ -123,17 +52,7 @@ def test_wibeth_simple_thresholds_and_accumulator_limits():
     n = 24
     link_kw = {l: confs[l % 4] for l in range(n)}
     nus = [ragged_units(201 + k, n, 16, (0, 1, 16)) for k in range(3)]
-    check("simple x4", "wibeth", {}, link_kw, host_batches("wibeth", 201, 0.3, n, 16, nus), min_tps=1000)
-
-
-def all_wibeth_policies():
-    any_taps = list(S.firwin_int(7, 0.1, 32))
-    return [dict(algorithm="SimpleThreshold", threshold=30),
-            dict(algorithm="AbsRS", threshold=30, rs_memory_factor=7, rs_scale_factor=2),
-            dict(algorithm="StandardRS", threshold=30, rs_memory_factor=6),
-            dict(algorithm="FIR", threshold=5),
-            dict(algorithm="FIR", threshold=5, fir_taps=any_taps),  # not the binomial taps: PackedFirIqrAnyTaps
-            dict(algorithm="SimpleThreshold", threshold=30, acc_limit=0)]  # the scalar fallback
+    check("simple x4", "wibeth", {}, host_batches("wibeth", 201, 0.3, n, 16, nus), link_kw=link_kw, min_tps=1000)
 
 
 @gpu
@@ -150,7 +69,8 @@ def test_every_wibeth_policy_in_one_handle():
         link_kw[l] = kw
     table = np.random.default_rng(202).integers(0, 13, 64).astype(np.uint16)
     nus = [ragged_units(202 + k, n, 16, (0, 1, 16)) for k in range(3)]
-    check("all WIBEth policies", "wibeth", {}, link_kw, host_batches("wibeth", 202, 0.3, n, 16, nus), tables={7: table}, min_tps=1000)
+    check("all WIBEth policies", "wibeth", {}, host_batches("wibeth", 202, 0.3, n, 16, nus), link_kw=link_kw, rs_tables={7: table},
+          min_tps=1000)
 
 
 @gpu
@@ -162,7 +82,7 @@ def test_wib2_policies_in_one_handle():
     n = 12
     link_kw = {l: confs[l % 4] for l in range(n)}
     nus = [ragged_units(203 + k, n, 8, (0, 1, 8)) for k in range(2)]
-    check("WIB2 policies", "wib2", {}, link_kw, host_batches("wib2", 203, 0.3, n, 8, nus), min_tps=100)
+    check("WIB2 policies", "wib2", {}, host_batches("wib2", 203, 0.3, n, 8, nus), link_kw=link_kw, min_tps=100)
 
 
 @gpu
@@ -170,12 +90,9 @@ def test_production_geometries_per_group():
     """Three groups in one handle, each sized from the SM count into a production regime of its own: SimpleThreshold with
     20 x SMs + 1 links (20 warps per SM, sliced), AbsRS above one round (sliced), FIR + IQR with 4k + 3 links (quads, the
     group's last one partial). Frames generated on the device; two launches, state carried."""
-    import torch
-
-    sms = torch.cuda.get_device_properties(0).multi_processor_count
-    n_simple, n_rs, n_fir = 20 * sms + 1, 20 * sms + 1, 4 * sms + 3
-    assert expected_geometry("SimpleThreshold", n_simple, 64, sms) == (20, 4)
-    assert expected_geometry("AbsRS", n_rs, 64, sms) == (20, 4)
+    n_simple, n_rs, n_fir = 20 * sms() + 1, 20 * sms() + 1, 4 * sms() + 3
+    assert expected_geometry("SimpleThreshold", n_simple, 64, sms()) == (20, 4)
+    assert expected_geometry("AbsRS", n_rs, 64, sms()) == (20, 4)
     assert n_fir % 4 == 3
     assert halving_slices(64, 4) == [(0, 32), (32, 48), (48, 56), (56, 64)]
     n = n_simple + n_rs + n_fir
@@ -183,35 +100,11 @@ def test_production_geometries_per_group():
     np.random.default_rng(204).shuffle(kinds)  # groups interleaved over the link range
     kinds_kw = [dict(threshold=30), dict(algorithm="AbsRS", threshold=30), dict(algorithm="FIR", threshold=5)]
     link_kw = {l: kinds_kw[int(k)] for l, k in enumerate(kinds)}
-    stride = 64
+    stride, nus = 64, [None, None]
     p = S.gen_params(204, 0.1)
-    buf = torch.empty(n * stride * F.WIBETH_FRAME_BYTES, dtype=torch.uint8, device="cuda")
-    got = []
-    try:
-        with S.TPGenerator(n, stride, tp_capacity=1 << 24) as g:
-            for l, kw in link_kw.items():
-                g.set_link_config(l, **kw)
-            g.start()
-            for k in range(2):
-                S.gen_wibeth_device(p, buf.data_ptr(), n, stride, unit0=k * stride)
-                torch.cuda.synchronize()
-                g.process_device(buf.data_ptr(), stride)
-                got.append(g.fetch_tps(cap=1 << 24))
-            gstate = np.stack([g.dump_state(l) for l in range(n)])
-            assert g.counters()["units_processed"] == 2 * n * stride
-    finally:
-        del buf
-        torch.cuda.empty_cache()
-
-    def one(l):
-        o = oracle_for("wibeth", full_conf({}, link_kw[l]), l)
-        tps = [o.process(S.gen_wibeth_host(p, 1, stride, link0=l, unit0=k * stride, n_threads=1)[0], cap=1 << 16) for k in range(2)]
-        return np.concatenate(tps), o.state()
-
-    with ThreadPoolExecutor(os.cpu_count() or 1) as ex:
-        res = list(ex.map(one, range(n)))
-    want = np.concatenate([r[0] for r in res])
-    assert_links_match("production geometries", "wibeth", {}, link_kw, np.concatenate(got), gstate, want, np.stack([r[1] for r in res]),
+    got, gstate, _ = run_device("wibeth", n, stride, nus, p, link_kw=link_kw)
+    want, ostate = replay_oracles("wibeth", n, stride, nus, p, configured_oracles("wibeth", {}, link_kw), cap=1 << 16)
+    assert_links_match("production geometries", "wibeth", {}, link_kw, np.concatenate(got), gstate, np.concatenate(want), ostate,
                        min_tps=10000)
 
 
@@ -223,7 +116,7 @@ def test_streaming_path_sorted_per_link_configs():
     confs = [dict(threshold=30), dict(threshold=45, acc_limit=4), dict(algorithm="AbsRS", threshold=30), dict(algorithm="FIR", threshold=5)]
     link_kw = {l: confs[l % 4] for l in range(n)}
     units = S.gen_wibeth_host(S.gen_params(205, 0.3), n, n_units)
-    want, _ = run_oracles("wibeth", {}, link_kw, [(units, None)])
+    want, _ = replay_batches([(units, None)], configured_oracles("wibeth", {}, link_kw))
     with S.TPGenerator(n, 4, sorted_tps=True) as g:
         for l, kw in link_kw.items():
             g.set_link_config(l, **kw)
@@ -246,10 +139,10 @@ def test_links_set_to_the_handle_configuration_change_nothing():
     nus = [ragged_units(206 + k, n, 16, (0, 1, 16)) for k in range(2)]
     batches = host_batches("wibeth", 206, 0.3, n, 16, nus)
     handle = dict(threshold=30)
-    a_tps, a_state = run_handle("wibeth", handle, {}, batches)
+    a_tps, a_state = run_host("wibeth", handle, batches)
     # every field the handle has, and fields SimpleThreshold does not read changed on some links: still one group
     link_kw = {l: (dict(fir_taps=[1, 2, 3], rs_scale_factor=3) if l % 2 else {}) for l in range(n)}
-    b_tps, b_state = run_handle("wibeth", handle, link_kw, batches)
+    b_tps, b_state = run_host("wibeth", handle, batches, link_kw=link_kw)
     assert a_tps.size > 100
     assert_same_tps(b_tps, a_tps, "links set to the handle's configuration")
     assert (a_state == b_state).all()
@@ -261,8 +154,8 @@ def test_every_link_set_to_b_equals_a_handle_created_with_b():
     nus = [ragged_units(207 + k, n, 16, (0, 1, 16)) for k in range(2)]
     batches = host_batches("wibeth", 207, 0.3, n, 16, nus)
     b = dict(algorithm="AbsRS", threshold=25, acc_limit=5, rs_memory_factor=7, rs_scale_factor=2)
-    want_tps, want_state = run_handle("wibeth", b, {}, batches)
-    got_tps, got_state = run_handle("wibeth", dict(threshold=60), {l: b for l in range(n)}, batches)
+    want_tps, want_state = run_host("wibeth", b, batches)
+    got_tps, got_state = run_host("wibeth", dict(threshold=60), batches, link_kw={l: b for l in range(n)})
     assert want_tps.size > 100
     assert_same_tps(got_tps, want_tps, "all links set to B")
     assert (got_state == want_state).all()
@@ -271,15 +164,6 @@ def test_every_link_set_to_b_equals_a_handle_created_with_b():
 # ---- call rules -----------------------------------------------------------------------------------------------------------------
 def raw_set(g, link, c):
     return _lib.lib.swtpg_set_link_config(g._h, link, None if c is None else C.byref(c))
-
-
-def link_config(**kw):
-    c = _lib.SwtpgLinkConfig()
-    c.struct_size = C.sizeof(c)
-    c.algorithm, c.threshold, c.frugal_acc_limit, c.rs_memory_factor, c.rs_scale_factor = 0, 60, 10, 8, 5
-    for k, v in kw.items():
-        setattr(c, k, v)
-    return c
 
 
 @gpu
@@ -329,10 +213,10 @@ def test_stop_reconfigure_start_and_reset():
             g.set_link_config(l, **kw)
         g.start()
         tps2 = g.process_host(batches[0][0])
-        state2 = np.stack([g.dump_state(l) for l in range(n)])
+        state2 = dump_states(g)
     handle = dict(threshold=40)
-    want1, _ = run_oracles("wibeth", handle, first, batches)
-    want2, ostate2 = run_oracles("wibeth", handle, second, batches)
+    want1, _ = replay_batches(batches, configured_oracles("wibeth", handle, first))
+    want2, ostate2 = replay_batches(batches, configured_oracles("wibeth", handle, second))
     assert_same_tps(tps1, want1, "first configuration")
     assert_links_match("after reconfiguration", "wibeth", handle, second, tps2, state2, want2, ostate2, min_tps=100)
 

@@ -12,7 +12,7 @@ import cases
 import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import frames as F
 from oracle import binding as B
-from util import assert_same_as_reference, assert_same_tps, oracle_config
+from util import assert_same_as_reference, assert_same_state, assert_same_tps, dump_states, oracle_config
 
 pytestmark = pytest.mark.gpu
 
@@ -86,9 +86,7 @@ def test_fir_thresholds_beyond_the_packed_comparator_range(fmt, thr):
         got = np.concatenate(parts)
         assert got.size > 20
         assert_same_tps(got, want, f"{fmt} FIR thr {thr}")
-        st, so = g.dump_state(1), oracles[1].state()
-        for f in ("pedestal", "quantile25", "quantile75", "accum25", "accum75", "prev_was_over", "hit_charge", "hit_tover", "prev_samp"):
-            assert (st[f] == so[f]).all(), f
+        assert_same_state(g.dump_state(1)[None], oracles[1].state()[None], fmt, "FIR", f"{fmt} FIR thr {thr}, link 1")
 
 
 def test_unpack_known_answer_through_the_abi():
@@ -150,17 +148,7 @@ def test_against_oracle_with_state_and_dumps(algorithm, thr, L):
         assert_same_tps(np.concatenate(got), np.concatenate(want), algorithm)
         assert (np.concatenate(gp, axis=1) == np.stack(peds)).all(), "pedestal dump"
         assert (np.concatenate(gw, axis=1) == np.stack(wavs)).all(), "waveform dump"
-        fields = ["pedestal", "accum", "prev_was_over", "hit_charge", "hit_tover", "initialized"]
-        if algorithm in ("SimpleThreshold", "AbsRS", "StandardRS"):
-            fields += ["hit_peak_adc", "hit_peak_time"]
-        if algorithm in ("AbsRS", "StandardRS"):
-            fields += ["rs", "pedestal_rs", "accum_rs", "rs_memory_factor"]
-        if algorithm == "FIR":
-            fields += ["quantile25", "quantile75", "accum25", "accum75", "prev_samp"]
-        for l in range(n_links):
-            sg, so = g.dump_state(l), oracles[l].state()
-            for f in fields:
-                assert (sg[f] == so[f]).all(), f"link {l} state field {f}"
+        assert_same_state(dump_states(g), np.stack([o.state() for o in oracles]), "wibeth", algorithm, algorithm)
 
 
 ANY_TAPS = [([2, 5, 11, 17, 9, 4, 1], 6), ([-3, 7, 20, 31, 20, 7, -3], 6), ([1, 3, 8, 10, 8, 3, 1], 5), ([300, -700, 1200, 2000, 1200, -700, 300], 6)]
@@ -193,10 +181,7 @@ def test_fir_with_arbitrary_taps(fmt, taps, exponent):
         assert (np.concatenate(gw, axis=1) == np.stack(wavs)).all(), "waveform dump"
         assert (np.concatenate(gp, axis=1) == np.stack(peds)).all(), "pedestal dump"
         assert_same_tps(np.concatenate(got), np.concatenate(want), f"{fmt} taps {taps}")
-        for l in range(n_links):
-            sg, so = g.dump_state(l), oracles[l].state()
-            for f in ["pedestal", "accum", "prev_was_over", "hit_charge", "hit_tover", "quantile25", "quantile75", "accum25", "accum75", "prev_samp"]:
-                assert (sg[f] == so[f]).all(), f"link {l} state field {f}"
+        assert_same_state(dump_states(g), np.stack([o.state() for o in oracles]), fmt, "FIR", f"{fmt} taps {taps}")
 
 
 @pytest.mark.parametrize("algorithm,thr", [("SimpleThreshold", 30), ("SimpleThreshold", 2), ("SimpleThreshold", 40000), ("FIR", 5), ("FIR", 2),
@@ -222,13 +207,7 @@ def test_wib2_against_oracle_with_state_and_dumps(algorithm, thr):
         assert_same_tps(np.concatenate(got), np.concatenate(want), f"wib2 {algorithm}")
         assert (np.concatenate(gp, axis=1) == np.stack(peds)).all(), "pedestal dump"
         assert (np.concatenate(gw, axis=1) == np.stack(wavs)).all(), "waveform dump"
-        fields = ["pedestal", "accum", "prev_was_over", "hit_charge", "hit_tover", "initialized"]
-        if algorithm == "FIR":
-            fields += ["quantile25", "quantile75", "accum25", "accum75", "prev_samp"]
-        for l in range(n_links):
-            sg, so = g.dump_state(l), oracles[l].state()
-            for f in fields:
-                assert (sg[f] == so[f]).all(), f"link {l} state field {f}"
+        assert_same_state(dump_states(g), np.stack([o.state() for o in oracles]), "wib2", algorithm, f"wib2 {algorithm}")
 
 
 @pytest.mark.parametrize("fmt,algorithm,thr,kw", [
@@ -264,10 +243,7 @@ def test_extreme_amplitudes_wrap_and_saturate_like_the_reference(fmt, algorithm,
         assert (np.concatenate(gp, axis=1) == np.stack(peds)).all(), "pedestal dump"
         assert (np.concatenate(gw, axis=1) == np.stack(wavs)).all(), "waveform dump"
         assert_same_tps(np.concatenate(got), np.concatenate(want), f"{fmt} {algorithm}")
-        for l in range(n_links):
-            sg, so = g.dump_state(l), oracles[l].state()
-            for f in ("pedestal", "accum", "prev_was_over", "hit_charge", "hit_tover"):
-                assert (sg[f] == so[f]).all(), f"link {l} state field {f}"
+        assert_same_state(dump_states(g), np.stack([o.state() for o in oracles]), fmt, algorithm, f"{fmt} {algorithm}")
     allt = np.concatenate(want)
     assert allt.size > 200
     if algorithm == "SimpleThreshold" and fmt == "wibeth":
@@ -308,10 +284,7 @@ def test_per_link_memory_factor_after_start(algorithm):
         for u in range(step, n_units, step):
             got.append(g.process_host(np.ascontiguousarray(units[:, u:u + step])))
         assert_same_tps(np.concatenate(got), np.concatenate(want), "per-link memory factor")
-        for l in range(n_links):
-            st, so = g.dump_state(l), oracles[l].state()
-            for f in ("rs", "pedestal_rs", "accum_rs", "rs_memory_factor"):
-                assert (st[f] == so[f]).all(), f"link {l} {f}"
+        assert_same_state(dump_states(g), np.stack([o.state() for o in oracles]), "wibeth", algorithm, "per-link memory factor")
 
 
 def test_wib2_many_links_ragged_and_streaming():

@@ -9,13 +9,9 @@ import pytest
 
 import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import hostshim as H
+from fdreadoutlibs_b200 import frames as F
 from oracle import binding as B
-
-PERM = [0, 1, 2, 3, 4, 5, 6, 7, 15, 8, 9, 10, 11, 12, 13, 14]
-
-
-def linear_map(crate, slot, stream, chan):
-    return ((crate * 8 + slot) * 64 + stream) * 64 + chan
+from util import as_tuples, expected_host_tps, linear_map
 
 
 def test_host_library_exports():
@@ -103,28 +99,6 @@ def test_tpset_windows_heartbeats_and_tardy_cutoff():
     h.close()
 
 
-def expected_host_tps(tps, link_stream, *, mask=(), tp_timeout=10 ** 9, correct=False, crate=1, slot=0, wib2=False):
-    """What process_swtpg_hits makes of device/oracle TP records of one link."""
-    out = []
-    for r in tps:
-        c = int(r["channel"])
-        if wib2 or correct:
-            off = linear_map(crate, slot, link_stream, c)
-        else:  # H2: position-ordered LUT indexed by the frame channel
-            off = linear_map(crate, slot, link_stream, (c & ~15) | PERM[c & 15])
-        if off in mask:
-            continue
-        if int(r["time_over_threshold"]) > tp_timeout:
-            continue
-        out.append((int(r["time_start"]), int(r["time_peak"]), int(r["time_over_threshold"]), off, int(r["adc_integral"]), int(r["adc_peak"])))
-    return sorted(out)
-
-
-def as_tuples(h):
-    return sorted((int(r["time_start"]), int(r["time_peak"]), int(r["time_over_threshold"]), int(r["channel"]), int(r["adc_integral"]),
-                   int(r["adc_peak"])) for r in h)
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("algorithm,algo_id,correct", [("SimpleThreshold", 0, False), ("SimpleThreshold", 0, True), ("AbsRS", 1, False)])
 def test_wibeth_frame_processor_end_to_end(algorithm, algo_id, correct):
@@ -153,11 +127,11 @@ def test_wibeth_frame_processor_end_to_end(algorithm, algo_id, correct):
             assert info["num_tps_sent"] == got.size and info["num_ts_errors"] == 1  # first frame: previous_ts = 0
             assert info["num_seq_id_errors"] == 1 and info["num_frames_dropped_busy"] == 0  # first frame: previous_seq_id = 0, seq 0 != 1
             n_long = sum(1 for r in w if int(r["time_over_threshold"]) > timeout and
-                         linear_map(1, 0, l, (int(r["channel"]) & ~15) | PERM[int(r["channel"]) & 15] if not correct else int(r["channel"])) not in mask)
+                         linear_map(1, 0, l, int(F.position_to_channel(int(r["channel"]))) if not correct else int(r["channel"])) not in mask)
             assert info["num_tps_suppressed_too_long"] == n_long
             assert fp.misconfigurations(l) == 0
             # RegisterToChannelNumber: position p holds frame channel 16(p/16) + perm[p%16]
-            assert (fp.register_channel_map(l) == [linear_map(1, 0, l, (p & ~15) | PERM[p & 15]) for p in range(64)]).all()
+            assert (fp.register_channel_map(l) == [linear_map(1, 0, l, int(F.position_to_channel(p))) for p in range(64)]).all()
             top = info["top"]
             assert len(top) == 10 and all(top[i][1] >= top[i + 1][1] for i in range(9))
             total_sent += got.size

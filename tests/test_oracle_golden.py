@@ -4,9 +4,12 @@ import numpy as np
 import pytest
 
 import cases
+import fdreadoutlibs_b200 as S
+from fdreadoutlibs_b200 import _lib
+from fdreadoutlibs_b200 import api as A
 from fdreadoutlibs_b200 import frames as F
 from oracle import binding as B
-from util import assert_same_tps, oracle_config
+from util import assert_same_tps, create_status, oracle_config, state_fields
 
 
 @pytest.mark.parametrize("name", sorted(cases.GOLDEN_CASES))
@@ -137,3 +140,24 @@ def test_oracle_empty_and_state_carry():
     assert o.process(fr[:0]).size == 0
     two = np.concatenate([o.process(fr[:13]), o.process(fr[13:])])
     assert_same_tps(two, one, "split")
+
+
+# every (format, algorithm) swtpg_create accepts (WIB2 has no StandardRS)
+ACCEPTED = [(fmt, a) for fmt in A.FORMATS for a in S.ALGORITHMS if create_status(fmt, a, 30) != _lib.SWTPG_ERR_UNSUPPORTED]
+
+
+@pytest.mark.parametrize("fmt,algorithm", ACCEPTED)
+def test_state_fields_cover_what_moves(fmt, algorithm):
+    """util.state_fields, which the GPU tests compare, names every field of the carried state that the oracle moves: every field
+    that differs on some channel between the state after the first of 16 generated units and the state after the last. The
+    fields left out keep their seeds, such as SimpleThreshold's quartiles and the RS memory factor."""
+    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
+    units = gen(S.gen_params(1, 0.3), 1, 16)[0]
+    o = B.Oracle(B.make_config(fmt=fmt, algorithm=S.ALGORITHMS[algorithm], threshold=5 if algorithm == "FIR" else 30))
+    o.process(units[:1])
+    first = o.state()
+    o.process(units[1:])
+    last = o.state()
+    moved = {f for f in F.STATE_DTYPE.names if (first[f] != last[f]).any()}
+    assert "pedestal" in moved
+    assert moved <= set(state_fields(fmt, algorithm)), f"moved but not compared: {sorted(moved - set(state_fields(fmt, algorithm)))}"
