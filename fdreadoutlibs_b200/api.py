@@ -27,8 +27,11 @@ FLAG_ADC_STATS = 2  # SWTPG_FLAG_ADC_STATS
 
 
 class SwtpgError(RuntimeError):
-    def __init__(self, status: int, detail: str):
+    """`tps`: the records the failing call delivered all the same (poll on SWTPG_ERR_OVERFLOW), else None."""
+
+    def __init__(self, status: int, detail: str, tps: Optional[np.ndarray] = None):
         self.status = status
+        self.tps = tps
         super().__init__(f"{lib.swtpg_status_string(status).decode()} ({status}): {detail}")
 
 
@@ -253,12 +256,17 @@ class TPGenerator:
         self._check(lib.swtpg_sync(self._h))
 
     def poll(self, cap: int = 1 << 16, wait_us: int = 0) -> np.ndarray:
+        """SWTPG_ERR_OVERFLOW (a batch found more TPs than tp_capacity) raises SwtpgError with the records this call delivered
+        in its `tps`: they are true records, and no later poll returns them."""
         out = np.zeros(cap, dtype=F.TP_DTYPE)
         n = C.c_size_t(0)
         if wait_us:
-            self._check(lib.swtpg_poll_wait(self._h, out.ctypes.data, cap, C.byref(n), wait_us))
+            st = lib.swtpg_poll_wait(self._h, out.ctypes.data, cap, C.byref(n), wait_us)
         else:
-            self._check(lib.swtpg_poll(self._h, out.ctypes.data, cap, C.byref(n)))
+            st = lib.swtpg_poll(self._h, out.ctypes.data, cap, C.byref(n))
+        if st == SWTPG_ERR_OVERFLOW:
+            raise SwtpgError(st, (lib.swtpg_last_error(self._h) or b"").decode(), tps=out[: n.value].copy())
+        self._check(st)
         return out[: n.value].copy()
 
     def drain(self) -> np.ndarray:

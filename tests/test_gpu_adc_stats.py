@@ -16,7 +16,7 @@ from fdreadoutlibs_b200 import _lib
 from fdreadoutlibs_b200 import api as A
 from fdreadoutlibs_b200 import frames as F
 from fdreadoutlibs_b200 import hostshim as H
-from util import all_wibeth_policies, channels, create_status, linear_map, ragged_units, run_device, sms
+from util import adc_of, all_wibeth_policies, channels, combine, create_status, expected, linear_map, ragged_units, run_device, sms, stats_of
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -51,45 +51,6 @@ def test_create_accepts_the_flag_and_still_refuses_unknown_bits():
 
 
 # ---- expected values --------------------------------------------------------------------------------------------------------------
-def adc_of(fmt, units, adc_offset=F.WIB2_ADC_OFFSET):
-    """(samples, channels) raw ADC values of a link's units."""
-    if len(units) == 0:
-        return np.zeros((0, channels(fmt)), dtype=np.uint16)
-    if fmt == "wib2":
-        return F.unpack_wib2_superchunks(units, adc_offset)[0].reshape(-1, F.WIB2_CHANNELS)
-    return F.unpack_wibeth_frames(units)[0].reshape(-1, F.WIBETH_CHANNELS)
-
-
-def stats_of(a):
-    """ADC_STATS_DTYPE row of (samples, channels) ADC values."""
-    out = np.zeros(a.shape[1], dtype=F.ADC_STATS_DTYPE)
-    if a.shape[0]:
-        v = a.astype(np.uint64)
-        out["samples"] = a.shape[0]
-        out["sum"] = v.sum(0)
-        out["sum_sq"] = (v * v).sum(0)
-        out["min"] = a.min(0)
-        out["max"] = a.max(0)
-    return out
-
-
-def expected(fmt, frames, nu=None, adc_offset=F.WIB2_ADC_OFFSET):
-    """(n_links, channels) statistics of one batch: frames [n_links, stride, unit_bytes], nu valid units per link (None = all)."""
-    n, stride = frames.shape[:2]
-    return np.stack([stats_of(adc_of(fmt, frames[l, : (stride if nu is None else int(nu[l]))], adc_offset)) for l in range(n)])
-
-
-def combine(a, b):
-    """Statistics of two windows together."""
-    out = a.copy()
-    for f in ("samples", "sum", "sum_sq"):
-        out[f] = a[f] + b[f]
-    both = (a["samples"] > 0) & (b["samples"] > 0)
-    out["min"] = np.where(both, np.minimum(a["min"], b["min"]), np.where(a["samples"] > 0, a["min"], b["min"]))
-    out["max"] = np.maximum(a["max"], b["max"])
-    return out
-
-
 def zeros(n_links, fmt):
     return np.zeros((n_links, channels(fmt)), dtype=F.ADC_STATS_DTYPE)
 

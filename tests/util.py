@@ -106,6 +106,46 @@ def assert_same_state(gstate, ostate, fmt, algorithm, what):
                             f"channel {ch}: GPU {g[i][ch]}, oracle {o[i][ch]}")
 
 
+# ---- ADC statistics ---------------------------------------------------------------------------------------------------------
+def adc_of(fmt, units, adc_offset=F.WIB2_ADC_OFFSET):
+    """(samples, channels) raw ADC values of a link's units."""
+    if len(units) == 0:
+        return np.zeros((0, channels(fmt)), dtype=np.uint16)
+    if fmt == "wib2":
+        return F.unpack_wib2_superchunks(units, adc_offset)[0].reshape(-1, F.WIB2_CHANNELS)
+    return F.unpack_wibeth_frames(units)[0].reshape(-1, F.WIBETH_CHANNELS)
+
+
+def stats_of(a):
+    """ADC_STATS_DTYPE row of (samples, channels) ADC values."""
+    out = np.zeros(a.shape[1], dtype=F.ADC_STATS_DTYPE)
+    if a.shape[0]:
+        v = a.astype(np.uint64)
+        out["samples"] = a.shape[0]
+        out["sum"] = v.sum(0)
+        out["sum_sq"] = (v * v).sum(0)
+        out["min"] = a.min(0)
+        out["max"] = a.max(0)
+    return out
+
+
+def expected(fmt, frames, nu=None, adc_offset=F.WIB2_ADC_OFFSET):
+    """(n_links, channels) statistics of one batch: frames [n_links, stride, unit_bytes], nu valid units per link (None = all)."""
+    n, stride = frames.shape[:2]
+    return np.stack([stats_of(adc_of(fmt, frames[l, : (stride if nu is None else int(nu[l]))], adc_offset)) for l in range(n)])
+
+
+def combine(a, b):
+    """Statistics of two windows together."""
+    out = a.copy()
+    for f in ("samples", "sum", "sum_sq"):
+        out[f] = a[f] + b[f]
+    both = (a["samples"] > 0) & (b["samples"] > 0)
+    out["min"] = np.where(both, np.minimum(a["min"], b["min"]), np.where(a["samples"] > 0, a["min"], b["min"]))
+    out["max"] = np.maximum(a["max"], b["max"])
+    return out
+
+
 # ---- configurations ---------------------------------------------------------------------------------------------------------
 # what TPGenerator's own configuration defaults to
 HANDLE = dict(algorithm="SimpleThreshold", threshold=60, acc_limit=10, rs_memory_factor=8, rs_scale_factor=5, fir_taps=None, tap_exponent=6)
@@ -243,24 +283,32 @@ def run_device(fmt, n_links, stride, nus, params, *, link_kw=None, thresholds=No
     return got, states, info
 
 
-def replay_oracles(fmt, n_links, stride, nus, params, oracle_of, cap=1 << 18):
-    """run_device's launches on the CPU. The generator is counter-based, so each link's units are generated on the host and run
-    through that link's oracle_of(link), one link per worker of a thread pool (ctypes releases the GIL). Returns (TPs of each
-    link, per-link state)."""
-    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
-
+def replay_links(n_links, oracle_of, units_of, cap=1 << 20):
+    """Link l's unit arrays units_of(l) (an iterable, in order) through oracle_of(l), one link per worker of a thread pool (ctypes
+    releases the GIL). Returns (TPs of each link, per-link state)."""
     def one(l):
         o = oracle_of(l)
-        parts = [np.zeros(0, dtype=F.TP_DTYPE)]
-        for k, nu in enumerate(nus):
-            n = stride if nu is None else int(nu[l])
-            if n:
-                parts.append(o.process(gen(params, 1, n, link0=l, unit0=k * stride, n_threads=1)[0], cap=cap))
+        parts = [np.zeros(0, dtype=F.TP_DTYPE)] + [o.process(u, cap=cap) for u in units_of(l) if len(u)]
         return np.concatenate(parts), o.state()
 
     with ThreadPoolExecutor(os.cpu_count() or 1) as ex:
         res = list(ex.map(one, range(n_links)))
     return [r[0] for r in res], np.stack([r[1] for r in res])
+
+
+def replay_oracles(fmt, n_links, stride, nus, params, oracle_of, cap=1 << 18):
+    """run_device's launches on the CPU. The generator is counter-based, so each link's units are generated on the host, in
+    replay_links's worker of that link, and run through that link's oracle_of(link). Returns (TPs of each link, per-link
+    state)."""
+    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
+
+    def units_of(l):
+        for k, nu in enumerate(nus):
+            n = stride if nu is None else int(nu[l])
+            if n:
+                yield gen(params, 1, n, link0=l, unit0=k * stride, n_threads=1)[0]
+
+    return replay_links(n_links, oracle_of, units_of, cap)
 
 
 def run_host(fmt, handle, batches, *, link_kw=None, thresholds=None, rs_tables=None):
@@ -282,9 +330,11 @@ def run_host(fmt, handle, batches, *, link_kw=None, thresholds=None, rs_tables=N
 
 def replay_batches(batches, oracle_of):
     """host_batches on the CPU, link l through oracle_of(l): (TPs of all batches, per-link state)."""
-    oracles = [oracle_of(l) for l in range(batches[0][0].shape[0])]
-    want = np.concatenate([B.oracle_process_links(None, u, nu, oracles=oracles)[0] for u, nu in batches])
-    return want, np.stack([o.state() for o in oracles])
+    def units_of(l):
+        return [u[l, : (u.shape[1] if nu is None else int(nu[l]))] for u, nu in batches]
+
+    tps, state = replay_links(batches[0][0].shape[0], oracle_of, units_of)
+    return np.concatenate(tps), state
 
 
 def assert_links_match(what, fmt, handle, link_kw, got, gstate, want, ostate, min_tps=1):
