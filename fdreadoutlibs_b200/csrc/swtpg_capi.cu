@@ -14,12 +14,12 @@
 #include <new>
 #include <string>
 #include <thread>
-#include <type_traits>
 #include <vector>
 
 using namespace swtpg;
 using swtpg_internal::ConfGroup;
 using swtpg_internal::fail;
+using swtpg_internal::Policy;
 using swtpg_internal::TpgConf;
 
 // Layouts the ctypes binding (fdreadoutlibs_b200/_lib.py, frames.py) relies on.
@@ -77,32 +77,27 @@ residency(int threads, size_t smem, int cap, unsigned* resident, unsigned* sms)
   return cudaSuccess;
 }
 
-// Geometry of the WIBEth kernel: one link-warp per CTA with a ring of 2 stages x 32 ticks (7 KB) + 2.5 KB hit staging. Measured
-// best on B200 (profiles/r01_geometry_sweep.txt): the kernel is issue-bound, so deeper rings do not help, and single-warp CTAs
-// let the block scheduler spread the 20 resident warps per SM evenly over the four sub-partitions.
-constexpr int kGeoStages = 2, kGeoChunk = 32;
-
-// WARPS_PER_SM: 0 = the policy's own measured optimum (Algo::kWarpsPerSm). SLICE_WHOLE_ROUNDS: hand the links out in slices
-// even when their number is a whole multiple of the persistent warps.
-template<class Algo, bool DUMP, int WARPS_PER_SM = 0, bool SLICE_WHOLE_ROUNDS = false>
+// One-warp-per-CTA form of the WIBEth kernel, persistent: at most as many CTAs as the device holds at once; warps claim links
+// dynamically (wibeth_kernel), so the grid only has to load every SM sub-partition alike: a multiple of 4 single-warp CTAs per
+// SM, capped at the policy's warps per SM (20 on B200: 5 warps per sub-partition; a 21st warp would make one sub-partition of
+// every SM 20 % slower than its neighbours — profiles/README.md). From the policy's full-load link count on it runs its
+// full-load warps per SM and slices the links even when their number is a whole multiple of the persistent warps.
+template<class Algo, bool DUMP>
 cudaError_t
 launch_wibeth_geo(const KernelParams& kp, cudaStream_t s)
 {
-  constexpr auto k = wibeth_kernel<Algo, 1, kGeoStages, kGeoChunk, DUMP, 1>;
-  constexpr size_t smem = WibEthSmem<1, kGeoStages, kGeoChunk>::total;
-  // Persistent grid: at most as many CTAs as the device holds at once; warps walk the links.
+  constexpr auto k = wibeth_kernel<Algo, DUMP>;
+  constexpr size_t smem = WibEthSmem::total;
   unsigned resident = 0, sms = 0;
   const cudaError_t e = residency<k>(32, smem, 0, &resident, &sms);
   if (e != cudaSuccess)
     return e;
-  // Persistent warps claim links dynamically (wibeth_kernel), so the grid only has to load every SM sub-partition alike:
-  // a multiple of 4 single-warp CTAs per SM (20 on B200: 5 warps per sub-partition; a 21st warp would make one
-  // sub-partition of every SM 20 % slower than its neighbours — profiles/README.md).
+  const bool full_load = Algo::kFullLoadWarpsPerSm > 0 && kp.n_links >= Algo::kFullLoadWarpsPerSm * sms + Algo::kFullLoadExtraLinks;
+  const unsigned warps_per_sm = full_load ? Algo::kFullLoadWarpsPerSm : Algo::kWarpsPerSm;
   const unsigned per_sm = resident / sms;
   unsigned even = per_sm >= 4 ? per_sm / 4 * 4 : per_sm;
-  constexpr int kWarpsPerSm = WARPS_PER_SM > 0 ? WARPS_PER_SM : Algo::kWarpsPerSm;
-  if (kWarpsPerSm > 0) // the measured optimum, if the device holds that many
-    even = std::min<unsigned>(even, unsigned(kWarpsPerSm));
+  if (warps_per_sm > 0) // the measured optimum, if the device holds that many
+    even = std::min(even, warps_per_sm);
   const unsigned grid = std::min<unsigned>(std::min<unsigned>(kp.n_links, even * sms), resident);
   // More links than persistent warps = several rounds of links per warp, and whatever the last round leaves idle is lost (round 2,
   // straight-line SimpleThreshold policy: 6000 links on 4144 warps 64.9 % of the HBM peak, 8288 = two full rounds 73.0 %). Handing
@@ -111,12 +106,12 @@ launch_wibeth_geo(const KernelParams& kp, cudaStream_t s)
   // the tail without more round trips per link than four equal ones (pipelined SimpleThreshold policy at 20 warps per SM, 5920
   // links: whole links 68.9 %, equal slices 70.8 %, halving 73.1 %; 6000 links 71.0 -> 73.3 %; AbsRS + 2.5 %;
   // profiles/r02_halving_slices_probe.txt).
-  //   * For most policies a link count that is a whole number of rounds keeps whole links (straight-line form, 8288 links: 73.0 %
-  //     against 70.8 % sliced); the pipelined SimpleThreshold policy gains from slices even then (SLICE_WHOLE_ROUNDS).
+  //   * Below full load a link count that is a whole number of rounds keeps whole links (straight-line form, 8288 links: 73.0 %
+  //     against 70.8 % sliced); at full load the policies gain from slices even then.
   // A launch that cannot fill the GPU keeps whole links: time is sequential per link, slices could only wait for each other.
   KernelParams kq = kp;
   unsigned parts = 1;
-  if (kp.n_links > grid && (SLICE_WHOLE_ROUNDS || kp.n_links % grid != 0))
+  if (kp.n_links > grid && (full_load || kp.n_links % grid != 0))
     parts = std::max(1u, std::min(4u, kp.units_stride / 16u));
   // Test hook: SWTPG_PARTS=n hands every launch out in n slices (at most 8), so that the GPU suite can run its cases with every
   // link sliced (tests/test_gpu_parity.py::test_links_handed_out_in_slices).
@@ -131,14 +126,13 @@ launch_wibeth_geo(const KernelParams& kp, cudaStream_t s)
   return cudaGetLastError();
 }
 
-// CTA form of the WIBEth kernel (wibeth_quad_kernel): 4 consumer warps + 1 producer warp per quad of links, ring of 2 x 32 ticks.
+// CTA form of the WIBEth kernel (wibeth_quad_kernel): 4 consumer warps + 1 producer warp per quad of links.
 template<class Algo, bool DUMP>
 cudaError_t
 launch_wibeth_quad(const KernelParams& kp, cudaStream_t s)
 {
-  constexpr int kStages = 2, kChunk = 32;
-  constexpr auto k = wibeth_quad_kernel<Algo, kStages, kChunk, DUMP>;
-  constexpr size_t smem = WibEthQuadSmem<kStages, kChunk>::total;
+  constexpr auto k = wibeth_quad_kernel<Algo, DUMP>;
+  constexpr size_t smem = WibEthQuadSmem::total;
   unsigned resident = 0, sms = 0;
   const cudaError_t e = residency<k>((kQuad + 1) * 32, smem, Algo::kQuadCtasPerSm, &resident, &sms);
   if (e != cudaSuccess)
@@ -153,51 +147,20 @@ launch_wibeth_quad(const KernelParams& kp, cudaStream_t s)
 // for FIR + IQR (ptxas needs 64 registers instead of 109 for it, so 20 consumer warps fit an SM), the one-warp-per-CTA form
 // 2-5 % faster for SimpleThreshold and the running sums (the quad's lock-step costs more than the producer bookkeeping it
 // saves).
-// WIBEth SimpleThreshold, the production algorithm: which form of its policy runs and with how many persistent warps is a
-// measured choice (profiles/r02_simple_pipeline_sweep.txt, profiles/r02_halving_slices_probe.txt).
-//   * The software-pipelined form (prefetch of the next group's rows + deferred quiet test, PackedSimpleT<true>, 92 registers) on
-//     the 2 x 32-tick ring runs every launch since its dependent chain lost an instruction (the accumulator reset as one IMAD):
-//     with 20 warps per SM and halving slices it beats the straight-line form with 28 at every link count — 5920 links 73.1 %
-//     against 67.8 % of the HBM peak, 6000 links 73.3 / 67.8 %, 8288 links 74.3 / 73.2 %, 4440 links 72.1 / 67.6 % — except on
-//     a dense-hit batch (20.2 / 21.0 %).
-//   * Below one link per warp of the 20-per-SM grid (2960 links on B200: a 750-link shard of an 8-GPU module, the streaming
-//     path's 240 links, one APA) a launch is bound by what ONE warp does per tick and keeps at most 16 warps per SM (measured
-//     optimum of the round-2 sweep); beyond that 20 warps per SM and slices even for whole rounds.
-template<bool DUMP>
-cudaError_t
-launch_wibeth_simple(const KernelParams& kp, cudaStream_t s)
-{
-  int sms = 148, dev = 0;
-  if (cudaGetDevice(&dev) == cudaSuccess)
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  constexpr int kFullWarpsPerSm = 20;
-  if (kp.n_links >= unsigned(kFullWarpsPerSm * sms)) // 2960 links: 66.5 % with 20 warps per SM against 64.2 % with 16; 2500: 56.7 / 58.2 %
-    return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, kFullWarpsPerSm, true>(kp, s);
-  return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP>(kp, s);
-}
-
+// WIBEth SimpleThreshold, the production algorithm, runs the software-pipelined form of its policy (prefetch of the next group's
+// rows + deferred quiet test, PackedSimpleT<true>, 92 registers) on every launch since its dependent chain lost an instruction
+// (the accumulator reset as one IMAD): with 20 warps per SM and halving slices it beats the straight-line form with 28 at every
+// link count — 5920 links 73.1 % against 67.8 % of the HBM peak, 6000 links 73.3 / 67.8 %, 8288 links 74.3 / 73.2 %, 4440 links
+// 72.1 / 67.6 % — except on a dense-hit batch (20.2 / 21.0 %) (profiles/r02_simple_pipeline_sweep.txt,
+// profiles/r02_halving_slices_probe.txt).
 template<class Algo, bool DUMP>
 cudaError_t
 launch_wibeth(const KernelParams& kp, cudaStream_t s)
 {
-  if constexpr (std::is_same<Algo, PackedSimpleWibEth>::value) {
-    return launch_wibeth_simple<DUMP>(kp, s);
-  } else if constexpr (Algo::kQuadCtasPerSm > 0) {
+  if constexpr (Algo::kQuadCtasPerSm > 0)
     return launch_wibeth_quad<Algo, DUMP>(kp, s);
-  } else {
-    // The running sums (AbsRS, StandardRS; one-warp-per-CTA form): a launch of more than one round of a 20-per-SM grid runs 20
-    // warps per SM with halving slices, whole rounds included — AbsRS 28.7 -> 30.4 % of the HBM peak at 5920 links (its own
-    // optimum of 16 warps per SM holds for whole links: 20 unsliced 26.9 %), StandardRS 35.4 -> 36.7 %
-    // (profiles/r02_warps_crossover_probe.txt).
-    if constexpr (std::is_same<Algo, PackedRsWibEth<false>>::value || std::is_same<Algo, PackedRsWibEth<true>>::value) {
-      int sms = 148, dev = 0;
-      if (cudaGetDevice(&dev) == cudaSuccess)
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      if (kp.n_links > unsigned(20 * sms))
-        return launch_wibeth_geo<Algo, DUMP, 20, true>(kp, s);
-    }
+  else
     return launch_wibeth_geo<Algo, DUMP>(kp, s);
-  }
 }
 
 // WIB2: one CTA (4 consumer warps + 1 producer warp) per link at a time, ring of 4 superchunks; persistent over links.
@@ -219,37 +182,25 @@ launch_wib2(const KernelParams& kp, cudaStream_t s)
 
 template<bool DUMP>
 cudaError_t
-launch(const swtpg_handle* h, const TpgConf& c, const KernelParams& kp, cudaStream_t s)
+launch(Policy policy, const KernelParams& kp, cudaStream_t s)
 {
-  if (h->cfg.format == SWTPG_FORMAT_WIB2) {
-    switch (c.algorithm) {
-      case SWTPG_ALGO_SIMPLE_THRESHOLD:
-        return c.fast_simple ? launch_wib2<PackedSimpleWib2, DUMP>(kp, s)
-                              : launch_wib2<ScalarAlgo<SWTPG_ALGO_SIMPLE_THRESHOLD, true>, DUMP>(kp, s);
-      case SWTPG_ALGO_FIR_IQR:
-        return c.fast_fir       ? launch_wib2<PackedFirIqr, DUMP>(kp, s)
-               : c.fast_fir_any ? launch_wib2<PackedFirIqrAnyTaps, DUMP>(kp, s)
-                                 : launch_wib2<ScalarAlgo<SWTPG_ALGO_FIR_IQR, true>, DUMP>(kp, s);
-      case SWTPG_ALGO_ABS_RS:
-        return c.fast_rs_wib2 ? launch_wib2<PackedRsIqrWib2, DUMP>(kp, s) : launch_wib2<ScalarAlgo<SWTPG_ALGO_ABS_RS, true>, DUMP>(kp, s);
-      default: return cudaErrorNotSupported;
-    }
-  }
-  if (h->cfg.format == SWTPG_FORMAT_WIBETH) {
-    switch (c.algorithm) {
-      case SWTPG_ALGO_SIMPLE_THRESHOLD:
-        return c.fast_simple ? launch_wibeth<PackedSimpleWibEth, DUMP>(kp, s)
-                              : launch_wibeth<ScalarAlgo<SWTPG_ALGO_SIMPLE_THRESHOLD, false>, DUMP>(kp, s);
-      case SWTPG_ALGO_ABS_RS:
-        return c.fast_rs ? launch_wibeth<PackedRsWibEth<false>, DUMP>(kp, s) : launch_wibeth<ScalarAlgo<SWTPG_ALGO_ABS_RS, false>, DUMP>(kp, s);
-      case SWTPG_ALGO_STANDARD_RS:
-        return c.fast_rs ? launch_wibeth<PackedRsWibEth<true>, DUMP>(kp, s)
-                          : launch_wibeth<ScalarAlgo<SWTPG_ALGO_STANDARD_RS, false>, DUMP>(kp, s);
-      case SWTPG_ALGO_FIR_IQR:
-        return c.fast_fir       ? launch_wibeth<PackedFirIqr, DUMP>(kp, s)
-               : c.fast_fir_any ? launch_wibeth<PackedFirIqrAnyTaps, DUMP>(kp, s)
-                                 : launch_wibeth<ScalarAlgo<SWTPG_ALGO_FIR_IQR, false>, DUMP>(kp, s);
-    }
+  switch (policy) {
+    case Policy::WibEthSimple: return launch_wibeth<PackedSimpleWibEthPipe, DUMP>(kp, s);
+    case Policy::WibEthAbsRs: return launch_wibeth<PackedRsWibEth<false>, DUMP>(kp, s);
+    case Policy::WibEthStandardRs: return launch_wibeth<PackedRsWibEth<true>, DUMP>(kp, s);
+    case Policy::WibEthFir: return launch_wibeth<PackedFirIqr, DUMP>(kp, s);
+    case Policy::WibEthFirAnyTaps: return launch_wibeth<PackedFirIqrAnyTaps, DUMP>(kp, s);
+    case Policy::WibEthScalarSimple: return launch_wibeth<ScalarAlgo<SWTPG_ALGO_SIMPLE_THRESHOLD, false>, DUMP>(kp, s);
+    case Policy::WibEthScalarAbsRs: return launch_wibeth<ScalarAlgo<SWTPG_ALGO_ABS_RS, false>, DUMP>(kp, s);
+    case Policy::WibEthScalarStandardRs: return launch_wibeth<ScalarAlgo<SWTPG_ALGO_STANDARD_RS, false>, DUMP>(kp, s);
+    case Policy::WibEthScalarFir: return launch_wibeth<ScalarAlgo<SWTPG_ALGO_FIR_IQR, false>, DUMP>(kp, s);
+    case Policy::Wib2Simple: return launch_wib2<PackedSimpleWib2, DUMP>(kp, s);
+    case Policy::Wib2AbsRs: return launch_wib2<PackedRsIqrWib2, DUMP>(kp, s);
+    case Policy::Wib2Fir: return launch_wib2<PackedFirIqr, DUMP>(kp, s);
+    case Policy::Wib2FirAnyTaps: return launch_wib2<PackedFirIqrAnyTaps, DUMP>(kp, s);
+    case Policy::Wib2ScalarSimple: return launch_wib2<ScalarAlgo<SWTPG_ALGO_SIMPLE_THRESHOLD, true>, DUMP>(kp, s);
+    case Policy::Wib2ScalarAbsRs: return launch_wib2<ScalarAlgo<SWTPG_ALGO_ABS_RS, true>, DUMP>(kp, s);
+    case Policy::Wib2ScalarFir: return launch_wib2<ScalarAlgo<SWTPG_ALGO_FIR_IQR, true>, DUMP>(kp, s);
   }
   return cudaErrorNotSupported;
 }
@@ -300,7 +251,7 @@ launch_groups(const swtpg_handle* h, const void* d_frames, const uint32_t* d_nun
               int16_t* ped, int16_t* wav, cudaStream_t s)
 {
   for (const ConfGroup& g : h->conf_groups) {
-    const cudaError_t e = launch<DUMP>(h, h->confs[g.conf], make_params(h, g, d_frames, d_nunits, stride, d_tps, d_count, ped, wav), s);
+    const cudaError_t e = launch<DUMP>(h->confs[g.conf].policy, make_params(h, g, d_frames, d_nunits, stride, d_tps, d_count, ped, wav), s);
     if (e != cudaSuccess)
       return e;
   }
@@ -338,6 +289,23 @@ form_conf_groups(swtpg_handle* h)
   return SWTPG_OK;
 }
 
+// The SV_RS_FACTOR row (u16x2 by lane) of 64-channel state group g: the link's per-channel table h->h_rs_factor where it has one,
+// else its configuration's factor.
+void
+rs_factor_row(const swtpg_handle* h, uint32_t g, uint32_t* row)
+{
+  const uint32_t link = g / h->groups_per_link, sub = g % h->groups_per_link;
+  for (uint32_t lane = 0; lane < 32; ++lane) {
+    uint32_t lo = h->link_rs_factor[link], hi = lo;
+    if (h->h_rs_factor && h->rs_table_link[link]) {
+      const uint16_t* f = h->h_rs_factor + size_t(link) * h->channels + sub * 64 + 2 * lane;
+      lo = f[0];
+      hi = f[1];
+    }
+    row[lane] = lo | (hi << 16);
+  }
+}
+
 swtpg_status
 reset_state(swtpg_handle* h)
 {
@@ -345,17 +313,11 @@ reset_state(swtpg_handle* h)
   // hit threshold: the link's table, else its configuration's threshold, so that every link has a valid row
   std::vector<uint32_t> st(size_t(h->n_groups) * kStateWordsPerGroup, 0u);
   for (uint32_t g = 0; g < h->n_groups; ++g) {
+    rs_factor_row(h, g, &st[size_t(g) * kStateWordsPerGroup + SV_RS_FACTOR * 32]);
     const uint32_t link = g / h->groups_per_link, sub = g % h->groups_per_link;
     const std::vector<uint16_t>& table = h->link_thresholds[link];
     for (uint32_t lane = 0; lane < 32; ++lane) {
-      uint32_t lo = h->link_rs_factor[link], hi = lo;
-      if (h->h_rs_factor && h->rs_table_link[link]) {
-        const uint16_t* f = h->h_rs_factor + size_t(link) * h->channels + sub * 64 + 2 * lane;
-        lo = f[0];
-        hi = f[1];
-      }
-      st[size_t(g) * kStateWordsPerGroup + SV_RS_FACTOR * 32 + lane] = lo | (hi << 16);
-      lo = hi = h->confs[h->link_conf[link]].threshold;
+      uint32_t lo = h->confs[h->link_conf[link]].threshold, hi = lo;
       if (!table.empty()) {
         lo = table[sub * 64 + 2 * lane];
         hi = table[sub * 64 + 2 * lane + 1];
@@ -383,7 +345,7 @@ reset_adc_stats(swtpg_handle* h)
   return SWTPG_OK;
 }
 
-// Rewrites the SV_RS_FACTOR rows of links [link0, link0 + n) from h->h_rs_factor (or each link's configured factor): ONE strided
+// Rewrites the SV_RS_FACTOR rows of links [link0, link0 + n) (rs_factor_row): ONE strided
 // asynchronous copy on the compute stream, i.e. ordered before every kernel launched after this call and after every kernel
 // launched before it. The source is pageable, so the runtime has staged it when the call returns.
 swtpg_status
@@ -391,18 +353,8 @@ upload_rs_factor_rows(swtpg_handle* h, uint32_t link0, uint32_t n)
 {
   const uint32_t g0 = link0 * h->groups_per_link, ng = n * h->groups_per_link;
   std::vector<uint32_t> rows(size_t(ng) * 32);
-  for (uint32_t g = 0; g < ng; ++g) {
-    const uint32_t link = (g0 + g) / h->groups_per_link, sub = (g0 + g) % h->groups_per_link;
-    for (uint32_t lane = 0; lane < 32; ++lane) {
-      uint32_t lo = h->link_rs_factor[link], hi = lo;
-      if (h->h_rs_factor && h->rs_table_link[link]) {
-        const uint16_t* f = h->h_rs_factor + size_t(link) * h->channels + sub * 64 + 2 * lane;
-        lo = f[0];
-        hi = f[1];
-      }
-      rows[size_t(g) * 32 + lane] = lo | (hi << 16);
-    }
-  }
+  for (uint32_t g = 0; g < ng; ++g)
+    rs_factor_row(h, g0 + g, &rows[size_t(g) * 32]);
   SW_CUDA(h, cudaMemcpy2DAsync(h->d_state + size_t(g0) * kStateWordsPerGroup + SV_RS_FACTOR * 32, size_t(kStateWordsPerGroup) * 4, rows.data(), 128,
                                128, ng, cudaMemcpyHostToDevice, h->stream));
   return SWTPG_OK;
@@ -527,44 +479,42 @@ classify_config(int32_t format, const swtpg_link_config& in, TpgConf* out, const
     swtpg_firwin_int(7, 0.1, 1 << c.tap_exponent, c.fir_taps);
     c.fir_taps[7] = 0;
   }
-  // Packed fast path validity (see PackedSimpleWibEth)
-  c.fast_simple = c.algorithm == SWTPG_ALGO_SIMPLE_THRESHOLD && c.threshold <= 32767 &&
-                  (wib2 || (c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000));
-
-  c.fast_rs = !wib2 && (c.algorithm == SWTPG_ALGO_ABS_RS || c.algorithm == SWTPG_ALGO_STANDARD_RS) && c.threshold <= 32767 &&
-              c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000;
-  // WIB2 AbsRS fast path validity (see PackedRsIqrWib2); threshold >= 1 is enforced above for the algorithm as such
-  if (wib2 && c.algorithm == SWTPG_ALGO_ABS_RS && c.threshold >= 1) {
-    const uint32_t e = c.tap_exponent, mult = 1u << e;
-    const uint64_t sigma_max = (1u << 15) / (uint64_t(mult) * c.threshold);
-    // thresholds sigma * threshold are compared by the bf16 comparator (valid up to 32640) and built by a packed multiply-add
-    // (no carry between the halves while (sigmaMax + 3) * threshold < 2^16); outside that range every group takes the
-    // exact-threshold tier (plain signed compares on the 64-bit-lane product, like the reference's _mm256_cmpgt_epi16)
-    const bool packed_ok = e >= 1 && e <= 10;
-    const bool range_ok = (sigma_max + 3) * c.threshold < 65536 && sigma_max * c.threshold <= 32640;
-    c.fast_rs_wib2 = packed_ok;
-    c.fir_force_exact = packed_ok && !range_ok;
-  }
-  // Packed FIR fast path validity (see PackedFirIqr): binomial taps, and (sigmaMax + 3) * multiplier * threshold < 2^16
-  {
-    static const int16_t kBinomial[8] = { 1, 6, 15, 20, 15, 6, 1, 0 };
-    bool taps_ok = true;
-    for (int i = 0; i < 8; ++i)
-      taps_ok &= c.fir_taps[i] == kBinomial[i];
-    const uint32_t e = c.tap_exponent, mult = 1u << e;
-    const uint64_t sigma_max = (1u << 15) / (mult * 5u);
-    // The packed policies build sigma * multiplier * threshold with one multiply-add (no carry between the halves while
-    // (sigmaMax + 3) * K < 2^16) and compare through the bf16 comparator, which orders like signed int16 only up to 32640:
-    // K = multiplier * threshold with sigmaMax * K <= 32640 (threshold <= 5 at the reference's exponent 6). Beyond that the
-    // reference's _mm256_cmpgt_epi16 sees the product as a NEGATIVE int16 once a channel's IQR is large enough, so such
-    // configurations run the same packed trackers and filter with the exact-threshold tier forced on for every group.
-    const uint64_t K = uint64_t(mult) * c.threshold;
-    const bool packed_ok = c.algorithm == SWTPG_ALGO_FIR_IQR && e >= 1 && e <= 10;
-    const bool range_ok = (sigma_max + 3) * K < 65536 && sigma_max * K <= 32640;
-    c.fast_fir = packed_ok && taps_ok;      // binomial cascade
-    c.fast_fir_any = packed_ok && !taps_ok; // any other taps[0..6]: packed multiply-add chain (PackedFirIqrAnyTaps)
-    if (packed_ok && !range_ok)
-      c.fir_force_exact = true;
+  // The policy: a packed fast path where the configuration is inside its validity range (see the policy), else the reference
+  // arithmetic (ScalarAlgo).
+  auto by_format = [wib2](Policy wibeth, Policy wib2_policy) { return wib2 ? wib2_policy : wibeth; };
+  const bool acc_ok = c.frugal_acc_limit >= 1 && c.frugal_acc_limit <= 1000;
+  const bool thr_ok = c.threshold <= 32767;
+  // The packed IQR-threshold trackers (FIR + IQR, WIB2 AbsRS) need 1 <= tap_exponent <= 10. They build sigma * K with one
+  // multiply-add (no carry between the halves while (sigmaMax + 3) * K < 2^16) and compare through the bf16 comparator, which
+  // orders like signed int16 only up to 32640. Beyond that the reference's _mm256_cmpgt_epi16 sees the product as a NEGATIVE
+  // int16 once a channel's IQR is large enough, so such configurations run the same packed trackers with the exact-threshold
+  // tier (plain signed compares on the 64-bit-lane product) forced on for every group.
+  const bool iqr_ok = c.tap_exponent >= 1 && c.tap_exponent <= 10;
+  const uint32_t mult = 1u << c.tap_exponent;
+  auto exact_tier = [](uint64_t sigma_max, uint64_t K) { return !((sigma_max + 3) * K < 65536 && sigma_max * K <= 32640); };
+  switch (c.algorithm) {
+    case SWTPG_ALGO_SIMPLE_THRESHOLD:
+      c.policy = thr_ok && (wib2 || acc_ok) ? by_format(Policy::WibEthSimple, Policy::Wib2Simple)
+                                            : by_format(Policy::WibEthScalarSimple, Policy::Wib2ScalarSimple);
+      break;
+    case SWTPG_ALGO_ABS_RS:
+      if (wib2) { // K = threshold (>= 1, checked above), sigmaMax = 2^15 / (multiplier * threshold)
+        c.policy = iqr_ok ? Policy::Wib2AbsRs : Policy::Wib2ScalarAbsRs;
+        c.fir_force_exact = iqr_ok && exact_tier((1u << 15) / (uint64_t(mult) * c.threshold), c.threshold);
+      } else {
+        c.policy = thr_ok && acc_ok ? Policy::WibEthAbsRs : Policy::WibEthScalarAbsRs;
+      }
+      break;
+    case SWTPG_ALGO_STANDARD_RS: c.policy = thr_ok && acc_ok ? Policy::WibEthStandardRs : Policy::WibEthScalarStandardRs; break;
+    case SWTPG_ALGO_FIR_IQR: { // K = multiplier * threshold, sigmaMax = 2^15 / (multiplier * 5): threshold <= 5 at exponent 6
+      static const int16_t kBinomial[8] = { 1, 6, 15, 20, 15, 6, 1, 0 };
+      const bool binomial = memcmp(c.fir_taps, kBinomial, sizeof kBinomial) == 0; // the cascade, else the multiply-add chain
+      c.policy = !iqr_ok  ? by_format(Policy::WibEthScalarFir, Policy::Wib2ScalarFir)
+                 : binomial ? by_format(Policy::WibEthFir, Policy::Wib2Fir)
+                            : by_format(Policy::WibEthFirAnyTaps, Policy::Wib2FirAnyTaps);
+      c.fir_force_exact = iqr_ok && exact_tier((1u << 15) / (mult * 5u), uint64_t(mult) * c.threshold);
+      break;
+    }
   }
   *out = c;
   return SWTPG_OK;
@@ -580,7 +530,7 @@ threshold_table_allowed(int32_t format, int32_t algorithm)
 }
 
 // Whether links of configurations a and b can run in one launch: they agree in every field their algorithm reads (the kernel
-// parameters the policies of launch() consume). The policy flags follow from those fields. rs_memory_factor is per-link state
+// parameters the policies of launch() consume). The policy follows from those fields. rs_memory_factor is per-link state
 // (SV_RS_FACTOR rows), not a kernel parameter, so it never splits a group.
 bool
 same_group(int32_t format, const TpgConf& a, const TpgConf& b)

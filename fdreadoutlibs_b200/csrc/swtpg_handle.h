@@ -24,6 +24,28 @@ struct TpSorter;
 // One TPG configuration (swtpg_create's or a link's, swtpg_set_link_config), normalised — default taps and tap exponent
 // filled in — and classified: which policy of the launch table runs it. classify_config (swtpg_capi.cu) is the only place
 // that makes one.
+// The kernel policy a configuration runs (launch, swtpg_capi.cu): a packed fast path (swtpg_kernels.cuh) where the configuration
+// is inside its validity range, else ScalarAlgo, the reference arithmetic.
+enum class Policy : uint8_t
+{
+  WibEthSimple,     // PackedSimpleWibEthPipe
+  WibEthAbsRs,      // PackedRsWibEth<false>
+  WibEthStandardRs, // PackedRsWibEth<true>
+  WibEthFir,        // PackedFirIqr: binomial taps
+  WibEthFirAnyTaps, // PackedFirIqrAnyTaps
+  WibEthScalarSimple,
+  WibEthScalarAbsRs,
+  WibEthScalarStandardRs,
+  WibEthScalarFir,
+  Wib2Simple,     // PackedSimpleWib2
+  Wib2AbsRs,      // PackedRsIqrWib2
+  Wib2Fir,        // PackedFirIqr
+  Wib2FirAnyTaps, // PackedFirIqrAnyTaps
+  Wib2ScalarSimple,
+  Wib2ScalarAbsRs,
+  Wib2ScalarFir,
+};
+
 struct TpgConf
 {
   int32_t algorithm = 0;
@@ -32,7 +54,7 @@ struct TpgConf
   uint16_t rs_scale_factor = 0;
   int16_t fir_taps[SWTPG_MAX_TAPS] = {};
   uint8_t tap_exponent = 0;
-  bool fast_simple = false, fast_fir = false, fast_rs = false, fast_rs_wib2 = false, fast_fir_any = false;
+  Policy policy = Policy::WibEthScalarSimple;
   bool fir_force_exact = false; // packed FIR / WIB2-AbsRS trackers with the exact-threshold tier on every group (classify_config)
 };
 

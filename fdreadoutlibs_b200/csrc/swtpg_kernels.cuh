@@ -9,12 +9,10 @@
 //   struct Algo { load(state, lane); seed(S); tick<...>(S, ctx, t); store(state, lane); }
 // `Scalar*` policies do the arithmetic one channel at a time in 32-bit registers, exactly as written in the
 // reference (any configuration); `Packed*` policies are the production fast paths on packed s16x2 registers and are
-// selected by the host only for configurations inside their documented validity range (swtpg_capi.cu: pick_kernel).
+// selected by the host only for configurations inside their documented validity range (swtpg_capi.cu: classify_config).
 #pragma once
 
 #include "swtpg_device.cuh"
-
-#include <type_traits>
 
 namespace swtpg {
 
@@ -185,7 +183,13 @@ template<int ALGO, bool WIB2>
 struct ScalarAlgo
 {
   static constexpr int kGroupUnroll = 1;
-  static constexpr int kWarpsPerSm = 0; // persistent single-warp CTAs per SM the WIBEth launch aims for; 0 = as many as fit
+  static constexpr bool kNeedsUnitTs = true; // tick() emits TPs with TickCtx::ts; the packed policies stage hits, and
+                                             // HitStage::flush reads the unit's timestamp itself
+  // One-warp-per-CTA WIBEth launch (launch_wibeth_geo): kWarpsPerSm persistent warps per SM (0 = as many as fit); from
+  // kFullLoadWarpsPerSm x SMs + kFullLoadExtraLinks links on, kFullLoadWarpsPerSm and slices even for whole rounds (0 = never).
+  static constexpr int kWarpsPerSm = 0;
+  static constexpr int kFullLoadWarpsPerSm = 0;
+  static constexpr int kFullLoadExtraLinks = 0;
   static constexpr int kQuadCtasPerSm = 0; // WIBEth: > 0 = run wibeth_quad_kernel (CTA of 4 links + producer warp) with that many CTAs per SM
   static constexpr int kWib2MinCtas = 1;   // WIB2: minimum CTAs per SM the register allocation must allow
   ChanRegs c[2];
@@ -443,15 +447,20 @@ struct ScalarAlgo
 // PIPE = true: the two-stage software pipeline, the form every WIBEth SimpleThreshold launch runs (a warp runs at the speed of
 // its dependent chain; since the accumulator reset is one IMAD that chain is short enough for 20 such warps per SM to beat 28
 // straight-line ones); PIPE = false: straight-line groups, fewer registers and instructions — the WIB2 kernel's form and the
-// base of the running-sum policies. The host picks per launch (launch_wibeth_simple, swtpg_capi.cu).
+// base of the running-sum policies.
 template<bool PIPE>
 struct PackedSimpleT
 {
   static constexpr int kGroupUnroll = 4;
-  // persistent warps per SM, measured: 5 per sub-partition for the straight-line form (profiles/r01_warps_sweep.txt), 4 for the
-  // pipelined one below one round of links (92 registers; profiles/r02_simple_pipeline_sweep.txt); from 2960 links on the host
-  // asks for 20 (profiles/r02_pipelined_full_load_probe.txt, r02_warps_crossover_probe.txt)
-  static constexpr int kWarpsPerSm = PIPE ? 16 : 20;
+  static constexpr bool kNeedsUnitTs = false;
+  // Launch of the pipelined form (see ScalarAlgo; the running sums set their own): 4 persistent warps per sub-partition below one
+  // round of links (92 registers; profiles/r02_simple_pipeline_sweep.txt), from 2960 links on B200 (20 x 148 SMs) 5 and slices
+  // for whole rounds too (profiles/r02_pipelined_full_load_probe.txt, r02_warps_crossover_probe.txt): a launch below one link per
+  // warp of the 20-per-SM grid is bound by what ONE warp does per tick. 2960 links: 66.5 % of the HBM peak with 20 warps per SM
+  // against 64.2 % with 16; 2500 links: 56.7 / 58.2 %.
+  static constexpr int kWarpsPerSm = 16;
+  static constexpr int kFullLoadWarpsPerSm = 20;
+  static constexpr int kFullLoadExtraLinks = 0;
   static constexpr int kQuadCtasPerSm = 0; // one warp per CTA: the CTA form measured slower for this policy (65.4 % against
                                            // 68.2 % of the HBM peak at 5920 links, profiles/r02_quad_form_probe.txt)
   static constexpr int kWib2MinCtas = 5;
@@ -763,7 +772,11 @@ template<bool STANDARD>
 struct PackedRsWibEth : PackedSimpleWibEth
 {
   static constexpr int kGroupUnroll = 2;
-  static constexpr int kWarpsPerSm = STANDARD ? 20 : 16; // AbsRS: 4 warps per sub-partition beat 5 by 3 % (same sweep)
+  // AbsRS: 4 warps per sub-partition beat 5 by 3 % (same sweep). Above one round of a 20-per-SM grid, 20 warps per SM with
+  // halving slices, whole rounds included: AbsRS 28.7 -> 30.4 % of the HBM peak at 5920 links (its own 16 per SM hold for whole
+  // links: 20 unsliced 26.9 %), StandardRS 35.4 -> 36.7 % (profiles/r02_warps_crossover_probe.txt).
+  static constexpr int kWarpsPerSm = STANDARD ? 20 : 16;
+  static constexpr int kFullLoadExtraLinks = 1;
   uint32_t RS1, MRq, AR;     // RS + 1 (carried value, after median subtraction); 1 - median_RS; (acc_RS - 1) as fp16 subnormal
   int f_lo, f_hi, nf_lo, nf_hi, scale;
   template<int ROW_WORDS = 28>
@@ -922,6 +935,7 @@ struct PackedRsWibEth : PackedSimpleWibEth
 struct PackedFirIqr
 {
   static constexpr int kGroupUnroll = 2;
+  static constexpr bool kNeedsUnitTs = false;
   static constexpr int kWarpsPerSm = 12; // 3 warps per sub-partition: 3 % faster than the 16 its 128 registers allow (same sweep)
   static constexpr int kWib2MinCtas = 5;
   static constexpr int kQuadCtasPerSm = 4; // CTA form, 16 consumer warps per SM (measured: 4 CTAs 29.8 %, 5 CTAs 27.8 %, profiles/r02_fir_forms.txt)
@@ -1435,27 +1449,91 @@ struct PackedRsIqrWib2 : PackedFirIqr
 };
 
 // =====================================================================================================================
-// WIBEth kernel: persistent warps, one link (64 channels) at a time per warp, per-warp TMA ring of CHUNK_TICKS-tick stages.
+// What the three kernels share: a link's place in the batch, the shared-memory layout, and the consumer side of a work item
+// (its close, the cursor re-arm). Each kernel keeps its own producer and hand-out logic, and its own chunk step (seed, group
+// loop, debug dumps): as one shared function it changed ptxas's register allocation of the one-warp-per-CTA kernel (92 -> 94
+// registers for the production policy) and of the WIB2 kernel. For the same reason the one-warp-per-CTA kernel also writes out
+// its hit-staging placement and cursor re-arm; every instance compiles to the same SASS as with them written out per kernel.
+// =====================================================================================================================
+__device__ __forceinline__ uint32_t
+units_of(const KernelParams& p, uint32_t link)
+{
+  return p.n_units ? p.n_units[link] : p.units_stride;
+}
+template<uint32_t UNIT_BYTES> // a WIBEth frame or a WIB2 superchunk
+__device__ __forceinline__ const uint8_t*
+base_of(const KernelParams& p, uint32_t link)
+{
+  return p.frames + size_t(link) * p.units_stride * UNIT_BYTES;
+}
+
+// Dynamic shared memory of one CTA: [stages | mbarriers | hit staging (16 B + 4 B per record) of each consumer warp | hit
+// counters | link FIFO].
+template<size_t STAGE_BYTES, size_t BAR_BYTES, int HIT_WARPS, size_t FIFO_BYTES>
+struct SmemLayout
+{
+  static constexpr size_t align16(size_t x) { return (x + 15) & ~size_t(15); }
+  static constexpr size_t bars = align16(STAGE_BYTES);
+  static constexpr size_t hits = align16(bars + BAR_BYTES);
+  static constexpr size_t aux = hits + size_t(HIT_WARPS) * HitStage::kCap * 16;
+  static constexpr size_t counts = aux + size_t(HIT_WARPS) * HitStage::kCap * 4;
+  static constexpr size_t fifo = align16(counts + size_t(HIT_WARPS) * 4);
+  static constexpr size_t total = fifo + FIFO_BYTES;
+
+  static __device__ __forceinline__ void place_hits(HitStage& h, uint8_t* smem, uint32_t warp)
+  {
+    h.buf = reinterpret_cast<uint4*>(smem + hits) + size_t(warp) * HitStage::kCap;
+    h.aux = reinterpret_cast<uint32_t*>(smem + aux) + size_t(warp) * HitStage::kCap;
+    h.cnt = reinterpret_cast<uint32_t*>(smem + counts) + warp;
+  }
+};
+
+// End of a work item: drain the policy's software pipeline, flush the staged hits (records carry unit indices of THIS link),
+// store the state of 64-channel group `group` and its FIR ring phase after `ticks` ticks.
+template<bool WIB2_UNITS, class Algo>
+__device__ __forceinline__ void
+close_item(Algo& algo, const TickCtx& ctx, const HitStage& hits, uint32_t* st, uint32_t group, uint32_t ticks, uint32_t lane)
+{
+  const KernelParams& p = *ctx.p;
+  algo.template finish_link<WIB2_UNITS>(ctx);
+  Algo::template flush<WIB2_UNITS>(hits, p.sink, ctx.link_base, ctx.link, lane);
+  const uint32_t k_end = algo.phase_after(ticks);
+  algo.store(st, lane, k_end);
+  if (lane == 0)
+    p.group_flags[group] = kFlagInitialized | (k_end << 8);
+}
+
+// One lane of each of the launch's `participants` calls this after its last claim: the last one out re-arms the cursor for the
+// next launch (launches of one handle are stream-ordered: state is carried).
+__device__ __forceinline__ void
+rearm_cursor(const KernelParams& p, uint32_t participants)
+{
+  __threadfence();
+  if (atomicAdd(p.link_cursor + 1, 1u) == participants - 1u) {
+    p.link_cursor[0] = 0u;
+    p.link_cursor[1] = 0u;
+  }
+}
+
+// Ring of both WIBEth forms: 2 stages of 32 ticks per link (7 KB). Measured best on B200 (profiles/r01_geometry_sweep.txt): the
+// kernels are issue-bound, so deeper rings do not help.
+constexpr int kWibEthRowBytes = 112;
+constexpr int kWibEthStages = 2, kWibEthChunkTicks = 32;
+constexpr uint32_t kWibEthChunkBytes = kWibEthRowBytes * kWibEthChunkTicks;
+constexpr uint32_t kWibEthChunksPerUnit = 64 / kWibEthChunkTicks;
+static_assert(64 % kWibEthChunkTicks == 0, "chunk must divide the frame");
+
+// =====================================================================================================================
+// WIBEth kernel: persistent single-warp CTAs, one link (64 channels) at a time per warp, private TMA ring of chunk stages.
 // Warp w of the grid starts on link w; every further link is CLAIMED from a global cursor when the warp's producer runs
 // out of chunks, so links go to whichever warp is free first: a warp that shares its SM sub-partition with one more
 // neighbour, or that drew longer links in a ragged batch, simply takes fewer of them. The ring is refilled by lane 0 from
-// a producer cursor that runs NSTAGE chunks ahead of the consumer ACROSS link boundaries, so a warp never drains its
-// pipeline between links; the producer hands the links it chose to the consumer through a small warp-uniform FIFO.
+// a producer cursor that runs kWibEthStages chunks ahead of the consumer ACROSS link boundaries, so a warp never drains its
+// pipeline between links; the producer hands the links it chose to the consumer through a small warp-uniform FIFO. Single-warp
+// CTAs let the block scheduler spread the resident warps evenly over an SM's four sub-partitions.
 // =====================================================================================================================
-constexpr int kWibEthRowBytes = 112;
-
-// Dynamic shared memory of one CTA: [stages | mbarriers | hit staging (16 B + 4 B per record) | hit counters | link FIFOs].
-template<int WARPS, int NSTAGE, int CHUNK_TICKS>
-struct WibEthSmem
-{
-  static constexpr size_t align16(size_t x) { return (x + 15) & ~size_t(15); }
-  static constexpr size_t bars = align16(size_t(WARPS) * NSTAGE * kWibEthRowBytes * CHUNK_TICKS);
-  static constexpr size_t hits = align16(bars + size_t(WARPS) * NSTAGE * 8);
-  static constexpr size_t aux = hits + size_t(WARPS) * HitStage::kCap * 16;
-  static constexpr size_t counts = aux + size_t(WARPS) * HitStage::kCap * 4;
-  static constexpr size_t fifo = align16(counts + size_t(WARPS) * 4);
-  static constexpr size_t total = fifo + size_t(WARPS) * 32; // 8-entry link FIFO per warp
-};
+constexpr uint32_t kWibEthFifo = 8; // links in flight; power of two; in shared memory so the tick loop carries no registers for it
+using WibEthSmem = SmemLayout<size_t(kWibEthStages) * kWibEthChunkBytes, size_t(kWibEthStages) * 8, 1, kWibEthFifo * 4>;
 
 // Whole warp: wait until *counter == want (acquire: what the publishing warp stored before its release is visible afterwards).
 __device__ __noinline__ void
@@ -1470,52 +1548,47 @@ wait_for_slices(const uint32_t* counter, uint32_t want)
   }
 }
 
-template<class Algo, int WARPS, int NSTAGE, int CHUNK_TICKS, bool DUMP, int MIN_CTAS = 1>
-__global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
+template<class Algo, bool DUMP>
+__global__ void __launch_bounds__(32, 1)
 wibeth_kernel(const KernelParams p)
 {
-  static_assert(64 % CHUNK_TICKS == 0, "chunk must divide the frame");
-  constexpr int kChunkBytes = kWibEthRowBytes * CHUNK_TICKS;
-  constexpr int kChunksPerUnit = 64 / CHUNK_TICKS;
+  constexpr int NSTAGE = kWibEthStages;
+  constexpr uint32_t kChunkBytes = kWibEthChunkBytes, kChunksPerUnit = kWibEthChunksPerUnit;
   extern __shared__ __align__(128) uint8_t smem[];
 
-  // warp index through a shuffle: tells the compiler it is warp-uniform, so the ring bookkeeping runs on the uniform datapath
+  // the warp's index (0) through a shuffle: without it ptxas allocates the tick loop's registers differently (92 -> 94 for the
+  // production policy)
   const uint32_t warp = __shfl_sync(0xFFFFFFFFu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31u;
-  const uint32_t warps_total = gridDim.x * WARPS;
-  const uint32_t first_link = blockIdx.x * WARPS + warp; // this warp's first work item
+  const uint32_t warps_total = gridDim.x;
+  const uint32_t first_link = blockIdx.x + warp; // this warp's first work item
   const uint32_t n_items = p.n_links << p.parts_log2;
   if (first_link >= n_items)
-    return; // warps are fully independent: no block-level barrier anywhere below
+    return;
 
-  using L = WibEthSmem<WARPS, NSTAGE, CHUNK_TICKS>;
   uint8_t* stages = smem + size_t(warp) * NSTAGE * kChunkBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L::bars) + warp * NSTAGE;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + WibEthSmem::bars) + warp * NSTAGE;
   HitStage hits;
-  hits.buf = reinterpret_cast<uint4*>(smem + L::hits) + size_t(warp) * HitStage::kCap;
-  hits.aux = reinterpret_cast<uint32_t*>(smem + L::aux) + size_t(warp) * HitStage::kCap;
-  hits.cnt = reinterpret_cast<uint32_t*>(smem + L::counts) + warp;
-
-  auto units_of = [&](uint32_t link) -> uint32_t { return p.n_units ? p.n_units[link] : p.units_stride; };
-  auto base_of = [&](uint32_t link) -> const uint8_t* { return p.frames + size_t(link) * p.units_stride * SWTPG_WIBETH_FRAME_BYTES; };
+  hits.buf = reinterpret_cast<uint4*>(smem + WibEthSmem::hits) + size_t(warp) * HitStage::kCap;
+  hits.aux = reinterpret_cast<uint32_t*>(smem + WibEthSmem::aux) + size_t(warp) * HitStage::kCap;
+  hits.cnt = reinterpret_cast<uint32_t*>(smem + WibEthSmem::counts) + warp;
 
   // Producer cursor: the next chunk to request is pr_src; pr_left chunks remain in link pr_link. Every lane keeps the same
   // (warp-uniform) copy, so the bookkeeping runs on the uniform datapath; only lane 0 talks to the mbarrier / copy engine
   // and to the global link cursor.
   // FIFO of links the producer has started and the consumer has not: the producer is at most NSTAGE chunks ahead and every
   // link it starts has >= kChunksPerUnit chunks, so at most ceil(NSTAGE / kChunksPerUnit) + 1 links are in flight.
-  constexpr uint32_t kFifo = 8; // power of two; lives in shared memory so the tick loop carries no registers for it
-  static_assert((NSTAGE + kChunksPerUnit - 1) / kChunksPerUnit + 1 <= int(kFifo), "link FIFO too short for this ring geometry");
-  volatile uint32_t* fifo = reinterpret_cast<volatile uint32_t*>(smem + L::fifo) + warp * kFifo;
+  static_assert((NSTAGE + kChunksPerUnit - 1) / kChunksPerUnit + 1 <= kWibEthFifo, "link FIFO too short for this ring geometry");
+  volatile uint32_t* fifo = reinterpret_cast<volatile uint32_t*>(smem + WibEthSmem::fifo) + warp * kWibEthFifo;
   uint32_t fifo_head = 0, fifo_n = 0;
   auto fifo_push = [&](uint32_t link) { // whole warp, converged; every lane holds the same `link`
     if (lane == 0)
-      fifo[(fifo_head + fifo_n) & (kFifo - 1u)] = link;
+      fifo[(fifo_head + fifo_n) & (kWibEthFifo - 1u)] = link;
     ++fifo_n;
     __syncwarp();
   };
   auto fifo_pop = [&]() -> uint32_t {
     const uint32_t link = fifo[fifo_head];
-    fifo_head = (fifo_head + 1u) & (kFifo - 1u);
+    fifo_head = (fifo_head + 1u) & (kWibEthFifo - 1u);
     --fifo_n;
     return link;
   };
@@ -1532,7 +1605,7 @@ wibeth_kernel(const KernelParams p)
     }
     if (p.link_ids != nullptr) // one configuration group of several: its (item mod n_links)-th link
       link = p.link_ids[link];
-    const uint32_t n = units_of(link);
+    const uint32_t n = units_of(p, link);
     if (p.slice_geom) { // halving slices: n/2, n/4, ... and the rest (slice k starts ceil(n / 2^k) units before the end)
       u0 = n - ((n + (1u << part) - 1u) >> part);
       u1 = part + 1u == (1u << p.parts_log2) ? n : n - ((n + (2u << part) - 1u) >> (part + 1u));
@@ -1548,7 +1621,7 @@ wibeth_kernel(const KernelParams p)
   auto slices_before = [&](uint32_t link, uint32_t part, uint32_t u0) -> uint32_t {
     if (!p.slice_geom)
       return min(part, u0);
-    const uint32_t n = units_of(link);
+    const uint32_t n = units_of(p, link);
     return min(part, n > 1u ? 32u - uint32_t(__clz(int(n - 1u))) : 0u);
   };
   // same value in every lane -> uniform register, so that the producer's per-chunk bookkeeping stays on the uniform datapath
@@ -1562,7 +1635,7 @@ wibeth_kernel(const KernelParams p)
     pr_left = uniform((u1 - u0) * kChunksPerUnit);
     if (pr_left != 0) {
       fifo_push(item);
-      pr_src = base_of(uniform(link)) + size_t(uniform(u0)) * SWTPG_WIBETH_FRAME_BYTES + 32;
+      pr_src = base_of<SWTPG_WIBETH_FRAME_BYTES>(p, uniform(link)) + size_t(uniform(u0)) * SWTPG_WIBETH_FRAME_BYTES + 32;
       pr_in_unit = 0;
     }
   };
@@ -1623,7 +1696,7 @@ wibeth_kernel(const KernelParams p)
   while (fifo_n != 0) { // the producer started this link NSTAGE chunks ago (or at start-up)
     uint32_t link, u0, n_units; // n_units: end of the slice
     const uint32_t part = slice_of(fifo_pop(), link, u0, n_units);
-    const uint8_t* link_base = base_of(link);
+    const uint8_t* link_base = base_of<SWTPG_WIBETH_FRAME_BYTES>(p, link);
     uint32_t* st = p.state + size_t(link) * kStateWordsPerGroup;
     // A later slice of a link continues from the state its predecessor stored: wait until the NON-EMPTY slices before it are
     // done (with fewer units than slices some are empty and never run: exactly min(part, u0) of the earlier ones are not). By
@@ -1642,12 +1715,10 @@ wibeth_kernel(const KernelParams p)
     for (uint32_t unit = u0; unit < n_units; ++unit) {
       ctx.tick_base = 0u; // 64 ticks per unit = 0 mod 8: the FIR ring phase at a unit's first tick is the slice's initial one
       ctx.unit = unit;
-      if constexpr (!std::is_same<Algo, PackedSimpleWibEth>::value && !std::is_same<Algo, PackedSimpleWibEthPipe>::value) {
-        // DAQEthHeader word 1 = timestamp (docs/README.md:81); the packed path reads it when it flushes hits
+      if constexpr (Algo::kNeedsUnitTs) // DAQEthHeader word 1 = timestamp (docs/README.md:81)
         ctx.ts = *reinterpret_cast<const unsigned long long*>(link_base + size_t(unit) * SWTPG_WIBETH_FRAME_BYTES + 8);
-      }
 #pragma unroll 1
-      for (int t0 = 0; t0 < 64; t0 += CHUNK_TICKS) {
+      for (int t0 = 0; t0 < 64; t0 += kWibEthChunkTicks) {
         mbar_wait(&bars[stg], phase);
         const uint32_t* rows = reinterpret_cast<const uint32_t*>(stages + stg * kChunkBytes);
         if (need_seed) {
@@ -1655,13 +1726,12 @@ wibeth_kernel(const KernelParams p)
           need_seed = false;
         }
         constexpr int G = 4;
-        static_assert(CHUNK_TICKS % G == 0, "group must divide the chunk");
         constexpr int kGroupUnroll = Algo::kGroupUnroll;
         algo.begin_chunk(rows, pp);
 #pragma unroll kGroupUnroll
-        for (int tt = 0; tt < CHUNK_TICKS; tt += G) {
+        for (int tt = 0; tt < kWibEthChunkTicks; tt += G) {
           uint32_t ped[G], wav[G];
-          algo.template group<G, DUMP>(rows + tt * (kWibEthRowBytes / 4), pp, ctx, t0 + tt, ped, wav, tt + G < CHUNK_TICKS);
+          algo.template group<G, DUMP>(rows + tt * (kWibEthRowBytes / 4), pp, ctx, t0 + tt, ped, wav, tt + G < kWibEthChunkTicks);
           if constexpr (DUMP) {
 #pragma unroll
             for (int g = 0; g < G; ++g) {
@@ -1684,12 +1754,7 @@ wibeth_kernel(const KernelParams p)
       }
     }
 
-    algo.template finish_link<false>(ctx); // drains the policy's software pipeline (deferred hit bookkeeping of the last group)
-    Algo::template flush<false>(hits, p.sink, link_base, link, lane); // records carry unit indices of THIS link
-    const uint32_t k_end = algo.phase_after((n_units - u0) * 64u);
-    algo.store(st, lane, k_end);
-    if (lane == 0)
-      p.group_flags[link] = kFlagInitialized | (k_end << 8);
+    close_item<false>(algo, ctx, hits, st, link, (n_units - u0) * 64u, lane);
     if (p.parts_log2 != 0u) { // publish the state to the warp that runs the link's next slice; the last slice re-arms the counter
       __threadfence(); // every lane's (the release alone measured the same, profiles/r02_step_form_probe.txt)
       __syncwarp();    // orders the lanes' stores before lane 0's release, which is cumulative
@@ -1699,7 +1764,6 @@ wibeth_kernel(const KernelParams p)
       }
     }
   }
-  // Last warp out re-arms the cursor for the next launch (launches of one handle are stream-ordered: state is carried).
   if (lane == 0) {
     const uint32_t active = min(warps_total, n_items);
     __threadfence();
@@ -1712,8 +1776,8 @@ wibeth_kernel(const KernelParams p)
 
 // =====================================================================================================================
 // WIBEth kernel, CTA form: 4 consumer warps + 1 producer warp work on a QUAD of 4 links in lock-step (the structure of the
-// WIB2 kernel below, where one link is four warps wide). A stage of the CTA-wide ring holds one CHUNK_TICKS-tick chunk of
-// each of the four links (four bulk copies signalled on ONE `full` barrier, released through ONE `empty` barrier with an
+// WIB2 kernel below, where one link is four warps wide). A stage of the CTA-wide ring holds one chunk of each of the four links
+// (four bulk copies signalled on ONE `full` barrier, released through ONE `empty` barrier with an
 // arrival per consumer), so a consumer's per-chunk bookkeeping is a barrier wait and an arrive — the ring cursor, the
 // source addresses and the link hand-out (first quad by block index, every further one claimed from the device-side cursor
 // four links at a time, published through a small FIFO) live in the producer warp, once per quad instead of once per link.
@@ -1722,42 +1786,26 @@ wibeth_kernel(const KernelParams p)
 constexpr int kQuad = 4;
 constexpr uint32_t kNoLink = 0xFFFFFFFFu; // quad position without a link (past the end of the group)
 constexpr uint32_t kQuadFifo = 4; // quads in flight: the producer is at most NSTAGE chunks ahead, a quad has >= kChunksPerUnit chunks
+// per stage one chunk of each link and the two barriers; per FIFO entry 4 link ids, the quad's length in units, padding
+using WibEthQuadSmem = SmemLayout<size_t(kWibEthStages) * kQuad * kWibEthChunkBytes, size_t(kWibEthStages) * 16, kQuad, kQuadFifo * 32>;
 
-template<int NSTAGE, int CHUNK_TICKS>
-struct WibEthQuadSmem
-{
-  static constexpr size_t align16(size_t x) { return (x + 15) & ~size_t(15); }
-  static constexpr size_t chunk = size_t(kWibEthRowBytes) * CHUNK_TICKS;
-  static constexpr size_t bars = align16(size_t(NSTAGE) * kQuad * chunk);
-  static constexpr size_t hits = align16(bars + size_t(NSTAGE) * 16);
-  static constexpr size_t aux = hits + size_t(kQuad) * HitStage::kCap * 16;
-  static constexpr size_t counts = aux + size_t(kQuad) * HitStage::kCap * 4;
-  static constexpr size_t fifo = align16(counts + size_t(kQuad) * 4);
-  static constexpr size_t total = fifo + kQuadFifo * 32; // per quad: 4 link ids, its length in units, padding
-};
-
-template<class Algo, int NSTAGE, int CHUNK_TICKS, bool DUMP>
+template<class Algo, bool DUMP>
 __global__ void __launch_bounds__((kQuad + 1) * 32)
 wibeth_quad_kernel(const KernelParams p)
 {
-  static_assert(64 % CHUNK_TICKS == 0, "chunk must divide the frame");
-  constexpr uint32_t kChunkBytes = kWibEthRowBytes * CHUNK_TICKS;
-  constexpr uint32_t kChunksPerUnit = 64 / CHUNK_TICKS;
+  constexpr int NSTAGE = kWibEthStages;
+  constexpr uint32_t kChunkBytes = kWibEthChunkBytes, kChunksPerUnit = kWibEthChunksPerUnit;
   static_assert((NSTAGE + kChunksPerUnit - 1) / kChunksPerUnit + 2 <= kQuadFifo, "quad FIFO too short for this ring geometry");
   extern __shared__ __align__(128) uint8_t smem[];
-  using L = WibEthQuadSmem<NSTAGE, CHUNK_TICKS>;
+  using L = WibEthQuadSmem;
   const uint32_t warp = __shfl_sync(0xFFFFFFFFu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31u;
   uint8_t* stages = smem;
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + L::bars);
   uint64_t* empty = full + NSTAGE;
   volatile uint32_t* fifo = reinterpret_cast<volatile uint32_t*>(smem + L::fifo); // [kQuadFifo][8]: links[4], units of the longest
   HitStage hits;
-  hits.buf = reinterpret_cast<uint4*>(smem + L::hits) + size_t(warp) * HitStage::kCap;
-  hits.aux = reinterpret_cast<uint32_t*>(smem + L::aux) + size_t(warp) * HitStage::kCap;
-  hits.cnt = reinterpret_cast<uint32_t*>(smem + L::counts) + warp;
+  L::place_hits(hits, smem, warp);
 
-  auto units_of = [&](uint32_t link) -> uint32_t { return p.n_units ? p.n_units[link] : p.units_stride; };
-  auto base_of = [&](uint32_t link) -> const uint8_t* { return p.frames + size_t(link) * p.units_stride * SWTPG_WIBETH_FRAME_BYTES; };
   auto link_of = [&](uint32_t item) -> uint32_t { return p.link_ids != nullptr ? p.link_ids[item] : item; }; // the group's item-th link
 
   if (threadIdx.x == 0) {
@@ -1792,7 +1840,7 @@ wibeth_quad_kernel(const KernelParams p)
           break;
 #pragma unroll
         for (int c = 0; c < kQuad; ++c) { // a group's last quad may be partial
-          nu[c] = first_link + c < p.n_links ? units_of(link_of(first_link + c)) : 0u;
+          nu[c] = first_link + c < p.n_links ? units_of(p, link_of(first_link + c)) : 0u;
           longest = max(longest, nu[c]);
         }
         if (longest != 0)
@@ -1836,11 +1884,7 @@ wibeth_quad_kernel(const KernelParams p)
         }
       }
     }
-    __threadfence(); // last CTA out re-arms the cursor for the next launch
-    if (atomicAdd(p.link_cursor + 1, 1u) == gridDim.x - 1u) {
-      p.link_cursor[0] = 0u;
-      p.link_cursor[1] = 0u;
-    }
+    rearm_cursor(p, gridDim.x);
     return;
   }
 
@@ -1863,8 +1907,8 @@ wibeth_quad_kernel(const KernelParams p)
     // the position's link through a reduction: a uniform register, as the link index was before groups (ptxas otherwise
     // needs up to 7 more registers for this kernel)
     const uint32_t link = __reduce_max_sync(0xFFFFFFFFu, entry[warp]), longest = entry[4];
-    const uint32_t n_units = link != kNoLink ? units_of(link) : 0u;
-    const uint8_t* link_base = base_of(link != kNoLink ? link : 0u);
+    const uint32_t n_units = link != kNoLink ? units_of(p, link) : 0u;
+    const uint8_t* link_base = base_of<SWTPG_WIBETH_FRAME_BYTES>(p, link != kNoLink ? link : 0u);
     uint32_t* st = p.state + size_t(link) * kStateWordsPerGroup;
     uint32_t flags = 0;
     bool need_seed = false;
@@ -1880,12 +1924,12 @@ wibeth_quad_kernel(const KernelParams p)
       const bool mine = unit < n_units;
       ctx.tick_base = unit * 64u;
       ctx.unit = unit;
-      if constexpr (!std::is_same<Algo, PackedSimpleWibEth>::value && !std::is_same<Algo, PackedSimpleWibEthPipe>::value) {
-        if (mine) // DAQEthHeader word 1 = timestamp (docs/README.md:81); the packed path reads it when it flushes hits
+      if constexpr (Algo::kNeedsUnitTs) {
+        if (mine) // DAQEthHeader word 1 = timestamp (docs/README.md:81)
           ctx.ts = *reinterpret_cast<const unsigned long long*>(link_base + size_t(unit) * SWTPG_WIBETH_FRAME_BYTES + 8);
       }
 #pragma unroll 1
-      for (int t0 = 0; t0 < 64; t0 += CHUNK_TICKS) {
+      for (int t0 = 0; t0 < 64; t0 += kWibEthChunkTicks) {
         if (unit != 0 || t0 != 0)
           mbar_wait(&full[stg], phase);
         if (mine) {
@@ -1895,13 +1939,12 @@ wibeth_quad_kernel(const KernelParams p)
             need_seed = false;
           }
           constexpr int G = 4;
-          static_assert(CHUNK_TICKS % G == 0, "group must divide the chunk");
           constexpr int kGroupUnroll = Algo::kGroupUnroll;
           algo.begin_chunk(rows, pp);
 #pragma unroll kGroupUnroll
-          for (int tt = 0; tt < CHUNK_TICKS; tt += G) {
+          for (int tt = 0; tt < kWibEthChunkTicks; tt += G) {
             uint32_t ped[G], wav[G];
-            algo.template group<G, DUMP>(rows + tt * (kWibEthRowBytes / 4), pp, ctx, t0 + tt, ped, wav, tt + G < CHUNK_TICKS);
+            algo.template group<G, DUMP>(rows + tt * (kWibEthRowBytes / 4), pp, ctx, t0 + tt, ped, wav, tt + G < kWibEthChunkTicks);
             if constexpr (DUMP) {
 #pragma unroll
               for (int g = 0; g < G; ++g) {
@@ -1926,14 +1969,8 @@ wibeth_quad_kernel(const KernelParams p)
       }
     }
 
-    if (n_units != 0) {
-      algo.template finish_link<false>(ctx);
-      Algo::template flush<false>(hits, p.sink, link_base, link, lane); // records carry unit indices of THIS link
-      const uint32_t k_end = algo.phase_after(n_units * 64u);
-      algo.store(st, lane, k_end);
-      if (lane == 0)
-        p.group_flags[link] = kFlagInitialized | (k_end << 8);
-    }
+    if (n_units != 0)
+      close_item<false>(algo, ctx, hits, st, link, n_units * 64u, lane);
   }
 }
 
@@ -1952,17 +1989,8 @@ constexpr int kWib2Warps = 4;
 constexpr uint32_t kWib2Fifo = 8;           // links in flight: the producer is at most NSTAGE superchunks ahead (+ the end marker)
 constexpr uint32_t kNoMoreLinks = 0xFFFFFFFFu;
 
-template<int NSTAGE>
-struct Wib2Smem
-{
-  static constexpr size_t align16(size_t x) { return (x + 15) & ~size_t(15); }
-  static constexpr size_t bars = align16(size_t(NSTAGE) * SWTPG_WIB2_SUPERCHUNK_BYTES);
-  static constexpr size_t hits = align16(bars + size_t(NSTAGE) * 16);
-  static constexpr size_t aux = hits + size_t(kWib2Warps) * HitStage::kCap * 16;
-  static constexpr size_t counts = aux + size_t(kWib2Warps) * HitStage::kCap * 4;
-  static constexpr size_t fifo = align16(counts + size_t(kWib2Warps) * 4);
-  static constexpr size_t total = fifo + kWib2Fifo * 4; // link FIFO, producer -> consumers
-};
+template<int NSTAGE> // per stage one superchunk and the two barriers
+using Wib2Smem = SmemLayout<size_t(NSTAGE) * SWTPG_WIB2_SUPERCHUNK_BYTES, size_t(NSTAGE) * 16, kWib2Warps, kWib2Fifo * 4>;
 
 // Algo::kWib2MinCtas caps the registers so that that many CTAs fit an SM (5 = 25 warps): +1 % for SimpleThreshold, +2 % for
 // FIR + IQR, -3.5 % for the running sum, which therefore leaves it at 1 (gpurun_out/var30: measured per policy).
@@ -1978,12 +2006,7 @@ wib2_kernel(const KernelParams p)
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + L::bars);
   uint64_t* empty = full + NSTAGE;
   HitStage hits;
-  hits.buf = reinterpret_cast<uint4*>(smem + L::hits) + size_t(warp) * HitStage::kCap;
-  hits.aux = reinterpret_cast<uint32_t*>(smem + L::aux) + size_t(warp) * HitStage::kCap;
-  hits.cnt = reinterpret_cast<uint32_t*>(smem + L::counts) + warp;
-
-  auto units_of = [&](uint32_t link) -> uint32_t { return p.n_units ? p.n_units[link] : p.units_stride; };
-  auto base_of = [&](uint32_t link) -> const uint8_t* { return p.frames + size_t(link) * p.units_stride * kUnit; };
+  L::place_hits(hits, smem, warp);
 
   if (threadIdx.x == 0) {
 #pragma unroll
@@ -2017,7 +2040,7 @@ wib2_kernel(const KernelParams p)
         if (item >= p.n_links)
           break;
         link = p.link_ids != nullptr ? p.link_ids[item] : item; // the group's item-th link
-        n_units = units_of(link);
+        n_units = units_of(p, link);
         if (n_units != 0)
           break;
       }
@@ -2027,7 +2050,7 @@ wib2_kernel(const KernelParams p)
         mbar_arrive(&full[slot]);
         break;
       }
-      const uint8_t* src = base_of(link);
+      const uint8_t* src = base_of<kUnit>(p, link);
       for (uint32_t unit = 0; unit < n_units; ++unit, src += kUnit) {
         wait_slot();
         if (unit == 0) // published before the arrive below releases it to the consumers
@@ -2040,12 +2063,7 @@ wib2_kernel(const KernelParams p)
         }
       }
     }
-    // last CTA out re-arms the cursor for the next launch
-    __threadfence();
-    if (atomicAdd(p.link_cursor + 1, 1u) == gridDim.x - 1u) {
-      p.link_cursor[0] = 0u;
-      p.link_cursor[1] = 0u;
-    }
+    rearm_cursor(p, gridDim.x);
     return;
   }
 
@@ -2065,8 +2083,8 @@ wib2_kernel(const KernelParams p)
     const uint32_t link = fifo[popped & (kWib2Fifo - 1u)];
     if (link == kNoMoreLinks)
       break;
-    const uint32_t n_units = units_of(link);
-    const uint8_t* link_base = base_of(link);
+    const uint32_t n_units = units_of(p, link);
+    const uint8_t* link_base = base_of<kUnit>(p, link);
     const uint32_t group = link * kWib2Warps + warp;
     uint32_t* st = p.state + size_t(group) * kStateWordsPerGroup;
     const uint32_t flags = p.group_flags[group];
@@ -2081,7 +2099,7 @@ wib2_kernel(const KernelParams p)
       if (unit != 0)
         mbar_wait(&full[stg], phase);
       const uint32_t* sc = reinterpret_cast<const uint32_t*>(stages + stg * kUnit);
-      if constexpr (!std::is_same<Algo, PackedSimpleWib2>::value)
+      if constexpr (Algo::kNeedsUnitTs)
         ctx.ts = uint64_t(sc[1]) | (uint64_t(sc[2]) << 32); // WIB2Frame::get_timestamp, first frame (:350-351)
       const uint32_t* rows = sc + row0;
       if (need_seed) {
@@ -2114,12 +2132,7 @@ wib2_kernel(const KernelParams p)
       }
     }
 
-    algo.template finish_link<true>(ctx);
-    Algo::template flush<true>(hits, p.sink, link_base, link, lane);
-    const uint32_t k_end = algo.phase_after(n_units * 12u);
-    algo.store(st, lane, k_end);
-    if (lane == 0)
-      p.group_flags[group] = kFlagInitialized | (k_end << 8);
+    close_item<true>(algo, ctx, hits, st, group, n_units * 12u, lane);
   }
 }
 

@@ -1,7 +1,7 @@
 """GPU (B200): the launch geometries production runs, every link against the oracle.
 
 The launch layer picks a geometry from the link count and the batch length (fdreadoutlibs_b200/csrc/swtpg_capi.cu:
-launch_wibeth_geo, launch_wibeth_simple, launch_wibeth, launch_wibeth_quad, launch_wib2): 16 or 20 persistent warps per SM,
+launch, launch_wibeth, launch_wibeth_geo, launch_wibeth_quad, launch_wib2): 16 or 20 persistent warps per SM,
 whole links or every link handed out in halving slices, the CTA form with dynamic quad claims for FIR + IQR, persistent WIB2
 CTAs whose producer warp claims further links from the cursor. Each case below is sized from the device's SM count so that it
 lands in one of those regimes (the headline one: pipelined SimpleThreshold, 20 warps per SM, 4 halving slices, 40 links per
@@ -31,29 +31,35 @@ WIDE_PULSES = dict(amp_min=3000, amp_max=15000, hw_min=6, hw_max=16, ped_base=30
 
 
 # ---- the launch rules util.py restates --------------------------------------------------------------------------------------
-def test_restated_launch_rules_match_the_source():
+def test_restated_launch_rules_match_the_policy_constants():
     """CPU: the source lines `expected_geometry` restates. If one of them changes, update the restatement (and the cases)."""
     capi = re.sub(r"\s+", " ", open(os.path.join(CSRC, "swtpg_capi.cu")).read())
     kern = re.sub(r"\s+", " ", open(os.path.join(CSRC, "swtpg_kernels.cuh")).read())
-    for line in ("constexpr auto k = wibeth_kernel<Algo, 1, kGeoStages, kGeoChunk, DUMP, 1>;",
+    for line in ("constexpr auto k = wibeth_kernel<Algo, DUMP>;",
+                 "const bool full_load = Algo::kFullLoadWarpsPerSm > 0 && "
+                 "kp.n_links >= Algo::kFullLoadWarpsPerSm * sms + Algo::kFullLoadExtraLinks;",
+                 "const unsigned warps_per_sm = full_load ? Algo::kFullLoadWarpsPerSm : Algo::kWarpsPerSm;",
                  "unsigned even = per_sm >= 4 ? per_sm / 4 * 4 : per_sm;",
-                 "even = std::min<unsigned>(even, unsigned(kWarpsPerSm));",
+                 "if (warps_per_sm > 0) // the measured optimum, if the device holds that many even = std::min(even, warps_per_sm);",
                  "const unsigned grid = std::min<unsigned>(std::min<unsigned>(kp.n_links, even * sms), resident);",
-                 "if (kp.n_links > grid && (SLICE_WHOLE_ROUNDS || kp.n_links % grid != 0))",
+                 "if (kp.n_links > grid && (full_load || kp.n_links % grid != 0))",
                  "parts = std::max(1u, std::min(4u, kp.units_stride / 16u));",
                  "kq.slice_geom = 1u; // halving slices",
-                 f"constexpr int kFullWarpsPerSm = {FULL_WARPS_PER_SM};",
-                 "if (kp.n_links >= unsigned(kFullWarpsPerSm * sms))",
-                 "return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP, kFullWarpsPerSm, true>(kp, s);",
-                 "return launch_wibeth_geo<PackedSimpleWibEthPipe, DUMP>(kp, s); }",
-                 "if constexpr (std::is_same<Algo, PackedSimpleWibEth>::value) { return launch_wibeth_simple<DUMP>(kp, s); } "
-                 "else if constexpr (Algo::kQuadCtasPerSm > 0) { return launch_wibeth_quad<Algo, DUMP>(kp, s); }",
-                 f"if (kp.n_links > unsigned({FULL_WARPS_PER_SM} * sms)) return launch_wibeth_geo<Algo, DUMP, {FULL_WARPS_PER_SM}, true>(kp, s);"):
+                 "if constexpr (Algo::kQuadCtasPerSm > 0) return launch_wibeth_quad<Algo, DUMP>(kp, s); "
+                 "else return launch_wibeth_geo<Algo, DUMP>(kp, s);",
+                 "case Policy::WibEthSimple: return launch_wibeth<PackedSimpleWibEthPipe, DUMP>(kp, s);",
+                 "case Policy::WibEthAbsRs: return launch_wibeth<PackedRsWibEth<false>, DUMP>(kp, s);",
+                 "case Policy::WibEthStandardRs: return launch_wibeth<PackedRsWibEth<true>, DUMP>(kp, s);"):
         assert line in capi, f"swtpg_capi.cu no longer has `{line}`"
-    for line in ("static constexpr int kWarpsPerSm = PIPE ? 16 : 20;", "static constexpr int kWarpsPerSm = STANDARD ? 20 : 16;",
-                 "static constexpr int kWarpsPerSm = 0;",
-                 # PackedSimpleT runs the one-warp-per-CTA form
-                 "static constexpr int kWarpsPerSm = PIPE ? 16 : 20; static constexpr int kQuadCtasPerSm = 0;",
+    for line in (# ScalarAlgo: as many warps as fit, never full load
+                 "static constexpr int kWarpsPerSm = 0; static constexpr int kFullLoadWarpsPerSm = 0; "
+                 "static constexpr int kFullLoadExtraLinks = 0; static constexpr int kQuadCtasPerSm = 0;",
+                 # PackedSimpleT (the pipelined form) runs the one-warp-per-CTA form: 16 per SM, from 20 * SMs links on 20
+                 f"static constexpr int kWarpsPerSm = 16; static constexpr int kFullLoadWarpsPerSm = {FULL_WARPS_PER_SM}; "
+                 "static constexpr int kFullLoadExtraLinks = 0; static constexpr int kQuadCtasPerSm = 0;",
+                 # PackedRsWibEth (derives from PackedSimpleT): its own warps, full load from 20 * SMs + 1 links on
+                 "static constexpr int kWarpsPerSm = STANDARD ? 20 : 16; static constexpr int kFullLoadExtraLinks = 1;",
+                 "struct PackedRsWibEth : PackedSimpleWibEth",
                  # the halving slices halving_slices restates
                  "u0 = n - ((n + (1u << part) - 1u) >> part); "
                  "u1 = part + 1u == (1u << p.parts_log2) ? n : n - ((n + (2u << part) - 1u) >> (part + 1u));"):

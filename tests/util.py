@@ -353,11 +353,12 @@ def check(what, fmt, handle, batches, *, link_kw=None, thresholds=None, rs_table
 
 
 # ---- the launch rules, restated ---------------------------------------------------------------------------------------------
-# swtpg_capi.cu: launch_wibeth_geo, launch_wibeth_simple, launch_wibeth, and the policies' constants kWarpsPerSm /
-# kQuadCtasPerSm (swtpg_kernels.cuh: PackedSimpleT, PackedRsWibEth, ScalarAlgo, PackedFirIqr, PackedFirIqrAnyTaps).
-# tests/test_gpu_launch_geometry.py::test_restated_launch_rules_match_the_source pins the source lines this depends on, so the
+# swtpg_capi.cu: launch, launch_wibeth, launch_wibeth_geo, and the policies' constants kWarpsPerSm / kFullLoadWarpsPerSm /
+# kFullLoadExtraLinks / kQuadCtasPerSm (swtpg_kernels.cuh: PackedSimpleT, PackedRsWibEth, ScalarAlgo, PackedFirIqr,
+# PackedFirIqrAnyTaps).
+# tests/test_gpu_launch_geometry.py::test_restated_launch_rules_match_the_policy_constants pins the source lines this depends on, so the
 # restatement has to be updated together with the rules.
-FULL_WARPS_PER_SM = 20   # kFullWarpsPerSm, and the running sums' 20 warps per SM above one round
+FULL_WARPS_PER_SM = 20   # kFullLoadWarpsPerSm of PackedSimpleT and (inherited) PackedRsWibEth
 QUAD_CTAS_PER_SM = 4     # PackedFirIqr / PackedFirIqrAnyTaps::kQuadCtasPerSm
 MAX_CTAS_PER_SM = 32     # what an sm_100 SM holds at most
 
