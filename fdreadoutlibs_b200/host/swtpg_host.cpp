@@ -7,6 +7,7 @@
 #include <cstring>
 #include <ctime>
 #include <thread>
+#include <variant>
 
 namespace swtpg {
 namespace host {
@@ -168,6 +169,13 @@ TpgEngine::set_link_thresholds(uint32_t link, const uint16_t* by_channel, uint32
   check(m_h, swtpg_set_link_thresholds(m_h, link, by_channel), "swtpg_set_link_thresholds");
 }
 
+static bool
+has_plane_thresholds(const RawDataProcessorConf& config)
+{
+  const auto& plane = config.tpg_plane_threshold;
+  return plane[0] >= 0 || plane[1] >= 0 || plane[2] >= 0;
+}
+
 // The per-frame-channel table of RawDataProcessorConf::tpg_plane_threshold: channel c of the link (crate, slot, link) takes the
 // threshold of its plane, or tpg_threshold where that is -1. Empty when no plane has its own.
 static std::vector<uint16_t>
@@ -175,7 +183,7 @@ plane_threshold_table(const RawDataProcessorConf& config, const ChannelMap& map,
 {
   std::vector<uint16_t> table;
   const auto& plane = config.tpg_plane_threshold;
-  if (plane[0] < 0 && plane[1] < 0 && plane[2] < 0)
+  if (!has_plane_thresholds(config))
     return table;
   for (int32_t t : plane)
     if (t > 32767)
@@ -280,186 +288,7 @@ TpgEngine::drain(bool wait)
   }
 }
 
-// ---- WIBEthFrameProcessor ---------------------------------------------------------------------------------------------
-WIBEthFrameProcessor::WIBEthFrameProcessor(std::unique_ptr<FrameErrorRegistry>& error_registry, std::shared_ptr<TpgEngine> engine)
-  : inherited(error_registry)
-  , m_engine(std::move(engine))
-  , m_wibeth_frame_handler(std::make_unique<WIBEthFrameHandler>())
-{
-}
-
-WIBEthFrameProcessor::~WIBEthFrameProcessor()
-{
-  m_wibeth_frame_handler->reset();
-}
-
-void
-WIBEthFrameProcessor::conf(const RawDataProcessorConf& config)
-{
-  m_tpg_algorithm = config.tpg_algorithm;
-  swtpg_config a{};
-  if (m_tpg_algorithm == "SimpleThreshold") {
-    m_tp_algo = TriggerPrimitive::Algorithm::kSimpleThreshold;
-    a.algorithm = SWTPG_ALGO_SIMPLE_THRESHOLD;
-  } else if (m_tpg_algorithm == "AbsRS") {
-    m_tp_algo = TriggerPrimitive::Algorithm::kAbsRunningSum;
-    a.algorithm = SWTPG_ALGO_ABS_RS;
-    m_enable_simple_threshold_on_collection = config.enable_simple_threshold_on_collection;
-  } else if (m_tpg_algorithm == "StandardRS") {
-    m_tp_algo = TriggerPrimitive::Algorithm::kRunningSum;
-    a.algorithm = SWTPG_ALGO_STANDARD_RS;
-    m_enable_simple_threshold_on_collection = config.enable_simple_threshold_on_collection;
-  } else {
-    throw TPGAlgorithmInexistent(m_tpg_algorithm);
-  }
-  // Running-sum factors travel as integers x10 (src/wibeth/WIBEthFrameProcessor.cpp:199-206)
-  m_tpg_rs_memory_factor = uint16_t(10 * config.tpg_rs_memory_factor);
-  m_tpg_rs_scale_factor = config.tpg_rs_scale_factor != 0 ? uint16_t(10 / config.tpg_rs_scale_factor) : 0;
-  m_tpg_frugal_streaming_accumulator_limit = config.tpg_frugal_streaming_accumulator_limit;
-  m_tp_max_width = config.tp_timeout;
-  m_channel_mask_set.insert(config.tpg_channel_mask.begin(), config.tpg_channel_mask.end());
-  m_tpg_threshold = config.tpg_threshold;
-  m_crate_no = config.crate_id;
-  m_slot_no = config.slot_id;
-  m_stream_id = config.link_id;
-  m_correct_lookup = config.correct_channel_lookup;
-  m_block = config.block_on_backpressure;
-
-  inherited::reset_tasks();
-  inherited::add_preprocess_task([this](frameptr fp) { sequence_check(fp); });
-  inherited::add_preprocess_task([this](frameptr fp) { timestamp_check(fp); });
-  if (config.enable_tpg) {
-    m_tpg_enabled = true;
-    m_channel_map = make_map(config.channel_map_name);
-    a.threshold = m_tpg_threshold;
-    a.frugal_acc_limit = m_tpg_frugal_streaming_accumulator_limit;
-    a.rs_memory_factor = m_tpg_rs_memory_factor;
-    a.rs_scale_factor = m_tpg_rs_scale_factor;
-    m_wibeth_frame_handler->link = m_engine->attach(this);
-    m_engine->configure(m_wibeth_frame_handler->link, a);
-    // the table must be in place before start(), so it comes from the configured ids rather than the first frame's header (a link
-    // whose frames carry other ids is reported as a LinkMisconfiguration)
-    const std::vector<uint16_t> table = plane_threshold_table(config, m_channel_map, SWTPG_WIBETH_CHANNELS);
-    m_engine->set_link_thresholds(m_wibeth_frame_handler->link, table.empty() ? nullptr : table.data(), uint32_t(table.size()));
-    inherited::add_postprocess_task([this](constframeptr fp) { find_hits(fp, m_wibeth_frame_handler.get()); });
-  }
-  inherited::conf(config);
-}
-
-void
-WIBEthFrameProcessor::start()
-{
-  if (m_tpg_enabled) {
-    m_tps_suppressed_too_long = 0;
-    m_tps_send_failed = 0;
-    m_frames_dropped = 0;
-    m_wibeth_frame_handler->reset(); // = initialize(): fresh per-link resources; the device state is zeroed by swtpg_start
-    m_engine->start();
-  }
-  m_previous_ts = m_current_ts = 0;
-  m_first_ts_missmatch = true;
-  m_ts_error_ctr = 0;
-  m_first_seq_id_mismatch = true;
-  m_seq_id_error_ctr = 0;
-  m_t0 = std::chrono::high_resolution_clock::now();
-  m_new_tps = 0;
-  m_tpg_hits_count = 0;
-  inherited::start();
-}
-
-void
-WIBEthFrameProcessor::stop()
-{
-  inherited::stop();
-  if (m_tpg_enabled) {
-    m_engine->stop(); // flushes the partially filled superchunk and delivers the remaining TPs through process_swtpg_hits
-    m_wibeth_frame_handler->reset();
-  }
-}
-
-void
-WIBEthFrameProcessor::get_info(RawDataProcessorInfo& info)
-{
-  info = RawDataProcessorInfo{};
-  info.num_seq_id_errors = m_seq_id_error_ctr.load();
-  info.min_seq_id_jump = m_seq_id_min_jump.exchange(0);
-  info.max_seq_id_jump = m_seq_id_max_jump.exchange(0);
-  info.num_ts_errors = m_ts_error_ctr.load();
-  const auto now = std::chrono::high_resolution_clock::now();
-  if (m_tpg_enabled) {
-    const uint64_t new_hits = m_tpg_hits_count.exchange(0);
-    const double seconds = std::chrono::duration_cast<std::chrono::microseconds>(now - m_t0).count() / 1000000.;
-    info.rate_tp_hits = seconds > 0 ? new_hits / seconds / 1000. : 0;
-    info.num_tps_sent = m_new_tps.exchange(0);
-    info.num_tps_suppressed_too_long = m_tps_suppressed_too_long.exchange(0);
-    info.num_tps_send_failed = m_tps_send_failed.exchange(0);
-    info.num_frames_dropped_busy = m_frames_dropped.exchange(0);
-    // the ten channels with the most TPs since the last call, then reset (:263-284): the reference keeps a std::map keyed by
-    // offline channel and sorts its pairs by count; ties keep the map's (ascending channel) order
-    if (m_maps_ready.load(std::memory_order_acquire)) {
-      std::map<uint32_t, int> rate;
-      for (uint32_t c = 0; c < 64; ++c)
-        rate[m_offline_of_channel[c]] += int(m_tp_channel_rate[c].exchange(0, std::memory_order_relaxed));
-      std::vector<std::pair<uint32_t, int>> v(rate.begin(), rate.end());
-      std::stable_sort(v.begin(), v.end(), [](const auto& x, const auto& y) { return x.second > y.second; });
-      info.n_top = uint32_t(std::min<size_t>(10, v.size()));
-      for (uint32_t i = 0; i < info.n_top; ++i) {
-        info.top_channels[i] = v[i].first;
-        info.top_channel_tps[i] = uint32_t(v[i].second);
-      }
-    }
-  }
-  m_t0 = now;
-}
-
-void
-WIBEthFrameProcessor::sequence_check(frameptr fp)
-{
-  if (inherited::m_emulator_mode) { // emulated data: stamp the geo id and a perfectly incrementing sequence id
-    DAQEthHeader* h = fp->header();
-    h->crate_id = m_crate_no;
-    h->slot_id = m_slot_no;
-    h->stream_id = m_stream_id;
-    h->seq_id = m_previous_seq_id & 0xfff; // one frame per payload: (previous + i) with i = 0, as in the reference (:311)
-  }
-  m_current_seq_id = uint16_t(fp->header()->seq_id);
-  const uint16_t expected_seq_id = uint16_t((m_previous_seq_id + fp->get_num_frames()) & 0xfff);
-  int16_t delta_seq_id = int16_t(m_current_seq_id - expected_seq_id);
-  if (delta_seq_id > 0x800)
-    delta_seq_id -= 0x1000;
-  else if (delta_seq_id < -0x7ff)
-    delta_seq_id += 0x1000;
-  if (delta_seq_id != 0) {
-    ++m_seq_id_error_ctr;
-    m_seq_id_max_jump = std::max(delta_seq_id, m_seq_id_max_jump.load());
-    m_seq_id_min_jump = std::min(delta_seq_id, m_seq_id_min_jump.load());
-    m_error_registry->add_error("SEQUENCE_ID_JUMP", FrameErrorRegistry::ErrorInterval{ expected_seq_id, m_current_seq_id });
-    m_first_seq_id_mismatch = false;
-  }
-  m_previous_seq_id = m_current_seq_id;
-}
-
-void
-WIBEthFrameProcessor::timestamp_check(frameptr fp)
-{
-  const uint64_t frame_tick_difference = DUNEWIBEthTypeAdapter::expected_tick_difference * fp->get_num_frames();
-  if (inherited::m_emulator_mode) {
-    DAQEthHeader* h = fp->header();
-    h->crate_id = m_crate_no;
-    h->slot_id = m_slot_no;
-    h->stream_id = m_stream_id;
-    h->timestamp = m_previous_ts + frame_tick_difference;
-  }
-  m_current_ts = fp->get_first_timestamp();
-  if (m_current_ts - m_previous_ts != frame_tick_difference) {
-    ++m_ts_error_ctr;
-    m_error_registry->add_error("MISSING_FRAMES", FrameErrorRegistry::ErrorInterval{ m_previous_ts + frame_tick_difference, m_current_ts });
-    m_first_ts_missmatch = false;
-  }
-  m_previous_ts = m_current_ts;
-  m_last_processed_daq_ts = m_current_ts;
-}
-
+// ---- TpcFrameProcessor ------------------------------------------------------------------------------------------------
 namespace {
 ChannelAdcStats
 channel_adc_stats(uint32_t offline_channel, const swtpg_adc_stats& a)
@@ -479,16 +308,248 @@ channel_adc_stats(uint32_t offline_channel, const swtpg_adc_stats& a)
 }
 } // namespace
 
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::TpcFrameProcessor(std::unique_ptr<FrameErrorRegistry>& error_registry,
+                                                                     std::shared_ptr<TpgEngine> engine)
+  : inherited(error_registry)
+  , m_engine(std::move(engine))
+  , m_frame_handler(std::make_unique<H>())
+{
+}
+
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
 void
-WIBEthFrameProcessor::get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset)
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::conf_link(const RawDataProcessorConf& config, const swtpg_config& a,
+                                                             std::function<void(constframeptr)> find_hits)
+{
+  m_tp_max_width = config.tp_timeout;
+  m_channel_mask_set.insert(config.tpg_channel_mask.begin(), config.tpg_channel_mask.end());
+  m_crate_no = config.crate_id;
+  m_slot_no = config.slot_id;
+  m_link_no = config.link_id;
+  m_block = config.block_on_backpressure;
+  if (config.enable_tpg) {
+    m_tpg_enabled = true;
+    m_channel_map = make_map(config.channel_map_name);
+    m_frame_handler->link = m_engine->attach(this);
+    m_engine->configure(m_frame_handler->link, a);
+    // the table must be in place before start(), so it comes from the configured ids rather than the first frame's header (a
+    // WIBEth link whose frames carry other ids is reported as a LinkMisconfiguration)
+    const std::vector<uint16_t> table = plane_threshold_table(config, m_channel_map, kChannels);
+    m_engine->set_link_thresholds(m_frame_handler->link, table.empty() ? nullptr : table.data(), uint32_t(table.size()));
+    inherited::add_postprocess_task(std::move(find_hits));
+  }
+  inherited::conf(config);
+}
+
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
+void
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::start()
+{
+  if (m_tpg_enabled) {
+    m_tps_suppressed_too_long = 0;
+    m_tps_send_failed = 0;
+    m_frames_dropped = 0;
+    m_frame_handler->reset(); // = initialize(): fresh per-link resources; the device state is zeroed by swtpg_start
+    m_engine->start();
+  }
+  m_previous_ts = m_current_ts = 0;
+  m_ts_error_ctr = 0;
+  m_t0 = std::chrono::high_resolution_clock::now();
+  m_new_tps = 0;
+  m_tpg_hits_count = 0;
+  inherited::start();
+}
+
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
+void
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::stop()
+{
+  inherited::stop();
+  if (m_tpg_enabled) {
+    m_engine->stop(); // flushes the partially filled superchunk and delivers the remaining TPs through process_swtpg_hits
+    m_frame_handler->reset();
+  }
+}
+
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
+void
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::get_info(RawDataProcessorInfo& info)
+{
+  info = RawDataProcessorInfo{};
+  info.num_ts_errors = m_ts_error_ctr.load();
+  const auto now = std::chrono::high_resolution_clock::now();
+  if (m_tpg_enabled) {
+    const uint64_t new_hits = m_tpg_hits_count.exchange(0);
+    const double seconds = std::chrono::duration_cast<std::chrono::microseconds>(now - m_t0).count() / 1000000.;
+    info.rate_tp_hits = seconds > 0 ? new_hits / seconds / 1000. : 0;
+    info.num_tps_sent = m_new_tps.exchange(0);
+    info.num_tps_suppressed_too_long = m_tps_suppressed_too_long.exchange(0);
+    info.num_tps_send_failed = m_tps_send_failed.exchange(0);
+    info.num_frames_dropped_busy = m_frames_dropped.exchange(0);
+    // the ten channels with the most TPs since the last call, then reset (src/wibeth/WIBEthFrameProcessor.cpp:263-284): the
+    // reference keeps a std::map keyed by offline channel and sorts its pairs by count; ties keep the map's (ascending channel) order
+    if (m_maps_ready.load(std::memory_order_acquire)) {
+      std::map<uint32_t, int> rate;
+      for (uint32_t c = 0; c < kChannels; ++c)
+        rate[m_offline_of_channel[c]] += int(m_tp_channel_rate[c].exchange(0, std::memory_order_relaxed));
+      std::vector<std::pair<uint32_t, int>> v(rate.begin(), rate.end());
+      std::stable_sort(v.begin(), v.end(), [](const auto& x, const auto& y) { return x.second > y.second; });
+      info.n_top = uint32_t(std::min<size_t>(10, v.size()));
+      for (uint32_t i = 0; i < info.n_top; ++i) {
+        info.top_channels[i] = v[i].first;
+        info.top_channel_tps[i] = uint32_t(v[i].second);
+      }
+    }
+  }
+  m_t0 = now;
+}
+
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
+void
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset)
 {
   out.clear();
   if (!m_maps_ready.load(std::memory_order_acquire))
     return;
-  swtpg_adc_stats s[64];
-  m_engine->read_adc_stats(m_wibeth_frame_handler->link, s, 64, reset);
-  for (uint32_t c = 0; c < 64; ++c)
+  swtpg_adc_stats s[kChannels];
+  m_engine->read_adc_stats(m_frame_handler->link, s, kChannels, reset);
+  for (uint32_t c = 0; c < kChannels; ++c)
     out.push_back(channel_adc_stats(m_offline_of_channel[c], s[c]));
+}
+
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
+void
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::process_swtpg_hits(const swtpg_tp* tps, size_t n)
+{
+  uint64_t nhits = 0;
+  for (size_t i = 0; i < n; ++i) {
+    const swtpg_tp& r = tps[i];
+    const uint32_t c = r.channel & (kChannels - 1);
+    if (m_masked[c]) // offline channel in tpg_channel_mask (src/wibeth/WIBEthFrameProcessor.cpp:528)
+      continue;
+    TriggerPrimitiveTypeAdapter tp;
+    tp.tp.time_start = r.time_start;
+    tp.tp.time_peak = r.time_peak;
+    tp.tp.time_over_threshold = r.time_over_threshold;
+    tp.tp.channel = m_offline_of_channel[c];
+    tp.tp.adc_integral = r.adc_integral;
+    tp.tp.adc_peak = r.adc_peak;
+    tp.tp.detid = uint16_t(m_det_id);
+    tp.tp.type = TriggerPrimitive::Type::kTPC;
+    tp.tp.algorithm = m_tp_algo;
+    tp.tp.version = 1;
+    bool sent = false;
+    if (tp.tp.time_over_threshold > m_tp_max_width)
+      m_tps_suppressed_too_long++; // reference: ers::warning(TPTooLong)
+    else if (!m_tp_sink || !m_tp_sink(std::move(tp)))
+      m_tps_send_failed++; // reference: ers::warning(FailedToSendTP)
+    else
+      sent = true;
+    if (kCountEveryTp || sent) {
+      m_new_tps++;
+      ++nhits;
+    }
+    m_tp_channel_rate[c].fetch_add(1, std::memory_order_relaxed);
+  }
+  m_tpg_hits_count += nhits;
+}
+
+template class TpcFrameProcessor<DUNEWIBEthTypeAdapter, WIBEthFrameHandler, SWTPG_WIBETH_CHANNELS, false>;
+template class TpcFrameProcessor<DUNEWIBSuperChunkTypeAdapter, WIB2FrameHandler, SWTPG_WIB2_CHANNELS, true>;
+
+// ---- WIBEthFrameProcessor ---------------------------------------------------------------------------------------------
+void
+WIBEthFrameProcessor::conf(const RawDataProcessorConf& config)
+{
+  swtpg_config a{};
+  if (config.tpg_algorithm == "SimpleThreshold") {
+    m_tp_algo = TriggerPrimitive::Algorithm::kSimpleThreshold;
+    a.algorithm = SWTPG_ALGO_SIMPLE_THRESHOLD;
+  } else if (config.tpg_algorithm == "AbsRS") {
+    m_tp_algo = TriggerPrimitive::Algorithm::kAbsRunningSum;
+    a.algorithm = SWTPG_ALGO_ABS_RS;
+    m_enable_simple_threshold_on_collection = config.enable_simple_threshold_on_collection;
+  } else if (config.tpg_algorithm == "StandardRS") {
+    m_tp_algo = TriggerPrimitive::Algorithm::kRunningSum;
+    a.algorithm = SWTPG_ALGO_STANDARD_RS;
+    m_enable_simple_threshold_on_collection = config.enable_simple_threshold_on_collection;
+  } else {
+    throw TPGAlgorithmInexistent(config.tpg_algorithm);
+  }
+  // Running-sum factors travel as integers x10 (src/wibeth/WIBEthFrameProcessor.cpp:199-206)
+  m_tpg_rs_memory_factor = uint16_t(10 * config.tpg_rs_memory_factor);
+  a.rs_memory_factor = m_tpg_rs_memory_factor;
+  a.rs_scale_factor = config.tpg_rs_scale_factor != 0 ? uint16_t(10 / config.tpg_rs_scale_factor) : 0;
+  a.frugal_acc_limit = config.tpg_frugal_streaming_accumulator_limit;
+  a.threshold = config.tpg_threshold;
+  m_correct_lookup = config.correct_channel_lookup;
+  inherited::reset_tasks();
+  inherited::add_preprocess_task([this](frameptr fp) { sequence_check(fp); });
+  inherited::add_preprocess_task([this](frameptr fp) { timestamp_check(fp); });
+  conf_link(config, a, [this](constframeptr fp) { find_hits(fp, m_frame_handler.get()); });
+}
+
+void
+WIBEthFrameProcessor::start()
+{
+  TpcFrameProcessor::start();
+  m_seq_id_error_ctr = 0;
+}
+
+void
+WIBEthFrameProcessor::get_info(RawDataProcessorInfo& info)
+{
+  TpcFrameProcessor::get_info(info);
+  info.num_seq_id_errors = m_seq_id_error_ctr.load();
+  info.min_seq_id_jump = m_seq_id_min_jump.exchange(0);
+  info.max_seq_id_jump = m_seq_id_max_jump.exchange(0);
+}
+
+void
+WIBEthFrameProcessor::sequence_check(frameptr fp)
+{
+  if (inherited::m_emulator_mode) { // emulated data: stamp the geo id and a perfectly incrementing sequence id
+    DAQEthHeader* h = fp->header();
+    h->crate_id = m_crate_no;
+    h->slot_id = m_slot_no;
+    h->stream_id = m_link_no;
+    h->seq_id = m_previous_seq_id & 0xfff; // one frame per payload: (previous + i) with i = 0, as in the reference (:311)
+  }
+  m_current_seq_id = uint16_t(fp->header()->seq_id);
+  const uint16_t expected_seq_id = uint16_t((m_previous_seq_id + fp->get_num_frames()) & 0xfff);
+  int16_t delta_seq_id = int16_t(m_current_seq_id - expected_seq_id);
+  if (delta_seq_id > 0x800)
+    delta_seq_id -= 0x1000;
+  else if (delta_seq_id < -0x7ff)
+    delta_seq_id += 0x1000;
+  if (delta_seq_id != 0) {
+    ++m_seq_id_error_ctr;
+    m_seq_id_max_jump = std::max(delta_seq_id, m_seq_id_max_jump.load());
+    m_seq_id_min_jump = std::min(delta_seq_id, m_seq_id_min_jump.load());
+    m_error_registry->add_error("SEQUENCE_ID_JUMP", FrameErrorRegistry::ErrorInterval{ expected_seq_id, m_current_seq_id });
+  }
+  m_previous_seq_id = m_current_seq_id;
+}
+
+void
+WIBEthFrameProcessor::timestamp_check(frameptr fp)
+{
+  const uint64_t frame_tick_difference = DUNEWIBEthTypeAdapter::expected_tick_difference * fp->get_num_frames();
+  if (inherited::m_emulator_mode) {
+    DAQEthHeader* h = fp->header();
+    h->crate_id = m_crate_no;
+    h->slot_id = m_slot_no;
+    h->stream_id = m_link_no;
+    h->timestamp = m_previous_ts + frame_tick_difference;
+  }
+  m_current_ts = fp->get_first_timestamp();
+  if (m_current_ts - m_previous_ts != frame_tick_difference) {
+    ++m_ts_error_ctr;
+    m_error_registry->add_error("MISSING_FRAMES", FrameErrorRegistry::ErrorInterval{ m_previous_ts + frame_tick_difference, m_current_ts });
+  }
+  m_previous_ts = m_current_ts;
+  m_last_processed_daq_ts = m_current_ts;
 }
 
 void
@@ -503,17 +564,12 @@ WIBEthFrameProcessor::find_hits(constframeptr fp, WIBEthFrameHandler* frame_hand
     for (uint32_t p = 0; p < 64; ++p)
       frame_handler->register_channel_map[p] = m_channel_map(hdr->crate_id, hdr->slot_id, hdr->stream_id, position_to_frame_channel(p));
     m_det_id = uint32_t(hdr->det_id);
-    if (hdr->crate_id != m_crate_no || hdr->slot_id != m_slot_no || hdr->stream_id != m_stream_id)
-      m_misconf.push_back({ uint32_t(hdr->crate_id), uint32_t(hdr->slot_id), uint32_t(hdr->stream_id), m_crate_no, m_slot_no, m_stream_id });
-    for (uint32_t p = 0; p < 64; ++p)
-      m_register_channels[p] = frame_handler->register_channel_map[p];
-    for (uint32_t c = 0; c < 64; ++c) { // per FRAME channel: the offline channel a record of that channel is reported with, masked or not
-      // H2 (SURVEY.md): production indexes the POSITION-ordered map with the FRAME channel the AVX2 code emits (:527)
-      m_offline_of_channel[c] = m_correct_lookup ? m_channel_map(hdr->crate_id, hdr->slot_id, hdr->stream_id, c) : m_register_channels[c];
-      m_masked[c] = m_channel_mask_set.count(m_offline_of_channel[c]) ? 1 : 0;
-      m_tp_channel_rate[c].store(0, std::memory_order_relaxed);
-    }
-    m_maps_ready.store(true, std::memory_order_release);
+    if (hdr->crate_id != m_crate_no || hdr->slot_id != m_slot_no || hdr->stream_id != m_link_no)
+      m_misconf.push_back({ uint32_t(hdr->crate_id), uint32_t(hdr->slot_id), uint32_t(hdr->stream_id), m_crate_no, m_slot_no, m_link_no });
+    // H2 (SURVEY.md): production indexes the POSITION-ordered map with the FRAME channel the AVX2 code emits (:527)
+    set_channel_tables([&](uint32_t c) {
+      return m_correct_lookup ? m_channel_map(hdr->crate_id, hdr->slot_id, hdr->stream_id, c) : frame_handler->register_channel_map[c];
+    });
     if (m_enable_simple_threshold_on_collection) { // collection channels run with R = 0, i.e. a plain threshold (:441-450)
       uint16_t factor[64];
       for (uint32_t c = 0; c < 64; ++c) {
@@ -524,64 +580,10 @@ WIBEthFrameProcessor::find_hits(constframeptr fp, WIBEthFrameHandler* frame_hand
     }
     frame_handler->first_hit = false;
   }
-  // The frame is only borrowed for the duration of this call: swtpg_submit copies it into the pinned staging slot — unless it
-  // lies in a latency buffer registered with the engine, which the copy engine then reads directly (zero-copy ingest).
-  // Non-blocking by default, like the reference's try_send: a full ring drops the frame and counts it. With
-  // block_on_backpressure the thread SLEEPS until the completion thread has freed ring space (swtpg_submit_wait). TPs come
-  // back through the engine's delivery thread (process_swtpg_hits below), never through this thread.
-  if (!m_block) {
-    if (!m_engine->submit(frame_handler->link, fp->data, sizeof fp->data))
-      ++m_frames_dropped;
-  } else {
-    while (!m_engine->submit(frame_handler->link, fp->data, sizeof fp->data, 100000)) {
-    }
-  }
-}
-
-void
-WIBEthFrameProcessor::process_swtpg_hits(const swtpg_tp* tps, size_t n)
-{
-  uint64_t nhits = 0;
-  for (size_t i = 0; i < n; ++i) {
-    const swtpg_tp& r = tps[i];
-    const uint32_t c = r.channel & 63u;
-    if (m_masked[c]) // offline channel in tpg_channel_mask (:528)
-      continue;
-    const uint32_t offline_channel = m_offline_of_channel[c];
-    TriggerPrimitiveTypeAdapter tp;
-    tp.tp.time_start = r.time_start;
-    tp.tp.time_peak = r.time_peak;
-    tp.tp.time_over_threshold = r.time_over_threshold;
-    tp.tp.channel = offline_channel;
-    tp.tp.adc_integral = r.adc_integral;
-    tp.tp.adc_peak = r.adc_peak;
-    tp.tp.detid = uint16_t(m_det_id);
-    tp.tp.type = TriggerPrimitive::Type::kTPC;
-    tp.tp.algorithm = m_tp_algo;
-    tp.tp.version = 1;
-    if (tp.tp.time_over_threshold > m_tp_max_width) {
-      m_tps_suppressed_too_long++; // reference: ers::warning(TPTooLong)
-    } else if (!m_tp_sink || !m_tp_sink(std::move(tp))) {
-      m_tps_send_failed++;         // reference: ers::warning(FailedToSendTP)
-    } else {
-      m_new_tps++;
-      ++nhits;
-    }
-    m_tp_channel_rate[c].fetch_add(1, std::memory_order_relaxed);
-  }
-  m_tpg_hits_count += nhits;
+  submit(fp, frame_handler->link);
 }
 
 // ---- WIB2FrameProcessor ---------------------------------------------------------------------------------------------
-WIB2FrameProcessor::WIB2FrameProcessor(std::unique_ptr<FrameErrorRegistry>& error_registry, std::shared_ptr<TpgEngine> engine)
-  : inherited(error_registry)
-  , m_engine(std::move(engine))
-  , m_handler(std::make_unique<WIB2FrameHandler>())
-{
-}
-
-WIB2FrameProcessor::~WIB2FrameProcessor() = default;
-
 void
 WIB2FrameProcessor::conf(const RawDataProcessorConf& config)
 {
@@ -594,85 +596,14 @@ WIB2FrameProcessor::conf(const RawDataProcessorConf& config)
     a.algorithm = SWTPG_ALGO_FIR_IQR;
   else
     throw TPGAlgorithmInexistent(config.tpg_algorithm);
-  m_tp_max_width = config.tp_timeout;
-  m_channel_mask_set.insert(config.tpg_channel_mask.begin(), config.tpg_channel_mask.end());
-  m_crate_no = config.crate_id;
-  m_slot_no = config.slot_id;
-  m_link = config.link_id;
-  m_block = config.block_on_backpressure;
+  // FIR + IQR and AbsRS multiply the threshold by an IQR sigma
+  if (config.enable_tpg && has_plane_thresholds(config) && a.algorithm != SWTPG_ALGO_SIMPLE_THRESHOLD)
+    throw std::invalid_argument("tpg_plane_threshold: WIB2 supports per-plane thresholds with SimpleThreshold only");
+  a.threshold = config.tpg_threshold;
+  a.frugal_acc_limit = 10;
   inherited::reset_tasks();
   inherited::add_preprocess_task([this](frameptr fp) { timestamp_check(fp); });
-  if (config.enable_tpg) {
-    m_tpg_enabled = true;
-    m_channel_map = make_map(config.channel_map_name);
-    const std::vector<uint16_t> table = plane_threshold_table(config, m_channel_map, SWTPG_WIB2_CHANNELS);
-    if (!table.empty() && a.algorithm != SWTPG_ALGO_SIMPLE_THRESHOLD) // FIR + IQR and AbsRS multiply the threshold by an IQR sigma
-      throw std::invalid_argument("tpg_plane_threshold: WIB2 supports per-plane thresholds with SimpleThreshold only");
-    a.threshold = config.tpg_threshold;
-    a.frugal_acc_limit = 10;
-    m_handler->link = m_engine->attach(this);
-    m_engine->configure(m_handler->link, a);
-    m_engine->set_link_thresholds(m_handler->link, table.empty() ? nullptr : table.data(), uint32_t(table.size()));
-    inherited::add_postprocess_task([this](constframeptr fp) { find_hits(fp, m_handler.get()); });
-  }
-  inherited::conf(config);
-}
-
-void
-WIB2FrameProcessor::start()
-{
-  if (m_tpg_enabled) {
-    m_tps_suppressed_too_long = 0;
-    m_tps_send_failed = 0;
-    m_frames_dropped = 0;
-    m_handler->reset();
-    m_engine->start();
-  }
-  m_previous_ts = m_current_ts = 0;
-  m_first_ts_missmatch = true;
-  m_ts_error_ctr = 0;
-  m_t0 = std::chrono::high_resolution_clock::now();
-  m_new_tps = 0;
-  m_tpg_hits_count = 0;
-}
-
-void
-WIB2FrameProcessor::stop()
-{
-  if (m_tpg_enabled) {
-    m_engine->stop();
-    m_handler->reset();
-  }
-}
-
-void
-WIB2FrameProcessor::get_info(RawDataProcessorInfo& info)
-{
-  info = RawDataProcessorInfo{};
-  info.num_ts_errors = m_ts_error_ctr.load();
-  const auto now = std::chrono::high_resolution_clock::now();
-  if (m_tpg_enabled) {
-    const uint64_t new_hits = m_tpg_hits_count.exchange(0);
-    const double seconds = std::chrono::duration_cast<std::chrono::microseconds>(now - m_t0).count() / 1000000.;
-    info.rate_tp_hits = seconds > 0 ? new_hits / seconds / 1000. : 0;
-    info.num_tps_sent = m_new_tps.exchange(0);
-    info.num_tps_suppressed_too_long = m_tps_suppressed_too_long.exchange(0);
-    info.num_tps_send_failed = m_tps_send_failed.exchange(0);
-    info.num_frames_dropped_busy = m_frames_dropped.exchange(0);
-    if (m_maps_ready.load(std::memory_order_acquire)) {
-      std::map<uint32_t, int> rate;
-      for (uint32_t c = 0; c < 256; ++c)
-        rate[m_register_channels[c]] += int(m_tp_channel_rate[c].exchange(0, std::memory_order_relaxed));
-      std::vector<std::pair<uint32_t, int>> v(rate.begin(), rate.end());
-      std::stable_sort(v.begin(), v.end(), [](const auto& x, const auto& y) { return x.second > y.second; });
-      info.n_top = uint32_t(std::min<size_t>(10, v.size()));
-      for (uint32_t i = 0; i < info.n_top; ++i) {
-        info.top_channels[i] = v[i].first;
-        info.top_channel_tps[i] = uint32_t(v[i].second);
-      }
-    }
-  }
-  m_t0 = now;
+  conf_link(config, a, [this](constframeptr fp) { find_hits(fp, m_frame_handler.get()); });
 }
 
 void
@@ -686,7 +617,7 @@ WIB2FrameProcessor::timestamp_check(frameptr fp)
       WIB2Header* h = fp->header(i);
       h->crate = m_crate_no;
       h->slot = m_slot_no;
-      h->link = m_link;
+      h->link = m_link_no;
       fp->set_timestamp(i, ts_next);
       ts_next += tick;
     }
@@ -695,22 +626,9 @@ WIB2FrameProcessor::timestamp_check(frameptr fp)
   if (m_current_ts - m_previous_ts != superchunk_tick_difference) {
     ++m_ts_error_ctr;
     m_error_registry->add_error("MISSING_FRAMES", FrameErrorRegistry::ErrorInterval{ m_previous_ts + superchunk_tick_difference, m_current_ts });
-    m_first_ts_missmatch = false;
   }
   m_previous_ts = m_current_ts;
   m_last_processed_daq_ts = m_current_ts;
-}
-
-void
-WIB2FrameProcessor::get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset)
-{
-  out.clear();
-  if (!m_maps_ready.load(std::memory_order_acquire))
-    return;
-  swtpg_adc_stats s[256];
-  m_engine->read_adc_stats(m_handler->link, s, 256, reset);
-  for (uint32_t c = 0; c < 256; ++c)
-    out.push_back(channel_adc_stats(m_register_channels[c], s[c]));
 }
 
 void
@@ -723,53 +641,10 @@ WIB2FrameProcessor::find_hits(constframeptr fp, WIB2FrameHandler* frame_handler)
     m_det_id = h->detector_id;
     // WIB2's AVX2 code emits the register POSITION and the map is position-ordered (src/wib2/WIB2FrameProcessor.cpp:367-368),
     // so the reported channel is the true offline channel of the frame channel: a frame-channel-ordered map is equivalent.
-    for (uint32_t c = 0; c < 256; ++c) {
-      m_register_channels[c] = m_channel_map(h->crate, h->slot, h->link, c);
-      m_masked[c] = m_channel_mask_set.count(m_register_channels[c]) ? 1 : 0;
-      m_tp_channel_rate[c].store(0, std::memory_order_relaxed);
-    }
-    m_maps_ready.store(true, std::memory_order_release);
+    set_channel_tables([&](uint32_t c) { return m_channel_map(h->crate, h->slot, h->link, c); });
     frame_handler->first_hit = false;
   }
-  if (!m_block) {
-    if (!m_engine->submit(frame_handler->link, fp->data, sizeof fp->data))
-      ++m_frames_dropped;
-  } else {
-    while (!m_engine->submit(frame_handler->link, fp->data, sizeof fp->data, 100000)) {
-    }
-  }
-}
-
-void
-WIB2FrameProcessor::process_swtpg_hits(const swtpg_tp* tps, size_t n)
-{
-  uint64_t nhits = 0;
-  for (size_t i = 0; i < n; ++i) {
-    const swtpg_tp& r = tps[i];
-    const uint32_t c = r.channel & 255u;
-    if (m_masked[c])
-      continue;
-    const uint32_t offline_channel = m_register_channels[c];
-    TriggerPrimitiveTypeAdapter tp;
-    tp.tp.time_start = r.time_start;
-    tp.tp.time_peak = r.time_peak;
-    tp.tp.time_over_threshold = r.time_over_threshold;
-    tp.tp.channel = offline_channel;
-    tp.tp.adc_integral = r.adc_integral;
-    tp.tp.adc_peak = r.adc_peak;
-    tp.tp.detid = uint16_t(m_det_id);
-    tp.tp.type = TriggerPrimitive::Type::kTPC;
-    tp.tp.algorithm = TriggerPrimitive::Algorithm::kUnknown; // never assigned in the reference (wib2/WIB2FrameProcessor.hpp:137)
-    tp.tp.version = 1;
-    if (tp.tp.time_over_threshold > m_tp_max_width)
-      m_tps_suppressed_too_long++;
-    else if (!m_tp_sink || !m_tp_sink(std::move(tp)))
-      m_tps_send_failed++;
-    m_new_tps++; // counted regardless of the outcome, as the reference does (:469-470)
-    ++nhits;
-    m_tp_channel_rate[c].fetch_add(1, std::memory_order_relaxed);
-  }
-  m_tpg_hits_count += nhits;
+  submit(fp, frame_handler->link);
 }
 
 // ---- TPCTPRequestHandler ----------------------------------------------------------------------------------------------
@@ -914,7 +789,7 @@ struct swtpg_host_conf
   uint32_t sink_capacity; // per link; try_send fails beyond it (0 = unbounded)
 };
 
-// The TPG fields of one link's RawDataProcessorConf, overriding those of swtpg_host_conf (swtpg_host_create_links).
+// The TPG fields of one link's RawDataProcessorConf, overriding those of swtpg_host_conf (swtpg_host_create with links).
 struct swtpg_host_link_conf
 {
   char tpg_algorithm[32];
@@ -933,12 +808,14 @@ struct swtpg_host_tp
   uint16_t version, flag;
 };
 
+using WIBEthProcessors = std::vector<std::unique_ptr<WIBEthFrameProcessor>>;
+using WIB2Processors = std::vector<std::unique_ptr<WIB2FrameProcessor>>;
+
 struct swtpg_host
 {
   std::shared_ptr<TpgEngine> engine;
   std::vector<std::unique_ptr<FrameErrorRegistry>> regs;
-  std::vector<std::unique_ptr<WIBEthFrameProcessor>> eth;
-  std::vector<std::unique_ptr<WIB2FrameProcessor>> wib2;
+  std::variant<WIBEthProcessors, WIB2Processors> procs; // one processor per link, all of the engine's format
   std::vector<std::vector<TriggerPrimitiveTypeAdapter>> queues;
   std::vector<std::unique_ptr<std::mutex>> qmu;
   uint32_t sink_capacity = 0;
@@ -949,6 +826,26 @@ struct swtpg_host
 
 static thread_local std::string g_host_error;
 
+// f(processors) with the handle's processor vector: the format is resolved once per C call, not once per payload.
+template<class F>
+static decltype(auto)
+with_processors(swtpg_host* h, F&& f)
+{
+  return std::visit(std::forward<F>(f), h->procs);
+}
+
+// Payload `index` of an array of P's frames through the consumer path of processor p: the pre-process tasks (may rewrite the
+// header in emulator mode — the buffer is the caller's, as the latency buffer element is in the reference), then the
+// post-process task.
+template<class P>
+static void
+push_payload(P& p, void* payloads, size_t index)
+{
+  auto* fp = static_cast<typename P::frameptr>(payloads) + index;
+  p.preprocess_item(fp);
+  p.postprocess_item(fp);
+}
+
 extern "C" {
 
 const char*
@@ -957,8 +854,10 @@ swtpg_host_last_error(void)
   return g_host_error.c_str();
 }
 
-static swtpg_host*
-host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_t flags = SWTPG_FLAG_NONE)
+// links: NULL, or links[n_links], each frame processor's conf() with its own TPG fields (one engine, links with different
+// configurations). flags: SWTPG_FLAG_* for the engine's handle (SWTPG_FLAG_ADC_STATS: the processors' get_adc_stats).
+swtpg_host*
+swtpg_host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_t flags)
 {
   try {
     auto h = std::make_unique<swtpg_host>();
@@ -968,6 +867,8 @@ host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_
     h->count_only = c->count_only_sink != 0;
     h->queues.resize(c->n_links);
     h->regs.resize(c->n_links); // the processors keep REFERENCES to these unique_ptrs (as the reference's model does): no reallocation later
+    if (c->format != SWTPG_FORMAT_WIBETH)
+      h->procs.emplace<WIB2Processors>();
     for (uint32_t l = 0; l < c->n_links; ++l) {
       h->qmu.push_back(std::make_unique<std::mutex>());
       h->regs[l] = std::make_unique<FrameErrorRegistry>();
@@ -1008,15 +909,12 @@ host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_
         hp->queues[l].push_back(std::move(tp));
         return true;
       };
-      if (c->format == SWTPG_FORMAT_WIBETH) {
-        h->eth.push_back(std::make_unique<WIBEthFrameProcessor>(h->regs[l], h->engine));
-        h->eth[l]->init(sink);
-        h->eth[l]->conf(rc);
-      } else {
-        h->wib2.push_back(std::make_unique<WIB2FrameProcessor>(h->regs[l], h->engine));
-        h->wib2[l]->init(sink);
-        h->wib2[l]->conf(rc);
-      }
+      with_processors(hp, [&](auto& procs) {
+        using P = typename std::decay_t<decltype(procs)>::value_type::element_type;
+        procs.push_back(std::make_unique<P>(h->regs[l], h->engine));
+        procs.back()->init(sink);
+        procs.back()->conf(rc);
+      });
     }
     return h.release();
   } catch (const TPGAlgorithmInexistent& e) {
@@ -1025,26 +923,6 @@ host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_
     g_host_error = e.what();
   }
   return nullptr;
-}
-
-swtpg_host*
-swtpg_host_create(const swtpg_host_conf* c)
-{
-  return host_create(c, nullptr);
-}
-
-// links[n_links]: each frame processor's conf() gets its own TPG fields (one engine, links with different configurations)
-swtpg_host*
-swtpg_host_create_links(const swtpg_host_conf* c, const swtpg_host_link_conf* links)
-{
-  return host_create(c, links);
-}
-
-// The same with SWTPG_FLAG_* for the engine's handle (SWTPG_FLAG_ADC_STATS: the processors' get_adc_stats); links may be NULL.
-swtpg_host*
-swtpg_host_create_flags(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_t flags)
-{
-  return host_create(c, links, flags);
 }
 
 void
@@ -1057,10 +935,10 @@ int
 swtpg_host_start(swtpg_host* h)
 {
   try {
-    for (auto& p : h->eth)
-      p->start();
-    for (auto& p : h->wib2)
-      p->start();
+    with_processors(h, [](auto& procs) {
+      for (auto& p : procs)
+        p->start();
+    });
     return 0;
   } catch (const std::exception& e) {
     g_host_error = e.what();
@@ -1072,10 +950,10 @@ int
 swtpg_host_stop(swtpg_host* h)
 {
   try {
-    for (auto& p : h->eth)
-      p->stop();
-    for (auto& p : h->wib2)
-      p->stop();
+    with_processors(h, [](auto& procs) {
+      for (auto& p : procs)
+        p->stop();
+    });
     return 0;
   } catch (const std::exception& e) {
     g_host_error = e.what();
@@ -1083,21 +961,12 @@ swtpg_host_stop(swtpg_host* h)
   }
 }
 
-// One payload of one link through the consumer path: pre-process tasks (may rewrite the header in emulator mode — the
-// buffer is the caller's, as the latency buffer element is in the reference), then the post-process task.
+// One payload of one link through the consumer path
 int
 swtpg_host_push(swtpg_host* h, uint32_t link, void* payload)
 {
   try {
-    if (!h->eth.empty()) {
-      auto* fp = static_cast<DUNEWIBEthTypeAdapter*>(payload);
-      h->eth[link]->preprocess_item(fp);
-      h->eth[link]->postprocess_item(fp);
-    } else {
-      auto* fp = static_cast<DUNEWIBSuperChunkTypeAdapter*>(payload);
-      h->wib2[link]->preprocess_item(fp);
-      h->wib2[link]->postprocess_item(fp);
-    }
+    with_processors(h, [&](auto& procs) { push_payload(*procs[link], payload, 0); });
     return 0;
   } catch (const std::exception& e) {
     g_host_error = e.what();
@@ -1110,31 +979,22 @@ swtpg_host_push(swtpg_host* h, uint32_t link, void* payload)
 int
 swtpg_host_push_parallel(swtpg_host* h, void* payloads, uint32_t n_units)
 {
-  const size_t n_links = h->eth.empty() ? h->wib2.size() : h->eth.size();
-  const size_t unit_bytes = h->eth.empty() ? sizeof(DUNEWIBSuperChunkTypeAdapter) : sizeof(DUNEWIBEthTypeAdapter);
-  std::vector<std::thread> threads;
+  const size_t n_links = h->queues.size();
   std::vector<std::string> errors(n_links);
-  for (size_t l = 0; l < n_links; ++l)
-    threads.emplace_back([=, &errors]() {
-      try {
-        for (uint32_t u = 0; u < n_units; ++u) {
-          char* p = static_cast<char*>(payloads) + (l * n_units + u) * unit_bytes;
-          if (!h->eth.empty()) {
-            auto* fp = reinterpret_cast<DUNEWIBEthTypeAdapter*>(p);
-            h->eth[l]->preprocess_item(fp);
-            h->eth[l]->postprocess_item(fp);
-          } else {
-            auto* fp = reinterpret_cast<DUNEWIBSuperChunkTypeAdapter*>(p);
-            h->wib2[l]->preprocess_item(fp);
-            h->wib2[l]->postprocess_item(fp);
-          }
+  with_processors(h, [&](auto& procs) {
+    std::vector<std::thread> threads;
+    for (size_t l = 0; l < n_links; ++l)
+      threads.emplace_back([=, &errors, &procs]() {
+        try {
+          for (uint32_t u = 0; u < n_units; ++u)
+            push_payload(*procs[l], payloads, l * n_units + u);
+        } catch (const std::exception& e) {
+          errors[l] = e.what();
         }
-      } catch (const std::exception& e) {
-        errors[l] = e.what();
-      }
-    });
-  for (auto& t : threads)
-    t.join();
+      });
+    for (auto& t : threads)
+      t.join();
+  });
   for (auto& e : errors)
     if (!e.empty()) {
       g_host_error = e;
@@ -1160,54 +1020,44 @@ int
 swtpg_host_push_feeders(swtpg_host* h, void* payloads, uint32_t n_units, uint32_t n_threads, uint32_t burst, double pace, uint32_t passes,
                         swtpg_host_feed_stats* out)
 {
-  const size_t n_links = h->eth.empty() ? h->wib2.size() : h->eth.size();
-  const bool eth = !h->eth.empty();
-  const size_t unit_bytes = eth ? sizeof(DUNEWIBEthTypeAdapter) : sizeof(DUNEWIBSuperChunkTypeAdapter);
-  const double period_s = (eth ? 2048.0 : 12.0 * 32.0) / 62.5e6;
+  const size_t n_links = h->queues.size();
+  const double period_s = (std::holds_alternative<WIBEthProcessors>(h->procs) ? 2048.0 : 12.0 * 32.0) / 62.5e6;
   n_threads = std::max<uint32_t>(1, std::min<uint32_t>(n_threads, uint32_t(n_links)));
   burst = std::max<uint32_t>(1, std::min(burst, n_units));
-  std::vector<std::thread> threads;
   std::vector<std::string> errors(n_threads);
   std::vector<double> cpu(n_threads, 0.0);
   std::vector<uint64_t> late(n_threads, 0);
   const auto t_start = std::chrono::steady_clock::now() + std::chrono::milliseconds(2);
-  for (uint32_t t = 0; t < n_threads; ++t)
-    threads.emplace_back([=, &errors, &cpu, &late]() {
-      try {
-        for (uint32_t pass = 0; pass < passes; ++pass)
-          for (uint32_t u0 = 0; u0 < n_units; u0 += burst) {
-            const uint32_t u1 = std::min(n_units, u0 + burst);
-            if (pace > 0) {
-              const double due_s = (double(pass) * n_units + u1) * period_s / pace;
-              const auto due = t_start + std::chrono::duration_cast<std::chrono::steady_clock::duration>(std::chrono::duration<double>(due_s));
-              if (std::chrono::steady_clock::now() < due)
-                std::this_thread::sleep_until(due);
-              else
-                ++late[t];
-            }
-            for (size_t l = t; l < n_links; l += n_threads)
-              for (uint32_t u = u0; u < u1; ++u) {
-                char* p = static_cast<char*>(payloads) + (l * n_units + u) * unit_bytes;
-                if (eth) {
-                  auto* fp = reinterpret_cast<DUNEWIBEthTypeAdapter*>(p);
-                  h->eth[l]->preprocess_item(fp);
-                  h->eth[l]->postprocess_item(fp);
-                } else {
-                  auto* fp = reinterpret_cast<DUNEWIBSuperChunkTypeAdapter*>(p);
-                  h->wib2[l]->preprocess_item(fp);
-                  h->wib2[l]->postprocess_item(fp);
-                }
+  with_processors(h, [&](auto& procs) {
+    std::vector<std::thread> threads;
+    for (uint32_t t = 0; t < n_threads; ++t)
+      threads.emplace_back([=, &errors, &cpu, &late, &procs]() {
+        try {
+          for (uint32_t pass = 0; pass < passes; ++pass)
+            for (uint32_t u0 = 0; u0 < n_units; u0 += burst) {
+              const uint32_t u1 = std::min(n_units, u0 + burst);
+              if (pace > 0) {
+                const double due_s = (double(pass) * n_units + u1) * period_s / pace;
+                const auto due = t_start + std::chrono::duration_cast<std::chrono::steady_clock::duration>(std::chrono::duration<double>(due_s));
+                if (std::chrono::steady_clock::now() < due)
+                  std::this_thread::sleep_until(due);
+                else
+                  ++late[t];
               }
-          }
-        timespec ts{};
-        clock_gettime(CLOCK_THREAD_CPUTIME_ID, &ts);
-        cpu[t] = double(ts.tv_sec) + 1e-9 * double(ts.tv_nsec);
-      } catch (const std::exception& e) {
-        errors[t] = e.what();
-      }
-    });
-  for (auto& th : threads)
-    th.join();
+              for (size_t l = t; l < n_links; l += n_threads)
+                for (uint32_t u = u0; u < u1; ++u)
+                  push_payload(*procs[l], payloads, l * n_units + u);
+            }
+          timespec ts{};
+          clock_gettime(CLOCK_THREAD_CPUTIME_ID, &ts);
+          cpu[t] = double(ts.tv_sec) + 1e-9 * double(ts.tv_nsec);
+        } catch (const std::exception& e) {
+          errors[t] = e.what();
+        }
+      });
+    for (auto& th : threads)
+      th.join();
+  });
   const double wall = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
   for (auto& e : errors)
     if (!e.empty()) {
@@ -1266,10 +1116,7 @@ swtpg_host_take_tps(swtpg_host* h, uint32_t link, swtpg_host_tp* out, size_t cap
 void
 swtpg_host_get_info(swtpg_host* h, uint32_t link, RawDataProcessorInfo* info)
 {
-  if (!h->eth.empty())
-    h->eth[link]->get_info(*info);
-  else
-    h->wib2[link]->get_info(*info);
+  with_processors(h, [&](auto& procs) { procs[link]->get_info(*info); });
 }
 
 uint64_t
@@ -1283,13 +1130,14 @@ swtpg_host_error_count(swtpg_host* h, uint32_t link, const char* name)
 uint32_t
 swtpg_host_misconfigurations(swtpg_host* h, uint32_t link)
 {
-  return h->eth.empty() ? 0u : uint32_t(h->eth[link]->misconfigurations().size());
+  const auto* eth = std::get_if<WIBEthProcessors>(&h->procs);
+  return eth ? uint32_t((*eth)[link]->misconfigurations().size()) : 0u;
 }
 
 uint64_t
 swtpg_host_last_daq_time(swtpg_host* h, uint32_t link)
 {
-  return h->eth.empty() ? h->wib2[link]->get_last_daq_time() : h->eth[link]->get_last_daq_time();
+  return with_processors(h, [&](auto& procs) { return procs[link]->get_last_daq_time(); });
 }
 
 // Zero-copy ingest: register / unregister the array the pushed payloads live in (the "latency buffer")
@@ -1315,10 +1163,7 @@ swtpg_host_adc_stats(swtpg_host* h, uint32_t link, int reset, ChannelAdcStats* o
 {
   try {
     std::vector<ChannelAdcStats> v;
-    if (!h->eth.empty())
-      h->eth.at(link)->get_adc_stats(v, reset != 0);
-    else
-      h->wib2.at(link)->get_adc_stats(v, reset != 0);
+    with_processors(h, [&](auto& procs) { procs.at(link)->get_adc_stats(v, reset != 0); });
     const size_t n = std::min<size_t>(v.size(), cap);
     std::copy(v.begin(), v.begin() + n, out);
     return int(n);
@@ -1332,10 +1177,9 @@ swtpg_host_adc_stats(swtpg_host* h, uint32_t link, int reset, ChannelAdcStats* o
 void
 swtpg_host_register_channel_map(swtpg_host* h, uint32_t link, uint32_t* out64)
 {
-  if (h->eth.empty())
-    return;
-  for (int p = 0; p < 64; ++p)
-    out64[p] = h->eth[link]->handler()->register_channel_map[size_t(p)];
+  if (const auto* eth = std::get_if<WIBEthProcessors>(&h->procs))
+    for (int p = 0; p < 64; ++p)
+      out64[p] = (*eth)[link]->handler()->register_channel_map[size_t(p)];
 }
 
 // ---- TPCTPRequestHandler harness ---------------------------------------------------------------------------------------------

@@ -287,6 +287,87 @@ public:
   virtual void process_swtpg_hits(const swtpg_tp* tps, size_t n) = 0; // records of THIS link, any order
 };
 
+// ---- the link plumbing both TPC formats share ----------------------------------------------------------------------------
+// What WIBEthFrameProcessor and WIB2FrameProcessor of the reference each write out in full: the link's attachment in conf(),
+// the TPG part of start / stop / get_info, the per-channel tables built on the first frame, the submit of find_hits and the
+// TriggerPrimitive tail of process_swtpg_hits. kChannels: frame channels of one payload. kCountEveryTp: num_tps_sent and the
+// hit rate count every record that passed the mask, whatever tp_timeout or tp_out made of it (WIB2,
+// src/wib2/WIB2FrameProcessor.cpp:469-470), rather than only the records tp_out accepted (WIBEth).
+template<class ReadoutType, class FrameHandler, uint32_t kChannels, bool kCountEveryTp>
+class TpcFrameProcessor : public TaskRawDataProcessorModel<ReadoutType>, public FrameProcessorBase
+{
+  static_assert((kChannels & (kChannels - 1)) == 0, "a record's frame channel is its channel field modulo kChannels");
+
+public:
+  using inherited = TaskRawDataProcessorModel<ReadoutType>;
+  using frameptr = ReadoutType*;
+  using constframeptr = const ReadoutType*;
+
+  void init(TpSink tp_out) { m_tp_sink = std::move(tp_out); } // reference: get_iom_sender("tp_out")
+  void start() override;
+  void stop() override;
+  void get_info(RawDataProcessorInfo& info);
+  // Not in the reference: the ADC statistics of this link's channels since the last reset (engine flag SWTPG_FLAG_ADC_STATS), by
+  // the offline channel its TPs carry, masked channels included. Empty until the first frame has built the channel map.
+  void get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset);
+  void process_swtpg_hits(const swtpg_tp* tps, size_t n) override; // fed with device TP records
+  FrameHandler* handler() { return m_frame_handler.get(); }
+
+protected:
+  TpcFrameProcessor(std::unique_ptr<FrameErrorRegistry>& error_registry, std::shared_ptr<TpgEngine> engine);
+  // The rest of conf() once the caller has parsed its algorithm into `a` and registered its pre-process tasks: the link's
+  // tp_timeout, channel mask, ids and back-pressure policy, and with enable_tpg its engine link, configuration, threshold
+  // table and the post-process task find_hits.
+  void conf_link(const RawDataProcessorConf& config, const swtpg_config& a, std::function<void(constframeptr)> find_hits);
+  // First frame: the offline channel offline_of(c) that records of frame channel c are reported with, its mask flag, a zeroed
+  // rate counter; then get_info and get_adc_stats may read them.
+  template<class OfflineOf>
+  void set_channel_tables(OfflineOf offline_of)
+  {
+    for (uint32_t c = 0; c < kChannels; ++c) {
+      m_offline_of_channel[c] = offline_of(c);
+      m_masked[c] = m_channel_mask_set.count(m_offline_of_channel[c]) ? 1 : 0;
+      m_tp_channel_rate[c].store(0, std::memory_order_relaxed);
+    }
+    m_maps_ready.store(true, std::memory_order_release);
+  }
+  // The frame is only borrowed for the duration of find_hits: swtpg_submit copies it into the pinned staging slot — unless it
+  // lies in a latency buffer registered with the engine, which the copy engine then reads directly (zero-copy ingest).
+  // Non-blocking by default, like the reference's try_send: a full ring drops the frame and counts it. With
+  // block_on_backpressure the thread SLEEPS until the completion thread has freed ring space (swtpg_submit_wait). TPs come
+  // back through the engine's delivery thread (process_swtpg_hits), never through this thread.
+  void submit(constframeptr fp, uint32_t link)
+  {
+    if (!m_block) {
+      if (!m_engine->submit(link, fp->data, sizeof fp->data))
+        ++m_frames_dropped;
+    } else {
+      while (!m_engine->submit(link, fp->data, sizeof fp->data, 100000)) {
+      }
+    }
+  }
+
+  std::shared_ptr<TpgEngine> m_engine;
+  std::unique_ptr<FrameHandler> m_frame_handler;
+  TpSink m_tp_sink;
+  ChannelMap m_channel_map;
+  bool m_tpg_enabled = false, m_block = false;
+  TriggerPrimitive::Algorithm m_tp_algo = TriggerPrimitive::Algorithm::kUnknown; // never assigned for WIB2 (wib2/WIB2FrameProcessor.hpp:137)
+  uint64_t m_tp_max_width = 0;
+  std::set<uint32_t> m_channel_mask_set;
+  uint32_t m_crate_no = 0, m_slot_no = 0, m_link_no = 0, m_det_id = 0;
+  // m_tp_channel_rate_map of the reference, kept as one counter per FRAME channel (the key of every record) and turned into
+  // (offline channel -> count) pairs in get_info; the channel mask likewise is looked up once per channel
+  std::array<std::atomic<uint32_t>, kChannels> m_tp_channel_rate{};
+  std::array<uint32_t, kChannels> m_offline_of_channel{};
+  std::array<uint8_t, kChannels> m_masked{};
+  std::atomic<bool> m_maps_ready{ false };
+  uint64_t m_previous_ts = 0, m_current_ts = 0;
+  std::atomic<uint64_t> m_ts_error_ctr{ 0 }, m_new_tps{ 0 }, m_tpg_hits_count{ 0 }, m_tps_suppressed_too_long{ 0 }, m_tps_send_failed{ 0 },
+    m_frames_dropped{ 0 };
+  std::chrono::time_point<std::chrono::high_resolution_clock> m_t0;
+};
+
 // ---- WIBEth ---------------------------------------------------------------------------------------------------------------
 // include/fdreadoutlibs/wibeth/WIBEthFrameProcessor.hpp:45-71. The handler keeps its role (per-link TPG resources) but the
 // resources are now a link slot of the engine instead of a hit buffer + ProcessingInfo.
@@ -300,63 +381,30 @@ public:
 };
 
 // include/fdreadoutlibs/wibeth/WIBEthFrameProcessor.hpp:73-205
-class WIBEthFrameProcessor : public TaskRawDataProcessorModel<DUNEWIBEthTypeAdapter>, public FrameProcessorBase
+class WIBEthFrameProcessor : public TpcFrameProcessor<DUNEWIBEthTypeAdapter, WIBEthFrameHandler, SWTPG_WIBETH_CHANNELS, false>
 {
 public:
-  using inherited = TaskRawDataProcessorModel<DUNEWIBEthTypeAdapter>;
-  using frameptr = DUNEWIBEthTypeAdapter*;
-  using constframeptr = const DUNEWIBEthTypeAdapter*;
+  WIBEthFrameProcessor(std::unique_ptr<FrameErrorRegistry>& error_registry, std::shared_ptr<TpgEngine> engine)
+    : TpcFrameProcessor(error_registry, std::move(engine))
+  {
+  }
 
-  WIBEthFrameProcessor(std::unique_ptr<FrameErrorRegistry>& error_registry, std::shared_ptr<TpgEngine> engine);
-  ~WIBEthFrameProcessor() override;
-
-  void init(TpSink tp_out) { m_tp_sink = std::move(tp_out); } // reference: get_iom_sender("tp_out") (:158-170)
-  void conf(const RawDataProcessorConf& cfg) override;         // (:172-235)
-  void start() override;                                        // (:111-144)
-  void stop() override;                                         // (:146-154)
-  void get_info(RawDataProcessorInfo& info);                    // (:237-292)
-  // Not in the reference: the ADC statistics of this link's channels since the last reset (engine flag SWTPG_FLAG_ADC_STATS), by
-  // the offline channel its TPs carry, masked channels included. Empty until the first frame has built the channel map.
-  void get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset);
-
-  void sequence_check(frameptr fp);                             // (:298-353)
-  void timestamp_check(frameptr fp);                            // (:359-405)
+  void conf(const RawDataProcessorConf& cfg) override;                 // (:172-235)
+  void start() override;                                                // (:111-144)
+  void get_info(RawDataProcessorInfo& info);                            // (:237-292)
+  void sequence_check(frameptr fp);                                     // (:298-353)
+  void timestamp_check(frameptr fp);                                    // (:359-405)
   void find_hits(constframeptr fp, WIBEthFrameHandler* frame_handler); // (:410-476)
-  void process_swtpg_hits(const swtpg_tp* tps, size_t n) override;     // (:478-572), fed with device TP records
 
   const std::vector<LinkMisconfiguration>& misconfigurations() const { return m_misconf; }
-  WIBEthFrameHandler* handler() { return m_wibeth_frame_handler.get(); }
 
 private:
-  std::shared_ptr<TpgEngine> m_engine;
-  std::unique_ptr<WIBEthFrameHandler> m_wibeth_frame_handler;
-  TpSink m_tp_sink;
-  ChannelMap m_channel_map;
-  bool m_tpg_enabled = false, m_enable_simple_threshold_on_collection = false, m_correct_lookup = false, m_block = false;
-  std::string m_tpg_algorithm;
-  TriggerPrimitive::Algorithm m_tp_algo = TriggerPrimitive::Algorithm::kUnknown;
-  uint16_t m_tpg_threshold = 0, m_tpg_rs_memory_factor = 0, m_tpg_rs_scale_factor = 0;
-  int16_t m_tpg_frugal_streaming_accumulator_limit = 0;
-  uint64_t m_tp_max_width = 0;
-  std::set<uint32_t> m_channel_mask_set;
-  uint32_t m_crate_no = 0, m_slot_no = 0, m_stream_id = 0, m_det_id = 0;
-  std::array<uint32_t, 64> m_register_channels{};
-  // m_tp_channel_rate_map of the reference (:263-284), kept as one counter per FRAME channel (the key of every record) and
-  // turned into (offline channel -> count) pairs in get_info; the channel mask likewise is looked up once per channel
-  std::array<std::atomic<uint32_t>, 64> m_tp_channel_rate{};
-  std::array<uint32_t, 64> m_offline_of_channel{};
-  std::array<uint8_t, 64> m_masked{};
-  std::atomic<bool> m_maps_ready{ false };
-  std::mutex m_rate_mu;
+  bool m_enable_simple_threshold_on_collection = false, m_correct_lookup = false;
+  uint16_t m_tpg_rs_memory_factor = 0;
   std::vector<LinkMisconfiguration> m_misconf;
-
-  uint64_t m_previous_ts = 0, m_current_ts = 0;
   uint16_t m_previous_seq_id = 0, m_current_seq_id = 0;
-  bool m_first_ts_missmatch = true, m_first_seq_id_mismatch = true;
-  std::atomic<uint64_t> m_ts_error_ctr{ 0 }, m_seq_id_error_ctr{ 0 };
+  std::atomic<uint64_t> m_seq_id_error_ctr{ 0 };
   std::atomic<int16_t> m_seq_id_min_jump{ 0 }, m_seq_id_max_jump{ 0 };
-  std::atomic<uint64_t> m_new_tps{ 0 }, m_tpg_hits_count{ 0 }, m_tps_suppressed_too_long{ 0 }, m_tps_send_failed{ 0 }, m_frames_dropped{ 0 };
-  std::chrono::time_point<std::chrono::high_resolution_clock> m_t0;
 };
 
 // ---- WIB2 -----------------------------------------------------------------------------------------------------------------
@@ -370,46 +418,21 @@ public:
   void reset() { first_hit = true; }
 };
 
-class WIB2FrameProcessor : public TaskRawDataProcessorModel<DUNEWIBSuperChunkTypeAdapter>, public FrameProcessorBase
+class WIB2FrameProcessor : public TpcFrameProcessor<DUNEWIBSuperChunkTypeAdapter, WIB2FrameHandler, SWTPG_WIB2_CHANNELS, true>
 {
 public:
-  using inherited = TaskRawDataProcessorModel<DUNEWIBSuperChunkTypeAdapter>;
-  using frameptr = DUNEWIBSuperChunkTypeAdapter*;
-  using constframeptr = const DUNEWIBSuperChunkTypeAdapter*;
+  WIB2FrameProcessor(std::unique_ptr<FrameErrorRegistry>& error_registry, std::shared_ptr<TpgEngine> engine)
+    : TpcFrameProcessor(error_registry, std::move(engine))
+  {
+  }
 
-  WIB2FrameProcessor(std::unique_ptr<FrameErrorRegistry>& error_registry, std::shared_ptr<TpgEngine> engine);
-  ~WIB2FrameProcessor() override;
-  void init(TpSink tp_out) { m_tp_sink = std::move(tp_out); }
-  void conf(const RawDataProcessorConf& cfg) override; // src/wib2/WIB2FrameProcessor.cpp:196-229
-  void start() override;
-  void stop() override;
-  void get_info(RawDataProcessorInfo& info);
-  void get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset); // as WIBEthFrameProcessor::get_adc_stats
-  void timestamp_check(frameptr fp);                                  // (:293-340)
-  void find_hits(constframeptr fp, WIB2FrameHandler* frame_handler);  // (:345-396)
-  void process_swtpg_hits(const swtpg_tp* tps, size_t n) override;    // (:398-479)
-  WIB2FrameHandler* handler() { return m_handler.get(); }
-
-private:
-  std::shared_ptr<TpgEngine> m_engine;
-  std::unique_ptr<WIB2FrameHandler> m_handler;
-  TpSink m_tp_sink;
-  ChannelMap m_channel_map;
-  bool m_tpg_enabled = false, m_block = false;
-  uint64_t m_tp_max_width = 0;
-  std::set<uint32_t> m_channel_mask_set;
-  uint32_t m_crate_no = 0, m_slot_no = 0, m_link = 0, m_det_id = 0;
-  std::array<uint32_t, 256> m_register_channels{};
-  std::array<std::atomic<uint32_t>, 256> m_tp_channel_rate{};
-  std::array<uint8_t, 256> m_masked{};
-  std::atomic<bool> m_maps_ready{ false };
-  std::mutex m_rate_mu;
-  uint64_t m_previous_ts = 0, m_current_ts = 0;
-  bool m_first_ts_missmatch = true;
-  std::atomic<uint64_t> m_ts_error_ctr{ 0 }, m_new_tps{ 0 }, m_tpg_hits_count{ 0 }, m_tps_suppressed_too_long{ 0 }, m_tps_send_failed{ 0 },
-    m_frames_dropped{ 0 };
-  std::chrono::time_point<std::chrono::high_resolution_clock> m_t0;
+  void conf(const RawDataProcessorConf& cfg) override;                // src/wib2/WIB2FrameProcessor.cpp:196-229
+  void timestamp_check(frameptr fp);                                   // (:293-340)
+  void find_hits(constframeptr fp, WIB2FrameHandler* frame_handler); // (:345-396)
 };
+
+extern template class TpcFrameProcessor<DUNEWIBEthTypeAdapter, WIBEthFrameHandler, SWTPG_WIBETH_CHANNELS, false>;
+extern template class TpcFrameProcessor<DUNEWIBSuperChunkTypeAdapter, WIB2FrameHandler, SWTPG_WIB2_CHANNELS, true>;
 
 // ---- downstream of the path: TPs -> time-ordered TPSets -------------------------------------------------------------------
 // trigger::TPSet as send_tp_sets fills it (src/TPCTPRequestHandler.cpp:145-165)

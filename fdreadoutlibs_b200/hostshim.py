@@ -61,10 +61,9 @@ class TpHandlerInfo(C.Structure):
 
 EXPORTS = ["swtpg_host_tpsets_create", "swtpg_host_tpsets_destroy", "swtpg_host_tpsets_receive", "swtpg_host_tpsets_cycle",
            "swtpg_host_tpsets_cutoff", "swtpg_host_tpsets_count", "swtpg_host_tpsets_get", "swtpg_host_tpsets_info",
-           "swtpg_host_push_parallel", "swtpg_host_push_feeders", "swtpg_host_tp_count", "swtpg_host_counters", "swtpg_host_stream_timing", "swtpg_host_last_error", "swtpg_host_create", "swtpg_host_create_links", "swtpg_host_destroy", "swtpg_host_start", "swtpg_host_stop", "swtpg_host_push",
+           "swtpg_host_push_parallel", "swtpg_host_push_feeders", "swtpg_host_tp_count", "swtpg_host_counters", "swtpg_host_stream_timing", "swtpg_host_last_error", "swtpg_host_create", "swtpg_host_destroy", "swtpg_host_start", "swtpg_host_stop", "swtpg_host_push",
            "swtpg_host_take_tps", "swtpg_host_get_info", "swtpg_host_error_count", "swtpg_host_misconfigurations",
-           "swtpg_host_last_daq_time", "swtpg_host_register_channel_map", "swtpg_host_register_buffer", "swtpg_host_adc_stats",
-           "swtpg_host_create_flags"]
+           "swtpg_host_last_daq_time", "swtpg_host_register_channel_map", "swtpg_host_register_buffer", "swtpg_host_adc_stats"]
 
 _lib = None
 
@@ -75,9 +74,7 @@ def host_lib():
         lib = C.CDLL(HOST_LIB_PATH)
         lib.swtpg_host_last_error.restype = C.c_char_p
         lib.swtpg_host_create.restype = C.c_void_p
-        lib.swtpg_host_create.argtypes = [C.POINTER(HostConf)]
-        lib.swtpg_host_create_links.restype = C.c_void_p
-        lib.swtpg_host_create_links.argtypes = [C.POINTER(HostConf), C.POINTER(HostLinkConf)]
+        lib.swtpg_host_create.argtypes = [C.POINTER(HostConf), C.POINTER(HostLinkConf), C.c_uint32]
         lib.swtpg_host_destroy.argtypes = [C.c_void_p]
         lib.swtpg_host_start.argtypes = [C.c_void_p]
         lib.swtpg_host_stop.argtypes = [C.c_void_p]
@@ -100,8 +97,6 @@ def host_lib():
         lib.swtpg_host_last_daq_time.argtypes = [C.c_void_p, C.c_uint32]
         lib.swtpg_host_register_channel_map.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
         lib.swtpg_host_register_buffer.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int]
-        lib.swtpg_host_create_flags.restype = C.c_void_p
-        lib.swtpg_host_create_flags.argtypes = [C.POINTER(HostConf), C.POINTER(HostLinkConf), C.c_uint32]
         lib.swtpg_host_adc_stats.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p, C.c_uint32]
         lib.swtpg_host_tpsets_create.restype = C.c_void_p
         lib.swtpg_host_tpsets_create.argtypes = [C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32, C.c_uint32]
@@ -153,12 +148,8 @@ class FrameProcessors:
         c.n_slots = n_slots
         self.lib = host_lib()
         self.n_links = n_links
-        if adc_stats:
-            assert link_confs is None
-            self.h = self.lib.swtpg_host_create_flags(C.byref(c), None, 2)  # SWTPG_FLAG_ADC_STATS
-        elif link_confs is None:
-            self.h = self.lib.swtpg_host_create(C.byref(c))
-        else:
+        links = None
+        if link_confs is not None:
             assert len(link_confs) == n_links
             links = (HostLinkConf * n_links)()
             for l, lc in enumerate(link_confs):
@@ -169,7 +160,7 @@ class FrameProcessors:
                 links[l].tpg_frugal_streaming_accumulator_limit = lc.get("acc_limit", acc_limit)
                 for p, t in enumerate(lc.get("plane_threshold", (-1, -1, -1))):
                     links[l].tpg_plane_threshold[p] = t
-            self.h = self.lib.swtpg_host_create_links(C.byref(c), links)
+        self.h = self.lib.swtpg_host_create(C.byref(c), links, 2 if adc_stats else 0)  # SWTPG_FLAG_ADC_STATS
         if not self.h:
             raise HostError(self.lib.swtpg_host_last_error().decode())
 

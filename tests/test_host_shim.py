@@ -3,6 +3,7 @@ sequence_check + timestamp_check pre-tasks, find_hits post-task, process_swtpg_h
 CPU part: the library loads, exports its harness, refuses unknown algorithms the way the reference does and fails loudly
 without a device. GPU part: TriggerPrimitives equal the oracle's TPs pushed through the same LUT / mask / timeout logic."""
 import ctypes as C
+from collections import Counter
 
 import numpy as np
 import pytest
@@ -11,7 +12,7 @@ import fdreadoutlibs_b200 as S
 from fdreadoutlibs_b200 import hostshim as H
 from fdreadoutlibs_b200 import frames as F
 from oracle import binding as B
-from util import as_tuples, expected_host_tps, linear_map
+from util import HANDLE, adc_of, as_tuples, expected_host_tps, linear_map, oracle_for
 
 
 def test_host_library_exports():
@@ -223,6 +224,116 @@ def test_wib2_frame_processor_end_to_end(algorithm, algo_id):
             assert as_tuples(got) == expected_host_tps(want[want["link"] == l], l, wib2=True), f"link {l}"
             assert (got["algorithm"] == 0).all()  # kUnknown: never assigned in the reference (wib2/WIB2FrameProcessor.hpp:137)
             assert fp.get_info(l)["num_ts_errors"] == 1
+
+
+def wib2_masked_case(seed, n_links=2, n_units=40, threshold=30):
+    """WIB2 units of n_links links, the oracle's records of them, a channel mask holding the two busiest channels of every link
+    and a tp_timeout that about a quarter of the records exceed."""
+    units = S.gen_wib2_host(S.gen_params(seed, 0.5), n_links, n_units)
+    want, _ = B.oracle_process_links(B.make_config(fmt="wib2", threshold=threshold), units)
+    mask = []
+    for l in range(n_links):
+        ch, n = np.unique(want[want["link"] == l]["channel"], return_counts=True)
+        mask += [linear_map(1, 0, l, int(c)) for c in ch[np.argsort(-n, kind="stable")[:2]]]
+    return units, want, tuple(mask), int(np.percentile(want["time_over_threshold"], 75))
+
+
+def push_all(fp, units):
+    fp.start()
+    for u in range(units.shape[1]):
+        for l in range(units.shape[0]):
+            fp.push(l, units[l, u].copy())
+    fp.stop()
+
+
+@pytest.mark.gpu
+def test_wib2_mask_timeout_and_bounded_sink():
+    """WIB2FrameProcessor::process_swtpg_hits (src/wib2/WIB2FrameProcessor.cpp:398-479): a masked channel's records are skipped,
+    one over tp_timeout is suppressed, one that tp_out refuses is counted as failed, and num_tps_sent counts every record that
+    passed the mask whatever became of it (:469-470). The TriggerPrimitives carry Algorithm::kUnknown."""
+    units, want, mask, timeout = wib2_masked_case(68)
+    n_links = units.shape[0]
+    wants = [want[want["link"] == l] for l in range(n_links)]
+    unmasked = [[r for r in w if linear_map(1, 0, l, int(r["channel"])) not in mask] for l, w in enumerate(wants)]
+    exp = [expected_host_tps(w, l, mask=mask, tp_timeout=timeout, wib2=True) for l, w in enumerate(wants)]
+    cap = min(len(e) for e in exp) // 2
+    with H.FrameProcessors(n_links, 8, fmt="wib2", threshold=30, channel_mask=mask, tp_timeout=timeout, sink_capacity=cap) as fp:
+        push_all(fp, units)
+        for l in range(n_links):
+            got, info = fp.take_tps(l), fp.get_info(l)
+            n_long = sum(1 for r in unmasked[l] if int(r["time_over_threshold"]) > timeout)
+            assert cap > 10 and n_long > 0 and len(unmasked[l]) < wants[l].size
+            # which records the sink takes depends on the delivery order: each is one of the expected ones
+            assert got.size == cap and not Counter(as_tuples(got)) - Counter(exp[l]), f"link {l}"
+            assert (got["algorithm"] == 0).all()
+            assert info["num_tps_suppressed_too_long"] == n_long and info["num_tps_send_failed"] == len(exp[l]) - cap
+            assert info["num_tps_sent"] == len(unmasked[l]) and info["num_frames_dropped_busy"] == 0
+
+
+@pytest.mark.gpu
+def test_wib2_get_info_top_channels():
+    """WIB2FrameProcessor::get_info's top channels: the ten offline channels with the most unmasked records
+    since the last call, too-long ones included, most first and ties in ascending channel order. The call resets the counts."""
+    units, want, mask, timeout = wib2_masked_case(69)
+    with H.FrameProcessors(units.shape[0], 8, fmt="wib2", threshold=30, channel_mask=mask, tp_timeout=timeout) as fp:
+        push_all(fp, units)
+        for l in range(units.shape[0]):
+            offline = [linear_map(1, 0, l, c) for c in range(256)]
+            n = Counter(linear_map(1, 0, l, int(r["channel"])) for r in want[want["link"] == l])
+            n = Counter({c: k for c, k in n.items() if c not in mask})
+            info = fp.get_info(l)
+            assert info["top"] == [(c, n[c]) for c in sorted(offline, key=lambda c: (-n[c], c))[:10]], f"link {l}"
+            assert info["num_tps_sent"] == sum(n.values()) and info["rate_tp_hits"] > 0
+            again = fp.get_info(l)
+            assert again["top"] == [(c, 0) for c in sorted(offline)[:10]]
+            assert again["num_tps_sent"] == again["num_tps_suppressed_too_long"] == again["num_tps_send_failed"] == 0
+            assert again["rate_tp_hits"] == 0
+
+
+@pytest.mark.gpu
+def test_wib2_adc_stats_by_offline_channel():
+    """get_adc_stats of each WIB2 processor: 256 entries under the offline channels of the frame channels (the direct map), a
+    masked channel too; mean, RMS, minimum and maximum as numpy computes them."""
+    n_links, n_units = 2, 16
+    units = S.gen_wib2_host(S.gen_params(591, 0.3), n_links, n_units)
+    masked = linear_map(1, 0, 0, 9)
+    with H.FrameProcessors(n_links, 8, fmt="wib2", channel_mask=(masked,), adc_stats=True) as fp:
+        assert fp.adc_stats(0).size == 0  # no frame yet: no channel map
+        push_all(fp, units)
+        got = [fp.adc_stats(l) for l in range(n_links)]
+    assert masked in got[0]["offline_channel"]
+    for l in range(n_links):
+        a = adc_of("wib2", units[l]).astype(np.float64)
+        g = got[l]
+        assert g.size == 256 and g["offline_channel"].tolist() == [linear_map(1, 0, l, c) for c in range(256)]
+        assert (g["samples"] == a.shape[0]).all()
+        np.testing.assert_allclose(g["mean"], a.mean(0), rtol=1e-12)
+        np.testing.assert_allclose(g["rms"], a.std(0), rtol=1e-9)
+        assert g["min"].tolist() == a.min(0).astype(int).tolist() and g["max"].tolist() == a.max(0).astype(int).tolist()
+
+
+@pytest.mark.gpu
+def test_adc_stats_with_per_link_configurations():
+    """adc_stats=True together with link_confs: two WIBEth links of one engine with different algorithms. Each link's
+    TriggerPrimitives equal the oracle's for its own configuration, and each link's ADC statistics equal numpy's."""
+    n_links, n_units = 2, 16
+    units = S.gen_wibeth_host(S.gen_params(592, 0.5), n_links, n_units)
+    confs = [dict(algorithm="SimpleThreshold", threshold=25), dict(algorithm="AbsRS", threshold=30)]
+    with H.FrameProcessors(n_links, 8, link_confs=confs, adc_stats=True) as fp:
+        push_all(fp, units)
+        got = [fp.take_tps(l) for l in range(n_links)]
+        stats = [fp.adc_stats(l) for l in range(n_links)]
+    for l, c in enumerate(confs):
+        want = oracle_for("wibeth", {**HANDLE, **c}, l).process(units[l])
+        assert want.size > 10 and as_tuples(got[l]) == expected_host_tps(want, l), f"link {l} ({c})"
+        assert (got[l]["algorithm"] == {"SimpleThreshold": 2, "AbsRS": 3}[c["algorithm"]]).all()
+        a = adc_of("wibeth", units[l]).astype(np.float64)
+        g = stats[l]
+        assert g["offline_channel"].tolist() == [linear_map(1, 0, l, int(F.position_to_channel(c))) for c in range(64)]
+        assert (g["samples"] == a.shape[0]).all()
+        np.testing.assert_allclose(g["mean"], a.mean(0), rtol=1e-12)
+        np.testing.assert_allclose(g["rms"], a.std(0), rtol=1e-9)
+        assert g["min"].tolist() == a.min(0).astype(int).tolist() and g["max"].tolist() == a.max(0).astype(int).tolist()
 
 
 @pytest.mark.gpu
