@@ -6,7 +6,8 @@ fails loudly if it has not been built.
 """
 from . import frames  # noqa: F401
 from .api import (ALGORITHMS, PinnedBuffer, SwtpgError, TPGAlgorithmInexistent, TPGenerator, device_available, firwin_int, gen_params,  # noqa: F401
-                  gen_wib2_device, gen_wib2_host, gen_wibeth_device, gen_wibeth_host, merge_sorted, sort_tps)
+                  gen_wib2_device, gen_wib2_host, gen_wibeth_device, gen_wibeth_host, merge_sorted, noise_frequencies, noise_power, sort_tps)
 
 __all__ = ["frames", "TPGenerator", "PinnedBuffer", "SwtpgError", "TPGAlgorithmInexistent", "ALGORITHMS", "device_available", "firwin_int",
-           "gen_params", "gen_wibeth_host", "gen_wib2_host", "gen_wibeth_device", "gen_wib2_device", "merge_sorted", "sort_tps"]
+           "gen_params", "gen_wibeth_host", "gen_wib2_host", "gen_wibeth_device", "gen_wib2_device", "merge_sorted", "noise_frequencies",
+           "noise_power", "sort_tps"]

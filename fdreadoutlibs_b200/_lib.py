@@ -68,6 +68,10 @@ class SwtpgAdcStats(C.Structure):
     ]
 
 
+class SwtpgNoiseLags(C.Structure):
+    _fields_ = [("segments", C.c_uint64), ("lag", C.c_uint64 * 33)]
+
+
 class SwtpgCounters(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in (
         "units_processed", "samples_processed", "tps_emitted", "tps_dropped_overflow", "batches", "submit_busy",
@@ -106,6 +110,8 @@ EXPORTS = {
     "swtpg_sync": (C.c_int, [C.c_void_p]),
     "swtpg_dump_state": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p]),
     "swtpg_read_adc_stats": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int]),
+    "swtpg_read_noise_lags": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int]),
+    "swtpg_noise_power": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "swtpg_get_counters": (C.c_int, [C.c_void_p, C.POINTER(SwtpgCounters)]),
     "swtpg_sort_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "swtpg_alloc_pinned": (C.c_void_p, [C.c_size_t, C.c_int]),

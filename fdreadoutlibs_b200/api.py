@@ -24,6 +24,7 @@ ALGORITHMS = {
 FORMATS = {"wibeth": FORMAT_WIBETH, "wib2": FORMAT_WIB2}
 FLAG_SORTED_TPS = 1  # SWTPG_FLAG_SORTED_TPS
 FLAG_ADC_STATS = 2  # SWTPG_FLAG_ADC_STATS
+FLAG_NOISE_SPECTRA = 8  # SWTPG_FLAG_NOISE_SPECTRA
 
 
 class SwtpgError(RuntimeError):
@@ -57,10 +58,12 @@ class TPGenerator:
     def __init__(self, n_links: int, max_units: int, *, fmt: str = "wibeth", algorithm: str = "SimpleThreshold", threshold: int = 60,
                  acc_limit: int = 10, rs_memory_factor: int = 8, rs_scale_factor: int = 5, fir_taps: Optional[Sequence[int]] = None,
                  tap_exponent: int = 6, tp_capacity: int = 0, n_slots: int = 0, device: int = 0, wib2_adc_offset: int = 0,
-                 dispatch_timeout_us: int = 0, sorted_tps: bool = False, adc_stats: bool = False):
+                 dispatch_timeout_us: int = 0, sorted_tps: bool = False, adc_stats: bool = False,
+                 noise_spectra: bool = False):
         """sorted_tps: SWTPG_FLAG_SORTED_TPS — every batch's TP list comes back ordered by (time_start, link, channel), ordered on
         the device (include/swtpg.h). adc_stats: SWTPG_FLAG_ADC_STATS — per-channel ADC statistics of every batch, read by
-        read_adc_stats()."""
+        read_adc_stats(). noise_spectra: SWTPG_FLAG_NOISE_SPECTRA — per-channel noise lag sums of every batch, read by
+        read_noise_lags() and turned into power spectra by noise_power()."""
         if algorithm not in ALGORITHMS:
             raise TPGAlgorithmInexistent(algorithm)
         cfg = SwtpgConfig()
@@ -82,7 +85,7 @@ class TPGenerator:
         cfg.tap_exponent = tap_exponent
         cfg.wib2_adc_offset = wib2_adc_offset
         cfg.dispatch_timeout_us = dispatch_timeout_us
-        cfg.flags = (FLAG_SORTED_TPS if sorted_tps else 0) | (FLAG_ADC_STATS if adc_stats else 0)
+        cfg.flags = (FLAG_SORTED_TPS if sorted_tps else 0) | (FLAG_ADC_STATS if adc_stats else 0) | (FLAG_NOISE_SPECTRA if noise_spectra else 0)
         self.cfg = cfg
         self.fmt = fmt
         self.n_links = n_links
@@ -311,6 +314,15 @@ class TPGenerator:
         self._check(lib.swtpg_read_adc_stats(self._h, link0, n_links, out.ctypes.data, 1 if reset else 0))
         return out
 
+    def read_noise_lags(self, link0: int = 0, n_links: Optional[int] = None, reset: bool = False) -> np.ndarray:
+        """swtpg_read_noise_lags: the current window of links [link0, link0 + n_links) (default: to the last link) as an
+        (n_links, channels) NOISE_LAGS_DTYPE array, by frame channel. reset=True starts a new window of those links."""
+        if n_links is None:
+            n_links = max(0, self.n_links - link0)
+        out = np.zeros((n_links, self.channels), dtype=F.NOISE_LAGS_DTYPE)
+        self._check(lib.swtpg_read_noise_lags(self._h, link0, n_links, out.ctypes.data, 1 if reset else 0))
+        return out
+
     def sort_stats(self) -> dict:
         """Device-side ordering (sorted_tps=True): ms of the last list, ms of all lists, lists ordered, lists the host finished."""
         a, b, n, f = C.c_double(0), C.c_double(0), C.c_uint64(0), C.c_uint64(0)
@@ -340,6 +352,24 @@ class PinnedBuffer:
             self.ptr = None
 
     __del__ = close
+
+
+def noise_power(lags: np.ndarray, fmt: str = "wibeth") -> np.ndarray:
+    """swtpg_noise_power: the averaged periodogram of NOISE_LAGS_DTYPE entries of a `fmt` handle, shape lags.shape + (N/2 + 1,),
+    in ADC counts^2 per bin (the mean over segments of |rfft(x)|^2 / N); bin k is at noise_frequencies(fmt)[k]. Entries without
+    segments give zeros."""
+    lags = np.ascontiguousarray(lags, dtype=F.NOISE_LAGS_DTYPE)
+    out = np.zeros(lags.shape + (F.NOISE_SEGMENT_TICKS[fmt] // 2 + 1,), dtype=np.float64)
+    st = lib.swtpg_noise_power(lags.ctypes.data, lags.size, FORMATS[fmt], out.ctypes.data)
+    if st != SWTPG_OK:
+        raise SwtpgError(st, "swtpg_noise_power")
+    return out
+
+
+def noise_frequencies(fmt: str = "wibeth") -> np.ndarray:
+    """Frequency in Hz of each bin of noise_power(.., fmt): k x 1.953125 MHz / N, k = 0 .. N/2."""
+    n = F.NOISE_SEGMENT_TICKS[fmt]
+    return np.arange(n // 2 + 1) * (F.SAMPLE_RATE_HZ / n)
 
 
 def sort_tps(tps: np.ndarray) -> np.ndarray:

@@ -29,6 +29,7 @@ static_assert(sizeof(swtpg_channel_state) == 48, "swtpg_channel_state layout cha
 static_assert(sizeof(swtpg_counters) == 80, "swtpg_counters layout changed");
 static_assert(sizeof(swtpg_link_config) == 36, "swtpg_link_config layout changed");
 static_assert(sizeof(swtpg_adc_stats) == 32, "swtpg_adc_stats layout changed");
+static_assert(sizeof(swtpg_noise_lags) == 272, "swtpg_noise_lags layout changed");
 
 namespace {
 thread_local std::string g_create_error;
@@ -334,12 +335,16 @@ reset_state(swtpg_handle* h)
 
 // swtpg_start: every window starts empty, after the statistics work of the previous run (reset_state then waits for the stream).
 swtpg_status
-reset_adc_stats(swtpg_handle* h)
+reset_channel_stats(swtpg_handle* h)
 {
   std::lock_guard<std::mutex> lk(h->stats_mu);
   if (h->stats_stream && h->stats_stream != h->stream)
     SW_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_stats, 0));
-  SW_CUDA(h, cudaMemsetAsync(h->d_adc_stats, 0, size_t(h->cfg.n_links) * h->channels * sizeof(swtpg_adc_stats), h->stream));
+  const size_t n = size_t(h->cfg.n_links) * h->channels;
+  if (h->d_adc_stats)
+    SW_CUDA(h, cudaMemsetAsync(h->d_adc_stats, 0, n * sizeof(swtpg_adc_stats), h->stream));
+  if (h->d_noise_lags)
+    SW_CUDA(h, cudaMemsetAsync(h->d_noise_lags, 0, n * sizeof(swtpg_noise_lags), h->stream));
   SW_CUDA(h, cudaEventRecord(h->ev_stats, h->stream));
   h->stats_stream = h->stream;
   return SWTPG_OK;
@@ -406,8 +411,8 @@ enqueue_batch(swtpg_handle* h, const void* d_frames, const uint32_t* n_units, ui
                     : launch_groups<false>(h, d_frames, d_nu, stride, h->d_tps, h->d_count, ped, wav, s));
     SW_CUDA(h, cudaEventRecord(h->ev1, s));
     h->timed = true;
-    if (h->d_adc_stats)
-      SW_CUDA(h, swtpg_internal::launch_adc_stats(h, d_frames, d_nu, stride, s));
+    if (h->channel_stats())
+      SW_CUDA(h, swtpg_internal::launch_channel_stats(h, d_frames, d_nu, stride, s));
   }
   h->last_stream = s;
   h->counters.units_processed += units;
@@ -553,6 +558,44 @@ same_group(int32_t format, const TpgConf& a, const TpgConf& b)
   return true;
 }
 
+// swtpg_read_adc_stats / swtpg_read_noise_lags: copies the window of links [link0, link0 + n_links) of a device accumulator
+// d[n_links][channels] to the pinned mirror hbuf and, on reset, zeroes it, in stream order. The caller holds read_mu and has checked
+// the arguments; returns when hbuf holds the window.
+template<typename T>
+swtpg_status
+read_window(swtpg_handle* h, T* d, T* hbuf, uint32_t link0, uint32_t n_links, int reset)
+{
+  const size_t first = size_t(link0) * h->channels, n = size_t(n_links) * h->channels;
+  {
+    // Copy and reset are enqueued back to back on the stream of the last batch: a batch enqueued meanwhile falls after both.
+    std::lock_guard<std::mutex> lk(h->stats_mu);
+    const cudaStream_t s = h->stats_stream ? h->stats_stream : h->stream;
+    SW_CUDA(h, cudaMemcpyAsync(hbuf + first, d + first, n * sizeof(T), cudaMemcpyDeviceToHost, s));
+    if (reset) {
+      SW_CUDA(h, cudaMemsetAsync(d + first, 0, n * sizeof(T), s));
+      SW_CUDA(h, cudaEventRecord(h->ev_stats, s));
+      h->stats_stream = s;
+    }
+    SW_CUDA(h, cudaEventRecord(h->ev_stats_read, s));
+  }
+  SW_CUDA(h, cudaEventSynchronize(h->ev_stats_read));
+  return SWTPG_OK;
+}
+
+swtpg_status
+check_read_args(swtpg_handle* h, uint32_t link0, uint32_t n_links, const void* out, const void* acc, const char* no_flag)
+{
+  if (!h)
+    return fail(nullptr, SWTPG_ERR_INVALID_ARG, "handle is NULL");
+  if (!out)
+    return fail(h, SWTPG_ERR_INVALID_ARG, "out is NULL");
+  if (!acc)
+    return fail(h, SWTPG_ERR_STATE, no_flag);
+  if (uint64_t(link0) + n_links > h->cfg.n_links)
+    return fail(h, SWTPG_ERR_INVALID_ARG, "link0 + n_links exceeds cfg.n_links");
+  return SWTPG_OK;
+}
+
 } // namespace
 
 cudaError_t
@@ -644,7 +687,7 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
     return fail(nullptr, cs, why);
   if (cfg->wib2_adc_offset % 4 != 0 || cfg->wib2_adc_offset > SWTPG_WIB2_FRAME_BYTES - 448)
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "wib2_adc_offset must be a multiple of 4 and leave room for the 448-byte ADC block");
-  if (cfg->flags & ~(SWTPG_FLAG_SORTED_TPS | SWTPG_FLAG_ADC_STATS))
+  if (cfg->flags & ~(SWTPG_FLAG_SORTED_TPS | SWTPG_FLAG_ADC_STATS | SWTPG_FLAG_NOISE_SPECTRA))
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "unknown bits in swtpg_config.flags");
 
   int ndev = 0;
@@ -714,6 +757,14 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
     SW_CUDA(hp, cudaMalloc(&h->d_adc_stats, bytes));
     SW_CUDA(hp, cudaMemset(h->d_adc_stats, 0, bytes));
     SW_CUDA(hp, cudaMallocHost(&h->h_adc_stats, bytes));
+  }
+  if (cfg->flags & SWTPG_FLAG_NOISE_SPECTRA) {
+    const size_t bytes = size_t(cfg->n_links) * h->channels * sizeof(swtpg_noise_lags);
+    SW_CUDA(hp, cudaMalloc(&h->d_noise_lags, bytes));
+    SW_CUDA(hp, cudaMemset(h->d_noise_lags, 0, bytes));
+    SW_CUDA(hp, cudaMallocHost(&h->h_noise_lags, bytes));
+  }
+  if (h->channel_stats()) {
     SW_CUDA(hp, cudaEventCreateWithFlags(&h->ev_stats, cudaEventDisableTiming));
     SW_CUDA(hp, cudaEventCreateWithFlags(&h->ev_stats_read, cudaEventDisableTiming));
   }
@@ -758,6 +809,8 @@ swtpg_destroy(swtpg_handle* h)
   if (h->sorter) swtpg_internal::sorter_destroy(h->sorter);
   if (h->d_adc_stats) cudaFree(h->d_adc_stats);
   if (h->h_adc_stats) cudaFreeHost(h->h_adc_stats);
+  if (h->d_noise_lags) cudaFree(h->d_noise_lags);
+  if (h->h_noise_lags) cudaFreeHost(h->h_noise_lags);
   if (h->ev_stats) cudaEventDestroy(h->ev_stats);
   if (h->ev_stats_read) cudaEventDestroy(h->ev_stats_read);
   delete[] h->h_rs_factor;
@@ -773,7 +826,7 @@ swtpg_start(swtpg_handle* h)
   swtpg_status s = SWTPG_OK;
   if (h->conf_groups_stale && (s = form_conf_groups(h)) != SWTPG_OK)
     return s;
-  if (h->d_adc_stats && (s = reset_adc_stats(h)) != SWTPG_OK)
+  if (h->channel_stats() && (s = reset_channel_stats(h)) != SWTPG_OK)
     return s;
   s = reset_state(h);
   if (s != SWTPG_OK)
@@ -1145,32 +1198,14 @@ swtpg_dump_state(swtpg_handle* h, uint32_t link, swtpg_channel_state* out)
 swtpg_status
 swtpg_read_adc_stats(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_adc_stats* out, int reset)
 {
-  if (!h)
-    return fail(nullptr, SWTPG_ERR_INVALID_ARG, "handle is NULL");
-  if (!out)
-    return fail(h, SWTPG_ERR_INVALID_ARG, "out is NULL");
-  if (!h->d_adc_stats)
-    return fail(h, SWTPG_ERR_STATE, "the handle was created without SWTPG_FLAG_ADC_STATS");
-  if (uint64_t(link0) + n_links > h->cfg.n_links)
-    return fail(h, SWTPG_ERR_INVALID_ARG, "link0 + n_links exceeds cfg.n_links");
-  if (n_links == 0)
-    return SWTPG_OK;
+  swtpg_status st = check_read_args(h, link0, n_links, out, h ? h->d_adc_stats : nullptr, "the handle was created without SWTPG_FLAG_ADC_STATS");
+  if (st != SWTPG_OK || n_links == 0)
+    return st;
   SW_CUDA(h, cudaSetDevice(h->cfg.device));
   std::lock_guard<std::mutex> rd(h->read_mu);
+  if ((st = read_window(h, h->d_adc_stats, h->h_adc_stats, link0, n_links, reset)) != SWTPG_OK)
+    return st;
   const size_t first = size_t(link0) * h->channels, n = size_t(n_links) * h->channels;
-  {
-    // Copy and reset are enqueued back to back on the stream of the last batch: a batch enqueued meanwhile falls after both.
-    std::lock_guard<std::mutex> lk(h->stats_mu);
-    const cudaStream_t s = h->stats_stream ? h->stats_stream : h->stream;
-    SW_CUDA(h, cudaMemcpyAsync(h->h_adc_stats + first, h->d_adc_stats + first, n * sizeof(swtpg_adc_stats), cudaMemcpyDeviceToHost, s));
-    if (reset) {
-      SW_CUDA(h, cudaMemsetAsync(h->d_adc_stats + first, 0, n * sizeof(swtpg_adc_stats), s));
-      SW_CUDA(h, cudaEventRecord(h->ev_stats, s));
-      h->stats_stream = s;
-    }
-    SW_CUDA(h, cudaEventRecord(h->ev_stats_read, s));
-  }
-  SW_CUDA(h, cudaEventSynchronize(h->ev_stats_read));
   for (size_t i = 0; i < n; ++i) {
     const swtpg_adc_stats& a = h->h_adc_stats[first + i];
     uint32_t ext[2];
@@ -1183,6 +1218,20 @@ swtpg_read_adc_stats(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_ad
     o.max = a.samples ? uint16_t(ext[1]) : 0;
     o.reserved = 0;
   }
+  return SWTPG_OK;
+}
+
+swtpg_status
+swtpg_read_noise_lags(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_noise_lags* out, int reset)
+{
+  swtpg_status st = check_read_args(h, link0, n_links, out, h ? h->d_noise_lags : nullptr, "the handle was created without SWTPG_FLAG_NOISE_SPECTRA");
+  if (st != SWTPG_OK || n_links == 0)
+    return st;
+  SW_CUDA(h, cudaSetDevice(h->cfg.device));
+  std::lock_guard<std::mutex> rd(h->read_mu);
+  if ((st = read_window(h, h->d_noise_lags, h->h_noise_lags, link0, n_links, reset)) != SWTPG_OK)
+    return st;
+  memcpy(out, h->h_noise_lags + size_t(link0) * h->channels, size_t(n_links) * h->channels * sizeof(swtpg_noise_lags));
   return SWTPG_OK;
 }
 

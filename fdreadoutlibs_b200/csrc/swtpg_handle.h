@@ -2,7 +2,7 @@
 //   swtpg_capi.cu    create / destroy / start / stop, the batch entry points and the kernel launch table
 //   swtpg_stream.cu  the streaming path (swtpg_submit ... swtpg_poll): per-link rings, dispatcher and completion threads,
 //                    the gather kernel that pulls frames out of pinned host memory
-//   swtpg_stats.cu   the per-channel ADC statistics kernel (SWTPG_FLAG_ADC_STATS)
+//   swtpg_stats.cu   the per-channel statistics kernel (SWTPG_FLAG_ADC_STATS, SWTPG_FLAG_NOISE_SPECTRA)
 // Not installed; nothing outside csrc/ includes it.
 #pragma once
 
@@ -119,16 +119,21 @@ struct swtpg_handle
   std::vector<uint8_t> rs_table_link; // [n_links] 1 = the link's rows of h_rs_factor were set (else its configuration's factor)
   swtpg_internal::TpSorter* sorter = nullptr; // SWTPG_FLAG_SORTED_TPS: device-side ordering of TP lists (swtpg_sort.cu)
 
-  // SWTPG_FLAG_ADC_STATS (all null without it). d_adc_stats[n_links][channels] holds the current window of every channel in the
+  // SWTPG_FLAG_ADC_STATS (null without it). d_adc_stats[n_links][channels] holds the current window of every channel in the
   // layout of swtpg_adc_stats, except its last 8 bytes: {16383 - min, max} as two 32-bit words, so that zeroed memory is an empty
-  // window and both merge by atomicMax. Every statistics kernel and every read runs in one order: each waits for ev_stats, which
-  // is recorded after the last of them on stats_stream, when it runs on another stream. stats_mu guards those two and keeps a
-  // read's copy and reset together; read_mu serialises reads (h_adc_stats, ev_stats_read).
+  // window and both merge by atomicMax.
   swtpg_adc_stats* d_adc_stats = nullptr;
   swtpg_adc_stats* h_adc_stats = nullptr; // pinned, same size
+  // SWTPG_FLAG_NOISE_SPECTRA (null without it): d_noise_lags[n_links][channels], the current window in the layout of swtpg_noise_lags.
+  swtpg_noise_lags* d_noise_lags = nullptr;
+  swtpg_noise_lags* h_noise_lags = nullptr; // pinned, same size
+  // Either flag (all null without both). Every statistics kernel and every read runs in one order: each waits for ev_stats, which
+  // is recorded after the last of them on stats_stream, when it runs on another stream. stats_mu guards those two and keeps a
+  // read's copy and reset together; read_mu serialises reads (h_adc_stats, h_noise_lags, ev_stats_read).
   cudaEvent_t ev_stats = nullptr, ev_stats_read = nullptr;
   cudaStream_t stats_stream = nullptr;
   std::mutex stats_mu, read_mu;
+  bool channel_stats() const { return d_adc_stats || d_noise_lags; } // every batch gets a launch_channel_stats
 
   // streaming path (swtpg_stream.cu), created on the first swtpg_submit / swtpg_register_buffer
   std::mutex engine_mu;
@@ -195,9 +200,10 @@ fail(swtpg_handle* h, swtpg_status s, const char* msg)
 cudaError_t launch_batch_kernel(swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t units_stride, swtpg_tp* d_tps,
                                 unsigned* d_count, cudaStream_t s);
 
-// swtpg_stats.cu: adds one batch, laid out as for launch_batch_kernel, to the per-channel ADC statistics (SWTPG_FLAG_ADC_STATS) on
-// stream `s`, after the statistics work of earlier batches and reads whatever stream that ran on.
-cudaError_t launch_adc_stats(swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t units_stride, cudaStream_t s);
+// swtpg_stats.cu: adds one batch, laid out as for launch_batch_kernel, to the per-channel ADC statistics (SWTPG_FLAG_ADC_STATS)
+// and noise lags (SWTPG_FLAG_NOISE_SPECTRA) the handle keeps, in one read of the batch on stream `s`, after the statistics work of
+// earlier batches and reads whatever stream that ran on.
+cudaError_t launch_channel_stats(swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t units_stride, cudaStream_t s);
 
 // swtpg_sort.cu: device-side ordering of a batch's TP list (SWTPG_FLAG_SORTED_TPS)
 TpSorter* sorter_create();

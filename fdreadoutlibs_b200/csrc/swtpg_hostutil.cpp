@@ -1,5 +1,5 @@
-// Host-only pieces of libswtpg_b200.so (plain g++; no CUDA): the staging copy of swtpg_submit, the FIR tap design and the
-// host-side ordering / merge of TP lists.
+// Host-only pieces of libswtpg_b200.so (plain g++; no CUDA): the staging copy of swtpg_submit, the FIR tap design, the
+// host-side ordering / merge of TP lists and the noise power spectra of swtpg_noise_power.
 #include "../../include/swtpg.h"
 
 #include <algorithm>
@@ -238,4 +238,47 @@ swtpg_firwin_int(int n, double cutoff, int multiplier, int16_t* taps)
   for (int m = 0; m < n; ++m)
     taps[m] = int16_t(std::round(multiplier * (v[size_t(m)] / sum)));
   return n;
+}
+
+// ---- noise power spectra -------------------------------------------------------------------------------------------------
+// swtpg_noise_power (include/swtpg.h): the cosine transform of the circular lag sums of swtpg_read_noise_lags.
+extern "C" swtpg_status
+swtpg_noise_power(const swtpg_noise_lags* in, size_t n, int format, double* power)
+{
+  if ((!in || !power) && n)
+    return SWTPG_ERR_INVALID_ARG;
+  if (format != SWTPG_FORMAT_WIBETH && format != SWTPG_FORMAT_WIB2)
+    return SWTPG_ERR_UNSUPPORTED;
+  const int N = int(format == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_NOISE_SEGMENT_TICKS : SWTPG_WIBETH_NOISE_SEGMENT_TICKS);
+  const int bins = N / 2 + 1;
+  const double kPi = 3.14159265358979323846;
+  std::vector<double> c(size_t(bins) * bins); // c[k][tau]: weight of lag[tau] in bin k (1, 2 cos(2 pi k tau / N), cos(pi k))
+  for (int k = 0; k < bins; ++k)
+    for (int tau = 0; tau < bins; ++tau)
+      c[size_t(k) * bins + tau] = (tau == 0 || tau == N / 2 ? 1.0 : 2.0) * std::cos(2 * kPi * ((k * tau) % N) / N);
+  for (size_t i = 0; i < n; ++i) {
+    const swtpg_noise_lags& a = in[i];
+    double* p = power + i * size_t(bins);
+    if (a.segments == 0) {
+      std::fill(p, p + bins, 0.0);
+      continue;
+    }
+    const double scale = 1.0 / (double(N) * double(a.segments));
+    double p0 = 0;
+    for (int tau = 0; tau < bins; ++tau)
+      p0 += c[size_t(tau)] * double(a.lag[tau]);
+    p[0] = p0 * scale;
+    // k >= 1: the weights sum to 0, so lag[tau] - lag[0] (exact in int64: 0 <= lag[tau] <= lag[0] < 2^63) gives the same sum
+    // without the pedestal's N x 900^2 per segment drowning the noise in rounding.
+    double d[SWTPG_WIBETH_NOISE_SEGMENT_TICKS / 2 + 1];
+    for (int tau = 0; tau < bins; ++tau)
+      d[tau] = double(int64_t(a.lag[tau]) - int64_t(a.lag[0]));
+    for (int k = 1; k < bins; ++k) {
+      double s = 0;
+      for (int tau = 1; tau < bins; ++tau)
+        s += c[size_t(k) * bins + tau] * d[tau];
+      p[k] = s * scale;
+    }
+  }
+  return SWTPG_OK;
 }

@@ -122,7 +122,7 @@ struct Batch
   cudaEvent_t ev_gather = nullptr, ev_kernel = nullptr, ev_count = nullptr, ev_tps = nullptr;
   cudaEvent_t ev_up = nullptr;                  // pointer table and lengths are on the device (the gather stream waits for it)
   cudaEvent_t ev_g0 = nullptr, ev_k0 = nullptr; // timing: start of the gather / of the TPG kernel (device clocks, swtpg_stream_timing)
-  cudaEvent_t ev_stats = nullptr;               // the ADC statistics kernel has read d_frames (SWTPG_FLAG_ADC_STATS only)
+  cudaEvent_t ev_stats = nullptr;               // the statistics kernel has read d_frames (swtpg_handle::channel_stats only)
   uint32_t n_ready = 0, n_taken = 0;
   bool overflow = false;
   bool released = false; // the release thread has handed the batch's ring slots back (guarded by StreamEngine::mu)
@@ -254,11 +254,11 @@ StreamEngine::enqueue(Batch& b)
   TRY(cudaEventRecord(b.ev_k0, h->stream));
   TRY(launch_batch_kernel(h, b.d_frames, b.d_nunits, M, b.d_tps, b.d_count, h->stream));
   TRY(cudaEventRecord(b.ev_kernel, h->stream));
-  if (h->d_adc_stats) { // after ev_kernel (stream timing is the TPG kernel's alone), and before ev_count: the batch is not reused earlier
-    TRY(launch_adc_stats(h, b.d_frames, b.d_nunits, M, h->stream));
+  if (h->channel_stats()) { // after ev_kernel (stream timing is the TPG kernel's alone), and before ev_count: the batch is not reused earlier
+    TRY(launch_channel_stats(h, b.d_frames, b.d_nunits, M, h->stream));
     TRY(cudaEventRecord(b.ev_stats, h->stream));
   }
-  TRY(cudaStreamWaitEvent(b.stream, h->d_adc_stats ? b.ev_stats : b.ev_kernel, 0));
+  TRY(cudaStreamWaitEvent(b.stream, h->channel_stats() ? b.ev_stats : b.ev_kernel, 0));
   TRY(cudaMemcpyAsync(b.h_count, b.d_count, sizeof(unsigned), cudaMemcpyDeviceToHost, b.stream));
   TRY(cudaEventRecord(b.ev_count, b.stream));
 #undef TRY
@@ -527,7 +527,7 @@ engine_create(swtpg_handle* h, StreamEngine** out)
     ok(cudaEventCreate(&b.ev_k0));
     ok(cudaEventCreateWithFlags(&b.ev_count, cudaEventDisableTiming | cudaEventBlockingSync));
     ok(cudaEventCreateWithFlags(&b.ev_tps, cudaEventDisableTiming | cudaEventBlockingSync));
-    if (h->d_adc_stats)
+    if (h->channel_stats())
       ok(cudaEventCreateWithFlags(&b.ev_stats, cudaEventDisableTiming));
     if (ce != cudaSuccess) {
       cleanup();

@@ -59,6 +59,13 @@ ADC_STATS_DTYPE = np.dtype(
 )
 assert ADC_STATS_DTYPE.itemsize == 32
 
+# swtpg_noise_lags of include/swtpg.h: one channel over one window of swtpg_read_noise_lags (WIB2 fills lag[0..24])
+NOISE_LAGS_DTYPE = np.dtype([("segments", "<u8"), ("lag", "<u8", (33,))], align=True)
+assert NOISE_LAGS_DTYPE.itemsize == 272
+# SWTPG_*_NOISE_SEGMENT_TICKS: ticks per noise-spectrum segment (one WIBEth frame, four WIB2 superchunks)
+NOISE_SEGMENT_TICKS = {"wibeth": 64, "wib2": 48}
+SAMPLE_RATE_HZ = 62.5e6 / 32  # one ADC sample per channel every 32 ticks of the 62.5 MHz timing clock
+
 # Lane l of AVX2 register r holds frame channel 16r + LANE_PERM[l] (unittest/WIBEthFrameExpansion_test.cxx:111,124).
 LANE_PERM = np.array([0, 1, 2, 3, 4, 5, 6, 7, 15, 8, 9, 10, 11, 12, 13, 14], dtype=np.int64)
 

@@ -161,6 +161,15 @@ TpgEngine::read_adc_stats(uint32_t link, swtpg_adc_stats* out, uint32_t n_channe
 }
 
 void
+TpgEngine::read_noise_lags(uint32_t link, swtpg_noise_lags* out, uint32_t n_channels, bool reset)
+{
+  const uint32_t channels = m_cfg.format == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_CHANNELS : SWTPG_WIBETH_CHANNELS;
+  if (n_channels != channels)
+    throw std::invalid_argument("TpgEngine::read_noise_lags: one entry per frame channel of the link");
+  check(m_h, swtpg_read_noise_lags(m_h, link, 1, out, reset ? 1 : 0), "swtpg_read_noise_lags");
+}
+
+void
 TpgEngine::set_link_thresholds(uint32_t link, const uint16_t* by_channel, uint32_t n_channels)
 {
   const uint32_t channels = m_cfg.format == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_CHANNELS : SWTPG_WIBETH_CHANNELS;
@@ -416,6 +425,27 @@ TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::get_adc_stats(std::vector<Cha
   m_engine->read_adc_stats(m_frame_handler->link, s, kChannels, reset);
   for (uint32_t c = 0; c < kChannels; ++c)
     out.push_back(channel_adc_stats(m_offline_of_channel[c], s[c]));
+}
+
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
+void
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::get_noise_spectra(std::vector<ChannelNoiseSpectrum>& out, bool reset)
+{
+  out.clear();
+  if (!m_maps_ready.load(std::memory_order_acquire))
+    return;
+  std::vector<swtpg_noise_lags> lags(kChannels);
+  std::vector<double> power(kChannels * (SWTPG_WIBETH_NOISE_SEGMENT_TICKS / 2 + 1));
+  m_engine->read_noise_lags(m_frame_handler->link, lags.data(), kChannels, reset);
+  const swtpg_format fmt = m_engine->format();
+  const size_t bins = (fmt == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_NOISE_SEGMENT_TICKS : SWTPG_WIBETH_NOISE_SEGMENT_TICKS) / 2 + 1;
+  check(nullptr, swtpg_noise_power(lags.data(), kChannels, fmt, power.data()), "swtpg_noise_power");
+  out.resize(kChannels);
+  for (uint32_t c = 0; c < kChannels; ++c) {
+    out[c].offline_channel = m_offline_of_channel[c];
+    out[c].segments = lags[c].segments;
+    std::copy(power.begin() + c * bins, power.begin() + (c + 1) * bins, out[c].power);
+  }
 }
 
 template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
@@ -855,7 +885,8 @@ swtpg_host_last_error(void)
 }
 
 // links: NULL, or links[n_links], each frame processor's conf() with its own TPG fields (one engine, links with different
-// configurations). flags: SWTPG_FLAG_* for the engine's handle (SWTPG_FLAG_ADC_STATS: the processors' get_adc_stats).
+// configurations). flags: SWTPG_FLAG_* for the engine's handle (SWTPG_FLAG_ADC_STATS: the processors' get_adc_stats;
+// SWTPG_FLAG_NOISE_SPECTRA: their get_noise_spectra).
 swtpg_host*
 swtpg_host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_t flags)
 {
@@ -1164,6 +1195,23 @@ swtpg_host_adc_stats(swtpg_host* h, uint32_t link, int reset, ChannelAdcStats* o
   try {
     std::vector<ChannelAdcStats> v;
     with_processors(h, [&](auto& procs) { procs.at(link)->get_adc_stats(v, reset != 0); });
+    const size_t n = std::min<size_t>(v.size(), cap);
+    std::copy(v.begin(), v.begin() + n, out);
+    return int(n);
+  } catch (const std::exception& e) {
+    g_host_error = e.what();
+    return -1;
+  }
+}
+
+// ChannelNoiseSpectrum of a link's processor: out[cap] (64 WIBEth / 256 WIB2 entries, none before the first frame); the entry count, -1 on error
+static_assert(sizeof(ChannelNoiseSpectrum) == 280, "hostshim.HOST_NOISE_SPECTRUM_DTYPE mirrors ChannelNoiseSpectrum");
+int
+swtpg_host_noise_spectra(swtpg_host* h, uint32_t link, int reset, ChannelNoiseSpectrum* out, uint32_t cap)
+{
+  try {
+    std::vector<ChannelNoiseSpectrum> v;
+    with_processors(h, [&](auto& procs) { procs.at(link)->get_noise_spectra(v, reset != 0); });
     const size_t n = std::min<size_t>(v.size(), cap);
     std::copy(v.begin(), v.begin() + n, out);
     return int(n);

@@ -229,6 +229,17 @@ struct ChannelAdcStats
   uint16_t min = 0, max = 0;
 };
 
+// Not a reference type: the noise power spectrum of one channel of a link over one window of swtpg_read_noise_lags (swtpg_noise_power
+// of its lags), reported under the offline channel that channel's TPs carry. power[k] is bin k at k x 1.953125 MHz / N, in ADC
+// counts^2 (the mean over segments of |rfft|^2 / N): N / 2 + 1 = 33 bins for WIBEth, 25 for WIB2 (the rest zero); all zero when
+// segments == 0.
+struct ChannelNoiseSpectrum
+{
+  uint32_t offline_channel = 0;
+  uint64_t segments = 0;
+  double power[SWTPG_WIBETH_NOISE_SEGMENT_TICKS / 2 + 1] = {};
+};
+
 // ---- the GPU pipeline shared by the links of one device -------------------------------------------------------------------
 class FrameProcessorBase;
 // One swtpg_handle per GPU; every frame processor attached to it owns one link index. Any link's post-processing thread
@@ -254,6 +265,9 @@ public:
   void set_link_thresholds(uint32_t link, const uint16_t* by_channel, uint32_t n_channels);
   // swtpg_read_adc_stats of one link: out[n_channels] by frame channel (an engine created with SWTPG_FLAG_ADC_STATS). After conf().
   void read_adc_stats(uint32_t link, swtpg_adc_stats* out, uint32_t n_channels, bool reset);
+  // swtpg_read_noise_lags of one link: out[n_channels] by frame channel (an engine created with SWTPG_FLAG_NOISE_SPECTRA). After conf().
+  void read_noise_lags(uint32_t link, swtpg_noise_lags* out, uint32_t n_channels, bool reset);
+  swtpg_format format() const { return swtpg_format(m_cfg.format); }
   // false = back-pressure (the link's ring is full). wait_us > 0: sleep up to that long for room first (swtpg_submit_wait)
   bool submit(uint32_t link, const void* unit, size_t bytes, uint64_t wait_us = 0);
   // Zero-copy ingest: the latency buffer(s) the constframeptrs point into (swtpg_register_buffer). After conf().
@@ -310,6 +324,10 @@ public:
   // Not in the reference: the ADC statistics of this link's channels since the last reset (engine flag SWTPG_FLAG_ADC_STATS), by
   // the offline channel its TPs carry, masked channels included. Empty until the first frame has built the channel map.
   void get_adc_stats(std::vector<ChannelAdcStats>& out, bool reset);
+  // Not in the reference: the noise power spectra of this link's channels since the last reset (engine flag
+  // SWTPG_FLAG_NOISE_SPECTRA), by the offline channel its TPs carry, masked channels included. Empty until the first frame has
+  // built the channel map.
+  void get_noise_spectra(std::vector<ChannelNoiseSpectrum>& out, bool reset);
   void process_swtpg_hits(const swtpg_tp* tps, size_t n) override; // fed with device TP records
   FrameHandler* handler() { return m_frame_handler.get(); }
 
@@ -320,7 +338,7 @@ protected:
   // table and the post-process task find_hits.
   void conf_link(const RawDataProcessorConf& config, const swtpg_config& a, std::function<void(constframeptr)> find_hits);
   // First frame: the offline channel offline_of(c) that records of frame channel c are reported with, its mask flag, a zeroed
-  // rate counter; then get_info and get_adc_stats may read them.
+  // rate counter; then get_info, get_adc_stats and get_noise_spectra may read them.
   template<class OfflineOf>
   void set_channel_tables(OfflineOf offline_of)
   {

@@ -37,6 +37,10 @@ HOST_ADC_STATS_DTYPE = np.dtype([("offline_channel", "<u4"), ("samples", "<u8"),
                                  ("max", "<u2")], align=True)
 assert HOST_ADC_STATS_DTYPE.itemsize == 40
 
+# ChannelNoiseSpectrum of swtpg_host.hpp (WIB2 fills power[0..24])
+HOST_NOISE_SPECTRUM_DTYPE = np.dtype([("offline_channel", "<u4"), ("segments", "<u8"), ("power", "<f8", (33,))], align=True)
+assert HOST_NOISE_SPECTRUM_DTYPE.itemsize == 280
+
 
 class HostInfo(C.Structure):
     _fields_ = [("num_seq_id_errors", C.c_uint64), ("min_seq_id_jump", C.c_int32), ("max_seq_id_jump", C.c_int32),
@@ -63,7 +67,8 @@ EXPORTS = ["swtpg_host_tpsets_create", "swtpg_host_tpsets_destroy", "swtpg_host_
            "swtpg_host_tpsets_cutoff", "swtpg_host_tpsets_count", "swtpg_host_tpsets_get", "swtpg_host_tpsets_info",
            "swtpg_host_push_parallel", "swtpg_host_push_feeders", "swtpg_host_tp_count", "swtpg_host_counters", "swtpg_host_stream_timing", "swtpg_host_last_error", "swtpg_host_create", "swtpg_host_destroy", "swtpg_host_start", "swtpg_host_stop", "swtpg_host_push",
            "swtpg_host_take_tps", "swtpg_host_get_info", "swtpg_host_error_count", "swtpg_host_misconfigurations",
-           "swtpg_host_last_daq_time", "swtpg_host_register_channel_map", "swtpg_host_register_buffer", "swtpg_host_adc_stats"]
+           "swtpg_host_last_daq_time", "swtpg_host_register_channel_map", "swtpg_host_register_buffer", "swtpg_host_adc_stats",
+           "swtpg_host_noise_spectra"]
 
 _lib = None
 
@@ -98,6 +103,7 @@ def host_lib():
         lib.swtpg_host_register_channel_map.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
         lib.swtpg_host_register_buffer.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int]
         lib.swtpg_host_adc_stats.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p, C.c_uint32]
+        lib.swtpg_host_noise_spectra.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p, C.c_uint32]
         lib.swtpg_host_tpsets_create.restype = C.c_void_p
         lib.swtpg_host_tpsets_create.argtypes = [C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32, C.c_uint32]
         lib.swtpg_host_tpsets_destroy.argtypes = [C.c_void_p]
@@ -126,11 +132,13 @@ class FrameProcessors:
                  crate_id: int = 1, slot_id: int = 0, first_link_id: int = 0, enable_tpg: bool = True, emulator_mode: bool = False,
                  correct_channel_lookup: bool = False, reversed_map: bool = False, collection_simple_threshold: bool = False,
                  sink_capacity: int = 0, block_on_backpressure: bool = True, device: int = 0, count_only_sink: bool = False,
-                 n_slots: int = 4, link_confs=None, adc_stats: bool = False):
+                 n_slots: int = 4, link_confs=None, adc_stats: bool = False,
+                 noise_spectra: bool = False):
         """link_confs: optional list of n_links dicts, each overriding algorithm, threshold, rs_memory_factor, rs_scale_factor
         and acc_limit for its link's conf(); the keys it leaves out take the arguments above. A dict may also set
         plane_threshold: three thresholds by plane (0 = collection), -1 = the link's threshold (tpg_plane_threshold).
-        adc_stats: the engine's handle accumulates per-channel ADC statistics (SWTPG_FLAG_ADC_STATS), read by adc_stats()."""
+        adc_stats: the engine's handle accumulates per-channel ADC statistics (SWTPG_FLAG_ADC_STATS), read by adc_stats().
+        noise_spectra: it accumulates per-channel noise lags (SWTPG_FLAG_NOISE_SPECTRA), read as spectra by noise_spectra()."""
         c = HostConf()
         c.device, c.format, c.n_links, c.superchunk_units = device, 1 if fmt == "wib2" else 0, n_links, superchunk_units
         c.tpg_algorithm = algorithm.encode()
@@ -160,7 +168,8 @@ class FrameProcessors:
                 links[l].tpg_frugal_streaming_accumulator_limit = lc.get("acc_limit", acc_limit)
                 for p, t in enumerate(lc.get("plane_threshold", (-1, -1, -1))):
                     links[l].tpg_plane_threshold[p] = t
-        self.h = self.lib.swtpg_host_create(C.byref(c), links, 2 if adc_stats else 0)  # SWTPG_FLAG_ADC_STATS
+        flags = (2 if adc_stats else 0) | (8 if noise_spectra else 0)  # SWTPG_FLAG_ADC_STATS, SWTPG_FLAG_NOISE_SPECTRA
+        self.h = self.lib.swtpg_host_create(C.byref(c), links, flags)
         if not self.h:
             raise HostError(self.lib.swtpg_host_last_error().decode())
 
@@ -197,6 +206,15 @@ class FrameProcessors:
         first frame). reset=True starts a new window of the link."""
         out = np.zeros(256, dtype=HOST_ADC_STATS_DTYPE)
         n = self.lib.swtpg_host_adc_stats(self.h, link, 1 if reset else 0, out.ctypes.data, out.size)
+        if n < 0:
+            raise HostError(self.lib.swtpg_host_last_error().decode())
+        return out[:n].copy()
+
+    def noise_spectra(self, link: int, reset: bool = False) -> np.ndarray:
+        """The processor's get_noise_spectra: HOST_NOISE_SPECTRUM_DTYPE entries by the offline channel its TPs carry (empty
+        before its first frame). reset=True starts a new window of the link."""
+        out = np.zeros(256, dtype=HOST_NOISE_SPECTRUM_DTYPE)
+        n = self.lib.swtpg_host_noise_spectra(self.h, link, 1 if reset else 0, out.ctypes.data, out.size)
         if n < 0:
             raise HostError(self.lib.swtpg_host_last_error().decode())
         return out[:n].copy()

@@ -112,6 +112,13 @@ typedef struct swtpg_config
 /* Per-channel ADC statistics of every link (swtpg_read_adc_stats): one extra read of every batch on the device, after its TPG kernel
  * and on the same stream. Without the flag nothing is allocated or launched for them. */
 #define SWTPG_FLAG_ADC_STATS 2u
+/* Per-channel noise spectra of every link (swtpg_read_noise_lags, swtpg_noise_power): the circular lag sums of fixed segments of
+ * every channel, accumulated on the device by the same extra read of every batch as SWTPG_FLAG_ADC_STATS (with both flags the batch
+ * is read once). Without the flag nothing is allocated or launched for them. */
+#define SWTPG_FLAG_NOISE_SPECTRA 8u /* bit 4u stays unassigned: swtpg_create keeps refusing it */
+/* Noise-spectrum segment lengths in ticks: one WIBEth frame, four WIB2 superchunks. */
+#define SWTPG_WIBETH_NOISE_SEGMENT_TICKS 64u
+#define SWTPG_WIB2_NOISE_SEGMENT_TICKS 48u
 
 /* Per-channel carried state, by frame channel: ChanState of wibeth/tpg/ProcessingInfo.hpp:20-66 and
  * wib2/tpg/ProcessingInfo.hpp:20-68. Used for parity dumps only. */
@@ -314,6 +321,33 @@ typedef struct swtpg_adc_stats
  *   - SWTPG_ERR_STATE on a handle created without the flag; SWTPG_ERR_INVALID_ARG for a NULL handle or out, or for
  *     link0 + n_links > cfg.n_links. */
 swtpg_status swtpg_read_adc_stats(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_adc_stats* out, int reset);
+
+/* Noise lags of one channel (frame channel, as swtpg_tp.channel) over one window. 272 bytes. An extension of the reference: what
+ * the noise is (white, a coherent line, low-frequency pickup), from which a threshold or the FIR taps of a channel are chosen.
+ * A segment is N consecutive ticks of one batch: N = SWTPG_WIBETH_NOISE_SEGMENT_TICKS (one frame) or
+ * SWTPG_WIB2_NOISE_SEGMENT_TICKS (four superchunks; a WIB2 link's valid units of a batch are cut into groups of four from its
+ * first unit, and a remainder of 1-3 superchunks is not counted). A segment never spans two batches. With x the raw 14-bit ADC
+ * values of a segment,
+ *   lag[tau] = sum over segments of sum_{t<N} x[t] x[(t + tau) mod N],  tau = 0 .. N/2,
+ * the circular lags, whose cosine transform is the segment's |rfft(x)|^2 (swtpg_noise_power). WIB2 fills lag[0..24] and leaves
+ * the rest 0. The sums are exact while lag[0] < 2^63, i.e. segments < 5.3e8 (4.9 h of one channel's data at 1.953125 MHz). */
+typedef struct swtpg_noise_lags
+{
+  uint64_t segments; /* segments of this channel in the window */
+  uint64_t lag[33];  /* circular lag sums, tau = 0 .. N/2 */
+} swtpg_noise_lags;
+/* out[n_links][SWTPG_*_CHANNELS] for links link0 .. link0 + n_links - 1 (handles created with SWTPG_FLAG_NOISE_SPECTRA). Windows,
+ * their order against batches and the streaming path, resets, swtpg_start, swtpg_stop and the errors are those of
+ * swtpg_read_adc_stats; a read of one kind ends no window of the other kind. */
+swtpg_status swtpg_read_noise_lags(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_noise_lags* out, int reset);
+/* The averaged periodogram with a rectangular window of n entries of swtpg_read_noise_lags of a handle of `format`: power[n][N/2+1],
+ * bin k at k * 1.953125 MHz / N, the mean over segments of |rfft(x)_k|^2 / N:
+ *   P_k = (lag[0] + 2 sum_{tau=1}^{N/2-1} lag[tau] cos(2 pi k tau / N) + lag[N/2] cos(pi k)) / (N segments).
+ * For k >= 1 lag[0] is subtracted from every lag in exact integers first (the cosine weights sum to 0), so the pedestal does not
+ * swamp the noise. Bin 0 keeps the pedestal: by Parseval the N bins of the full periodogram sum to lag[0] / segments. An entry with
+ * no segments gives zeros. A pure host function; SWTPG_ERR_INVALID_ARG for NULL pointers, SWTPG_ERR_UNSUPPORTED for an unknown
+ * format. */
+swtpg_status swtpg_noise_power(const swtpg_noise_lags* in, size_t n, int format, double* power);
 swtpg_status swtpg_get_counters(swtpg_handle* h, swtpg_counters* out);
 /* SWTPG_FLAG_SORTED_TPS bookkeeping: device time (CUDA events, includes the 16-byte read-back of the key range) of the last
  * ordered list and of all lists since swtpg_create, how many lists were ordered on the device, and how many of them the host
