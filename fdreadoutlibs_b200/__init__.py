@@ -5,9 +5,9 @@ host C++ mirror of the reference's FrameProcessor interface (`host/`). Importing
 fails loudly if it has not been built.
 """
 from . import frames  # noqa: F401
-from .api import (ALGORITHMS, PinnedBuffer, SwtpgError, TPGAlgorithmInexistent, TPGenerator, device_available, firwin_int, gen_params,  # noqa: F401
-                  gen_wib2_device, gen_wib2_host, gen_wibeth_device, gen_wibeth_host, merge_sorted, noise_frequencies, noise_power, sort_tps)
+from .api import (ALGORITHMS, PinnedBuffer, SwtpgError, TPGAlgorithmInexistent, TPGenerator, channel_covariance, device_available,  # noqa: F401
+                  firwin_int, gen_params, gen_wib2_device, gen_wib2_host, gen_wibeth_device, gen_wibeth_host, merge_sorted, noise_frequencies, noise_power, sort_tps)
 
-__all__ = ["frames", "TPGenerator", "PinnedBuffer", "SwtpgError", "TPGAlgorithmInexistent", "ALGORITHMS", "device_available", "firwin_int",
+__all__ = ["frames", "TPGenerator", "PinnedBuffer", "SwtpgError", "TPGAlgorithmInexistent", "ALGORITHMS", "channel_covariance", "device_available", "firwin_int",
            "gen_params", "gen_wibeth_host", "gen_wib2_host", "gen_wibeth_device", "gen_wib2_device", "merge_sorted", "noise_frequencies",
            "noise_power", "sort_tps"]

@@ -112,6 +112,8 @@ EXPORTS = {
     "swtpg_read_adc_stats": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int]),
     "swtpg_read_noise_lags": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int]),
     "swtpg_noise_power": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "swtpg_read_channel_products": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int]),
+    "swtpg_channel_covariance": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p]),
     "swtpg_get_counters": (C.c_int, [C.c_void_p, C.POINTER(SwtpgCounters)]),
     "swtpg_sort_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "swtpg_alloc_pinned": (C.c_void_p, [C.c_size_t, C.c_int]),

@@ -25,6 +25,7 @@ FORMATS = {"wibeth": FORMAT_WIBETH, "wib2": FORMAT_WIB2}
 FLAG_SORTED_TPS = 1  # SWTPG_FLAG_SORTED_TPS
 FLAG_ADC_STATS = 2  # SWTPG_FLAG_ADC_STATS
 FLAG_NOISE_SPECTRA = 8  # SWTPG_FLAG_NOISE_SPECTRA
+FLAG_CHANNEL_COVARIANCE = 32  # SWTPG_FLAG_CHANNEL_COVARIANCE
 
 
 class SwtpgError(RuntimeError):
@@ -59,11 +60,13 @@ class TPGenerator:
                  acc_limit: int = 10, rs_memory_factor: int = 8, rs_scale_factor: int = 5, fir_taps: Optional[Sequence[int]] = None,
                  tap_exponent: int = 6, tp_capacity: int = 0, n_slots: int = 0, device: int = 0, wib2_adc_offset: int = 0,
                  dispatch_timeout_us: int = 0, sorted_tps: bool = False, adc_stats: bool = False,
-                 noise_spectra: bool = False):
+                 noise_spectra: bool = False, channel_covariance: bool = False):
         """sorted_tps: SWTPG_FLAG_SORTED_TPS — every batch's TP list comes back ordered by (time_start, link, channel), ordered on
         the device (include/swtpg.h). adc_stats: SWTPG_FLAG_ADC_STATS — per-channel ADC statistics of every batch, read by
         read_adc_stats(). noise_spectra: SWTPG_FLAG_NOISE_SPECTRA — per-channel noise lag sums of every batch, read by
-        read_noise_lags() and turned into power spectra by noise_power()."""
+        read_noise_lags() and turned into power spectra by noise_power(). channel_covariance: SWTPG_FLAG_CHANNEL_COVARIANCE — the
+        sums of products of every pair of channels of each link, read by read_channel_products() and turned into covariance and
+        correlation matrices by channel_covariance()."""
         if algorithm not in ALGORITHMS:
             raise TPGAlgorithmInexistent(algorithm)
         cfg = SwtpgConfig()
@@ -85,7 +88,8 @@ class TPGenerator:
         cfg.tap_exponent = tap_exponent
         cfg.wib2_adc_offset = wib2_adc_offset
         cfg.dispatch_timeout_us = dispatch_timeout_us
-        cfg.flags = (FLAG_SORTED_TPS if sorted_tps else 0) | (FLAG_ADC_STATS if adc_stats else 0) | (FLAG_NOISE_SPECTRA if noise_spectra else 0)
+        cfg.flags = ((FLAG_SORTED_TPS if sorted_tps else 0) | (FLAG_ADC_STATS if adc_stats else 0) | (FLAG_NOISE_SPECTRA if noise_spectra else 0)
+                     | (FLAG_CHANNEL_COVARIANCE if channel_covariance else 0))
         self.cfg = cfg
         self.fmt = fmt
         self.n_links = n_links
@@ -323,6 +327,16 @@ class TPGenerator:
         self._check(lib.swtpg_read_noise_lags(self._h, link0, n_links, out.ctypes.data, 1 if reset else 0))
         return out
 
+    def read_channel_products(self, link0: int = 0, n_links: Optional[int] = None, reset: bool = False) -> np.ndarray:
+        """swtpg_read_channel_products: the current window of links [link0, link0 + n_links) (default: to the last link) as an
+        (n_links, channel_products_words(fmt)) uint64 array in the header's layout (frames.unpack_channel_products splits a row).
+        reset=True starts a new window of those links."""
+        if n_links is None:
+            n_links = max(0, self.n_links - link0)
+        out = np.zeros((n_links, F.channel_products_words(self.fmt)), dtype=np.uint64)
+        self._check(lib.swtpg_read_channel_products(self._h, link0, n_links, out.ctypes.data, 1 if reset else 0))
+        return out
+
     def sort_stats(self) -> dict:
         """Device-side ordering (sorted_tps=True): ms of the last list, ms of all lists, lists ordered, lists the host finished."""
         a, b, n, f = C.c_double(0), C.c_double(0), C.c_uint64(0), C.c_uint64(0)
@@ -364,6 +378,22 @@ def noise_power(lags: np.ndarray, fmt: str = "wibeth") -> np.ndarray:
     if st != SWTPG_OK:
         raise SwtpgError(st, "swtpg_noise_power")
     return out
+
+
+def channel_covariance(products: np.ndarray, fmt: str = "wibeth"):
+    """swtpg_channel_covariance of (n_links, channel_products_words(fmt)) rows of read_channel_products: (covariance,
+    correlation), each (n_links, channels, channels) float64, by frame channel. Population covariance in ADC counts^2; the
+    correlation is NaN in the row and column of a channel without variance, the covariance 0 there."""
+    products = np.ascontiguousarray(products, dtype=np.uint64)
+    if products.ndim != 2 or products.shape[1] != F.channel_products_words(fmt):
+        raise ValueError(f"products must be (n_links, {F.channel_products_words(fmt)}) for {fmt}")
+    c = F.WIB2_CHANNELS if fmt == "wib2" else F.WIBETH_CHANNELS
+    cov = np.zeros((products.shape[0], c, c), dtype=np.float64)
+    corr = np.zeros_like(cov)
+    st = lib.swtpg_channel_covariance(products.ctypes.data, products.shape[0], FORMATS[fmt], cov.ctypes.data, corr.ctypes.data)
+    if st != SWTPG_OK:
+        raise SwtpgError(st, "swtpg_channel_covariance")
+    return cov, corr
 
 
 def noise_frequencies(fmt: str = "wibeth") -> np.ndarray:

@@ -30,6 +30,8 @@ static_assert(sizeof(swtpg_counters) == 80, "swtpg_counters layout changed");
 static_assert(sizeof(swtpg_link_config) == 36, "swtpg_link_config layout changed");
 static_assert(sizeof(swtpg_adc_stats) == 32, "swtpg_adc_stats layout changed");
 static_assert(sizeof(swtpg_noise_lags) == 272, "swtpg_noise_lags layout changed");
+static_assert(SWTPG_CHANNEL_PRODUCTS_WORDS(SWTPG_WIBETH_CHANNELS) == 2145 && SWTPG_CHANNEL_PRODUCTS_WORDS(SWTPG_WIB2_CHANNELS) == 33153,
+              "swtpg_read_channel_products layout changed");
 
 namespace {
 thread_local std::string g_create_error;
@@ -345,6 +347,8 @@ reset_channel_stats(swtpg_handle* h)
     SW_CUDA(h, cudaMemsetAsync(h->d_adc_stats, 0, n * sizeof(swtpg_adc_stats), h->stream));
   if (h->d_noise_lags)
     SW_CUDA(h, cudaMemsetAsync(h->d_noise_lags, 0, n * sizeof(swtpg_noise_lags), h->stream));
+  if (h->d_channel_products)
+    SW_CUDA(h, cudaMemsetAsync(h->d_channel_products, 0, size_t(h->cfg.n_links) * h->products_words * sizeof(uint64_t), h->stream));
   SW_CUDA(h, cudaEventRecord(h->ev_stats, h->stream));
   h->stats_stream = h->stream;
   return SWTPG_OK;
@@ -558,14 +562,14 @@ same_group(int32_t format, const TpgConf& a, const TpgConf& b)
   return true;
 }
 
-// swtpg_read_adc_stats / swtpg_read_noise_lags: copies the window of links [link0, link0 + n_links) of a device accumulator
-// d[n_links][channels] to the pinned mirror hbuf and, on reset, zeroes it, in stream order. The caller holds read_mu and has checked
-// the arguments; returns when hbuf holds the window.
+// swtpg_read_adc_stats / swtpg_read_noise_lags / swtpg_read_channel_products: copies the window of links [link0, link0 + n_links)
+// of a device accumulator d[n_links][per_link] to the pinned mirror hbuf and, on reset, zeroes it, in stream order. The caller
+// holds read_mu and has checked the arguments; returns when hbuf holds the window.
 template<typename T>
 swtpg_status
-read_window(swtpg_handle* h, T* d, T* hbuf, uint32_t link0, uint32_t n_links, int reset)
+read_window(swtpg_handle* h, T* d, T* hbuf, uint32_t link0, uint32_t n_links, size_t per_link, int reset)
 {
-  const size_t first = size_t(link0) * h->channels, n = size_t(n_links) * h->channels;
+  const size_t first = size_t(link0) * per_link, n = size_t(n_links) * per_link;
   {
     // Copy and reset are enqueued back to back on the stream of the last batch: a batch enqueued meanwhile falls after both.
     std::lock_guard<std::mutex> lk(h->stats_mu);
@@ -687,7 +691,7 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
     return fail(nullptr, cs, why);
   if (cfg->wib2_adc_offset % 4 != 0 || cfg->wib2_adc_offset > SWTPG_WIB2_FRAME_BYTES - 448)
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "wib2_adc_offset must be a multiple of 4 and leave room for the 448-byte ADC block");
-  if (cfg->flags & ~(SWTPG_FLAG_SORTED_TPS | SWTPG_FLAG_ADC_STATS | SWTPG_FLAG_NOISE_SPECTRA))
+  if (cfg->flags & ~(SWTPG_FLAG_SORTED_TPS | SWTPG_FLAG_ADC_STATS | SWTPG_FLAG_NOISE_SPECTRA | SWTPG_FLAG_CHANNEL_COVARIANCE))
     return fail(nullptr, SWTPG_ERR_INVALID_ARG, "unknown bits in swtpg_config.flags");
 
   int ndev = 0;
@@ -764,6 +768,13 @@ swtpg_create(const swtpg_config* cfg, swtpg_handle** out)
     SW_CUDA(hp, cudaMemset(h->d_noise_lags, 0, bytes));
     SW_CUDA(hp, cudaMallocHost(&h->h_noise_lags, bytes));
   }
+  h->products_words = SWTPG_CHANNEL_PRODUCTS_WORDS(h->channels);
+  if (cfg->flags & SWTPG_FLAG_CHANNEL_COVARIANCE) {
+    const size_t bytes = size_t(cfg->n_links) * h->products_words * sizeof(uint64_t);
+    SW_CUDA(hp, cudaMalloc(&h->d_channel_products, bytes));
+    SW_CUDA(hp, cudaMemset(h->d_channel_products, 0, bytes));
+    SW_CUDA(hp, cudaMallocHost(&h->h_channel_products, bytes));
+  }
   if (h->channel_stats()) {
     SW_CUDA(hp, cudaEventCreateWithFlags(&h->ev_stats, cudaEventDisableTiming));
     SW_CUDA(hp, cudaEventCreateWithFlags(&h->ev_stats_read, cudaEventDisableTiming));
@@ -811,6 +822,8 @@ swtpg_destroy(swtpg_handle* h)
   if (h->h_adc_stats) cudaFreeHost(h->h_adc_stats);
   if (h->d_noise_lags) cudaFree(h->d_noise_lags);
   if (h->h_noise_lags) cudaFreeHost(h->h_noise_lags);
+  if (h->d_channel_products) cudaFree(h->d_channel_products);
+  if (h->h_channel_products) cudaFreeHost(h->h_channel_products);
   if (h->ev_stats) cudaEventDestroy(h->ev_stats);
   if (h->ev_stats_read) cudaEventDestroy(h->ev_stats_read);
   delete[] h->h_rs_factor;
@@ -1203,7 +1216,7 @@ swtpg_read_adc_stats(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_ad
     return st;
   SW_CUDA(h, cudaSetDevice(h->cfg.device));
   std::lock_guard<std::mutex> rd(h->read_mu);
-  if ((st = read_window(h, h->d_adc_stats, h->h_adc_stats, link0, n_links, reset)) != SWTPG_OK)
+  if ((st = read_window(h, h->d_adc_stats, h->h_adc_stats, link0, n_links, h->channels, reset)) != SWTPG_OK)
     return st;
   const size_t first = size_t(link0) * h->channels, n = size_t(n_links) * h->channels;
   for (size_t i = 0; i < n; ++i) {
@@ -1229,9 +1242,24 @@ swtpg_read_noise_lags(swtpg_handle* h, uint32_t link0, uint32_t n_links, swtpg_n
     return st;
   SW_CUDA(h, cudaSetDevice(h->cfg.device));
   std::lock_guard<std::mutex> rd(h->read_mu);
-  if ((st = read_window(h, h->d_noise_lags, h->h_noise_lags, link0, n_links, reset)) != SWTPG_OK)
+  if ((st = read_window(h, h->d_noise_lags, h->h_noise_lags, link0, n_links, h->channels, reset)) != SWTPG_OK)
     return st;
   memcpy(out, h->h_noise_lags + size_t(link0) * h->channels, size_t(n_links) * h->channels * sizeof(swtpg_noise_lags));
+  return SWTPG_OK;
+}
+
+swtpg_status
+swtpg_read_channel_products(swtpg_handle* h, uint32_t link0, uint32_t n_links, uint64_t* out, int reset)
+{
+  swtpg_status st = check_read_args(h, link0, n_links, out, h ? h->d_channel_products : nullptr,
+                                    "the handle was created without SWTPG_FLAG_CHANNEL_COVARIANCE");
+  if (st != SWTPG_OK || n_links == 0)
+    return st;
+  SW_CUDA(h, cudaSetDevice(h->cfg.device));
+  std::lock_guard<std::mutex> rd(h->read_mu);
+  if ((st = read_window(h, h->d_channel_products, h->h_channel_products, link0, n_links, h->products_words, reset)) != SWTPG_OK)
+    return st;
+  memcpy(out, h->h_channel_products + size_t(link0) * h->products_words, size_t(n_links) * h->products_words * sizeof(uint64_t));
   return SWTPG_OK;
 }
 

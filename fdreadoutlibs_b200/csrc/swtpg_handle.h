@@ -2,7 +2,8 @@
 //   swtpg_capi.cu    create / destroy / start / stop, the batch entry points and the kernel launch table
 //   swtpg_stream.cu  the streaming path (swtpg_submit ... swtpg_poll): per-link rings, dispatcher and completion threads,
 //                    the gather kernel that pulls frames out of pinned host memory
-//   swtpg_stats.cu   the per-channel statistics kernel (SWTPG_FLAG_ADC_STATS, SWTPG_FLAG_NOISE_SPECTRA)
+//   swtpg_stats.cu   the per-channel statistics kernel (SWTPG_FLAG_ADC_STATS, SWTPG_FLAG_NOISE_SPECTRA) and the channel
+//                    products kernel (SWTPG_FLAG_CHANNEL_COVARIANCE)
 // Not installed; nothing outside csrc/ includes it.
 #pragma once
 
@@ -127,13 +128,18 @@ struct swtpg_handle
   // SWTPG_FLAG_NOISE_SPECTRA (null without it): d_noise_lags[n_links][channels], the current window in the layout of swtpg_noise_lags.
   swtpg_noise_lags* d_noise_lags = nullptr;
   swtpg_noise_lags* h_noise_lags = nullptr; // pinned, same size
-  // Either flag (all null without both). Every statistics kernel and every read runs in one order: each waits for ev_stats, which
-  // is recorded after the last of them on stats_stream, when it runs on another stream. stats_mu guards those two and keeps a
-  // read's copy and reset together; read_mu serialises reads (h_adc_stats, h_noise_lags, ev_stats_read).
+  // SWTPG_FLAG_CHANNEL_COVARIANCE (null without it): d_channel_products[n_links][SWTPG_CHANNEL_PRODUCTS_WORDS(channels)], the
+  // current window in the layout of swtpg_read_channel_products.
+  uint64_t* d_channel_products = nullptr;
+  uint64_t* h_channel_products = nullptr; // pinned, same size
+  uint32_t products_words = 0;            // SWTPG_CHANNEL_PRODUCTS_WORDS(channels)
+  // Any of the three flags (all null without them). Every statistics kernel and every read runs in one order: each waits for
+  // ev_stats, which is recorded after the last of them on stats_stream, when it runs on another stream. stats_mu guards those two
+  // and keeps a read's copy and reset together; read_mu serialises reads (the pinned mirrors, ev_stats_read).
   cudaEvent_t ev_stats = nullptr, ev_stats_read = nullptr;
   cudaStream_t stats_stream = nullptr;
   std::mutex stats_mu, read_mu;
-  bool channel_stats() const { return d_adc_stats || d_noise_lags; } // every batch gets a launch_channel_stats
+  bool channel_stats() const { return d_adc_stats || d_noise_lags || d_channel_products; } // every batch gets a launch_channel_stats
 
   // streaming path (swtpg_stream.cu), created on the first swtpg_submit / swtpg_register_buffer
   std::mutex engine_mu;
@@ -201,8 +207,9 @@ cudaError_t launch_batch_kernel(swtpg_handle* h, const void* d_frames, const uin
                                 unsigned* d_count, cudaStream_t s);
 
 // swtpg_stats.cu: adds one batch, laid out as for launch_batch_kernel, to the per-channel ADC statistics (SWTPG_FLAG_ADC_STATS)
-// and noise lags (SWTPG_FLAG_NOISE_SPECTRA) the handle keeps, in one read of the batch on stream `s`, after the statistics work of
-// earlier batches and reads whatever stream that ran on.
+// and noise lags (SWTPG_FLAG_NOISE_SPECTRA) the handle keeps, in one read of the batch on stream `s`, then to its channel products
+// (SWTPG_FLAG_CHANNEL_COVARIANCE) in a second kernel, after the statistics work of earlier batches and reads whatever stream that
+// ran on.
 cudaError_t launch_channel_stats(swtpg_handle* h, const void* d_frames, const uint32_t* d_nunits, uint32_t units_stride, cudaStream_t s);
 
 // swtpg_sort.cu: device-side ordering of a batch's TP list (SWTPG_FLAG_SORTED_TPS)

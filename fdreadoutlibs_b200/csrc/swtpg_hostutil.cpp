@@ -1,5 +1,6 @@
 // Host-only pieces of libswtpg_b200.so (plain g++; no CUDA): the staging copy of swtpg_submit, the FIR tap design, the
-// host-side ordering / merge of TP lists and the noise power spectra of swtpg_noise_power.
+// host-side ordering / merge of TP lists, the noise power spectra of swtpg_noise_power and the covariance matrices of
+// swtpg_channel_covariance.
 #include "../../include/swtpg.h"
 
 #include <algorithm>
@@ -7,6 +8,7 @@
 #include <cstddef>
 #include <cstdint>
 #include <cstring>
+#include <limits>
 #include <vector>
 
 // ---- staging copy ------------------------------------------------------------------------------------------------------
@@ -279,6 +281,42 @@ swtpg_noise_power(const swtpg_noise_lags* in, size_t n, int format, double* powe
         s += c[size_t(k) * bins + tau] * d[tau];
       p[k] = s * scale;
     }
+  }
+  return SWTPG_OK;
+}
+
+// ---- channel covariance ------------------------------------------------------------------------------------------------------
+// swtpg_channel_covariance (include/swtpg.h): covariance and correlation matrices of the channel products of
+// swtpg_read_channel_products.
+extern "C" swtpg_status
+swtpg_channel_covariance(const uint64_t* in, size_t n_links, int format, double* covariance, double* correlation)
+{
+  if (!in)
+    return SWTPG_ERR_INVALID_ARG;
+  if (format != SWTPG_FORMAT_WIBETH && format != SWTPG_FORMAT_WIB2)
+    return SWTPG_ERR_UNSUPPORTED;
+  const size_t C = format == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_CHANNELS : SWTPG_WIBETH_CHANNELS;
+  const size_t words = SWTPG_CHANNEL_PRODUCTS_WORDS(C);
+  const double nan = std::numeric_limits<double>::quiet_NaN();
+  std::vector<__int128> num(C * C);
+  for (size_t l = 0; l < n_links; ++l) {
+    const uint64_t* w = in + l * words;
+    const __int128 n = w[0];
+    const uint64_t* sum = w + 1;
+    // num_ij = n P_ij - S_i S_j exactly: n < 2^36, P_ij < 2^64 and S_i < 2^50 keep both terms below 2^100
+    for (size_t i = 0, k = 1 + C; i < C; ++i)
+      for (size_t j = i; j < C; ++j, ++k)
+        num[i * C + j] = num[j * C + i] = n * __int128(w[k]) - __int128(sum[i]) * __int128(sum[j]);
+    const double n2 = double(w[0]) * double(w[0]);
+    for (size_t i = 0; i < C; ++i)
+      for (size_t j = 0; j < C; ++j) {
+        const size_t o = (l * C + i) * C + j;
+        const __int128 vi = num[i * C + i], vj = num[j * C + j];
+        if (covariance)
+          covariance[o] = w[0] ? double(num[i * C + j]) / n2 : 0.0; // a variance of 0 makes num_ij 0 (Cauchy-Schwarz)
+        if (correlation)
+          correlation[o] = vi > 0 && vj > 0 ? std::clamp(double(num[i * C + j]) / std::sqrt(double(vi) * double(vj)), -1.0, 1.0) : nan;
+      }
   }
   return SWTPG_OK;
 }

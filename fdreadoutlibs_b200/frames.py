@@ -66,6 +66,24 @@ assert NOISE_LAGS_DTYPE.itemsize == 272
 NOISE_SEGMENT_TICKS = {"wibeth": 64, "wib2": 48}
 SAMPLE_RATE_HZ = 62.5e6 / 32  # one ADC sample per channel every 32 ticks of the 62.5 MHz timing clock
 
+
+def channel_products_words(fmt: str) -> int:
+    """SWTPG_CHANNEL_PRODUCTS_WORDS: uint64 words per link of swtpg_read_channel_products (2145 WIBEth, 33153 WIB2)."""
+    c = WIB2_CHANNELS if fmt == "wib2" else WIBETH_CHANNELS
+    return 1 + c + c * (c + 1) // 2
+
+
+def unpack_channel_products(words: np.ndarray, fmt: str):
+    """One link's row of swtpg_read_channel_products -> (samples, sums (C,) uint64, products (C, C) uint64, full and symmetric)."""
+    c = WIB2_CHANNELS if fmt == "wib2" else WIBETH_CHANNELS
+    words = np.asarray(words, dtype=np.uint64)
+    assert words.shape == (channel_products_words(fmt),), words.shape
+    i, j = np.triu_indices(c)  # row-major upper triangle, i = 0 first: the header's order
+    p = np.zeros((c, c), dtype=np.uint64)
+    p[i, j] = words[1 + c:]
+    p[j, i] = words[1 + c:]
+    return int(words[0]), words[1:1 + c].copy(), p
+
 # Lane l of AVX2 register r holds frame channel 16r + LANE_PERM[l] (unittest/WIBEthFrameExpansion_test.cxx:111,124).
 LANE_PERM = np.array([0, 1, 2, 3, 4, 5, 6, 7, 15, 8, 9, 10, 11, 12, 13, 14], dtype=np.int64)
 

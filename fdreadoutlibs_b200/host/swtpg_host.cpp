@@ -170,6 +170,15 @@ TpgEngine::read_noise_lags(uint32_t link, swtpg_noise_lags* out, uint32_t n_chan
 }
 
 void
+TpgEngine::read_channel_products(uint32_t link, uint64_t* out, size_t words, bool reset)
+{
+  const uint32_t channels = m_cfg.format == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_CHANNELS : SWTPG_WIBETH_CHANNELS;
+  if (words != SWTPG_CHANNEL_PRODUCTS_WORDS(channels))
+    throw std::invalid_argument("TpgEngine::read_channel_products: SWTPG_CHANNEL_PRODUCTS_WORDS words of the link");
+  check(m_h, swtpg_read_channel_products(m_h, link, 1, out, reset ? 1 : 0), "swtpg_read_channel_products");
+}
+
+void
 TpgEngine::set_link_thresholds(uint32_t link, const uint16_t* by_channel, uint32_t n_channels)
 {
   const uint32_t channels = m_cfg.format == SWTPG_FORMAT_WIB2 ? SWTPG_WIB2_CHANNELS : SWTPG_WIBETH_CHANNELS;
@@ -446,6 +455,23 @@ TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::get_noise_spectra(std::vector
     out[c].segments = lags[c].segments;
     std::copy(power.begin() + c * bins, power.begin() + (c + 1) * bins, out[c].power);
   }
+}
+
+template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
+void
+TpcFrameProcessor<R, H, kChannels, kCountEveryTp>::get_channel_covariance(ChannelCovariance& out, bool reset)
+{
+  out = ChannelCovariance{};
+  if (!m_maps_ready.load(std::memory_order_acquire))
+    return;
+  std::vector<uint64_t> products(SWTPG_CHANNEL_PRODUCTS_WORDS(kChannels));
+  m_engine->read_channel_products(m_frame_handler->link, products.data(), products.size(), reset);
+  out.samples = products[0];
+  out.offline_channel.assign(m_offline_of_channel.begin(), m_offline_of_channel.end());
+  out.covariance.resize(size_t(kChannels) * kChannels);
+  out.correlation.resize(size_t(kChannels) * kChannels);
+  check(nullptr, swtpg_channel_covariance(products.data(), 1, m_engine->format(), out.covariance.data(), out.correlation.data()),
+        "swtpg_channel_covariance");
 }
 
 template<class R, class H, uint32_t kChannels, bool kCountEveryTp>
@@ -886,7 +912,7 @@ swtpg_host_last_error(void)
 
 // links: NULL, or links[n_links], each frame processor's conf() with its own TPG fields (one engine, links with different
 // configurations). flags: SWTPG_FLAG_* for the engine's handle (SWTPG_FLAG_ADC_STATS: the processors' get_adc_stats;
-// SWTPG_FLAG_NOISE_SPECTRA: their get_noise_spectra).
+// SWTPG_FLAG_NOISE_SPECTRA: their get_noise_spectra; SWTPG_FLAG_CHANNEL_COVARIANCE: their get_channel_covariance).
 swtpg_host*
 swtpg_host_create(const swtpg_host_conf* c, const swtpg_host_link_conf* links, uint32_t flags)
 {
@@ -1214,6 +1240,33 @@ swtpg_host_noise_spectra(swtpg_host* h, uint32_t link, int reset, ChannelNoiseSp
     with_processors(h, [&](auto& procs) { procs.at(link)->get_noise_spectra(v, reset != 0); });
     const size_t n = std::min<size_t>(v.size(), cap);
     std::copy(v.begin(), v.begin() + n, out);
+    return int(n);
+  } catch (const std::exception& e) {
+    g_host_error = e.what();
+    return -1;
+  }
+}
+
+// ChannelCovariance of a link's processor into samples, offline[cap] and covariance / correlation [cap][cap] (either may be NULL):
+// the channel count (64 WIBEth / 256 WIB2, 0 before the first frame), -1 on error or when cap is too small
+int
+swtpg_host_channel_covariance(swtpg_host* h, uint32_t link, int reset, uint64_t* samples, uint32_t* offline, double* covariance,
+                              double* correlation, uint32_t cap)
+{
+  try {
+    ChannelCovariance v;
+    with_processors(h, [&](auto& procs) { procs.at(link)->get_channel_covariance(v, reset != 0); });
+    const size_t n = v.offline_channel.size();
+    if (n > cap)
+      throw std::invalid_argument("swtpg_host_channel_covariance: cap is below the link's channel count");
+    if (samples)
+      *samples = v.samples;
+    if (offline)
+      std::copy(v.offline_channel.begin(), v.offline_channel.end(), offline);
+    if (covariance)
+      std::copy(v.covariance.begin(), v.covariance.end(), covariance);
+    if (correlation)
+      std::copy(v.correlation.begin(), v.correlation.end(), correlation);
     return int(n);
   } catch (const std::exception& e) {
     g_host_error = e.what();

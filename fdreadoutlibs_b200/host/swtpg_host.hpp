@@ -240,6 +240,16 @@ struct ChannelNoiseSpectrum
   double power[SWTPG_WIBETH_NOISE_SEGMENT_TICKS / 2 + 1] = {};
 };
 
+// Not a reference type: the channel covariance of a link over one window of swtpg_read_channel_products (swtpg_channel_covariance
+// of its products). Row and column c are frame channel c, reported under the offline channel offline_channel[c] that its TPs
+// carry. covariance and correlation are C x C row-major, full and symmetric: ADC counts^2, and NaN where a channel has no variance.
+struct ChannelCovariance
+{
+  uint64_t samples = 0;
+  std::vector<uint32_t> offline_channel;
+  std::vector<double> covariance, correlation;
+};
+
 // ---- the GPU pipeline shared by the links of one device -------------------------------------------------------------------
 class FrameProcessorBase;
 // One swtpg_handle per GPU; every frame processor attached to it owns one link index. Any link's post-processing thread
@@ -267,6 +277,9 @@ public:
   void read_adc_stats(uint32_t link, swtpg_adc_stats* out, uint32_t n_channels, bool reset);
   // swtpg_read_noise_lags of one link: out[n_channels] by frame channel (an engine created with SWTPG_FLAG_NOISE_SPECTRA). After conf().
   void read_noise_lags(uint32_t link, swtpg_noise_lags* out, uint32_t n_channels, bool reset);
+  // swtpg_read_channel_products of one link: out[words], words = SWTPG_CHANNEL_PRODUCTS_WORDS of its channels (an engine created
+  // with SWTPG_FLAG_CHANNEL_COVARIANCE). After conf().
+  void read_channel_products(uint32_t link, uint64_t* out, size_t words, bool reset);
   swtpg_format format() const { return swtpg_format(m_cfg.format); }
   // false = back-pressure (the link's ring is full). wait_us > 0: sleep up to that long for room first (swtpg_submit_wait)
   bool submit(uint32_t link, const void* unit, size_t bytes, uint64_t wait_us = 0);
@@ -328,6 +341,10 @@ public:
   // SWTPG_FLAG_NOISE_SPECTRA), by the offline channel its TPs carry, masked channels included. Empty until the first frame has
   // built the channel map.
   void get_noise_spectra(std::vector<ChannelNoiseSpectrum>& out, bool reset);
+  // Not in the reference: the covariance and correlation of this link's channels since the last reset (engine flag
+  // SWTPG_FLAG_CHANNEL_COVARIANCE), rows in frame-channel order under the offline channel its TPs carry, masked channels
+  // included. Empty (no rows) until the first frame has built the channel map.
+  void get_channel_covariance(ChannelCovariance& out, bool reset);
   void process_swtpg_hits(const swtpg_tp* tps, size_t n) override; // fed with device TP records
   FrameHandler* handler() { return m_frame_handler.get(); }
 
@@ -338,7 +355,7 @@ protected:
   // table and the post-process task find_hits.
   void conf_link(const RawDataProcessorConf& config, const swtpg_config& a, std::function<void(constframeptr)> find_hits);
   // First frame: the offline channel offline_of(c) that records of frame channel c are reported with, its mask flag, a zeroed
-  // rate counter; then get_info, get_adc_stats and get_noise_spectra may read them.
+  // rate counter; then get_info, get_adc_stats, get_noise_spectra and get_channel_covariance may read them.
   template<class OfflineOf>
   void set_channel_tables(OfflineOf offline_of)
   {

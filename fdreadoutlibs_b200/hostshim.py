@@ -68,7 +68,7 @@ EXPORTS = ["swtpg_host_tpsets_create", "swtpg_host_tpsets_destroy", "swtpg_host_
            "swtpg_host_push_parallel", "swtpg_host_push_feeders", "swtpg_host_tp_count", "swtpg_host_counters", "swtpg_host_stream_timing", "swtpg_host_last_error", "swtpg_host_create", "swtpg_host_destroy", "swtpg_host_start", "swtpg_host_stop", "swtpg_host_push",
            "swtpg_host_take_tps", "swtpg_host_get_info", "swtpg_host_error_count", "swtpg_host_misconfigurations",
            "swtpg_host_last_daq_time", "swtpg_host_register_channel_map", "swtpg_host_register_buffer", "swtpg_host_adc_stats",
-           "swtpg_host_noise_spectra"]
+           "swtpg_host_noise_spectra", "swtpg_host_channel_covariance"]
 
 _lib = None
 
@@ -104,6 +104,8 @@ def host_lib():
         lib.swtpg_host_register_buffer.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int]
         lib.swtpg_host_adc_stats.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p, C.c_uint32]
         lib.swtpg_host_noise_spectra.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p, C.c_uint32]
+        lib.swtpg_host_channel_covariance.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                      C.c_uint32]
         lib.swtpg_host_tpsets_create.restype = C.c_void_p
         lib.swtpg_host_tpsets_create.argtypes = [C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32, C.c_uint32]
         lib.swtpg_host_tpsets_destroy.argtypes = [C.c_void_p]
@@ -133,12 +135,14 @@ class FrameProcessors:
                  correct_channel_lookup: bool = False, reversed_map: bool = False, collection_simple_threshold: bool = False,
                  sink_capacity: int = 0, block_on_backpressure: bool = True, device: int = 0, count_only_sink: bool = False,
                  n_slots: int = 4, link_confs=None, adc_stats: bool = False,
-                 noise_spectra: bool = False):
+                 noise_spectra: bool = False, channel_covariance: bool = False):
         """link_confs: optional list of n_links dicts, each overriding algorithm, threshold, rs_memory_factor, rs_scale_factor
         and acc_limit for its link's conf(); the keys it leaves out take the arguments above. A dict may also set
         plane_threshold: three thresholds by plane (0 = collection), -1 = the link's threshold (tpg_plane_threshold).
         adc_stats: the engine's handle accumulates per-channel ADC statistics (SWTPG_FLAG_ADC_STATS), read by adc_stats().
-        noise_spectra: it accumulates per-channel noise lags (SWTPG_FLAG_NOISE_SPECTRA), read as spectra by noise_spectra()."""
+        noise_spectra: it accumulates per-channel noise lags (SWTPG_FLAG_NOISE_SPECTRA), read as spectra by noise_spectra().
+        channel_covariance: it accumulates the channel products of every link (SWTPG_FLAG_CHANNEL_COVARIANCE), read as covariance
+        and correlation matrices by channel_covariance()."""
         c = HostConf()
         c.device, c.format, c.n_links, c.superchunk_units = device, 1 if fmt == "wib2" else 0, n_links, superchunk_units
         c.tpg_algorithm = algorithm.encode()
@@ -168,7 +172,8 @@ class FrameProcessors:
                 links[l].tpg_frugal_streaming_accumulator_limit = lc.get("acc_limit", acc_limit)
                 for p, t in enumerate(lc.get("plane_threshold", (-1, -1, -1))):
                     links[l].tpg_plane_threshold[p] = t
-        flags = (2 if adc_stats else 0) | (8 if noise_spectra else 0)  # SWTPG_FLAG_ADC_STATS, SWTPG_FLAG_NOISE_SPECTRA
+        # SWTPG_FLAG_ADC_STATS, SWTPG_FLAG_NOISE_SPECTRA, SWTPG_FLAG_CHANNEL_COVARIANCE
+        flags = (2 if adc_stats else 0) | (8 if noise_spectra else 0) | (32 if channel_covariance else 0)
         self.h = self.lib.swtpg_host_create(C.byref(c), links, flags)
         if not self.h:
             raise HostError(self.lib.swtpg_host_last_error().decode())
@@ -218,6 +223,21 @@ class FrameProcessors:
         if n < 0:
             raise HostError(self.lib.swtpg_host_last_error().decode())
         return out[:n].copy()
+
+    def channel_covariance(self, link: int, reset: bool = False) -> dict:
+        """The processor's get_channel_covariance: samples, offline_channel (C,) uint32 of each row in frame-channel order, and the
+        (C, C) covariance and correlation matrices (C = 0 before its first frame). reset=True starts a new window of the link."""
+        samples = C.c_uint64(0)
+        offline = np.zeros(256, dtype=np.uint32)
+        cov = np.zeros((256, 256), dtype=np.float64)
+        corr = np.zeros((256, 256), dtype=np.float64)
+        n = self.lib.swtpg_host_channel_covariance(self.h, link, 1 if reset else 0, C.byref(samples), offline.ctypes.data, cov.ctypes.data,
+                                                   corr.ctypes.data, offline.size)
+        if n < 0:
+            raise HostError(self.lib.swtpg_host_last_error().decode())
+        shape = (n, n)
+        return {"samples": samples.value, "offline_channel": offline[:n].copy(), "covariance": cov.reshape(-1)[:n * n].reshape(shape).copy(),
+                "correlation": corr.reshape(-1)[:n * n].reshape(shape).copy()}
 
     def counters(self) -> dict:
         """swtpg_get_counters of the engine behind the processors."""

@@ -119,6 +119,12 @@ typedef struct swtpg_config
 /* Noise-spectrum segment lengths in ticks: one WIBEth frame, four WIB2 superchunks. */
 #define SWTPG_WIBETH_NOISE_SEGMENT_TICKS 64u
 #define SWTPG_WIB2_NOISE_SEGMENT_TICKS 48u
+/* Channel-to-channel covariance of every link (swtpg_read_channel_products, swtpg_channel_covariance): the sums of products of
+ * every pair of channels of a link, accumulated on the device by a kernel of its own after the statistics read of every batch
+ * and on the same stream. Without the flag nothing is allocated or launched for them. */
+#define SWTPG_FLAG_CHANNEL_COVARIANCE 32u /* bits 4u and 16u stay unassigned: swtpg_create keeps refusing them */
+/* uint64_t words per link of swtpg_read_channel_products for a link of `channels` frame channels: 2145 (WIBEth), 33153 (WIB2). */
+#define SWTPG_CHANNEL_PRODUCTS_WORDS(channels) (1u + (channels) + (channels) * ((channels) + 1u) / 2u)
 
 /* Per-channel carried state, by frame channel: ChanState of wibeth/tpg/ProcessingInfo.hpp:20-66 and
  * wib2/tpg/ProcessingInfo.hpp:20-68. Used for parity dumps only. */
@@ -348,6 +354,30 @@ swtpg_status swtpg_read_noise_lags(swtpg_handle* h, uint32_t link0, uint32_t n_l
  * no segments gives zeros. A pure host function; SWTPG_ERR_INVALID_ARG for NULL pointers, SWTPG_ERR_UNSUPPORTED for an unknown
  * format. */
 swtpg_status swtpg_noise_power(const swtpg_noise_lags* in, size_t n, int format, double* power);
+
+/* Channel products of one link over one window: SWTPG_CHANNEL_PRODUCTS_WORDS(C) uint64_t words, C = SWTPG_*_CHANNELS, by frame
+ * channel (as swtpg_tp.channel). An extension of the reference: whether a channel's noise is shared with other channels (pickup
+ * common to the channels of one front-end ASIC or FEMB), which no per-channel statistic shows and which a threshold at k x RMS
+ * fires on whole groups of channels for. With x_c[t] the raw 14-bit ADC values of channel c over the window's ticks t,
+ *   [0]                   samples, the ticks counted (every channel of a link sees every tick)
+ *   [1 + c]               sum[c] = sum_t x_c[t],                      c = 0 .. C-1
+ *   [1 + C + k(i, j)]     products[i][j] = sum_t x_i[t] x_j[t],       i <= j, upper triangle row-major:
+ *                         k(i, j) = i C - i (i - 1) / 2 + (j - i)
+ * The sums are exact while samples < 2^36 (9.7 h of one link's data). They are of raw values, so hits and cosmic tracks, which
+ * correlate neighbouring channels too, are in them: read the matrix over quiet windows. */
+/* out[n_links][SWTPG_CHANNEL_PRODUCTS_WORDS(C)] for links link0 .. link0 + n_links - 1 (handles created with
+ * SWTPG_FLAG_CHANNEL_COVARIANCE). Windows, their order against batches and the streaming path, resets, swtpg_start, swtpg_stop and
+ * the errors are those of swtpg_read_adc_stats; a read of one kind ends no window of another kind. */
+swtpg_status swtpg_read_channel_products(swtpg_handle* h, uint32_t link0, uint32_t n_links, uint64_t* out, int reset);
+/* Covariance and Pearson correlation of n_links entries of swtpg_read_channel_products of a handle of `format`: covariance and
+ * correlation [n_links][C][C], full and symmetric, either may be NULL. With n = samples, S = sum, P = products,
+ *   num_ij = n P_ij - S_i S_j   (formed exactly in 128-bit integers: the pedestal's n x 900^2 per product would otherwise
+ *                                swamp the noise's covariance in rounding)
+ *   covariance_ij  = num_ij / n^2                 (population covariance, numpy.cov(bias=True))
+ *   correlation_ij = num_ij / sqrt(num_ii num_jj) (clipped to [-1, 1] against rounding, as numpy.corrcoef)
+ * Where a variance is 0 (a dead or constant channel, a link without samples) the covariance is 0 and the correlation NaN. A pure
+ * host function; SWTPG_ERR_INVALID_ARG for a NULL in, SWTPG_ERR_UNSUPPORTED for an unknown format. */
+swtpg_status swtpg_channel_covariance(const uint64_t* in, size_t n_links, int format, double* covariance, double* correlation);
 swtpg_status swtpg_get_counters(swtpg_handle* h, swtpg_counters* out);
 /* SWTPG_FLAG_SORTED_TPS bookkeeping: device time (CUDA events, includes the 16-byte read-back of the key range) of the last
  * ordered list and of all lists since swtpg_create, how many lists were ordered on the device, and how many of them the host
