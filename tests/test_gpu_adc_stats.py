@@ -16,7 +16,8 @@ from fdreadoutlibs_b200 import _lib
 from fdreadoutlibs_b200 import api as A
 from fdreadoutlibs_b200 import frames as F
 from fdreadoutlibs_b200 import hostshim as H
-from util import adc_of, all_wibeth_policies, channels, combine, create_status, expected, linear_map, ragged_units, run_device, sms, stats_of
+from util import (adc_of, all_wibeth_policies, channels, combine, create_status, expected, linear_map, ragged_batch, ragged_units, run_device,
+                  sms, stats_of)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -64,15 +65,6 @@ def assert_stats(got, want, what):
             raise AssertionError(f"{what}: {len(bad)} (link, channel) differ in {f}; first: link {l} channel {c}: "
                                  f"got {got[l, c]} want {want[l, c]}")
     assert not got["reserved"].any()
-
-
-def ragged_batch(fmt, seed, n_links, stride, nu, **gen_kw):
-    """Generated frames with every byte past each link's n_units set to 0xFF (an overread would count 16383s)."""
-    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
-    frames = gen(S.gen_params(seed, 0.3), n_links, stride, unit0=seed * stride, **gen_kw).copy()
-    for l in range(n_links):
-        frames[l, int(nu[l]):] = 0xFF
-    return frames
 
 
 # ---- batch entry points -----------------------------------------------------------------------------------------------------------

@@ -16,30 +16,13 @@ from fdreadoutlibs_b200 import _lib
 from fdreadoutlibs_b200 import api as A
 from fdreadoutlibs_b200 import frames as F
 from fdreadoutlibs_b200 import hostshim as H
-from util import adc_of, all_wibeth_policies, channels, create_status, expected, linear_map, ragged_units, run_device, sms
+from util import (adc_of, all_wibeth_policies, channels, create_status, expected, expected_products, linear_map, ragged_batch, ragged_units,
+                  run_device, sms, words_of)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 # ---- expected values --------------------------------------------------------------------------------------------------------------
-def words_of(fmt, a):
-    """One link's swtpg_read_channel_products row of (samples, channels) ADC values."""
-    c = channels(fmt)
-    x = np.asarray(a, dtype=np.int64).reshape(-1, c)
-    out = np.zeros(F.channel_products_words(fmt), dtype=np.uint64)
-    out[0] = x.shape[0]
-    out[1:1 + c] = x.sum(axis=0)
-    i, j = np.triu_indices(c)
-    out[1 + c:] = (x.T @ x)[i, j]  # below 2^63 for every window of these tests: ticks x 16383^2
-    return out
-
-
-def expected_products(fmt, frames, nu=None, adc_offset=F.WIB2_ADC_OFFSET):
-    """(n_links, words) of one batch: frames [n_links, stride, unit_bytes], nu valid units per link (None = all)."""
-    n, stride = frames.shape[:2]
-    return np.stack([words_of(fmt, adc_of(fmt, frames[l, : (stride if nu is None else int(nu[l]))], adc_offset)) for l in range(n)])
-
-
 def zeros(n_links, fmt):
     return np.zeros((n_links, F.channel_products_words(fmt)), dtype=np.uint64)
 
@@ -59,15 +42,6 @@ def assert_products(got, want, fmt, what):
             where = f"products[{i[k - 1 - c]}][{j[k - 1 - c]}]"
         raise AssertionError(f"{what}: {len(bad)} words differ on {len(np.unique(bad[:, 0]))} links; first: link {l} {where}: "
                              f"got {got[l, k]} want {want[l, k]}")
-
-
-def ragged_batch(fmt, seed, n_links, stride, nu, **gen_kw):
-    """Generated frames with every byte past each link's n_units set to 0xFF (an overread would count 16383s)."""
-    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
-    frames = gen(S.gen_params(seed, 0.3), n_links, stride, unit0=seed * stride, **gen_kw).copy()
-    for l in range(n_links):
-        frames[l, int(nu[l]):] = 0xFF
-    return frames
 
 
 def pack(fmt, adc, ts0=1 << 40):

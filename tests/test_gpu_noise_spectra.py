@@ -16,30 +16,13 @@ from fdreadoutlibs_b200 import _lib
 from fdreadoutlibs_b200 import api as A
 from fdreadoutlibs_b200 import frames as F
 from fdreadoutlibs_b200 import hostshim as H
-from util import adc_of, all_wibeth_policies, channels, create_status, expected, linear_map, ragged_units, run_device, sms
+from util import (adc_of, all_wibeth_policies, channels, create_status, expected, expected_lags, lags_of, linear_map, ragged_batch, ragged_units,
+                  run_device, sms)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 # ---- expected values --------------------------------------------------------------------------------------------------------------
-def lags_of(fmt, a):
-    """NOISE_LAGS_DTYPE row of (samples, channels) ADC values of one link in one batch: whole segments from the first sample."""
-    n = F.NOISE_SEGMENT_TICKS[fmt]
-    out = np.zeros(a.shape[1], dtype=F.NOISE_LAGS_DTYPE)
-    segs = a.shape[0] // n
-    x = a[: segs * n].astype(np.int64).reshape(segs, n, a.shape[1])
-    out["segments"] = segs
-    for tau in range(n // 2 + 1):
-        out["lag"][:, tau] = (x * np.roll(x, -tau, axis=1)).sum(axis=(0, 1))
-    return out
-
-
-def expected_lags(fmt, frames, nu=None, adc_offset=F.WIB2_ADC_OFFSET):
-    """(n_links, channels) lags of one batch: frames [n_links, stride, unit_bytes], nu valid units per link (None = all)."""
-    n, stride = frames.shape[:2]
-    return np.stack([lags_of(fmt, adc_of(fmt, frames[l, : (stride if nu is None else int(nu[l]))], adc_offset)) for l in range(n)])
-
-
 def zeros(n_links, fmt):
     return np.zeros((n_links, channels(fmt)), dtype=F.NOISE_LAGS_DTYPE)
 
@@ -59,15 +42,6 @@ def assert_lags(got, want, what):
             l, c = bad[0]
             raise AssertionError(f"{what}: {len(bad)} (link, channel) differ in {f}; first: link {l} channel {c}: "
                                  f"got {got[l, c]} want {want[l, c]}")
-
-
-def ragged_batch(fmt, seed, n_links, stride, nu, **gen_kw):
-    """Generated frames with every byte past each link's n_units set to 0xFF (an overread would count 16383s)."""
-    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
-    frames = gen(S.gen_params(seed, 0.3), n_links, stride, unit0=seed * stride, **gen_kw).copy()
-    for l in range(n_links):
-        frames[l, int(nu[l]):] = 0xFF
-    return frames
 
 
 # ---- CPU --------------------------------------------------------------------------------------------------------------------------

@@ -146,6 +146,53 @@ def combine(a, b):
     return out
 
 
+def ragged_batch(fmt, seed, n_links, stride, nu, **gen_kw):
+    """Generated frames with every byte past each link's n_units set to 0xFF (an overread would count 16383s)."""
+    gen = S.gen_wib2_host if fmt == "wib2" else S.gen_wibeth_host
+    frames = gen(S.gen_params(seed, 0.3), n_links, stride, unit0=seed * stride, **gen_kw).copy()
+    for l in range(n_links):
+        frames[l, int(nu[l]):] = 0xFF
+    return frames
+
+
+# ---- noise lags -------------------------------------------------------------------------------------------------------------
+def lags_of(fmt, a):
+    """NOISE_LAGS_DTYPE row of (samples, channels) ADC values of one link in one batch: whole segments from the first sample."""
+    n = F.NOISE_SEGMENT_TICKS[fmt]
+    out = np.zeros(a.shape[1], dtype=F.NOISE_LAGS_DTYPE)
+    segs = a.shape[0] // n
+    x = a[: segs * n].astype(np.int64).reshape(segs, n, a.shape[1])
+    out["segments"] = segs
+    for tau in range(n // 2 + 1):
+        out["lag"][:, tau] = (x * np.roll(x, -tau, axis=1)).sum(axis=(0, 1))
+    return out
+
+
+def expected_lags(fmt, frames, nu=None, adc_offset=F.WIB2_ADC_OFFSET):
+    """(n_links, channels) lags of one batch: frames [n_links, stride, unit_bytes], nu valid units per link (None = all)."""
+    n, stride = frames.shape[:2]
+    return np.stack([lags_of(fmt, adc_of(fmt, frames[l, : (stride if nu is None else int(nu[l]))], adc_offset)) for l in range(n)])
+
+
+# ---- channel products -------------------------------------------------------------------------------------------------------
+def words_of(fmt, a):
+    """One link's swtpg_read_channel_products row of (samples, channels) ADC values."""
+    c = channels(fmt)
+    x = np.asarray(a, dtype=np.int64).reshape(-1, c)
+    out = np.zeros(F.channel_products_words(fmt), dtype=np.uint64)
+    out[0] = x.shape[0]
+    out[1:1 + c] = x.sum(axis=0)
+    i, j = np.triu_indices(c)
+    out[1 + c:] = (x.T @ x)[i, j]  # below 2^63 for every window of these tests: ticks x 16383^2
+    return out
+
+
+def expected_products(fmt, frames, nu=None, adc_offset=F.WIB2_ADC_OFFSET):
+    """(n_links, words) of one batch: frames [n_links, stride, unit_bytes], nu valid units per link (None = all)."""
+    n, stride = frames.shape[:2]
+    return np.stack([words_of(fmt, adc_of(fmt, frames[l, : (stride if nu is None else int(nu[l]))], adc_offset)) for l in range(n)])
+
+
 # ---- configurations ---------------------------------------------------------------------------------------------------------
 # what TPGenerator's own configuration defaults to
 HANDLE = dict(algorithm="SimpleThreshold", threshold=60, acc_limit=10, rs_memory_factor=8, rs_scale_factor=5, fir_taps=None, tap_exponent=6)
